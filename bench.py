@@ -1,8 +1,8 @@
 #!/usr/bin/env python
 """bench.py -- disparity -> PointCloud2 throughput (BASELINE.json's metric) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
-    (N > 1 is launched by the driver under torch.distributed.run, one rank per GPU)
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--dump-outputs DIR]
+    (N > 1 is launched under torch.distributed.run, one rank per GPU)
 
 --config selects the BASELINE.json workload (numbered as SURVEY.md section 8 numbers them, = configs[N-1]); every
 config prints ONE JSON line with the same keys (value, e2e, roofline, cpu_baseline, clocks ...):
@@ -27,6 +27,16 @@ config prints ONE JSON line with the same keys (value, e2e, roofline, cpu_baseli
   roofline   algorithmic bytes (SURVEY.md 8(d)) / measured kernel time vs the measured HBM peak.
   cpu_baseline  the CPU oracle port of the same path on a bounded sample, timed on this host (N=1, rank 0).
 
+--dump-outputs DIR writes, after the timed steps, what the kernel-only leg computed in its last step, as its caller
+receives it: the clouds, (units, points, 4) {x, y, z, 1.0f} with one row per unit of the device-resident ring, and for
+config 5 also the per-lane results of the last frame set each lane ran (cropped_score.npy, fused_depth_map.npy,
+combined_score.npy, as float32).  A zero disparity reprojects to +-inf and NaN (the reference publishes such points),
+so a cloud is written as two finite float32 arrays of its shape: cloud.npy holds every finite component and 0 in place
+of a non-finite one, cloud_nonfinite.npy says which is which (0 finite, 1 +inf, -1 -inf, 2 NaN).  At most 64 MB in all:
+a cloud larger than what is left keeps a fixed, seeded sample of its points (the same points of every unit).  The
+inputs are seeded, so two builds run with the same arguments can be compared output for output.  Rank 0 writes;
+nothing is written in the repository unless DIR is in it.
+
 --impl reference times the CPU oracle port with all host threads on the same workload, a bounded sample per step
 (same sample rule as cpu_baseline).  The reference's own glue is compiled from its sources in oracle/_ref, but its
 arithmetic lives in OpenCV / PCL, which this image does not have: the timed code is the cv2-pinned C port.
@@ -49,6 +59,7 @@ sys.path.insert(0, ROOT)
 
 BORDER = 40
 METRIC = "Mpixels/s disparity->PointCloud2"
+DUMP_BYTES = 64 * 10**6  # --dump-outputs: all files together
 
 # name, frame size, entry, frames (frame sets) per step per GPU, device-resident ring, workload string (shared by
 # both arms, byte for byte), what one unit of work is
@@ -211,6 +222,30 @@ def max_over_ranks(x, world):
 def sum_over_ranks(x, world):
     from disparity_to_point_cloud_b200 import sharding
     return sharding.sum_over_ranks(x, device="cuda") if world > 1 else x
+
+
+def dump_outputs(out_dir, cloud, **small):
+    """Writes device tensors as <out_dir>/<name>.npy in float32, DUMP_BYTES at most in all.  `small` are written
+    whole; `cloud` (units, points, 4) keeps as many points as fit in what is left, a seeded sample taken at the same
+    indices in every unit, split into cloud.npy (finite components, 0 elsewhere) and cloud_nonfinite.npy (0 finite,
+    1 +inf, -1 -inf, 2 NaN)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    left = DUMP_BYTES
+    for name, t in small.items():
+        a = t.float().cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes + 4096  # 4096 B: more than an .npy header takes
+    units, npts, _ = cloud.shape
+    keep = min(npts, (left - 2 * 4096) // (units * 32))  # 16 B of values + 16 B of classes per point
+    if keep < npts:
+        idx = np.sort(np.random.default_rng(0).choice(npts, keep, replace=False))
+        cloud = cloud[:, torch.from_numpy(idx).to(cloud.device)]
+    c = cloud.cpu().numpy()
+    kind = np.zeros(c.shape, dtype=np.float32)
+    kind[np.isposinf(c)], kind[np.isneginf(c)], kind[np.isnan(c)] = 1, -1, 2
+    np.save(os.path.join(out_dir, "cloud.npy"), np.where(np.isfinite(c), c, np.float32(0)))
+    np.save(os.path.join(out_dir, "cloud_nonfinite.npy"), kind)
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -431,6 +466,13 @@ def run_ours(args):
     # one cloud checked on the device path so a broken kernel can not post a number
     probe = d_out[min(1, ring - 1), :64].cpu().numpy().view(np.float32)
     assert probe[3] == 1.0 and probe[7] == 1.0, "kernel output is not XYZ1 points"
+    if args.dump_outputs and rank == 0:
+        # every launch of a step writes ring slot i from ring input i, so the ring holds the last step's results
+        cloud = d_out.view(torch.float32).view(ring, npts, 4)
+        if entry == "fusion":
+            dump_outputs(args.dump_outputs, cloud, cropped_score=d_pre, fused_depth_map=d_fused, combined_score=d_comb)
+        else:
+            dump_outputs(args.dump_outputs, cloud)
 
     peak, peak_src = measured_peak()
     alg = algorithmic_bytes(cfg, dims)
@@ -576,7 +618,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-ceiling", action="store_true", help="skip the raw-copy ceiling of the e2e path")
     ap.add_argument("--append", default="", help="also append the JSON line to this file (profiles/configs_r2.json)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the last timed step's outputs to DIR/<name>.npy (float32, 64 MB at most)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the product path's outputs (--impl ours)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -586,4 +634,5 @@ def main():
 
 
 if __name__ == "__main__":
+    sys.dont_write_bytecode = True  # the benchmark leaves the tree it runs from as it found it
     main()
