@@ -16,7 +16,7 @@ import numpy as np
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libd2pc_b200.so")
 
-FILTER_CROP, FILTER_CROP_FINITE = 0, 1
+FILTER_CROP, FILTER_CROP_FINITE, FILTER_VOXEL = 0, 1, 2
 ARITH_EXACT, ARITH_FAST = 0, 1
 
 
@@ -62,6 +62,13 @@ class Cloud(C.Structure):
         return np.ctypeslib.as_array(self.data, shape=(n,))
 
 
+class VoxelGrid(C.Structure):
+    """d2pc_voxel_grid: pcl::VoxelGrid<PointXYZ> parameters of D2PC_FILTER_VOXEL."""
+    _fields_ = [("struct_size", C.c_uint32), ("leaf_x", C.c_float), ("leaf_y", C.c_float), ("leaf_z", C.c_float),
+                ("min_points_per_voxel", C.c_uint32), ("limit_field", C.c_int32), ("limit_min", C.c_double),
+                ("limit_max", C.c_double)]
+
+
 class Timing(C.Structure):
     _fields_ = [("h2d_us", C.c_float), ("kernels_us", C.c_float), ("d2h_us", C.c_float), ("total_us", C.c_float),
                 ("points", C.c_uint64)]
@@ -89,6 +96,9 @@ SYMBOLS = [
     ("d2pc_get_q", C.c_int, [_ctx, _f64p]),
     ("d2pc_set_filter_mode", C.c_int, [_ctx, C.c_int]),
     ("d2pc_set_arith_mode", C.c_int, [_ctx, C.c_int]),
+    ("d2pc_voxel_grid_default", None, [C.POINTER(VoxelGrid)]),
+    ("d2pc_set_voxel_grid", C.c_int, [_ctx, C.POINTER(VoxelGrid)]),
+    ("d2pc_get_voxel_grid", C.c_int, [_ctx, C.POINTER(VoxelGrid)]),
     ("d2pc_process_mono8", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_process_f32", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_submit_mono8", C.c_int, [_ctx, C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
@@ -284,6 +294,25 @@ class Context:
 
     def set_filter_mode(self, m):
         self._check(lib().d2pc_set_filter_mode(self._h, m), "d2pc_set_filter_mode")
+
+    def set_voxel_grid(self, leaf, min_points: int = 0, limit=None):
+        """pcl::VoxelGrid parameters for FILTER_VOXEL.  leaf: one size or (x, y, z); limit: None or
+        (field, lo, hi) with field "x", "y" or "z" (both ends inclusive)."""
+        g = VoxelGrid()
+        lib().d2pc_voxel_grid_default(C.byref(g))
+        lx, ly, lz = (leaf, leaf, leaf) if np.isscalar(leaf) else leaf
+        g.leaf_x, g.leaf_y, g.leaf_z = lx, ly, lz
+        g.min_points_per_voxel = int(min_points)
+        if limit is not None:
+            field, lo, hi = limit
+            g.limit_field = {"x": 0, "y": 1, "z": 2}[field]
+            g.limit_min, g.limit_max = float(lo), float(hi)
+        self._check(lib().d2pc_set_voxel_grid(self._h, C.byref(g)), "d2pc_set_voxel_grid")
+
+    def get_voxel_grid(self) -> VoxelGrid:
+        g = VoxelGrid()
+        self._check(lib().d2pc_get_voxel_grid(self._h, C.byref(g)), "d2pc_get_voxel_grid")
+        return g
 
     def set_arith_mode(self, m):
         self._check(lib().d2pc_set_arith_mode(self._h, m), "d2pc_set_arith_mode")

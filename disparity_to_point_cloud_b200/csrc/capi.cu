@@ -30,6 +30,7 @@
 #include "median.h"
 #include "reproject.h"
 #include "score.h"
+#include "voxel.h"
 
 using namespace d2pc;
 
@@ -50,9 +51,10 @@ struct PinBuf {
 struct Slot {
   PinBuf h_in, h_out;
   DevBuf d_in, d_med, d_out, d_scratch, d_tables;
+  DevBuf d_voxel;  // VOXEL mode: the CROP cloud and the voxel stage's keys / indices / sort temp (voxel.h)
   // fusion pipeline (d2pc_submit_fusion): the four input frames, the two preprocessed scores, merge outputs
   DevBuf d_fuse_in[4], d_pre[2], d_container, d_combined, d_fused;
-  uint32_t *d_count = nullptr;  // [0] = kept points, [1] = compaction ticket
+  uint32_t *d_count = nullptr;  // [0] = kept points, [1] = compaction ticket, [2] = VOXEL overflow fallback taken
   uint32_t *h_count = nullptr;  // pinned
   cudaEvent_t ev_h2d = nullptr, ev_kernel = nullptr, ev_d2h = nullptr;
   cudaEvent_t ev_start = nullptr;  // recorded in front of the H2D copy when per-call timing is on (d2pc_set_timing)
@@ -61,7 +63,8 @@ struct Slot {
   bool pending = false;
   uint32_t width = 0, height = 0;
   uint64_t n_points = 0;
-  bool compact = false;
+  bool compact = false;  // the count decides the bytes (CROP_FINITE, VOXEL)
+  bool voxel = false;    // VOXEL: is_dense comes from the fallback flag
   // caller-supplied destination of this submission (d2pc_submit_*_into); nullptr = library-owned h_out
   uint8_t *user_dst = nullptr;
   size_t user_cap = 0;
@@ -85,8 +88,10 @@ struct d2pc_ctx {
   uint64_t launches = 0;
   std::string last_cuda_error;
   // device-entry scratch
-  DevBuf d_scratch, d_tables, d_med_batch;
+  DevBuf d_scratch, d_tables, d_med_batch, d_voxel;
   uint32_t *d_ticket = nullptr;
+  d2pc_voxel_grid voxel;  // D2PC_FILTER_VOXEL parameters (d2pc_set_voxel_grid)
+  bool voxel_set = false;
   // fusion buffers
   DevBuf d_fuse_in[4], d_container, d_combined, d_fused;
   PinBuf h_fused, h_combined;
@@ -235,6 +240,15 @@ uint64_t crop_points(uint32_t w, uint32_t h, int border) {
   return (cw > 0 && ch > 0) ? (uint64_t)cw * (uint64_t)ch : 0;
 }
 
+// CROP_FINITE and VOXEL clouds have a size known only on the device: the kept count decides the bytes
+bool counted_mode(const d2pc_ctx *ctx) {
+  return ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE || ctx->cfg.filter_mode == D2PC_FILTER_VOXEL;
+}
+bool voxel_mode(const d2pc_ctx *ctx) { return ctx->cfg.filter_mode == D2PC_FILTER_VOXEL; }
+
+// a cloud's is_dense: 0 in CROP mode (cpp:81), 1 in CROP_FINITE, in VOXEL 1 unless the overflow fallback was taken
+bool cloud_is_dense(bool compact, bool voxel, const uint32_t *h_count) { return compact && !(voxel && h_count[2]); }
+
 uint32_t next_epoch(d2pc_ctx *ctx) {
   // 30-bit launch epoch inside the tile descriptors; 0 is "never written"
   if (++ctx->epoch >= (1u << 30)) {
@@ -247,7 +261,7 @@ uint32_t next_epoch(d2pc_ctx *ctx) {
   return ctx->epoch;
 }
 
-void fill_cloud(const d2pc_ctx *ctx, const uint8_t *data, uint64_t n, bool compact, d2pc_cloud *out) {
+void fill_cloud(const d2pc_ctx *ctx, const uint8_t *data, uint64_t n, bool is_dense, d2pc_cloud *out) {
   // src/disparity_to_point_cloud.cpp:79-85 + pcl::toROSMsg<PointXYZ> (SURVEY.md A.3)
   memset(out, 0, sizeof(*out));
   out->data = data;
@@ -256,7 +270,7 @@ void fill_cloud(const d2pc_ctx *ctx, const uint8_t *data, uint64_t n, bool compa
   out->point_step = 16;
   out->row_step = (uint32_t)(16 * n);
   out->is_bigendian = 0;
-  out->is_dense = compact ? 1 : 0;
+  out->is_dense = is_dense ? 1 : 0;
   out->n_fields = 3;
   static const char *names[3] = {"x", "y", "z"};
   for (int i = 0; i < 3; ++i) {
@@ -313,12 +327,51 @@ int upload_dense(d2pc_ctx *ctx, size_t stage_off, uint8_t *dst, const uint8_t *s
   return D2PC_OK;
 }
 
+// The VOXEL stage of a batch whose CROP clouds are in the head of `voxel_scratch` (voxel.h), with the context's grid.
+int enqueue_voxel(d2pc_ctx *ctx, uint32_t n_frames, uint64_t n, uint8_t *d_out, size_t out_stride, uint32_t *d_counts,
+                  uint32_t *fallback, void *voxel_scratch, cudaStream_t stream) {
+  const d2pc_voxel_grid &g = ctx->voxel;
+  VoxelLaunch V;
+  V.n_frames = n_frames;
+  V.n = (uint32_t)n;
+  V.p.inv[0] = 1.0f / g.leaf_x, V.p.inv[1] = 1.0f / g.leaf_y, V.p.inv[2] = 1.0f / g.leaf_z;
+  V.p.min_points = g.min_points_per_voxel;
+  V.p.limit_field = g.limit_field;
+  V.p.limit_min = g.limit_min, V.p.limit_max = g.limit_max;
+  V.out = d_out;
+  V.out_stride = out_stride;
+  V.counts = d_counts;
+  V.fallback = fallback;
+  V.scratch = voxel_scratch;
+  int nl = 0;
+  CU(ctx, launch_voxel(V, stream, &nl));
+  ctx->launches += nl;
+  return D2PC_OK;
+}
+
 // Enqueue [median] + reproject for one frame batch already on the device.
+// In VOXEL mode the CROP kernels write into the head of `voxel_scratch` (voxel_scratch_bytes(n_frames, crop)) and
+// the voxel stage writes d_out / d_counts / fallback (per frame; may be null).
 int enqueue_kernels(d2pc_ctx *ctx, const uint8_t *d_in, bool is_f32, uint32_t n_frames, uint32_t w, uint32_t h,
                     size_t step, size_t frame_stride, uint8_t *d_med, uint8_t *d_out, size_t out_stride,
-                    uint32_t *d_counts, void *scratch, void *tables, uint32_t *ticket, cudaStream_t stream) {
+                    uint32_t *d_counts, void *scratch, void *tables, uint32_t *ticket, cudaStream_t stream,
+                    void *voxel_scratch = nullptr, uint32_t *fallback = nullptr) {
   const d2pc_config &c = ctx->cfg;
   int nl = 0;
+  const bool voxel = voxel_mode(ctx);
+  uint8_t *const v_out = d_out;
+  const size_t v_stride = out_stride;
+  uint32_t *const v_counts = d_counts;
+  if (voxel) {  // the CROP cloud goes to scratch, dense, and is the voxel stage's input
+    d_out = reinterpret_cast<uint8_t *>(voxel_crop(voxel_scratch));
+    out_stride = crop_points(w, h, c.border) * 16;
+    d_counts = nullptr;
+  }
+  auto voxel_stage = [&]() {
+    return voxel ? enqueue_voxel(ctx, n_frames, crop_points(w, h, c.border), v_out, v_stride, v_counts, fallback,
+                                 voxel_scratch, stream)
+                 : (int)D2PC_OK;
+  };
   ReprojectLaunch L;
   L.in = d_in;
   L.in_is_f32 = is_f32;
@@ -380,13 +433,13 @@ int enqueue_kernels(d2pc_ctx *ctx, const uint8_t *d_in, bool is_f32, uint32_t n_
     }
     CU(ctx, launch_median_u8(M, stream, &nl));
     ctx->launches += nl;
-    if (fuse) return D2PC_OK;
+    if (fuse) return voxel_stage();
     L.in = d_med;
   }
   L.epoch = L.compact ? next_epoch(ctx) : 0;
   CU(ctx, launch_reproject(L, stream, &nl));
   ctx->launches += nl;
-  return D2PC_OK;
+  return voxel_stage();
 }
 
 int check_frame(const d2pc_ctx *ctx, const void *data, uint32_t w, uint32_t h, size_t step, int esz) {
@@ -424,7 +477,7 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   const size_t d_pitch = (row_bytes % 16 == 0 || !is_f32) ? row_bytes : align_up(row_bytes, kAlign);
   const uint64_t n = crop_points(w, h, ctx->cfg.border);
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // PointCloud2.row_step / width are uint32
-  const bool compact = ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE;
+  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx);
   if (user_dst && !compact && user_cap < n * 16) return D2PC_ERR_BUFFER_TOO_SMALL;
   const bool user_pinned = user_dst && reinterpret_cast<uintptr_t>(user_dst) % 16 == 0 && lookup_pinned(ctx, user_dst);
   if ((rc = grow_dev(ctx, s.d_in, d_pitch * h))) return rc;
@@ -444,9 +497,11 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
       cudaGetLastError();
   }
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
-  if (compact && ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, w, h, ctx->cfg.border), true)) ||
-                  (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(w, h)))))
+  if (compact && !voxel &&
+      ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, w, h, ctx->cfg.border), true)) ||
+       (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(w, h)))))
     return rc;
+  if (voxel && (rc = grow_dev(ctx, s.d_voxel, voxel_scratch_bytes(1, (uint32_t)n)))) return rc;
 
   // ---- H2D (stream 1).  Pinned caller memory is DMA'd in place; pageable memory is staged.
   const void *src = data;
@@ -482,7 +537,7 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
     NvtxRange nvtx_k("d2pc kernels");
     rc = enqueue_kernels(ctx, s.d_in.p, is_f32, 1, w, h, d_pitch, d_pitch * h, s.d_med.p,
                          d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count, s.d_scratch.p, s.d_tables.p,
-                         s.d_count + 1, ctx->s_compute);
+                         s.d_count + 1, ctx->s_compute, s.d_voxel.p, s.d_count + 2);
   }
   if (rc) return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, ctx->s_compute));
@@ -495,14 +550,16 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
     // (pageable destination of a synchronous call): the slot completes on the compute stream
     CU(ctx, cudaEventRecord(s.ev_d2h, ctx->s_compute));
     s.pending = true;
-    s.width = w, s.height = h, s.n_points = n, s.compact = false;
+    s.width = w, s.height = h, s.n_points = n, s.compact = false, s.voxel = false;
     s.user_dst = user_dst, s.user_cap = user_cap, s.user_pinned = user_pinned;
     return D2PC_OK;
   }
   CU(ctx, cudaStreamWaitEvent(ctx->s_d2h, s.ev_kernel, 0));
   if (compact) {
-    // the kept count decides how many bytes travel: fetch it, the payload copy is issued in d2pc_wait
-    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->s_d2h));
+    // the kept count decides how many bytes travel: fetch it (and the VOXEL fallback flag), the payload copy is
+    // issued in d2pc_wait
+    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, (voxel ? 3 : 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+                            ctx->s_d2h));
   } else if (n) {
     // a page-locked caller buffer receives the cloud by DMA directly; a pageable one is filled from h_out in wait
     CU(ctx, cudaMemcpyAsync(user_pinned ? user_dst : s.h_out.p, s.d_out.p, n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
@@ -513,6 +570,7 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   s.height = h;
   s.n_points = n;
   s.compact = compact;
+  s.voxel = voxel;
   s.user_dst = user_dst;
   s.user_cap = user_cap;
   s.user_pinned = user_pinned;
@@ -651,6 +709,7 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
   rc = d2pc_q_from_intrinsics(c.fx, c.fy, c.cx, c.cy, c.baseline, c.rect_width, c.rect_height, ctx->q);
   if (rc) return fail(rc);
   make_qparams(ctx->q, &ctx->Q);
+  d2pc_voxel_grid_default(&ctx->voxel);
 
   if (const char *v = getenv("D2PC_ROWS_PER_UNIT")) ctx->rows_per_unit = atoi(v);
   if (const char *v = getenv("D2PC_CTAS_PER_SM")) ctx->ctas_per_sm = atoi(v);
@@ -679,6 +738,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
   for (auto &s : ctx->slots) {
     free_pin(s.h_in), free_pin(s.h_out);
     free_dev(s.d_in), free_dev(s.d_med), free_dev(s.d_out), free_dev(s.d_scratch), free_dev(s.d_tables);
+    free_dev(s.d_voxel);
     for (auto &b : s.d_fuse_in) free_dev(b);
     free_dev(s.d_pre[0]), free_dev(s.d_pre[1]), free_dev(s.d_container), free_dev(s.d_combined), free_dev(s.d_fused);
     if (s.d_count) cudaFree(s.d_count);
@@ -689,7 +749,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
     if (s.ev_start) cudaEventDestroy(s.ev_start);
     if (s.s_kern) cudaStreamDestroy(s.s_kern);
   }
-  free_dev(ctx->d_scratch), free_dev(ctx->d_tables), free_dev(ctx->d_med_batch);
+  free_dev(ctx->d_scratch), free_dev(ctx->d_tables), free_dev(ctx->d_med_batch), free_dev(ctx->d_voxel);
   for (auto &b : ctx->d_fuse_in) free_dev(b);
   free_dev(ctx->d_container), free_dev(ctx->d_combined), free_dev(ctx->d_fused);
   free_pin(ctx->h_fused), free_pin(ctx->h_combined);
@@ -718,8 +778,30 @@ int d2pc_get_q(const d2pc_ctx *ctx, double q[16]) {
   return D2PC_OK;
 }
 int d2pc_set_filter_mode(d2pc_ctx *ctx, int m) {
-  if (!ctx || m < 0 || m > 1) return D2PC_ERR_INVALID_ARG;
+  if (!ctx || m < 0 || m > 2 || (m == D2PC_FILTER_VOXEL && !ctx->voxel_set)) return D2PC_ERR_INVALID_ARG;
   ctx->cfg.filter_mode = m;
+  return D2PC_OK;
+}
+
+void d2pc_voxel_grid_default(d2pc_voxel_grid *g) {
+  if (!g) return;
+  memset(g, 0, sizeof(*g));
+  g->struct_size = sizeof(*g);
+  g->limit_field = -1;
+}
+int d2pc_set_voxel_grid(d2pc_ctx *ctx, const d2pc_voxel_grid *g) {
+  if (!ctx || !g || g->struct_size != sizeof(*g)) return D2PC_ERR_INVALID_ARG;
+  for (float leaf : {g->leaf_x, g->leaf_y, g->leaf_z})
+    if (!(std::isfinite(leaf) && leaf > 0.0f)) return D2PC_ERR_INVALID_ARG;
+  if (g->limit_field < -1 || g->limit_field > 2) return D2PC_ERR_INVALID_ARG;
+  if (!(g->limit_min <= g->limit_max)) return D2PC_ERR_INVALID_ARG;
+  ctx->voxel = *g;
+  ctx->voxel_set = true;
+  return D2PC_OK;
+}
+int d2pc_get_voxel_grid(const d2pc_ctx *ctx, d2pc_voxel_grid *g) {
+  if (!ctx || !g) return D2PC_ERR_INVALID_ARG;
+  *g = ctx->voxel;
   return D2PC_OK;
 }
 int d2pc_set_arith_mode(d2pc_ctx *ctx, int m) {
@@ -805,7 +887,7 @@ int d2pc_wait(d2pc_ctx *ctx, int slot, d2pc_cloud *out) {
   s.late_copy = false;
   s.pending = false;
   if (ctx->cfg.verbose) printf("Cloud size: %llu\n", (unsigned long long)n);  // cpp:82
-  if (out) fill_cloud(ctx, s.user_dst ? s.user_dst : s.h_out.p, n, s.compact, out);
+  if (out) fill_cloud(ctx, s.user_dst ? s.user_dst : s.h_out.p, n, cloud_is_dense(s.compact, s.voxel, s.h_count), out);
   return D2PC_OK;
 }
 
@@ -952,12 +1034,21 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // per-frame counts and PointCloud2.row_step are uint32
   if (reinterpret_cast<uintptr_t>(d_points) % 16 || points_stride % 16 || (n_frames > 1 && points_stride < n * 16))
     return D2PC_ERR_BAD_DIMS;
-  const bool compact = ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE;
+  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx);
   if (compact && !d_counts) return D2PC_ERR_INVALID_ARG;
   if (n_frames == 0) return D2PC_OK;  // an empty batch: nothing to launch (and no size below may wrap)
   CU(ctx, cudaSetDevice(ctx->device));
   int rc;
-  if (compact) {
+  // VOXEL: the sort and scan index a batch with int, so a batch of more than 2^31 - 1 crop points runs in chunks
+  const uint32_t chunk = voxel ? (uint32_t)std::min<uint64_t>(n_frames, std::max<uint64_t>(1, 0x7fffffffull / std::max<uint64_t>(n, 1)))
+                               : n_frames;
+  if (voxel) {
+    const size_t need = voxel_scratch_bytes(chunk, (uint32_t)n);
+    if (need > ctx->d_voxel.cap) {
+      CU(ctx, cudaStreamSynchronize(ctx->s_compute));
+      if ((rc = grow_dev(ctx, ctx->d_voxel, need))) return rc;
+    }
+  } else if (compact) {
     const size_t need = reproject_scratch_bytes(n_frames, w, h, ctx->cfg.border);
     if (need > ctx->d_scratch.cap || reproject_table_bytes(w, h) > ctx->d_tables.cap) {
       CU(ctx, cudaStreamSynchronize(ctx->s_compute));
@@ -975,9 +1066,15 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
     }
     d_med = ctx->d_med_batch.p;
   }
-  return enqueue_kernels(ctx, static_cast<const uint8_t *>(d_in), is_f32, n_frames, w, h, step, frame_stride, d_med,
-                         d_points, points_stride, d_counts, ctx->d_scratch.p, ctx->d_tables.p, ctx->d_ticket,
-                         ctx->s_compute);
+  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
+    const uint32_t nf = std::min(chunk, n_frames - f0);
+    if ((rc = enqueue_kernels(ctx, static_cast<const uint8_t *>(d_in) + f0 * frame_stride, is_f32, nf, w, h, step,
+                              frame_stride, d_med, d_points + f0 * points_stride, points_stride,
+                              d_counts ? d_counts + f0 : nullptr, ctx->d_scratch.p, ctx->d_tables.p, ctx->d_ticket,
+                              ctx->s_compute, ctx->d_voxel.p)))
+      return rc;
+  }
+  return D2PC_OK;
 }
 
 int d2pc_reproject_f32_device(d2pc_ctx *ctx, const float *d_disp, uint32_t n_frames, uint32_t w, uint32_t h,
@@ -1303,7 +1400,7 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
   if ((rc = slot_wait_idle(ctx, s))) return rc;
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
   const uint64_t n = crop_points(fw, fh, ctx->cfg.border);
-  const bool compact = ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE;
+  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx);
   if ((rc = grow_dev(ctx, s.d_med, (size_t)fw * fh)) || (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
   // a synchronous call: the callback kernel stores the CROP cloud straight into the pinned buffer (see submit_common)
   uint8_t *d_direct = nullptr;
@@ -1315,16 +1412,18 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
       cudaGetLastError();
   }
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
-  if (compact && ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, fw, fh, ctx->cfg.border), true)) ||
-                  (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(fw, fh)))))
+  if (compact && !voxel &&
+      ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, fw, fh, ctx->cfg.border), true)) ||
+       (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(fw, fh)))))
     return rc;
+  if (voxel && (rc = grow_dev(ctx, s.d_voxel, voxel_scratch_bytes(1, (uint32_t)n)))) return rc;
   rc = enqueue_kernels(ctx, ctx->d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh, s.d_med.p,
                        d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count, s.d_scratch.p, s.d_tables.p,
-                       s.d_count + 1, ctx->s_compute);
+                       s.d_count + 1, ctx->s_compute, s.d_voxel.p, s.d_count + 2);
   if (rc) return rc;
   uint64_t kept = n;
   if (compact) {
-    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, 4, cudaMemcpyDeviceToHost, ctx->s_compute));
+    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, voxel ? 12 : 4, cudaMemcpyDeviceToHost, ctx->s_compute));
     CU(ctx, cudaStreamSynchronize(ctx->s_compute));
     kept = n ? s.h_count[0] : 0;
   }
@@ -1332,7 +1431,7 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
     CU(ctx, cudaMemcpyAsync(s.h_out.p, s.d_out.p, kept * 16, cudaMemcpyDeviceToHost, ctx->s_compute));
   CU(ctx, cudaStreamSynchronize(ctx->s_compute));
   if (ctx->cfg.verbose) printf("Cloud size: %llu\n", (unsigned long long)kept);
-  fill_cloud(ctx, s.h_out.p, kept, compact, out);
+  fill_cloud(ctx, s.h_out.p, kept, cloud_is_dense(compact, voxel, s.h_count), out);
   return D2PC_OK;
 }
 
@@ -1356,7 +1455,7 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
   const size_t pitch = w, frame_bytes = (size_t)w * h, nn = (size_t)g.n * g.n;
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
   const uint64_t n = crop_points(fw, fh, c.border);
-  const bool compact = c.filter_mode == D2PC_FILTER_CROP_FINITE;
+  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx);
   // the four input frames of a set live in one allocation, so that a contiguous pinned set is one DMA
   if ((rc = grow_dev(ctx, s.d_fuse_in[0], 4 * pitch * h))) return rc;
   uint8_t *const fin[4] = {s.d_fuse_in[0].p, s.d_fuse_in[0].p + pitch * h, s.d_fuse_in[0].p + 2 * pitch * h,
@@ -1366,9 +1465,13 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
       (rc = grow_dev(ctx, s.d_fused, (size_t)fw * fh)) || (rc = grow_dev(ctx, s.d_med, (size_t)fw * fh)) ||
       (rc = grow_dev(ctx, s.d_out, n * 16 + 16)) || (rc = grow_pin(ctx, s.h_out, n * 16 + 16)))
     return rc;
-  if (compact && ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, fw, fh, c.border), true)) ||
-                  (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(fw, fh)))))
+  if (compact && !voxel &&
+      ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, fw, fh, c.border), true)) ||
+       (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(fw, fh)))))
     return rc;
+  // (allocated without a clear: the voxel stage writes every word of its scratch before reading it, so it does
+  // not matter that this slot's kernels run on s_kern rather than on the stream grow_dev clears on)
+  if (voxel && (rc = grow_dev(ctx, s.d_voxel, voxel_scratch_bytes(1, (uint32_t)n)))) return rc;
 
   NvtxRange nvtx_submit("d2pc submit fusion set");
   s.timed = ctx->timing && s.ev_start;
@@ -1410,19 +1513,21 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
                              nullptr, preprocess_scores != 0, &s.d_container, sk)))
     return rc;
   rc = enqueue_kernels(ctx, s.d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh, s.d_med.p, s.d_out.p, n * 16 + 16, s.d_count,
-                       s.d_scratch.p, s.d_tables.p, s.d_count + 1, sk);
+                       s.d_scratch.p, s.d_tables.p, s.d_count + 1, sk, s.d_voxel.p, s.d_count + 2);
   if (rc) return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, sk));
 
   // ---- D2H (stream 3)
   CU(ctx, cudaStreamWaitEvent(ctx->s_d2h, s.ev_kernel, 0));
-  if (compact) CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->s_d2h));
+  if (compact)
+    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, (voxel ? 3 : 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->s_d2h));
   else if (n) CU(ctx, cudaMemcpyAsync(s.h_out.p, s.d_out.p, n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
   CU(ctx, cudaEventRecord(s.ev_d2h, ctx->s_d2h));
   s.pending = true;
   s.width = fw, s.height = fh;
   s.n_points = n;
   s.compact = compact;
+  s.voxel = voxel;
   s.user_dst = nullptr, s.user_cap = 0, s.user_pinned = false, s.late_copy = false;
   return D2PC_OK;
 }

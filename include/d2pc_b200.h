@@ -50,8 +50,14 @@ typedef enum d2pc_status {
 /* src/disparity_to_point_cloud.cpp:69-76: the reference's only point filter is
  * the fixed border crop (CROP).  CROP_FINITE is an extension: crop, then drop
  * points with a non-finite x, y or z, order preserved (decoupled look-back
- * stream compaction). */
-typedef enum d2pc_filter_mode { D2PC_FILTER_CROP = 0, D2PC_FILTER_CROP_FINITE = 1 } d2pc_filter_mode;
+ * stream compaction).  VOXEL is an extension too: pcl::VoxelGrid<pcl::PointXYZ>
+ * applied to the CROP cloud on the device (d2pc_voxel_grid below; selectable once
+ * a grid has been set with d2pc_set_voxel_grid). */
+typedef enum d2pc_filter_mode {
+  D2PC_FILTER_CROP = 0,
+  D2PC_FILTER_CROP_FINITE = 1,
+  D2PC_FILTER_VOXEL = 2
+} d2pc_filter_mode;
 
 /* EXACT reproduces cv::reprojectImageTo3D's float64 rounding sequence bit for
  * bit (src/disparity_to_point_cloud.cpp:63-64).  FAST is float32 only
@@ -117,7 +123,7 @@ typedef struct d2pc_cloud {
   uint32_t point_step; /* 16 */
   uint32_t row_step;   /* 16 * width */
   uint8_t is_bigendian; /* 0 */
-  uint8_t is_dense;     /* 0 in CROP mode (cpp:81); 1 in CROP_FINITE */
+  uint8_t is_dense;     /* 0 in CROP mode (cpp:81); 1 in CROP_FINITE; VOXEL: 1, 0 for the overflow fallback */
   uint32_t n_fields;    /* 3 */
   d2pc_point_field fields[3];
 } d2pc_cloud;
@@ -145,8 +151,53 @@ int d2pc_q_from_intrinsics(double fx, double fy, double cx, double cy, double ba
                            double q_out[16]);
 int d2pc_set_q(d2pc_ctx *ctx, const double q[16]);
 int d2pc_get_q(const d2pc_ctx *ctx, double q_out[16]);
-int d2pc_set_filter_mode(d2pc_ctx *ctx, int filter_mode);
+int d2pc_set_filter_mode(d2pc_ctx *ctx, int filter_mode); /* VOXEL: D2PC_ERR_INVALID_ARG until a grid is set */
 int d2pc_set_arith_mode(d2pc_ctx *ctx, int arith_mode);
+
+/* ---- voxel-grid downsampling (D2PC_FILTER_VOXEL) ------------------------------
+ *
+ * The published cloud is pcl::VoxelGrid<pcl::PointXYZ> (PCL 1.7.2 - 1.12, downsample_all_data = true,
+ * filter_limit_negative = false) applied to exactly the cloud CROP mode publishes for the same frame, +-inf and
+ * NaN points included.  The recipe, float32 throughout unless stated, no FMA contraction:
+ *   1. inv[a] = 1.0f / leaf[a] for a in {x, y, z}.
+ *   2. A point is included when x, y and z are finite and, with a limit field set, that coordinate widened to
+ *      double lies in [limit_min, limit_max] (both ends inclusive).
+ *   3. min_p / max_p: per-axis float min / max over the included points.  None included: the empty cloud
+ *      (width 0, is_dense 1).
+ *   4. Overflow guard: d[a] = (int64)((max_p[a] - min_p[a]) * inv[a]) + 1; when dx*dy*dz > INT32_MAX the output is
+ *      the input cloud unchanged (all N crop points, is_dense 0) -- PCL's `output = *input_` after its warning.
+ *   5. min_b[a] = (int)floorf(min_p[a] * inv[a]), max_b[a] = (int)floorf(max_p[a] * inv[a]),
+ *      div_b = max_b - min_b + 1, mul = (1, div_b.x, div_b.x * div_b.y).
+ *   6. ijk[a] = (int)(floorf(p[a] * inv[a]) - (float)min_b[a]); idx = ijk.x + ijk.y * mul.y + ijk.z * mul.z in
+ *      64 bits (PCL's int wherever PCL's does not overflow).  Where PCL's int arithmetic WOULD overflow -- a
+ *      floorf bound outside int32, or an idx that can reach 2^31 - 1 -- PCL's result is undefined; this library
+ *      then takes the step-4 fallback as well.
+ *   7. Voxels are emitted in ascending idx; a voxel with fewer than min_points_per_voxel points is dropped.
+ *   8. centroid = (sum x, sum y, sum z) / (float)count, each sum a float32 left fold, IEEE division; the point is
+ *      {cx, cy, cz, 1.0f}, 16 bytes with the same fields and point_step as every other mode.
+ *      Summation order: ascending point index (row-major crop order) within the voxel.  PCL orders a voxel's
+ *      points with std::sort, which is not stable, so its order -- and the last bits of its centroids -- is
+ *      unspecified; the stable order is the one a GPU and a CPU reference can both meet bit for bit.
+ *   9. height 1, width = number of voxels, is_dense 1 (0 only for the fallback), row_step = 16 * width.
+ * The size of a VOXEL cloud is known only when the frame has been processed, so the rules of CROP_FINITE apply:
+ * BUFFER_TOO_SMALL is reported by d2pc_wait, the kernel never stores into host memory ("direct_out" does not
+ * apply), d2pc_slot_timing's d2h_us covers the count, and the device batch entries need d_counts (frame f's voxels
+ * at d_points + f * points_stride; every frame of a batch is its own grid). */
+typedef struct d2pc_voxel_grid {
+  uint32_t struct_size;          /* sizeof(d2pc_voxel_grid) */
+  float leaf_x, leaf_y, leaf_z;  /* finite, > 0 */
+  uint32_t min_points_per_voxel; /* PCL default 0 */
+  int32_t limit_field;           /* -1 none, 0 x, 1 y, 2 z */
+  double limit_min, limit_max;   /* limit_min <= limit_max */
+} d2pc_voxel_grid;
+
+/* leaf 0 (not yet valid), no limit, min_points_per_voxel 0. */
+void d2pc_voxel_grid_default(d2pc_voxel_grid *grid);
+/* D2PC_ERR_INVALID_ARG for a leaf that is not finite and > 0, a limit_field outside -1..2, limit_min > limit_max
+ * (PCL would accept it and return nothing) or a wrong struct_size; the previous grid is kept then. */
+int d2pc_set_voxel_grid(d2pc_ctx *ctx, const d2pc_voxel_grid *grid);
+/* The grid last set (d2pc_voxel_grid_default's until then). */
+int d2pc_get_voxel_grid(const d2pc_ctx *ctx, d2pc_voxel_grid *grid);
 
 /* ---- the disparity callback, host buffers (the reference-facing calls) ------ */
 

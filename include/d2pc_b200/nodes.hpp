@@ -207,6 +207,20 @@ class Disparity2PCloud {
     border_ = cfg.border;
     d2pc_b200::check(d2pc_create(&cfg, device, &ctx_), "d2pc_create");
     d2pc_get_q(ctx_, Q_);
+    // optional, not in the reference: pcl::VoxelGrid on the device (D2PC_FILTER_VOXEL), with a z pass-through
+    // limit when voxel_z_min < voxel_z_max.  With the defaults the node publishes what the reference does.
+    double leaf = 0.0, z_min = 0.0, z_max = 0.0;
+    nh_.param<double>("voxel_leaf_size", leaf, 0.0);
+    nh_.param<double>("voxel_z_min", z_min, 0.0);
+    nh_.param<double>("voxel_z_max", z_max, 0.0);
+    if (leaf > 0.0) {
+      d2pc_voxel_grid g;
+      d2pc_voxel_grid_default(&g);
+      g.leaf_x = g.leaf_y = g.leaf_z = static_cast<float>(leaf);
+      if (z_min < z_max) g.limit_field = 2, g.limit_min = z_min, g.limit_max = z_max;
+      d2pc_b200::check(d2pc_set_voxel_grid(ctx_, &g), "d2pc_set_voxel_grid", ctx_);
+      d2pc_b200::check(d2pc_set_filter_mode(ctx_, D2PC_FILTER_VOXEL), "d2pc_set_filter_mode", ctx_);
+    }
   }
   ~Disparity2PCloud() {
     d2pc_destroy(ctx_);  // waits for the device: nothing writes into output_ any more
@@ -245,7 +259,7 @@ class Disparity2PCloud {
     output.point_step = cloud.point_step;
     output.row_step = cloud.row_step;
     output.is_dense = cloud.is_dense;
-    // CROP_FINITE keeps fewer points than the crop holds: shrink the view, never the storage
+    // CROP_FINITE / VOXEL keep fewer points than the crop holds: shrink the view, never the storage
     output.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
     output.header.stamp = msg->header.stamp;             // cpp:87
     output.header.frame_id = "/camera_optical_frame";    // cpp:89

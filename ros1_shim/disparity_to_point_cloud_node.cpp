@@ -34,6 +34,23 @@ class Disparity2PCloudGpu {
     if (rc != D2PC_OK) {
       ROS_FATAL("d2pc_create: %s", d2pc_strerror(rc));
       ros::shutdown();
+      return;
+    }
+    // optional, not in the reference: pcl::VoxelGrid on the device, with a z pass-through limit when
+    // voxel_z_min < voxel_z_max; with the defaults the node publishes what the reference does
+    double leaf = 0.0, z_min = 0.0, z_max = 0.0;
+    nh_.param<double>("voxel_leaf_size", leaf, 0.0);
+    nh_.param<double>("voxel_z_min", z_min, 0.0);
+    nh_.param<double>("voxel_z_max", z_max, 0.0);
+    if (leaf > 0.0) {
+      d2pc_voxel_grid g;
+      d2pc_voxel_grid_default(&g);
+      g.leaf_x = g.leaf_y = g.leaf_z = static_cast<float>(leaf);
+      if (z_min < z_max) g.limit_field = 2, g.limit_min = z_min, g.limit_max = z_max;
+      if (d2pc_set_voxel_grid(ctx_, &g) != D2PC_OK || d2pc_set_filter_mode(ctx_, D2PC_FILTER_VOXEL) != D2PC_OK) {
+        ROS_FATAL("voxel_leaf_size %g: not a valid voxel grid", leaf);
+        ros::shutdown();
+      }
     }
   }
   ~Disparity2PCloudGpu() {
