@@ -69,6 +69,11 @@ class VoxelGrid(C.Structure):
                 ("limit_max", C.c_double)]
 
 
+class RadiusOutlier(C.Structure):
+    """d2pc_radius_outlier: pcl::RadiusOutlierRemoval parameters of the stage behind every filter mode."""
+    _fields_ = [("struct_size", C.c_uint32), ("radius", C.c_double), ("min_neighbors", C.c_uint32)]
+
+
 class Timing(C.Structure):
     _fields_ = [("h2d_us", C.c_float), ("kernels_us", C.c_float), ("d2h_us", C.c_float), ("total_us", C.c_float),
                 ("points", C.c_uint64)]
@@ -99,6 +104,11 @@ SYMBOLS = [
     ("d2pc_voxel_grid_default", None, [C.POINTER(VoxelGrid)]),
     ("d2pc_set_voxel_grid", C.c_int, [_ctx, C.POINTER(VoxelGrid)]),
     ("d2pc_get_voxel_grid", C.c_int, [_ctx, C.POINTER(VoxelGrid)]),
+    ("d2pc_radius_outlier_default", None, [C.POINTER(RadiusOutlier)]),
+    ("d2pc_set_radius_outlier", C.c_int, [_ctx, C.POINTER(RadiusOutlier)]),
+    ("d2pc_get_radius_outlier", C.c_int, [_ctx, C.POINTER(RadiusOutlier)]),
+    ("d2pc_radius_outlier_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
+                                             C.c_void_p, C.c_size_t, C.c_void_p]),
     ("d2pc_process_mono8", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_process_f32", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_submit_mono8", C.c_int, [_ctx, C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
@@ -314,6 +324,21 @@ class Context:
         self._check(lib().d2pc_get_voxel_grid(self._h, C.byref(g)), "d2pc_get_voxel_grid")
         return g
 
+    def set_radius_outlier(self, radius: float, min_neighbors: int = 1):
+        """pcl::RadiusOutlierRemoval behind the filter mode: radius 0 turns the stage off."""
+        if not 0 <= int(min_neighbors) <= 0xFFFFFFFF:  # ctypes would wrap a negative count into a huge one
+            raise ValueError(f"set_radius_outlier: min_neighbors must be in [0, 2^32 - 1], got {min_neighbors}")
+        p = RadiusOutlier()
+        lib().d2pc_radius_outlier_default(C.byref(p))
+        p.radius = float(radius)
+        p.min_neighbors = int(min_neighbors)
+        self._check(lib().d2pc_set_radius_outlier(self._h, C.byref(p)), "d2pc_set_radius_outlier")
+
+    def get_radius_outlier(self) -> RadiusOutlier:
+        p = RadiusOutlier()
+        self._check(lib().d2pc_get_radius_outlier(self._h, C.byref(p)), "d2pc_get_radius_outlier")
+        return p
+
     def set_arith_mode(self, m):
         self._check(lib().d2pc_set_arith_mode(self._h, m), "d2pc_set_arith_mode")
 
@@ -423,6 +448,11 @@ class Context:
     def reproject_mono8_device(self, d_img, n_frames, w, h, step, frame_stride, d_points, points_stride, d_counts=0):
         self._check(lib().d2pc_reproject_mono8_device(self._h, d_img, n_frames, w, h, step, frame_stride, d_points,
                                                       points_stride, d_counts or None), "d2pc_reproject_mono8_device")
+
+    def radius_outlier_device(self, d_in, n_frames, n_max, in_stride, d_in_counts, d_out, out_stride, d_out_counts):
+        self._check(lib().d2pc_radius_outlier_device(self._h, d_in, n_frames, n_max, in_stride, d_in_counts or None,
+                                                     d_out, out_stride, d_out_counts or None),
+                    "d2pc_radius_outlier_device")
 
     def median_u8_device(self, d_src, w, h, src_step, d_dst, dst_step, ksize):
         self._check(lib().d2pc_median_u8_device(self._h, d_src, w, h, src_step, d_dst, dst_step, ksize),

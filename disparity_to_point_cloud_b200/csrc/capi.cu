@@ -28,6 +28,7 @@
 
 #include "fusion.h"
 #include "median.h"
+#include "radius_outlier.h"
 #include "reproject.h"
 #include "score.h"
 #include "voxel.h"
@@ -52,6 +53,7 @@ struct Slot {
   PinBuf h_in, h_out;
   DevBuf d_in, d_med, d_out, d_scratch, d_tables;
   DevBuf d_voxel;  // VOXEL mode: the CROP cloud and the voxel stage's keys / indices / sort temp (voxel.h)
+  DevBuf d_ror;    // radius outlier stage: the mode's cloud and counts, then the stage's scratch (radius_outlier.h)
   // fusion pipeline (d2pc_submit_fusion): the four input frames, the two preprocessed scores, merge outputs
   DevBuf d_fuse_in[4], d_pre[2], d_container, d_combined, d_fused;
   uint32_t *d_count = nullptr;  // [0] = kept points, [1] = compaction ticket, [2] = VOXEL overflow fallback taken
@@ -64,7 +66,7 @@ struct Slot {
   uint32_t width = 0, height = 0;
   uint64_t n_points = 0;
   bool compact = false;  // the count decides the bytes (CROP_FINITE, VOXEL)
-  bool voxel = false;    // VOXEL: is_dense comes from the fallback flag
+  bool voxel = false;    // VOXEL without the radius outlier stage: is_dense comes from the fallback flag
   // caller-supplied destination of this submission (d2pc_submit_*_into); nullptr = library-owned h_out
   uint8_t *user_dst = nullptr;
   size_t user_cap = 0;
@@ -88,10 +90,11 @@ struct d2pc_ctx {
   uint64_t launches = 0;
   std::string last_cuda_error;
   // device-entry scratch
-  DevBuf d_scratch, d_tables, d_med_batch, d_voxel;
+  DevBuf d_scratch, d_tables, d_med_batch, d_voxel, d_ror;
   uint32_t *d_ticket = nullptr;
   d2pc_voxel_grid voxel;  // D2PC_FILTER_VOXEL parameters (d2pc_set_voxel_grid)
   bool voxel_set = false;
+  d2pc_radius_outlier ror;  // the radius outlier stage behind every mode (d2pc_set_radius_outlier; radius 0: off)
   // fusion buffers
   DevBuf d_fuse_in[4], d_container, d_combined, d_fused;
   PinBuf h_fused, h_combined;
@@ -240,13 +243,17 @@ uint64_t crop_points(uint32_t w, uint32_t h, int border) {
   return (cw > 0 && ch > 0) ? (uint64_t)cw * (uint64_t)ch : 0;
 }
 
-// CROP_FINITE and VOXEL clouds have a size known only on the device: the kept count decides the bytes
+bool ror_on(const d2pc_ctx *ctx) { return ctx->ror.radius > 0.0; }
+// CROP_FINITE and VOXEL clouds, and every cloud of the radius outlier stage, have a size known only on the device:
+// the kept count decides the bytes
 bool counted_mode(const d2pc_ctx *ctx) {
-  return ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE || ctx->cfg.filter_mode == D2PC_FILTER_VOXEL;
+  return ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE || ctx->cfg.filter_mode == D2PC_FILTER_VOXEL || ror_on(ctx);
 }
 bool voxel_mode(const d2pc_ctx *ctx) { return ctx->cfg.filter_mode == D2PC_FILTER_VOXEL; }
+bool finite_mode(const d2pc_ctx *ctx) { return ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE; }
 
 // a cloud's is_dense: 0 in CROP mode (cpp:81), 1 in CROP_FINITE, in VOXEL 1 unless the overflow fallback was taken
+// (`voxel` is false behind the radius outlier stage, whose output is always dense)
 bool cloud_is_dense(bool compact, bool voxel, const uint32_t *h_count) { return compact && !(voxel && h_count[2]); }
 
 uint32_t next_epoch(d2pc_ctx *ctx) {
@@ -349,15 +356,52 @@ int enqueue_voxel(d2pc_ctx *ctx, uint32_t n_frames, uint64_t n, uint8_t *d_out, 
   return D2PC_OK;
 }
 
+// The radius outlier stage with the context's setting on n_frames clouds (frame f at in + f * in_stride, in_counts[f]
+// points; in_counts null: n_max each).
+int enqueue_ror(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n_max, const uint8_t *in, size_t in_stride,
+                const uint32_t *in_counts, uint8_t *d_out, size_t out_stride, uint32_t *d_counts, void *scratch,
+                cudaStream_t stream) {
+  RorLaunch R;
+  R.n_frames = n_frames;
+  R.n_max = n_max;
+  R.in = in;
+  R.in_stride = in_stride;
+  R.in_counts = in_counts;
+  R.radius = ctx->ror.radius;
+  R.min_neighbors = ctx->ror.min_neighbors;
+  R.out = d_out;
+  R.out_stride = out_stride;
+  R.counts = d_counts;
+  R.scratch = scratch;
+  int nl = 0;
+  CU(ctx, launch_radius_outlier(R, stream, &nl));
+  ctx->launches += nl;
+  return D2PC_OK;
+}
+
 // Enqueue [median] + reproject for one frame batch already on the device.
 // In VOXEL mode the CROP kernels write into the head of `voxel_scratch` (voxel_scratch_bytes(n_frames, crop)) and
 // the voxel stage writes d_out / d_counts / fallback (per frame; may be null).
+// With the radius outlier stage on, the mode's clouds and counts go to the head of `ror_buf`
+// (ror_stage_bytes(n_frames, crop)) and the stage writes d_out / d_counts.
 int enqueue_kernels(d2pc_ctx *ctx, const uint8_t *d_in, bool is_f32, uint32_t n_frames, uint32_t w, uint32_t h,
                     size_t step, size_t frame_stride, uint8_t *d_med, uint8_t *d_out, size_t out_stride,
                     uint32_t *d_counts, void *scratch, void *tables, uint32_t *ticket, cudaStream_t stream,
-                    void *voxel_scratch = nullptr, uint32_t *fallback = nullptr) {
+                    void *voxel_scratch = nullptr, uint32_t *fallback = nullptr, void *ror_buf = nullptr) {
   const d2pc_config &c = ctx->cfg;
   int nl = 0;
+  const bool ror = ror_on(ctx);
+  const uint32_t n_crop = (uint32_t)crop_points(w, h, c.border);
+  uint8_t *const r_out = d_out;
+  const size_t r_stride = out_stride;
+  uint32_t *const r_counts = d_counts;
+  RorStage rs{};
+  if (ror) {  // the mode's clouds go to the stage's buffer, dense, and are its input
+    rs = ror_stage(ror_buf, n_frames, n_crop);
+    d_out = rs.clouds;
+    out_stride = (size_t)n_crop * 16;
+    d_counts = rs.counts;
+  }
   const bool voxel = voxel_mode(ctx);
   uint8_t *const v_out = d_out;
   const size_t v_stride = out_stride;
@@ -371,6 +415,14 @@ int enqueue_kernels(d2pc_ctx *ctx, const uint8_t *d_in, bool is_f32, uint32_t n_
     return voxel ? enqueue_voxel(ctx, n_frames, crop_points(w, h, c.border), v_out, v_stride, v_counts, fallback,
                                  voxel_scratch, stream)
                  : (int)D2PC_OK;
+  };
+  auto filter_stages = [&]() {
+    const int rc = voxel_stage();
+    if (rc || !ror) return rc;
+    // a CROP cloud has all n_crop points; the other modes' counts are on the device
+    return enqueue_ror(ctx, n_frames, n_crop, rs.clouds, (size_t)n_crop * 16,
+                       c.filter_mode == D2PC_FILTER_CROP ? nullptr : rs.counts, r_out, r_stride, r_counts, rs.scratch,
+                       stream);
   };
   ReprojectLaunch L;
   L.in = d_in;
@@ -433,13 +485,13 @@ int enqueue_kernels(d2pc_ctx *ctx, const uint8_t *d_in, bool is_f32, uint32_t n_
     }
     CU(ctx, launch_median_u8(M, stream, &nl));
     ctx->launches += nl;
-    if (fuse) return voxel_stage();
+    if (fuse) return filter_stages();
     L.in = d_med;
   }
   L.epoch = L.compact ? next_epoch(ctx) : 0;
   CU(ctx, launch_reproject(L, stream, &nl));
   ctx->launches += nl;
-  return voxel_stage();
+  return filter_stages();
 }
 
 int check_frame(const d2pc_ctx *ctx, const void *data, uint32_t w, uint32_t h, size_t step, int esz) {
@@ -477,7 +529,7 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   const size_t d_pitch = (row_bytes % 16 == 0 || !is_f32) ? row_bytes : align_up(row_bytes, kAlign);
   const uint64_t n = crop_points(w, h, ctx->cfg.border);
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // PointCloud2.row_step / width are uint32
-  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx);
+  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx), ror = ror_on(ctx);
   if (user_dst && !compact && user_cap < n * 16) return D2PC_ERR_BUFFER_TOO_SMALL;
   const bool user_pinned = user_dst && reinterpret_cast<uintptr_t>(user_dst) % 16 == 0 && lookup_pinned(ctx, user_dst);
   if ((rc = grow_dev(ctx, s.d_in, d_pitch * h))) return rc;
@@ -497,11 +549,12 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
       cudaGetLastError();
   }
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
-  if (compact && !voxel &&
+  if (finite_mode(ctx) &&
       ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, w, h, ctx->cfg.border), true)) ||
        (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(w, h)))))
     return rc;
   if (voxel && (rc = grow_dev(ctx, s.d_voxel, voxel_scratch_bytes(1, (uint32_t)n)))) return rc;
+  if (ror && (rc = grow_dev(ctx, s.d_ror, ror_stage_bytes(1, (uint32_t)n)))) return rc;
 
   // ---- H2D (stream 1).  Pinned caller memory is DMA'd in place; pageable memory is staged.
   const void *src = data;
@@ -537,7 +590,7 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
     NvtxRange nvtx_k("d2pc kernels");
     rc = enqueue_kernels(ctx, s.d_in.p, is_f32, 1, w, h, d_pitch, d_pitch * h, s.d_med.p,
                          d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count, s.d_scratch.p, s.d_tables.p,
-                         s.d_count + 1, ctx->s_compute, s.d_voxel.p, s.d_count + 2);
+                         s.d_count + 1, ctx->s_compute, s.d_voxel.p, s.d_count + 2, s.d_ror.p);
   }
   if (rc) return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, ctx->s_compute));
@@ -570,7 +623,7 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   s.height = h;
   s.n_points = n;
   s.compact = compact;
-  s.voxel = voxel;
+  s.voxel = voxel && !ror;
   s.user_dst = user_dst;
   s.user_cap = user_cap;
   s.user_pinned = user_pinned;
@@ -710,6 +763,7 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
   if (rc) return fail(rc);
   make_qparams(ctx->q, &ctx->Q);
   d2pc_voxel_grid_default(&ctx->voxel);
+  d2pc_radius_outlier_default(&ctx->ror);
 
   if (const char *v = getenv("D2PC_ROWS_PER_UNIT")) ctx->rows_per_unit = atoi(v);
   if (const char *v = getenv("D2PC_CTAS_PER_SM")) ctx->ctas_per_sm = atoi(v);
@@ -738,7 +792,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
   for (auto &s : ctx->slots) {
     free_pin(s.h_in), free_pin(s.h_out);
     free_dev(s.d_in), free_dev(s.d_med), free_dev(s.d_out), free_dev(s.d_scratch), free_dev(s.d_tables);
-    free_dev(s.d_voxel);
+    free_dev(s.d_voxel), free_dev(s.d_ror);
     for (auto &b : s.d_fuse_in) free_dev(b);
     free_dev(s.d_pre[0]), free_dev(s.d_pre[1]), free_dev(s.d_container), free_dev(s.d_combined), free_dev(s.d_fused);
     if (s.d_count) cudaFree(s.d_count);
@@ -749,7 +803,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
     if (s.ev_start) cudaEventDestroy(s.ev_start);
     if (s.s_kern) cudaStreamDestroy(s.s_kern);
   }
-  free_dev(ctx->d_scratch), free_dev(ctx->d_tables), free_dev(ctx->d_med_batch), free_dev(ctx->d_voxel);
+  free_dev(ctx->d_scratch), free_dev(ctx->d_tables), free_dev(ctx->d_med_batch), free_dev(ctx->d_voxel), free_dev(ctx->d_ror);
   for (auto &b : ctx->d_fuse_in) free_dev(b);
   free_dev(ctx->d_container), free_dev(ctx->d_combined), free_dev(ctx->d_fused);
   free_pin(ctx->h_fused), free_pin(ctx->h_combined);
@@ -802,6 +856,23 @@ int d2pc_set_voxel_grid(d2pc_ctx *ctx, const d2pc_voxel_grid *g) {
 int d2pc_get_voxel_grid(const d2pc_ctx *ctx, d2pc_voxel_grid *g) {
   if (!ctx || !g) return D2PC_ERR_INVALID_ARG;
   *g = ctx->voxel;
+  return D2PC_OK;
+}
+void d2pc_radius_outlier_default(d2pc_radius_outlier *p) {
+  if (!p) return;
+  memset(p, 0, sizeof(*p));
+  p->struct_size = sizeof(*p);
+  p->min_neighbors = 1;
+}
+int d2pc_set_radius_outlier(d2pc_ctx *ctx, const d2pc_radius_outlier *p) {
+  if (!ctx || !p || p->struct_size != sizeof(*p)) return D2PC_ERR_INVALID_ARG;
+  if (!(std::isfinite(p->radius) && p->radius >= 0.0)) return D2PC_ERR_INVALID_ARG;
+  ctx->ror = *p;
+  return D2PC_OK;
+}
+int d2pc_get_radius_outlier(const d2pc_ctx *ctx, d2pc_radius_outlier *p) {
+  if (!ctx || !p) return D2PC_ERR_INVALID_ARG;
+  *p = ctx->ror;
   return D2PC_OK;
 }
 int d2pc_set_arith_mode(d2pc_ctx *ctx, int m) {
@@ -1034,21 +1105,32 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // per-frame counts and PointCloud2.row_step are uint32
   if (reinterpret_cast<uintptr_t>(d_points) % 16 || points_stride % 16 || (n_frames > 1 && points_stride < n * 16))
     return D2PC_ERR_BAD_DIMS;
-  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx);
+  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx), ror = ror_on(ctx);
   if (compact && !d_counts) return D2PC_ERR_INVALID_ARG;
   if (n_frames == 0) return D2PC_OK;  // an empty batch: nothing to launch (and no size below may wrap)
   CU(ctx, cudaSetDevice(ctx->device));
   int rc;
-  // VOXEL: the sort and scan index a batch with int, so a batch of more than 2^31 - 1 crop points runs in chunks
-  const uint32_t chunk = voxel ? (uint32_t)std::min<uint64_t>(n_frames, std::max<uint64_t>(1, 0x7fffffffull / std::max<uint64_t>(n, 1)))
-                               : n_frames;
+  // VOXEL and the radius outlier stage: the sort and scan index a batch with int, so a batch of more than
+  // 2^31 - 1 (2^31 - 2) crop points runs in chunks; VOXEL's bounds pass puts the frame on gridDim.y, so a VOXEL
+  // chunk also holds at most 65535 frames
+  const uint64_t max_points = ror ? kRorMaxPoints : 0x7fffffffull;
+  uint32_t chunk = (voxel || ror) ? (uint32_t)std::min<uint64_t>(n_frames, std::max<uint64_t>(1, max_points / std::max<uint64_t>(n, 1)))
+                                  : n_frames;
+  if (voxel) chunk = std::min<uint32_t>(chunk, 65535);
+  if (ror) {
+    const size_t need = ror_stage_bytes(chunk, (uint32_t)n);
+    if (need > ctx->d_ror.cap) {
+      CU(ctx, cudaStreamSynchronize(ctx->s_compute));
+      if ((rc = grow_dev(ctx, ctx->d_ror, need))) return rc;
+    }
+  }
   if (voxel) {
     const size_t need = voxel_scratch_bytes(chunk, (uint32_t)n);
     if (need > ctx->d_voxel.cap) {
       CU(ctx, cudaStreamSynchronize(ctx->s_compute));
       if ((rc = grow_dev(ctx, ctx->d_voxel, need))) return rc;
     }
-  } else if (compact) {
+  } else if (finite_mode(ctx)) {
     const size_t need = reproject_scratch_bytes(n_frames, w, h, ctx->cfg.border);
     if (need > ctx->d_scratch.cap || reproject_table_bytes(w, h) > ctx->d_tables.cap) {
       CU(ctx, cudaStreamSynchronize(ctx->s_compute));
@@ -1071,8 +1153,41 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
     if ((rc = enqueue_kernels(ctx, static_cast<const uint8_t *>(d_in) + f0 * frame_stride, is_f32, nf, w, h, step,
                               frame_stride, d_med, d_points + f0 * points_stride, points_stride,
                               d_counts ? d_counts + f0 : nullptr, ctx->d_scratch.p, ctx->d_tables.p, ctx->d_ticket,
-                              ctx->s_compute, ctx->d_voxel.p)))
+                              ctx->s_compute, ctx->d_voxel.p, nullptr, ctx->d_ror.p)))
       return rc;
+  }
+  return D2PC_OK;
+}
+
+int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
+                               size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
+                               uint32_t *d_out_counts) {
+  if (!ctx || !d_in || !d_out || !d_out_counts || !ror_on(ctx)) return D2PC_ERR_INVALID_ARG;
+  const uint64_t bytes = (uint64_t)n_max * 16;
+  if (bytes > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // per-frame counts and PointCloud2.row_step are uint32
+  if (reinterpret_cast<uintptr_t>(d_in) % 16 || reinterpret_cast<uintptr_t>(d_out) % 16 || in_stride % 16 ||
+      out_stride % 16 || (n_frames > 1 && (in_stride < bytes || out_stride < bytes)))
+    return D2PC_ERR_BAD_DIMS;
+  if (n_frames == 0) return D2PC_OK;
+  // kept points are copied from the input after every flag is known: the two must not share bytes
+  const uintptr_t in0 = reinterpret_cast<uintptr_t>(d_in), out0 = reinterpret_cast<uintptr_t>(d_out);
+  const uint64_t in_end = in0 + (uint64_t)(n_frames - 1) * in_stride + bytes;
+  const uint64_t out_end = out0 + (uint64_t)(n_frames - 1) * out_stride + bytes;
+  if (bytes && in0 < out_end && out0 < in_end) return D2PC_ERR_INVALID_ARG;
+  CU(ctx, cudaSetDevice(ctx->device));
+  const uint32_t chunk =
+      (uint32_t)std::min<uint64_t>(n_frames, std::max<uint64_t>(1, kRorMaxPoints / std::max<uint64_t>(n_max, 1)));
+  const size_t need = ror_scratch_bytes(chunk, n_max);
+  if (need > ctx->d_ror.cap) {
+    CU(ctx, cudaStreamSynchronize(ctx->s_compute));
+    const int rc = grow_dev(ctx, ctx->d_ror, need);
+    if (rc) return rc;
+  }
+  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
+    const uint32_t nf = std::min(chunk, n_frames - f0);
+    const int rc = enqueue_ror(ctx, nf, n_max, d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
+                               d_out + f0 * out_stride, out_stride, d_out_counts + f0, ctx->d_ror.p, ctx->s_compute);
+    if (rc) return rc;
   }
   return D2PC_OK;
 }
@@ -1400,7 +1515,7 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
   if ((rc = slot_wait_idle(ctx, s))) return rc;
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
   const uint64_t n = crop_points(fw, fh, ctx->cfg.border);
-  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx);
+  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx), ror = ror_on(ctx);
   if ((rc = grow_dev(ctx, s.d_med, (size_t)fw * fh)) || (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
   // a synchronous call: the callback kernel stores the CROP cloud straight into the pinned buffer (see submit_common)
   uint8_t *d_direct = nullptr;
@@ -1412,14 +1527,15 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
       cudaGetLastError();
   }
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
-  if (compact && !voxel &&
+  if (finite_mode(ctx) &&
       ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, fw, fh, ctx->cfg.border), true)) ||
        (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(fw, fh)))))
     return rc;
   if (voxel && (rc = grow_dev(ctx, s.d_voxel, voxel_scratch_bytes(1, (uint32_t)n)))) return rc;
+  if (ror && (rc = grow_dev(ctx, s.d_ror, ror_stage_bytes(1, (uint32_t)n)))) return rc;
   rc = enqueue_kernels(ctx, ctx->d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh, s.d_med.p,
                        d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count, s.d_scratch.p, s.d_tables.p,
-                       s.d_count + 1, ctx->s_compute, s.d_voxel.p, s.d_count + 2);
+                       s.d_count + 1, ctx->s_compute, s.d_voxel.p, s.d_count + 2, s.d_ror.p);
   if (rc) return rc;
   uint64_t kept = n;
   if (compact) {
@@ -1431,7 +1547,7 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
     CU(ctx, cudaMemcpyAsync(s.h_out.p, s.d_out.p, kept * 16, cudaMemcpyDeviceToHost, ctx->s_compute));
   CU(ctx, cudaStreamSynchronize(ctx->s_compute));
   if (ctx->cfg.verbose) printf("Cloud size: %llu\n", (unsigned long long)kept);
-  fill_cloud(ctx, s.h_out.p, kept, cloud_is_dense(compact, voxel, s.h_count), out);
+  fill_cloud(ctx, s.h_out.p, kept, cloud_is_dense(compact, voxel && !ror, s.h_count), out);
   return D2PC_OK;
 }
 
@@ -1455,7 +1571,7 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
   const size_t pitch = w, frame_bytes = (size_t)w * h, nn = (size_t)g.n * g.n;
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
   const uint64_t n = crop_points(fw, fh, c.border);
-  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx);
+  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx), ror = ror_on(ctx);
   // the four input frames of a set live in one allocation, so that a contiguous pinned set is one DMA
   if ((rc = grow_dev(ctx, s.d_fuse_in[0], 4 * pitch * h))) return rc;
   uint8_t *const fin[4] = {s.d_fuse_in[0].p, s.d_fuse_in[0].p + pitch * h, s.d_fuse_in[0].p + 2 * pitch * h,
@@ -1465,13 +1581,15 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
       (rc = grow_dev(ctx, s.d_fused, (size_t)fw * fh)) || (rc = grow_dev(ctx, s.d_med, (size_t)fw * fh)) ||
       (rc = grow_dev(ctx, s.d_out, n * 16 + 16)) || (rc = grow_pin(ctx, s.h_out, n * 16 + 16)))
     return rc;
-  if (compact && !voxel &&
+  if (finite_mode(ctx) &&
       ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, fw, fh, c.border), true)) ||
        (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(fw, fh)))))
     return rc;
-  // (allocated without a clear: the voxel stage writes every word of its scratch before reading it, so it does
-  // not matter that this slot's kernels run on s_kern rather than on the stream grow_dev clears on)
+  // (allocated without a clear: the voxel and radius outlier stages write every word of their scratch before
+  // reading it, so it does not matter that this slot's kernels run on s_kern rather than on the stream grow_dev
+  // clears on)
   if (voxel && (rc = grow_dev(ctx, s.d_voxel, voxel_scratch_bytes(1, (uint32_t)n)))) return rc;
+  if (ror && (rc = grow_dev(ctx, s.d_ror, ror_stage_bytes(1, (uint32_t)n)))) return rc;
 
   NvtxRange nvtx_submit("d2pc submit fusion set");
   s.timed = ctx->timing && s.ev_start;
@@ -1513,7 +1631,7 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
                              nullptr, preprocess_scores != 0, &s.d_container, sk)))
     return rc;
   rc = enqueue_kernels(ctx, s.d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh, s.d_med.p, s.d_out.p, n * 16 + 16, s.d_count,
-                       s.d_scratch.p, s.d_tables.p, s.d_count + 1, sk, s.d_voxel.p, s.d_count + 2);
+                       s.d_scratch.p, s.d_tables.p, s.d_count + 1, sk, s.d_voxel.p, s.d_count + 2, s.d_ror.p);
   if (rc) return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, sk));
 
@@ -1527,7 +1645,7 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
   s.width = fw, s.height = fh;
   s.n_points = n;
   s.compact = compact;
-  s.voxel = voxel;
+  s.voxel = voxel && !ror;
   s.user_dst = nullptr, s.user_cap = 0, s.user_pinned = false, s.late_copy = false;
   return D2PC_OK;
 }

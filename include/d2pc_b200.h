@@ -123,7 +123,8 @@ typedef struct d2pc_cloud {
   uint32_t point_step; /* 16 */
   uint32_t row_step;   /* 16 * width */
   uint8_t is_bigendian; /* 0 */
-  uint8_t is_dense;     /* 0 in CROP mode (cpp:81); 1 in CROP_FINITE; VOXEL: 1, 0 for the overflow fallback */
+  uint8_t is_dense;     /* 0 in CROP mode (cpp:81); 1 in CROP_FINITE; VOXEL: 1, 0 for the overflow fallback;
+                           1 behind the radius outlier stage */
   uint32_t n_fields;    /* 3 */
   d2pc_point_field fields[3];
 } d2pc_cloud;
@@ -198,6 +199,49 @@ void d2pc_voxel_grid_default(d2pc_voxel_grid *grid);
 int d2pc_set_voxel_grid(d2pc_ctx *ctx, const d2pc_voxel_grid *grid);
 /* The grid last set (d2pc_voxel_grid_default's until then). */
 int d2pc_get_voxel_grid(const d2pc_ctx *ctx, d2pc_voxel_grid *grid);
+
+/* ---- radius outlier removal (a stage behind every filter mode) -------------------
+ *
+ * Off by default (radius 0).  With a radius set, the published cloud is pcl::RadiusOutlierRemoval<pcl::PointXYZ>
+ * (setNegative(false), keep_organized false) applied on the device to exactly the cloud the current filter mode
+ * would publish for that frame: CROP's N points (+-inf and NaN included), CROP_FINITE's compacted cloud, VOXEL's
+ * centroids (or, for a frame that took VOXEL's overflow fallback, its CROP cloud).  So CROP + this stage and
+ * CROP_FINITE + this stage publish the same bytes.  The setting is independent of d2pc_set_filter_mode.  The recipe:
+ *   1. r2 = radius * radius, in double.
+ *   2. A point takes part only when x, y and z are all finite.  A non-finite point is dropped and is nobody's
+ *      neighbour (PCL's kd-tree does not index it).
+ *   3. The squared distance of points i and j is float32 with no FMA: dx = xi - xj (likewise dy, dz),
+ *      s = (dx*dx + dy*dy) + dz*dz, each operation rounded.  (FLANN's L2_Simple<float>, as PCL's KdTreeFLANN uses it.)
+ *   4. neighbours(i) = the number of finite j with (double)s(i, j) <= r2; it counts i itself and any duplicate of i.
+ *   5. i is kept when neighbours(i) >= min_neighbors + 1, so min_neighbors = 0 keeps every finite point.
+ *   6. Kept points are copied unchanged, all 16 bytes, in input order; height 1, width = kept, is_dense 1,
+ *      row_step = 16 * width.
+ * Relation to PCL (RadiusOutlierRemoval::applyFilterIndices, PCL 1.8 - 1.12; restated from memory, PCL's source was
+ * not at hand when this was written -- the same footing as DESIGN.md section 0.1 for the OpenCV dispatch):
+ *   - is_dense input (CROP_FINITE, VOXEL): PCL runs nearestKSearch(k = min_neighbors + 1) per point and keeps it when
+ *     k neighbours were found and nn_dists[k - 1] <= r2 in double.  The k-th smallest distance is <= r2 exactly when
+ *     at least k distances are, which is rules 4-5.
+ *   - non-dense input (CROP, the VOXEL fallback): PCL runs radiusSearch, whose FLANN result set is believed to
+ *     test dist < (float)r2.  This library applies rule 4 to every input; the two differ only for a pair whose
+ *     distance lies exactly on the boundary (s == (float)r2, or between r2 and (float)r2).
+ *   - is_dense of the output: PCL's filter path copies the kept points into a fresh cloud; whether that copy sets
+ *     is_dense is not verified here.  The library publishes 1 (every kept point is finite).
+ * With a radius set every mode is a counted mode, as CROP_FINITE is: BUFFER_TOO_SMALL is reported by d2pc_wait, the
+ * kernel never stores into host memory ("direct_out" does not apply), d2pc_slot_timing's d2h_us covers the count,
+ * and the device batch entries need d_counts.  With radius 0 nothing of this applies. */
+typedef struct d2pc_radius_outlier {
+  uint32_t struct_size;   /* sizeof(d2pc_radius_outlier) */
+  double radius;          /* 0: the stage is off (the default); otherwise finite and > 0 */
+  uint32_t min_neighbors; /* PCL's setMinNeighborsInRadius; default 1 */
+} d2pc_radius_outlier;
+
+/* radius 0 (off), min_neighbors 1. */
+void d2pc_radius_outlier_default(d2pc_radius_outlier *p);
+/* D2PC_ERR_INVALID_ARG for a radius that is negative, NaN or infinite, or a wrong struct_size; the previous
+ * setting is kept then. */
+int d2pc_set_radius_outlier(d2pc_ctx *ctx, const d2pc_radius_outlier *p);
+/* The setting last made (d2pc_radius_outlier_default's until then). */
+int d2pc_get_radius_outlier(const d2pc_ctx *ctx, d2pc_radius_outlier *p);
 
 /* ---- the disparity callback, host buffers (the reference-facing calls) ------ */
 
@@ -294,6 +338,17 @@ int d2pc_reproject_f32_device(d2pc_ctx *ctx, const float *d_disp, uint32_t n_fra
 int d2pc_reproject_mono8_device(d2pc_ctx *ctx, const uint8_t *d_img, uint32_t n_frames, uint32_t width,
                                 uint32_t height, size_t step, size_t frame_stride, uint8_t *d_points,
                                 size_t points_stride, uint32_t *d_counts);
+
+/* The radius outlier stage alone (the context's d2pc_radius_outlier, which must have a radius > 0), on clouds
+ * already on the device -- for chaining, and for clouds that did not come from a disparity frame.  Frame f's
+ * input is d_in + f*in_stride bytes, d_in_counts[f] points of 16 bytes (d_in_counts NULL: n_max each; a count
+ * above n_max counts as n_max); its kept points go to d_out + f*out_stride and their number to d_out_counts[f].
+ * Pointers and strides 16-byte aligned, strides >= 16*n_max when n_frames > 1, n_max*16 < 2^32; the input and the
+ * output must not overlap (D2PC_ERR_INVALID_ARG).  n_frames has no other limit: batches of more than 2^31 - 2
+ * points run in chunks of frames. */
+int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
+                               size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
+                               uint32_t *d_out_counts);
 
 /* cv::medianBlur on CV_8UC1, replicate border (cpp:55-57 with ksize 11,
  * depth_map_fusion.cpp:124 with ksize 3).  ksize odd, 3..15. */

@@ -221,6 +221,20 @@ class Disparity2PCloud {
       d2pc_b200::check(d2pc_set_voxel_grid(ctx_, &g), "d2pc_set_voxel_grid", ctx_);
       d2pc_b200::check(d2pc_set_filter_mode(ctx_, D2PC_FILTER_VOXEL), "d2pc_set_filter_mode", ctx_);
     }
+    // optional, not in the reference: pcl::RadiusOutlierRemoval on the device behind the filter mode, on when
+    // radius_outlier_radius > 0
+    double ror_radius = 0.0;
+    int ror_min = 1;
+    nh_.param<double>("radius_outlier_radius", ror_radius, 0.0);
+    nh_.param<int>("radius_outlier_min_neighbors", ror_min, 1);
+    if (ror_radius != 0.0) {
+      if (ror_min < 0) throw std::runtime_error("radius_outlier_min_neighbors must not be negative");
+      d2pc_radius_outlier r;
+      d2pc_radius_outlier_default(&r);
+      r.radius = ror_radius;
+      r.min_neighbors = static_cast<uint32_t>(ror_min);
+      d2pc_b200::check(d2pc_set_radius_outlier(ctx_, &r), "d2pc_set_radius_outlier", ctx_);
+    }
   }
   ~Disparity2PCloud() {
     d2pc_destroy(ctx_);  // waits for the device: nothing writes into output_ any more
@@ -259,7 +273,8 @@ class Disparity2PCloud {
     output.point_step = cloud.point_step;
     output.row_step = cloud.row_step;
     output.is_dense = cloud.is_dense;
-    // CROP_FINITE / VOXEL keep fewer points than the crop holds: shrink the view, never the storage
+    // CROP_FINITE / VOXEL / the radius outlier stage keep fewer points than the crop holds: shrink the view, never
+    // the storage
     output.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
     output.header.stamp = msg->header.stamp;             // cpp:87
     output.header.frame_id = "/camera_optical_frame";    // cpp:89

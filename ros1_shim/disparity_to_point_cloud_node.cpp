@@ -52,6 +52,23 @@ class Disparity2PCloudGpu {
         ros::shutdown();
       }
     }
+    // optional, not in the reference: pcl::RadiusOutlierRemoval on the device behind the filter mode, on when
+    // radius_outlier_radius > 0
+    double ror_radius = 0.0;
+    int ror_min = 1;
+    nh_.param<double>("radius_outlier_radius", ror_radius, 0.0);
+    nh_.param<int>("radius_outlier_min_neighbors", ror_min, 1);
+    if (ror_radius != 0.0) {
+      d2pc_radius_outlier r;
+      d2pc_radius_outlier_default(&r);
+      r.radius = ror_radius;
+      r.min_neighbors = static_cast<uint32_t>(ror_min);
+      if (ror_min < 0 || d2pc_set_radius_outlier(ctx_, &r) != D2PC_OK) {
+        ROS_FATAL("radius_outlier_radius %g / radius_outlier_min_neighbors %d: not a valid setting", ror_radius,
+                  ror_min);
+        ros::shutdown();
+      }
+    }
   }
   ~Disparity2PCloudGpu() {
     d2pc_destroy(ctx_);
