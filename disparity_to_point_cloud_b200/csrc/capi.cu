@@ -49,11 +49,30 @@ struct PinBuf {
   size_t cap = 0;
 };
 
+// What the filter mode and the radius outlier stage make of one frame geometry (plan_cloud), decided once per call.
+struct CloudPlan {
+  uint64_t n = 0;           // crop points per frame
+  bool compact = false;     // the reproject kernels keep only finite points (CROP_FINITE)
+  bool voxel = false;       // the VOXEL stage runs on the CROP cloud
+  bool ror = false;         // the radius outlier stage runs on the mode's cloud
+  bool counted = false;     // the cloud's size is known only on the device: the kept count decides the bytes
+  uint32_t count_words = 1; // count words a slot reads back (Slot::d_count)
+  bool fallback_decides_dense = false;  // VOXEL without the outlier stage: the overflow fallback flag clears is_dense
+};
+
+// The device buffers between a batch's input frames and its cloud: one set per slot, one for the device batch.
+struct StageBufs {
+  DevBuf med;      // median-filtered frames
+  DevBuf scratch;  // CROP_FINITE tile descriptors (epoch-tagged: zero when allocated, see next_epoch)
+  DevBuf tables;   // CROP_FINITE tables
+  DevBuf voxel;    // VOXEL: the CROP clouds, then the stage's keys / indices / sort temp (voxel.h)
+  DevBuf ror;      // radius outlier stage: the mode's clouds and counts, then the stage's scratch (radius_outlier.h)
+};
+
 struct Slot {
   PinBuf h_in, h_out;
-  DevBuf d_in, d_med, d_out, d_scratch, d_tables;
-  DevBuf d_voxel;  // VOXEL mode: the CROP cloud and the voxel stage's keys / indices / sort temp (voxel.h)
-  DevBuf d_ror;    // radius outlier stage: the mode's cloud and counts, then the stage's scratch (radius_outlier.h)
+  DevBuf d_in, d_out;
+  StageBufs stages;
   // fusion pipeline (d2pc_submit_fusion): the four input frames, the two preprocessed scores, merge outputs
   DevBuf d_fuse_in[4], d_pre[2], d_container, d_combined, d_fused;
   uint32_t *d_count = nullptr;  // [0] = kept points, [1] = compaction ticket, [2] = VOXEL overflow fallback taken
@@ -63,10 +82,7 @@ struct Slot {
   bool timed = false;              // the last submission on this slot recorded all four events with timing
   cudaStream_t s_kern = nullptr;  // fusion pipeline: this slot's own kernel stream (small kernels of consecutive sets overlap)
   bool pending = false;
-  uint32_t width = 0, height = 0;
-  uint64_t n_points = 0;
-  bool compact = false;  // the count decides the bytes (CROP_FINITE, VOXEL)
-  bool voxel = false;    // VOXEL without the radius outlier stage: is_dense comes from the fallback flag
+  CloudPlan plan;  // of the pending submission
   // caller-supplied destination of this submission (d2pc_submit_*_into); nullptr = library-owned h_out
   uint8_t *user_dst = nullptr;
   size_t user_cap = 0;
@@ -89,8 +105,7 @@ struct d2pc_ctx {
   uint32_t epoch = 0;
   uint64_t launches = 0;
   std::string last_cuda_error;
-  // device-entry scratch
-  DevBuf d_scratch, d_tables, d_med_batch, d_voxel, d_ror;
+  StageBufs batch;  // the device-batch entries' stage buffers (their kernels run on s_compute)
   uint32_t *d_ticket = nullptr;
   d2pc_voxel_grid voxel;  // D2PC_FILTER_VOXEL parameters (d2pc_set_voxel_grid)
   bool voxel_set = false;
@@ -151,16 +166,16 @@ int cuda_fail(d2pc_ctx *ctx, cudaError_t e, const char *what) {
     if (e__ != cudaSuccess) return cuda_fail(ctx, e__, #call); \
   } while (0)
 
-int grow_dev(d2pc_ctx *ctx, DevBuf &b, size_t bytes, bool zero = false) {
+// clear_on: a new buffer is zeroed on this stream, the one whose kernels read it, so the clear is ordered before
+// them (a legacy-stream cudaMemset is not ordered with cudaStreamNonBlocking streams)
+int grow_dev(d2pc_ctx *ctx, DevBuf &b, size_t bytes, cudaStream_t clear_on = nullptr) {
   if (bytes <= b.cap) return D2PC_OK;
   if (b.p) CU(ctx, cudaFree(b.p));
   b.p = nullptr;
   b.cap = 0;
   const size_t cap = align_up(bytes, 1 << 16);
   CU(ctx, cudaMalloc(&b.p, cap));
-  // cleared on the compute stream: every kernel that reads the buffer is enqueued there later, so the clear is
-  // ordered before it (a legacy-stream cudaMemset is not ordered with cudaStreamNonBlocking streams)
-  if (zero) CU(ctx, cudaMemsetAsync(b.p, 0, cap, ctx->s_compute));
+  if (clear_on) CU(ctx, cudaMemsetAsync(b.p, 0, cap, clear_on));
   b.cap = cap;
   return D2PC_OK;
 }
@@ -237,33 +252,45 @@ void free_pin(PinBuf &b) {
   if (b.p) pinned_free(b.p);
   b = PinBuf{};
 }
+void free_stages(StageBufs &b) {
+  for (DevBuf *d : {&b.med, &b.scratch, &b.tables, &b.voxel, &b.ror}) free_dev(*d);
+}
 
 uint64_t crop_points(uint32_t w, uint32_t h, int border) {
   const long cw = (long)w - 2L * border, ch = (long)h - 2L * border;
   return (cw > 0 && ch > 0) ? (uint64_t)cw * (uint64_t)ch : 0;
 }
 
-bool ror_on(const d2pc_ctx *ctx) { return ctx->ror.radius > 0.0; }
-// CROP_FINITE and VOXEL clouds, and every cloud of the radius outlier stage, have a size known only on the device:
-// the kept count decides the bytes
-bool counted_mode(const d2pc_ctx *ctx) {
-  return ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE || ctx->cfg.filter_mode == D2PC_FILTER_VOXEL || ror_on(ctx);
+CloudPlan plan_cloud(const d2pc_ctx *ctx, uint32_t w, uint32_t h) {
+  CloudPlan p;
+  p.n = crop_points(w, h, ctx->cfg.border);
+  p.compact = ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE;
+  p.voxel = ctx->cfg.filter_mode == D2PC_FILTER_VOXEL;
+  p.ror = ctx->ror.radius > 0.0;
+  p.counted = p.compact || p.voxel || p.ror;
+  p.count_words = p.voxel ? 3 : 1;  // the kept count [, the ticket, the VOXEL fallback flag]
+  p.fallback_decides_dense = p.voxel && !p.ror;  // the outlier stage's output is always dense
+  return p;
 }
-bool voxel_mode(const d2pc_ctx *ctx) { return ctx->cfg.filter_mode == D2PC_FILTER_VOXEL; }
-bool finite_mode(const d2pc_ctx *ctx) { return ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE; }
 
-// a cloud's is_dense: 0 in CROP mode (cpp:81), 1 in CROP_FINITE, in VOXEL 1 unless the overflow fallback was taken
-// (`voxel` is false behind the radius outlier stage, whose output is always dense)
-bool cloud_is_dense(bool compact, bool voxel, const uint32_t *h_count) { return compact && !(voxel && h_count[2]); }
+// a cloud's size: all crop points, or the count the device kept
+uint64_t kept_points(const CloudPlan &p, const uint32_t *h_count) { return p.counted && p.n ? h_count[0] : p.n; }
+// a cloud's is_dense: 0 in CROP mode (cpp:81); 1 for a counted cloud, except a VOXEL frame that took the overflow
+// fallback
+bool cloud_is_dense(const CloudPlan &p, const uint32_t *h_count) {
+  return p.counted && !(p.fallback_decides_dense && h_count[2]);
+}
 
 uint32_t next_epoch(d2pc_ctx *ctx) {
-  // 30-bit launch epoch inside the tile descriptors; 0 is "never written"
+  // 30-bit launch epoch inside the tile descriptors; 0 is "never written".  The wrap clears every descriptor buffer
+  // with the device idle and waits for the clear, so it precedes the next launch on any stream.
   if (++ctx->epoch >= (1u << 30)) {
     ctx->epoch = 1;
     cudaDeviceSynchronize();
     for (auto &s : ctx->slots)
-      if (s.d_scratch.p) cudaMemsetAsync(s.d_scratch.p, 0, s.d_scratch.cap, ctx->s_compute);
-    if (ctx->d_scratch.p) cudaMemsetAsync(ctx->d_scratch.p, 0, ctx->d_scratch.cap, ctx->s_compute);
+      if (s.stages.scratch.p) cudaMemsetAsync(s.stages.scratch.p, 0, s.stages.scratch.cap, ctx->s_compute);
+    if (ctx->batch.scratch.p) cudaMemsetAsync(ctx->batch.scratch.p, 0, ctx->batch.scratch.cap, ctx->s_compute);
+    cudaStreamSynchronize(ctx->s_compute);
   }
   return ctx->epoch;
 }
@@ -334,20 +361,70 @@ int upload_dense(d2pc_ctx *ctx, size_t stage_off, uint8_t *dst, const uint8_t *s
   return D2PC_OK;
 }
 
+// A batch of frames on the device: frame f at data + f * frame_stride, rows `step` bytes apart.
+struct FrameBatch {
+  const uint8_t *data;
+  bool is_f32;
+  uint32_t n_frames, w, h;
+  size_t step, frame_stride;
+};
+
+// Where a stage writes a batch's clouds: frame f at points + f * stride, its point count at counts[f].
+struct CloudDst {
+  uint8_t *points;
+  size_t stride;
+  uint32_t *counts;
+};
+
+// Grows a stage-buffer set for batch `in` under plan p.  `stream` is where the set's kernels run; a new CROP_FINITE
+// descriptor buffer is cleared there.  in_use: work queued on `stream` may still use the set, so the stream is
+// synchronised before the first buffer is replaced (and only then).
+int grow_stages(d2pc_ctx *ctx, StageBufs &b, const CloudPlan &p, const FrameBatch &in, cudaStream_t stream,
+                bool in_use) {
+  const uint32_t n = (uint32_t)p.n;
+  const bool median = !in.is_f32 && ctx->cfg.median_ksize > 1;
+  const struct {
+    DevBuf &buf;
+    size_t bytes;
+    bool zero;
+  } need[] = {
+      {b.med, median ? in.frame_stride * (in.n_frames - 1) + in.step * in.h : 0, false},
+      {b.scratch, p.compact ? reproject_scratch_bytes(in.n_frames, in.w, in.h, ctx->cfg.border) : 0, true},
+      {b.tables, p.compact ? reproject_table_bytes(in.w, in.h) : 0, false},
+      {b.voxel, p.voxel ? voxel_scratch_bytes(in.n_frames, n) : 0, false},
+      {b.ror, p.ror ? ror_stage_bytes(in.n_frames, n) : 0, false},
+  };
+  for (const auto &x : need) {
+    if (x.bytes <= x.buf.cap) continue;
+    if (in_use) CU(ctx, cudaStreamSynchronize(stream));
+    in_use = false;
+    const int rc = grow_dev(ctx, x.buf, x.bytes, x.zero ? stream : nullptr);
+    if (rc) return rc;
+  }
+  return D2PC_OK;
+}
+
+// Frames per launch for a stage whose sort and scan index a launch's points with int: at most max_points points (but
+// at least one frame) and max_frames frames.
+uint32_t frames_per_chunk(uint32_t n_frames, uint64_t points_per_frame, uint64_t max_points, uint32_t max_frames) {
+  const uint64_t by_points = std::max<uint64_t>(1, max_points / std::max<uint64_t>(points_per_frame, 1));
+  return (uint32_t)std::min<uint64_t>({n_frames, max_frames, by_points});
+}
+
 // The VOXEL stage of a batch whose CROP clouds are in the head of `voxel_scratch` (voxel.h), with the context's grid.
-int enqueue_voxel(d2pc_ctx *ctx, uint32_t n_frames, uint64_t n, uint8_t *d_out, size_t out_stride, uint32_t *d_counts,
-                  uint32_t *fallback, void *voxel_scratch, cudaStream_t stream) {
+int enqueue_voxel(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n, const CloudDst &dst, uint32_t *fallback,
+                  void *voxel_scratch, cudaStream_t stream) {
   const d2pc_voxel_grid &g = ctx->voxel;
   VoxelLaunch V;
   V.n_frames = n_frames;
-  V.n = (uint32_t)n;
+  V.n = n;
   V.p.inv[0] = 1.0f / g.leaf_x, V.p.inv[1] = 1.0f / g.leaf_y, V.p.inv[2] = 1.0f / g.leaf_z;
   V.p.min_points = g.min_points_per_voxel;
   V.p.limit_field = g.limit_field;
   V.p.limit_min = g.limit_min, V.p.limit_max = g.limit_max;
-  V.out = d_out;
-  V.out_stride = out_stride;
-  V.counts = d_counts;
+  V.out = dst.points;
+  V.out_stride = dst.stride;
+  V.counts = dst.counts;
   V.fallback = fallback;
   V.scratch = voxel_scratch;
   int nl = 0;
@@ -359,8 +436,7 @@ int enqueue_voxel(d2pc_ctx *ctx, uint32_t n_frames, uint64_t n, uint8_t *d_out, 
 // The radius outlier stage with the context's setting on n_frames clouds (frame f at in + f * in_stride, in_counts[f]
 // points; in_counts null: n_max each).
 int enqueue_ror(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n_max, const uint8_t *in, size_t in_stride,
-                const uint32_t *in_counts, uint8_t *d_out, size_t out_stride, uint32_t *d_counts, void *scratch,
-                cudaStream_t stream) {
+                const uint32_t *in_counts, const CloudDst &dst, void *scratch, cudaStream_t stream) {
   RorLaunch R;
   R.n_frames = n_frames;
   R.n_max = n_max;
@@ -369,9 +445,9 @@ int enqueue_ror(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n_max, const uint8_t 
   R.in_counts = in_counts;
   R.radius = ctx->ror.radius;
   R.min_neighbors = ctx->ror.min_neighbors;
-  R.out = d_out;
-  R.out_stride = out_stride;
-  R.counts = d_counts;
+  R.out = dst.points;
+  R.out_stride = dst.stride;
+  R.counts = dst.counts;
   R.scratch = scratch;
   int nl = 0;
   CU(ctx, launch_radius_outlier(R, stream, &nl));
@@ -379,69 +455,29 @@ int enqueue_ror(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n_max, const uint8_t 
   return D2PC_OK;
 }
 
-// Enqueue [median] + reproject for one frame batch already on the device.
-// In VOXEL mode the CROP kernels write into the head of `voxel_scratch` (voxel_scratch_bytes(n_frames, crop)) and
-// the voxel stage writes d_out / d_counts / fallback (per frame; may be null).
-// With the radius outlier stage on, the mode's clouds and counts go to the head of `ror_buf`
-// (ror_stage_bytes(n_frames, crop)) and the stage writes d_out / d_counts.
-int enqueue_kernels(d2pc_ctx *ctx, const uint8_t *d_in, bool is_f32, uint32_t n_frames, uint32_t w, uint32_t h,
-                    size_t step, size_t frame_stride, uint8_t *d_med, uint8_t *d_out, size_t out_stride,
-                    uint32_t *d_counts, void *scratch, void *tables, uint32_t *ticket, cudaStream_t stream,
-                    void *voxel_scratch = nullptr, uint32_t *fallback = nullptr, void *ror_buf = nullptr) {
+// [median] + reproject of a batch into dst.
+int enqueue_reproject(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, StageBufs &b, const CloudDst &dst,
+                      uint32_t *ticket, cudaStream_t stream) {
   const d2pc_config &c = ctx->cfg;
   int nl = 0;
-  const bool ror = ror_on(ctx);
-  const uint32_t n_crop = (uint32_t)crop_points(w, h, c.border);
-  uint8_t *const r_out = d_out;
-  const size_t r_stride = out_stride;
-  uint32_t *const r_counts = d_counts;
-  RorStage rs{};
-  if (ror) {  // the mode's clouds go to the stage's buffer, dense, and are its input
-    rs = ror_stage(ror_buf, n_frames, n_crop);
-    d_out = rs.clouds;
-    out_stride = (size_t)n_crop * 16;
-    d_counts = rs.counts;
-  }
-  const bool voxel = voxel_mode(ctx);
-  uint8_t *const v_out = d_out;
-  const size_t v_stride = out_stride;
-  uint32_t *const v_counts = d_counts;
-  if (voxel) {  // the CROP cloud goes to scratch, dense, and is the voxel stage's input
-    d_out = reinterpret_cast<uint8_t *>(voxel_crop(voxel_scratch));
-    out_stride = crop_points(w, h, c.border) * 16;
-    d_counts = nullptr;
-  }
-  auto voxel_stage = [&]() {
-    return voxel ? enqueue_voxel(ctx, n_frames, crop_points(w, h, c.border), v_out, v_stride, v_counts, fallback,
-                                 voxel_scratch, stream)
-                 : (int)D2PC_OK;
-  };
-  auto filter_stages = [&]() {
-    const int rc = voxel_stage();
-    if (rc || !ror) return rc;
-    // a CROP cloud has all n_crop points; the other modes' counts are on the device
-    return enqueue_ror(ctx, n_frames, n_crop, rs.clouds, (size_t)n_crop * 16,
-                       c.filter_mode == D2PC_FILTER_CROP ? nullptr : rs.counts, r_out, r_stride, r_counts, rs.scratch,
-                       stream);
-  };
   ReprojectLaunch L;
-  L.in = d_in;
-  L.in_is_f32 = is_f32;
-  L.step = step;
-  L.frame_stride = frame_stride;
-  L.n_frames = n_frames;
-  L.width = w;
-  L.height = h;
+  L.in = in.data;
+  L.in_is_f32 = in.is_f32;
+  L.step = in.step;
+  L.frame_stride = in.frame_stride;
+  L.n_frames = in.n_frames;
+  L.width = in.w;
+  L.height = in.h;
   L.border = c.border;
   L.scale = c.disparity_scale;
-  L.out = d_out;
-  L.out_stride_bytes = out_stride;
-  L.counts = d_counts;
+  L.out = dst.points;
+  L.out_stride_bytes = dst.stride;
+  L.counts = dst.counts;
   L.Q = &ctx->Q;
   L.arith_fast = c.arith_mode == D2PC_ARITH_FAST;
-  L.compact = c.filter_mode == D2PC_FILTER_CROP_FINITE;
-  L.scratch = scratch;
-  L.tables = tables;
+  L.compact = p.compact;
+  L.scratch = b.scratch.p;
+  L.tables = b.tables.p;
   L.ticket = ticket;
   L.sm_count = ctx->sm_count;
   L.rows_per_unit = ctx->rows_per_unit;
@@ -452,21 +488,21 @@ int enqueue_kernels(d2pc_ctx *ctx, const uint8_t *d_in, bool is_f32, uint32_t n_
   L.exact_variant = ctx->exact_variant;
   L.zero_numer = ctx->zero_numer;
   L.prefetch_dist = ctx->prefetch_dist;
-  if (!is_f32 && c.median_ksize > 1) {
+  if (!in.is_f32 && c.median_ksize > 1) {
     // cpp:55-57: only crop pixels are consumed downstream, so only those medians are produced
     // (the replicate border is still the image edge, which matters when border < ksize/2).
     MedianLaunch M;
-    M.src = d_in;
-    M.dst = d_med;
-    M.src_step = M.dst_step = step;
-    M.src_frame_stride = M.dst_frame_stride = frame_stride;
-    M.n_frames = n_frames;
-    M.width = (int)w;
-    M.height = (int)h;
+    M.src = in.data;
+    M.dst = b.med.p;
+    M.src_step = M.dst_step = in.step;
+    M.src_frame_stride = M.dst_frame_stride = in.frame_stride;
+    M.n_frames = in.n_frames;
+    M.width = (int)in.w;
+    M.height = (int)in.h;
     M.ox0 = c.border;
     M.oy0 = c.border;
-    M.ow = (int)w - 2 * c.border;
-    M.oh = (int)h - 2 * c.border;
+    M.ow = (int)in.w - 2 * c.border;
+    M.oh = (int)in.h - 2 * c.border;
     M.ksize = c.median_ksize;
     M.sm_count = ctx->sm_count;
     M.strip_rows = ctx->median_strip;
@@ -478,20 +514,40 @@ int enqueue_kernels(d2pc_ctx *ctx, const uint8_t *d_in, bool is_f32, uint32_t n_
                       reproject_fuses_with_median(L, &zero_numer);
     if (fuse) {
       M.zero_numer = zero_numer;
-      M.points = d_out;
-      M.points_stride_bytes = out_stride;
+      M.points = dst.points;
+      M.points_stride_bytes = dst.stride;
       M.Q = &ctx->Q;
       M.scale = c.disparity_scale;
     }
     CU(ctx, launch_median_u8(M, stream, &nl));
     ctx->launches += nl;
-    if (fuse) return filter_stages();
-    L.in = d_med;
+    if (fuse) return D2PC_OK;
+    L.in = b.med.p;
   }
   L.epoch = L.compact ? next_epoch(ctx) : 0;
   CU(ctx, launch_reproject(L, stream, &nl));
   ctx->launches += nl;
-  return filter_stages();
+  return D2PC_OK;
+}
+
+// Enqueue the plan's stages for one frame batch already on the device: [median] + reproject, then VOXEL, then the
+// radius outlier stage.  The last stage that runs writes `out`; each one before it writes its clouds dense into the
+// next stage's buffer.  fallback: VOXEL's per-frame overflow fallback flags (may be null).
+int enqueue_kernels(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, StageBufs &b, const CloudDst &out,
+                    uint32_t *fallback, uint32_t *ticket, cudaStream_t stream) {
+  const uint32_t n = (uint32_t)p.n;
+  const size_t dense = (size_t)n * 16;
+  const RorStage rs = p.ror ? ror_stage(b.ror.p, in.n_frames, n) : RorStage{};
+  const CloudDst voxel_dst = p.ror ? CloudDst{rs.clouds, dense, rs.counts} : out;
+  const CloudDst crop_dst =
+      p.voxel ? CloudDst{reinterpret_cast<uint8_t *>(voxel_crop(b.voxel.p)), dense, nullptr} : voxel_dst;
+  int rc = enqueue_reproject(ctx, p, in, b, crop_dst, ticket, stream);
+  if (!rc && p.voxel) rc = enqueue_voxel(ctx, in.n_frames, n, voxel_dst, fallback, b.voxel.p, stream);
+  // a CROP cloud has all n points; the other modes' counts are on the device
+  if (!rc && p.ror)
+    rc = enqueue_ror(ctx, in.n_frames, n, rs.clouds, dense, p.compact || p.voxel ? rs.counts : nullptr, out,
+                     rs.scratch, stream);
+  return rc;
 }
 
 int check_frame(const d2pc_ctx *ctx, const void *data, uint32_t w, uint32_t h, size_t step, int esz) {
@@ -508,6 +564,36 @@ int slot_wait_idle(d2pc_ctx *ctx, Slot &s) {
     s.pending = false;
   }
   return D2PC_OK;
+}
+
+// The device alias of page-locked host memory, for a kernel's point stores into it; null where there is none or it is
+// not 16-byte aligned.
+uint8_t *direct_alias(void *host) {
+  void *dp = nullptr;
+  if (cudaHostGetDevicePointer(&dp, host, 0) == cudaSuccess && reinterpret_cast<uintptr_t>(dp) % 16 == 0)
+    return static_cast<uint8_t *>(dp);
+  cudaGetLastError();
+  return nullptr;
+}
+
+// A slot's D2H (stream 3), behind its kernels: the count words when the count decides the bytes (the payload copy is
+// issued in d2pc_wait), else the whole cloud into dst.
+int enqueue_readback(d2pc_ctx *ctx, Slot &s, const CloudPlan &p, uint8_t *dst) {
+  CU(ctx, cudaStreamWaitEvent(ctx->s_d2h, s.ev_kernel, 0));
+  if (p.counted)
+    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, p.count_words * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+                            ctx->s_d2h));
+  else if (p.n)
+    CU(ctx, cudaMemcpyAsync(dst, s.d_out.p, p.n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
+  CU(ctx, cudaEventRecord(s.ev_d2h, ctx->s_d2h));
+  return D2PC_OK;
+}
+
+void arm_slot(Slot &s, const CloudPlan &p, uint8_t *user_dst, size_t user_cap, bool user_pinned, bool late_copy) {
+  s.pending = true;
+  s.plan = p;
+  s.user_dst = user_dst, s.user_cap = user_cap, s.user_pinned = user_pinned;
+  s.late_copy = late_copy;
 }
 
 int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_t h, uint32_t step, bool is_f32,
@@ -527,34 +613,23 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   // mono8 rows of any width (the callback kernel reads bytes; a 665-wide fused map is then one DMA instead of a
   // pitched 2-D copy); float rows that are not 16-byte multiples keep a 256-byte pitch for the vector loads.
   const size_t d_pitch = (row_bytes % 16 == 0 || !is_f32) ? row_bytes : align_up(row_bytes, kAlign);
-  const uint64_t n = crop_points(w, h, ctx->cfg.border);
+  const CloudPlan p = plan_cloud(ctx, w, h);
+  const uint64_t n = p.n;
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // PointCloud2.row_step / width are uint32
-  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx), ror = ror_on(ctx);
-  if (user_dst && !compact && user_cap < n * 16) return D2PC_ERR_BUFFER_TOO_SMALL;
+  if (user_dst && !p.counted && user_cap < n * 16) return D2PC_ERR_BUFFER_TOO_SMALL;
   const bool user_pinned = user_dst && reinterpret_cast<uintptr_t>(user_dst) % 16 == 0 && lookup_pinned(ctx, user_dst);
   if ((rc = grow_dev(ctx, s.d_in, d_pitch * h))) return rc;
-  if (!is_f32 && ctx->cfg.median_ksize > 1 && (rc = grow_dev(ctx, s.d_med, d_pitch * h))) return rc;
-  const bool late_copy = sync_call && user_dst && !user_pinned && !compact && n;
+  const bool late_copy = sync_call && user_dst && !user_pinned && !p.counted && n;
   if (!user_pinned && !late_copy && (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
   // direct output: the kernel's point stores go over PCIe into the page-locked destination while it runs, so a lone
   // frame no longer pays kernel + copy back to back (CROP only: a compacted cloud's size is not known up front)
   uint8_t *d_direct = nullptr;
-  if (!compact && n && !late_copy &&
-      (ctx->direct_out > 0 || (ctx->direct_out == 0 && sync_call && !is_f32 && ctx->cfg.median_ksize > 1))) {
-    void *dp = nullptr;
-    if (cudaHostGetDevicePointer(&dp, user_pinned ? user_dst : s.h_out.p, 0) == cudaSuccess &&
-        reinterpret_cast<uintptr_t>(dp) % 16 == 0)
-      d_direct = static_cast<uint8_t *>(dp);
-    else
-      cudaGetLastError();
-  }
+  if (!p.counted && n && !late_copy &&
+      (ctx->direct_out > 0 || (ctx->direct_out == 0 && sync_call && !is_f32 && ctx->cfg.median_ksize > 1)))
+    d_direct = direct_alias(user_pinned ? user_dst : s.h_out.p);
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
-  if (finite_mode(ctx) &&
-      ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, w, h, ctx->cfg.border), true)) ||
-       (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(w, h)))))
-    return rc;
-  if (voxel && (rc = grow_dev(ctx, s.d_voxel, voxel_scratch_bytes(1, (uint32_t)n)))) return rc;
-  if (ror && (rc = grow_dev(ctx, s.d_ror, ror_stage_bytes(1, (uint32_t)n)))) return rc;
+  const FrameBatch in{s.d_in.p, is_f32, 1, w, h, d_pitch, d_pitch * h};
+  if ((rc = grow_stages(ctx, s.stages, p, in, ctx->s_compute, false))) return rc;
 
   // ---- H2D (stream 1).  Pinned caller memory is DMA'd in place; pageable memory is staged.
   const void *src = data;
@@ -588,45 +663,22 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   CU(ctx, cudaStreamWaitEvent(ctx->s_compute, s.ev_h2d, 0));
   {
     NvtxRange nvtx_k("d2pc kernels");
-    rc = enqueue_kernels(ctx, s.d_in.p, is_f32, 1, w, h, d_pitch, d_pitch * h, s.d_med.p,
-                         d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count, s.d_scratch.p, s.d_tables.p,
-                         s.d_count + 1, ctx->s_compute, s.d_voxel.p, s.d_count + 2, s.d_ror.p);
+    rc = enqueue_kernels(ctx, p, in, s.stages, {d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count},
+                         s.d_count + 2, s.d_count + 1, ctx->s_compute);
   }
   if (rc) return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, ctx->s_compute));
 
-  // ---- D2H (stream 3)
   NvtxRange nvtx_d2h("d2pc D2H");
-  s.late_copy = late_copy;
   if (d_direct || late_copy) {
     // the cloud is already in host memory when the kernel ends (direct output), or leaves the device in d2pc_wait
     // (pageable destination of a synchronous call): the slot completes on the compute stream
     CU(ctx, cudaEventRecord(s.ev_d2h, ctx->s_compute));
-    s.pending = true;
-    s.width = w, s.height = h, s.n_points = n, s.compact = false, s.voxel = false;
-    s.user_dst = user_dst, s.user_cap = user_cap, s.user_pinned = user_pinned;
-    return D2PC_OK;
-  }
-  CU(ctx, cudaStreamWaitEvent(ctx->s_d2h, s.ev_kernel, 0));
-  if (compact) {
-    // the kept count decides how many bytes travel: fetch it (and the VOXEL fallback flag), the payload copy is
-    // issued in d2pc_wait
-    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, (voxel ? 3 : 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                            ctx->s_d2h));
-  } else if (n) {
+  } else {
     // a page-locked caller buffer receives the cloud by DMA directly; a pageable one is filled from h_out in wait
-    CU(ctx, cudaMemcpyAsync(user_pinned ? user_dst : s.h_out.p, s.d_out.p, n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    if ((rc = enqueue_readback(ctx, s, p, user_pinned ? user_dst : s.h_out.p))) return rc;
   }
-  CU(ctx, cudaEventRecord(s.ev_d2h, ctx->s_d2h));
-  s.pending = true;
-  s.width = w;
-  s.height = h;
-  s.n_points = n;
-  s.compact = compact;
-  s.voxel = voxel && !ror;
-  s.user_dst = user_dst;
-  s.user_cap = user_cap;
-  s.user_pinned = user_pinned;
+  arm_slot(s, p, user_dst, user_cap, user_pinned, late_copy);
   return D2PC_OK;
 }
 
@@ -775,7 +827,8 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
     for (auto &s : ctx->slots) {
       const size_t pitch = align_up((size_t)c.max_width * 4, kAlign);
       const uint64_t np = crop_points(c.max_width, c.max_height, c.border);
-      if ((rc = grow_dev(ctx, s.d_in, pitch * c.max_height)) || (rc = grow_dev(ctx, s.d_med, pitch * c.max_height)) ||
+      if ((rc = grow_dev(ctx, s.d_in, pitch * c.max_height)) ||
+          (rc = grow_dev(ctx, s.stages.med, pitch * c.max_height)) ||
           (rc = grow_dev(ctx, s.d_out, np * 16 + 16)) || (rc = grow_pin(ctx, s.h_out, np * 16 + 16)) ||
           (rc = grow_pin(ctx, s.h_in, (size_t)c.max_width * 4 * c.max_height)))
         return fail(rc);
@@ -791,8 +844,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
   cudaDeviceSynchronize();
   for (auto &s : ctx->slots) {
     free_pin(s.h_in), free_pin(s.h_out);
-    free_dev(s.d_in), free_dev(s.d_med), free_dev(s.d_out), free_dev(s.d_scratch), free_dev(s.d_tables);
-    free_dev(s.d_voxel), free_dev(s.d_ror);
+    free_dev(s.d_in), free_dev(s.d_out), free_stages(s.stages);
     for (auto &b : s.d_fuse_in) free_dev(b);
     free_dev(s.d_pre[0]), free_dev(s.d_pre[1]), free_dev(s.d_container), free_dev(s.d_combined), free_dev(s.d_fused);
     if (s.d_count) cudaFree(s.d_count);
@@ -803,7 +855,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
     if (s.ev_start) cudaEventDestroy(s.ev_start);
     if (s.s_kern) cudaStreamDestroy(s.s_kern);
   }
-  free_dev(ctx->d_scratch), free_dev(ctx->d_tables), free_dev(ctx->d_med_batch), free_dev(ctx->d_voxel), free_dev(ctx->d_ror);
+  free_stages(ctx->batch);
   for (auto &b : ctx->d_fuse_in) free_dev(b);
   free_dev(ctx->d_container), free_dev(ctx->d_combined), free_dev(ctx->d_fused);
   free_pin(ctx->h_fused), free_pin(ctx->h_combined);
@@ -933,32 +985,24 @@ int d2pc_wait(d2pc_ctx *ctx, int slot, d2pc_cloud *out) {
   if (!s.pending) return D2PC_ERR_NOT_READY;
   CU(ctx, cudaSetDevice(ctx->device));
   CU(ctx, cudaEventSynchronize(s.ev_d2h));
-  uint64_t n = s.n_points;
-  bool in_place = s.user_pinned;  // the caller's buffer already holds the cloud
-  if (s.compact) {
-    n = s.n_points ? s.h_count[0] : 0;
-    if (s.user_dst && s.user_cap < n * 16) {
-      s.pending = false;
-      return D2PC_ERR_BUFFER_TOO_SMALL;
-    }
-    // the payload copy is synchronous here anyway, so it goes straight to the caller's buffer, page-locked or not
-    if (n) {
-      CU(ctx, cudaMemcpyAsync(s.user_dst ? s.user_dst : s.h_out.p, s.d_out.p, n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
-      CU(ctx, cudaStreamSynchronize(ctx->s_d2h));
-    }
-    in_place = true;
-  } else if (s.late_copy) {
-    if (n) {
-      CU(ctx, cudaMemcpyAsync(s.user_dst, s.d_out.p, n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
-      CU(ctx, cudaStreamSynchronize(ctx->s_d2h));
-    }
-    in_place = true;
+  const uint64_t n = kept_points(s.plan, s.h_count);
+  if (s.plan.counted && s.user_dst && s.user_cap < n * 16) {
+    s.pending = false;
+    return D2PC_ERR_BUFFER_TOO_SMALL;
   }
-  if (s.user_dst && !in_place && n) memcpy(s.user_dst, s.h_out.p, n * 16);
+  // a counted cloud and a late copy leave the device here: the copy is synchronous anyway, so it goes straight to
+  // the caller's buffer, page-locked or not
+  const bool copy_here = s.plan.counted || s.late_copy;
+  if (copy_here && n) {
+    CU(ctx, cudaMemcpyAsync(s.user_dst ? s.user_dst : s.h_out.p, s.d_out.p, n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CU(ctx, cudaStreamSynchronize(ctx->s_d2h));
+  }
+  // otherwise a page-locked caller buffer already holds the cloud; a pageable one is filled from h_out
+  if (s.user_dst && !s.user_pinned && !copy_here && n) memcpy(s.user_dst, s.h_out.p, n * 16);
   s.late_copy = false;
   s.pending = false;
   if (ctx->cfg.verbose) printf("Cloud size: %llu\n", (unsigned long long)n);  // cpp:82
-  if (out) fill_cloud(ctx, s.user_dst ? s.user_dst : s.h_out.p, n, cloud_is_dense(s.compact, s.voxel, s.h_count), out);
+  if (out) fill_cloud(ctx, s.user_dst ? s.user_dst : s.h_out.p, n, cloud_is_dense(s.plan, s.h_count), out);
   return D2PC_OK;
 }
 
@@ -1027,7 +1071,7 @@ int d2pc_slot_timing(d2pc_ctx *ctx, int slot, d2pc_timing *out) {
   CU(ctx, cudaEventElapsedTime(&d2h, s.ev_kernel, s.ev_d2h));
   CU(ctx, cudaEventElapsedTime(&tot, s.ev_start, s.ev_d2h));
   out->h2d_us = h2d * 1e3f, out->kernels_us = ker * 1e3f, out->d2h_us = d2h * 1e3f, out->total_us = tot * 1e3f;
-  out->points = s.compact ? (s.n_points ? s.h_count[0] : 0) : s.n_points;
+  out->points = kept_points(s.plan, s.h_count);
   return D2PC_OK;
 }
 
@@ -1101,59 +1145,29 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
   const int esz = is_f32 ? 4 : 1;
   if (w == 0 || h == 0 || step < (size_t)w * esz || (n_frames > 1 && frame_stride < step * h))
     return D2PC_ERR_BAD_DIMS;
-  const uint64_t n = crop_points(w, h, ctx->cfg.border);
+  const CloudPlan p = plan_cloud(ctx, w, h);
+  const uint64_t n = p.n;
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // per-frame counts and PointCloud2.row_step are uint32
   if (reinterpret_cast<uintptr_t>(d_points) % 16 || points_stride % 16 || (n_frames > 1 && points_stride < n * 16))
     return D2PC_ERR_BAD_DIMS;
-  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx), ror = ror_on(ctx);
-  if (compact && !d_counts) return D2PC_ERR_INVALID_ARG;
+  if (p.counted && !d_counts) return D2PC_ERR_INVALID_ARG;
   if (n_frames == 0) return D2PC_OK;  // an empty batch: nothing to launch (and no size below may wrap)
   CU(ctx, cudaSetDevice(ctx->device));
-  int rc;
   // VOXEL and the radius outlier stage: the sort and scan index a batch with int, so a batch of more than
   // 2^31 - 1 (2^31 - 2) crop points runs in chunks; VOXEL's bounds pass puts the frame on gridDim.y, so a VOXEL
   // chunk also holds at most 65535 frames
-  const uint64_t max_points = ror ? kRorMaxPoints : 0x7fffffffull;
-  uint32_t chunk = (voxel || ror) ? (uint32_t)std::min<uint64_t>(n_frames, std::max<uint64_t>(1, max_points / std::max<uint64_t>(n, 1)))
-                                  : n_frames;
-  if (voxel) chunk = std::min<uint32_t>(chunk, 65535);
-  if (ror) {
-    const size_t need = ror_stage_bytes(chunk, (uint32_t)n);
-    if (need > ctx->d_ror.cap) {
-      CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-      if ((rc = grow_dev(ctx, ctx->d_ror, need))) return rc;
-    }
-  }
-  if (voxel) {
-    const size_t need = voxel_scratch_bytes(chunk, (uint32_t)n);
-    if (need > ctx->d_voxel.cap) {
-      CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-      if ((rc = grow_dev(ctx, ctx->d_voxel, need))) return rc;
-    }
-  } else if (finite_mode(ctx)) {
-    const size_t need = reproject_scratch_bytes(n_frames, w, h, ctx->cfg.border);
-    if (need > ctx->d_scratch.cap || reproject_table_bytes(w, h) > ctx->d_tables.cap) {
-      CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-      if ((rc = grow_dev(ctx, ctx->d_scratch, need, true)) ||
-          (rc = grow_dev(ctx, ctx->d_tables, reproject_table_bytes(w, h))))
-        return rc;
-    }
-  }
-  uint8_t *d_med = nullptr;
-  if (!is_f32 && ctx->cfg.median_ksize > 1) {
-    const size_t need = frame_stride * (n_frames - 1) + step * h;
-    if (need > ctx->d_med_batch.cap) {
-      CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-      if ((rc = grow_dev(ctx, ctx->d_med_batch, need))) return rc;
-    }
-    d_med = ctx->d_med_batch.p;
-  }
+  const uint32_t chunk = p.voxel || p.ror ? frames_per_chunk(n_frames, n, p.ror ? kRorMaxPoints : 0x7fffffffull,
+                                                             p.voxel ? 65535 : UINT32_MAX)
+                                          : n_frames;
+  FrameBatch in{static_cast<const uint8_t *>(d_in), is_f32, chunk, w, h, step, frame_stride};
+  int rc = grow_stages(ctx, ctx->batch, p, in, ctx->s_compute, true);
+  if (rc) return rc;
   for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
-    const uint32_t nf = std::min(chunk, n_frames - f0);
-    if ((rc = enqueue_kernels(ctx, static_cast<const uint8_t *>(d_in) + f0 * frame_stride, is_f32, nf, w, h, step,
-                              frame_stride, d_med, d_points + f0 * points_stride, points_stride,
-                              d_counts ? d_counts + f0 : nullptr, ctx->d_scratch.p, ctx->d_tables.p, ctx->d_ticket,
-                              ctx->s_compute, ctx->d_voxel.p, nullptr, ctx->d_ror.p)))
+    in.data = static_cast<const uint8_t *>(d_in) + f0 * frame_stride;
+    in.n_frames = std::min(chunk, n_frames - f0);
+    if ((rc = enqueue_kernels(ctx, p, in, ctx->batch,
+                              {d_points + f0 * points_stride, points_stride, d_counts ? d_counts + f0 : nullptr},
+                              nullptr, ctx->d_ticket, ctx->s_compute)))
       return rc;
   }
   return D2PC_OK;
@@ -1162,7 +1176,7 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
 int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
                                size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
                                uint32_t *d_out_counts) {
-  if (!ctx || !d_in || !d_out || !d_out_counts || !ror_on(ctx)) return D2PC_ERR_INVALID_ARG;
+  if (!ctx || !d_in || !d_out || !d_out_counts || !(ctx->ror.radius > 0.0)) return D2PC_ERR_INVALID_ARG;
   const uint64_t bytes = (uint64_t)n_max * 16;
   if (bytes > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // per-frame counts and PointCloud2.row_step are uint32
   if (reinterpret_cast<uintptr_t>(d_in) % 16 || reinterpret_cast<uintptr_t>(d_out) % 16 || in_stride % 16 ||
@@ -1175,18 +1189,18 @@ int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_fr
   const uint64_t out_end = out0 + (uint64_t)(n_frames - 1) * out_stride + bytes;
   if (bytes && in0 < out_end && out0 < in_end) return D2PC_ERR_INVALID_ARG;
   CU(ctx, cudaSetDevice(ctx->device));
-  const uint32_t chunk =
-      (uint32_t)std::min<uint64_t>(n_frames, std::max<uint64_t>(1, kRorMaxPoints / std::max<uint64_t>(n_max, 1)));
+  const uint32_t chunk = frames_per_chunk(n_frames, n_max, kRorMaxPoints, UINT32_MAX);
   const size_t need = ror_scratch_bytes(chunk, n_max);
-  if (need > ctx->d_ror.cap) {
+  if (need > ctx->batch.ror.cap) {
     CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-    const int rc = grow_dev(ctx, ctx->d_ror, need);
+    const int rc = grow_dev(ctx, ctx->batch.ror, need);
     if (rc) return rc;
   }
   for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
     const uint32_t nf = std::min(chunk, n_frames - f0);
     const int rc = enqueue_ror(ctx, nf, n_max, d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
-                               d_out + f0 * out_stride, out_stride, d_out_counts + f0, ctx->d_ror.p, ctx->s_compute);
+                               {d_out + f0 * out_stride, out_stride, d_out_counts + f0}, ctx->batch.ror.p,
+                               ctx->s_compute);
     if (rc) return rc;
   }
   return D2PC_OK;
@@ -1514,40 +1528,29 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
   Slot &s = ctx->slots[0];
   if ((rc = slot_wait_idle(ctx, s))) return rc;
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
-  const uint64_t n = crop_points(fw, fh, ctx->cfg.border);
-  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx), ror = ror_on(ctx);
-  if ((rc = grow_dev(ctx, s.d_med, (size_t)fw * fh)) || (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
+  const CloudPlan p = plan_cloud(ctx, fw, fh);
+  const uint64_t n = p.n;
+  if ((rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
   // a synchronous call: the callback kernel stores the CROP cloud straight into the pinned buffer (see submit_common)
-  uint8_t *d_direct = nullptr;
-  if (!compact && n && ctx->direct_out >= 0 && ctx->cfg.median_ksize > 1) {
-    void *dp = nullptr;
-    if (cudaHostGetDevicePointer(&dp, s.h_out.p, 0) == cudaSuccess && reinterpret_cast<uintptr_t>(dp) % 16 == 0)
-      d_direct = static_cast<uint8_t *>(dp);
-    else
-      cudaGetLastError();
-  }
+  uint8_t *const d_direct =
+      !p.counted && n && ctx->direct_out >= 0 && ctx->cfg.median_ksize > 1 ? direct_alias(s.h_out.p) : nullptr;
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
-  if (finite_mode(ctx) &&
-      ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, fw, fh, ctx->cfg.border), true)) ||
-       (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(fw, fh)))))
+  const FrameBatch fused{ctx->d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh};
+  if ((rc = grow_stages(ctx, s.stages, p, fused, ctx->s_compute, false)) ||
+      (rc = enqueue_kernels(ctx, p, fused, s.stages, {d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count},
+                            s.d_count + 2, s.d_count + 1, ctx->s_compute)))
     return rc;
-  if (voxel && (rc = grow_dev(ctx, s.d_voxel, voxel_scratch_bytes(1, (uint32_t)n)))) return rc;
-  if (ror && (rc = grow_dev(ctx, s.d_ror, ror_stage_bytes(1, (uint32_t)n)))) return rc;
-  rc = enqueue_kernels(ctx, ctx->d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh, s.d_med.p,
-                       d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count, s.d_scratch.p, s.d_tables.p,
-                       s.d_count + 1, ctx->s_compute, s.d_voxel.p, s.d_count + 2, s.d_ror.p);
-  if (rc) return rc;
-  uint64_t kept = n;
-  if (compact) {
-    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, voxel ? 12 : 4, cudaMemcpyDeviceToHost, ctx->s_compute));
+  if (p.counted) {
+    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, p.count_words * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+                            ctx->s_compute));
     CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-    kept = n ? s.h_count[0] : 0;
   }
+  const uint64_t kept = kept_points(p, s.h_count);
   if (kept && !d_direct)
     CU(ctx, cudaMemcpyAsync(s.h_out.p, s.d_out.p, kept * 16, cudaMemcpyDeviceToHost, ctx->s_compute));
   CU(ctx, cudaStreamSynchronize(ctx->s_compute));
   if (ctx->cfg.verbose) printf("Cloud size: %llu\n", (unsigned long long)kept);
-  fill_cloud(ctx, s.h_out.p, kept, cloud_is_dense(compact, voxel && !ror, s.h_count), out);
+  fill_cloud(ctx, s.h_out.p, kept, cloud_is_dense(p, s.h_count), out);
   return D2PC_OK;
 }
 
@@ -1570,26 +1573,19 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
   // (mono8 frames of any width: the fusion kernels read bytes, and a pitched 2-D copy is the slow way in)
   const size_t pitch = w, frame_bytes = (size_t)w * h, nn = (size_t)g.n * g.n;
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
-  const uint64_t n = crop_points(fw, fh, c.border);
-  const bool compact = counted_mode(ctx), voxel = voxel_mode(ctx), ror = ror_on(ctx);
+  const CloudPlan p = plan_cloud(ctx, fw, fh);
+  const uint64_t n = p.n;
   // the four input frames of a set live in one allocation, so that a contiguous pinned set is one DMA
   if ((rc = grow_dev(ctx, s.d_fuse_in[0], 4 * pitch * h))) return rc;
   uint8_t *const fin[4] = {s.d_fuse_in[0].p, s.d_fuse_in[0].p + pitch * h, s.d_fuse_in[0].p + 2 * pitch * h,
                            s.d_fuse_in[0].p + 3 * pitch * h};
   if ((rc = grow_dev(ctx, s.d_pre[0], nn)) || (rc = grow_dev(ctx, s.d_pre[1], nn)) ||
       (rc = grow_dev(ctx, s.d_container, (size_t)g.nc * g.nc)) || (rc = grow_dev(ctx, s.d_combined, nn)) ||
-      (rc = grow_dev(ctx, s.d_fused, (size_t)fw * fh)) || (rc = grow_dev(ctx, s.d_med, (size_t)fw * fh)) ||
-      (rc = grow_dev(ctx, s.d_out, n * 16 + 16)) || (rc = grow_pin(ctx, s.h_out, n * 16 + 16)))
+      (rc = grow_dev(ctx, s.d_fused, (size_t)fw * fh)) || (rc = grow_dev(ctx, s.d_out, n * 16 + 16)) ||
+      (rc = grow_pin(ctx, s.h_out, n * 16 + 16)))
     return rc;
-  if (finite_mode(ctx) &&
-      ((rc = grow_dev(ctx, s.d_scratch, reproject_scratch_bytes(1, fw, fh, c.border), true)) ||
-       (rc = grow_dev(ctx, s.d_tables, reproject_table_bytes(fw, fh)))))
-    return rc;
-  // (allocated without a clear: the voxel and radius outlier stages write every word of their scratch before
-  // reading it, so it does not matter that this slot's kernels run on s_kern rather than on the stream grow_dev
-  // clears on)
-  if (voxel && (rc = grow_dev(ctx, s.d_voxel, voxel_scratch_bytes(1, (uint32_t)n)))) return rc;
-  if (ror && (rc = grow_dev(ctx, s.d_ror, ror_stage_bytes(1, (uint32_t)n)))) return rc;
+  const FrameBatch fused{s.d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh};
+  if ((rc = grow_stages(ctx, s.stages, p, fused, s.s_kern, false))) return rc;
 
   NvtxRange nvtx_submit("d2pc submit fusion set");
   s.timed = ctx->timing && s.ev_start;
@@ -1630,23 +1626,12 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
   if ((rc = fuse_device_impl(ctx, fin[0], fin[1], sc1, sc2, w, h, pitch, s.d_fused.p, s.d_combined.p,
                              nullptr, preprocess_scores != 0, &s.d_container, sk)))
     return rc;
-  rc = enqueue_kernels(ctx, s.d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh, s.d_med.p, s.d_out.p, n * 16 + 16, s.d_count,
-                       s.d_scratch.p, s.d_tables.p, s.d_count + 1, sk, s.d_voxel.p, s.d_count + 2, s.d_ror.p);
-  if (rc) return rc;
+  if ((rc = enqueue_kernels(ctx, p, fused, s.stages, {s.d_out.p, n * 16 + 16, s.d_count}, s.d_count + 2,
+                            s.d_count + 1, sk)))
+    return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, sk));
-
-  // ---- D2H (stream 3)
-  CU(ctx, cudaStreamWaitEvent(ctx->s_d2h, s.ev_kernel, 0));
-  if (compact)
-    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, (voxel ? 3 : 1) * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->s_d2h));
-  else if (n) CU(ctx, cudaMemcpyAsync(s.h_out.p, s.d_out.p, n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
-  CU(ctx, cudaEventRecord(s.ev_d2h, ctx->s_d2h));
-  s.pending = true;
-  s.width = fw, s.height = fh;
-  s.n_points = n;
-  s.compact = compact;
-  s.voxel = voxel && !ror;
-  s.user_dst = nullptr, s.user_cap = 0, s.user_pinned = false, s.late_copy = false;
+  if ((rc = enqueue_readback(ctx, s, p, s.h_out.p))) return rc;
+  arm_slot(s, p, nullptr, 0, false, false);
   return D2PC_OK;
 }
 

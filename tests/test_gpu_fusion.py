@@ -115,10 +115,24 @@ def test_bad_geometry_is_an_error(ctx):
         ctx.set_tuning("offset_y", 15)
 
 
+def _expected_cloud(crop, mode):
+    """The cloud the filter mode publishes from the CROP cloud, and its is_dense."""
+    return (crop, 0) if mode == "crop" else (oracle.filter_finite(crop), 1)
+
+
+@pytest.fixture(params=["crop", "finite"])
+def mode(request, ctx):
+    import disparity_to_point_cloud_b200 as d2pc
+    ctx.set_filter_mode({"crop": d2pc.FILTER_CROP, "finite": d2pc.FILTER_CROP_FINITE}[request.param])
+    yield request.param
+    ctx.set_filter_mode(d2pc.FILTER_CROP)
+
+
 @pytest.mark.parametrize("direct", [0, -1])
-def test_config5_fuse_then_reproject(ctx, direct):
+def test_config5_fuse_then_reproject(ctx, mode, direct):
     """BASELINE config 5: four 1280x720 maps -> 665x665 fused -> DisparityCb -> 585x585 points (direct 0: the
-    callback kernel stores the cloud into the pinned buffer itself; -1: device buffer + D2H copy)."""
+    callback kernel stores the cloud into the pinned buffer itself; -1: device buffer + D2H copy), in CROP and
+    CROP_FINITE mode."""
     q = golden("q_golden.npz")["q"][0]
     d1, d2, s1, s2 = _four(720, 1280, 6)
     ctx.set_tuning("direct_out", direct)
@@ -126,10 +140,13 @@ def test_config5_fuse_then_reproject(ctx, direct):
         got = ctx.fuse_then_process(d1, d2, s1, s2)
     finally:
         ctx.set_tuning("direct_out", 0)
-    assert got.size == 342225 * 16
     fused, _ = oracle.fuse(d1, d2, s1, s2, -7, 15)
     assert fused.shape == (665, 665)
-    assert_same_bits(got, oracle.disparity_cb_mono8(fused, q), "config 5")
+    crop = oracle.disparity_cb_mono8(fused, q)
+    assert crop.size == 342225 * 16
+    want, dense = _expected_cloud(crop, mode)
+    assert_same_bits(got, want, f"config 5 {mode}")
+    assert ctx.last_cloud.is_dense == dense
 
 
 def _node_pass_oracle(d1, d2, s1, s2, q, preprocess):
@@ -146,9 +163,10 @@ def _node_pass_oracle(d1, d2, s1, s2, q, preprocess):
 
 @pytest.mark.parametrize("h,w", [(480, 752), (330, 430)])   # rows that are / are not 16-byte multiples
 @pytest.mark.parametrize("preprocess", [True, False])
-def test_fusion_pipeline_slots_and_stream(ctx, preprocess, h, w):
+def test_fusion_pipeline_slots_and_stream(ctx, mode, preprocess, h, w):
     """d2pc_submit_fusion / d2pc_process_fusion_stream: whole node passes (the four callbacks + DisparityCb on the
-    fused map) overlapped on the slot pipeline; clouds in order, bit-identical to the oracle's node."""
+    fused map) overlapped on the slot pipeline; clouds in order, bit-identical to the oracle's node, in CROP and
+    CROP_FINITE mode."""
     import disparity_to_point_cloud_b200 as d2pc
     q = golden("q_golden.npz")["q"][0]
     n_sets = 5
@@ -158,18 +176,23 @@ def test_fusion_pipeline_slots_and_stream(ctx, preprocess, h, w):
         pin.array[i, 0], pin.array[i, 1] = synth.s2_scene(h, w, 300 + i), synth.s2_scene(h, w, 400 + i)
         pin.array[i, 2] = rng.integers(0, 256, (h, w), dtype=np.uint8)
         pin.array[i, 3] = rng.integers(0, 256, (h, w), dtype=np.uint8)
-    want = [_node_pass_oracle(*pin.array[i], q, preprocess) for i in range(n_sets)]
-    clouds = ctx.process_fusion_stream(pin.array, preprocess_scores=preprocess, n_sets=2 * n_sets)
+    want = [_expected_cloud(_node_pass_oracle(*pin.array[i], q, preprocess), mode) for i in range(n_sets)]
+    dense = []
+    clouds = ctx.process_fusion_stream(pin.array, preprocess_scores=preprocess, n_sets=2 * n_sets,
+                                       sink=lambda i, c: dense.append(c.is_dense))
     assert len(clouds) == 2 * n_sets
     for i, c in enumerate(clouds):
-        assert_same_bits(c, want[i % n_sets], f"stream set {i}")
+        assert_same_bits(c, want[i % n_sets][0], f"stream set {i}")
+        assert dense[i] == want[i % n_sets][1], f"stream set {i}"
     # explicit slots, pageable frames, waited out of order
     a = [np.array(pin.array[0, k]) for k in range(4)]
     b = [np.array(pin.array[3, k]) for k in range(4)]
     ctx.submit_fusion(0, *a, preprocess_scores=preprocess)
     ctx.submit_fusion(1, *b, preprocess_scores=preprocess)
-    assert_same_bits(ctx.wait(1), want[3], "slot 1")
-    assert_same_bits(ctx.wait(0), want[0], "slot 0")
+    assert_same_bits(ctx.wait(1), want[3][0], "slot 1")
+    assert ctx.last_cloud.is_dense == want[3][1]
+    assert_same_bits(ctx.wait(0), want[0][0], "slot 0")
+    assert ctx.last_cloud.is_dense == want[0][1]
     pin.free()
 
 

@@ -223,7 +223,7 @@ def test_fusion_entries(env):
     with d2pc.Context(offset_x=-7, offset_y=15, n_slots=2) as ctx:
         crops_fused = [ctx.fuse_then_process(*sets[s]) for s in range(3)]
         crops_pipe = ctx.process_fusion_stream(sets)
-        for mode in ("crop", "voxel"):
+        for mode in ("crop", "finite", "voxel"):
             set_mode(d2pc, ctx, mode, (0.1, 0, ("z", 0.0, 10.0)))
             ctx.set_radius_outlier(0.15, 2)
             wf = [want(c, mode, 0.15, 2, (0.1, 0, ("z", 0.0, 10.0))) for c in crops_fused]
