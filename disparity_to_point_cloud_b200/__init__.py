@@ -74,6 +74,12 @@ class RadiusOutlier(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("radius", C.c_double), ("min_neighbors", C.c_uint32)]
 
 
+class CropBox(C.Structure):
+    """d2pc_crop_box: pcl::CropBox (setTransform) parameters of the stage in front of VOXEL and the outlier stage."""
+    _fields_ = [("struct_size", C.c_uint32), ("enabled", C.c_int32), ("min_pt", C.c_float * 3),
+                ("max_pt", C.c_float * 3), ("transform", C.c_float * 12)]
+
+
 class Timing(C.Structure):
     _fields_ = [("h2d_us", C.c_float), ("kernels_us", C.c_float), ("d2h_us", C.c_float), ("total_us", C.c_float),
                 ("points", C.c_uint64)]
@@ -109,6 +115,11 @@ SYMBOLS = [
     ("d2pc_get_radius_outlier", C.c_int, [_ctx, C.POINTER(RadiusOutlier)]),
     ("d2pc_radius_outlier_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
                                              C.c_void_p, C.c_size_t, C.c_void_p]),
+    ("d2pc_crop_box_default", None, [C.POINTER(CropBox)]),
+    ("d2pc_set_crop_box", C.c_int, [_ctx, C.POINTER(CropBox)]),
+    ("d2pc_get_crop_box", C.c_int, [_ctx, C.POINTER(CropBox)]),
+    ("d2pc_crop_box_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
+                                       C.c_void_p, C.c_size_t, C.c_void_p]),
     ("d2pc_process_mono8", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_process_f32", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_submit_mono8", C.c_int, [_ctx, C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
@@ -339,6 +350,34 @@ class Context:
         self._check(lib().d2pc_get_radius_outlier(self._h, C.byref(p)), "d2pc_get_radius_outlier")
         return p
 
+    def set_crop_box(self, min_pt, max_pt=None, transform=None):
+        """pcl::CropBox in front of VOXEL and the outlier stage: keep the points p with min_pt <= T p <= max_pt.
+        transform: None (the identity) or the camera -> box transform T as a 3x4 [R | t] or a 4x4 matrix whose last
+        row is (0, 0, 0, 1).  set_crop_box(None) turns the box off."""
+        b = CropBox()
+        lib().d2pc_crop_box_default(C.byref(b))
+        if min_pt is not None:
+            if max_pt is None:
+                raise ValueError("set_crop_box: max_pt is required with min_pt")
+            b.enabled = 1
+            b.min_pt[:] = [float(v) for v in np.asarray(min_pt, np.float32).reshape(3)]
+            b.max_pt[:] = [float(v) for v in np.asarray(max_pt, np.float32).reshape(3)]
+            if transform is not None:
+                t = np.asarray(transform, np.float32)
+                if t.shape == (4, 4):
+                    if not np.array_equal(t[3], np.float32([0, 0, 0, 1])):
+                        raise ValueError(f"set_crop_box: the last row of a 4x4 transform must be (0, 0, 0, 1), got {t[3]}")
+                    t = t[:3]
+                if t.shape != (3, 4):
+                    raise ValueError(f"set_crop_box: transform must be 3x4 or 4x4, got {t.shape}")
+                b.transform[:] = [float(v) for v in t.reshape(12)]
+        self._check(lib().d2pc_set_crop_box(self._h, C.byref(b)), "d2pc_set_crop_box")
+
+    def get_crop_box(self) -> CropBox:
+        b = CropBox()
+        self._check(lib().d2pc_get_crop_box(self._h, C.byref(b)), "d2pc_get_crop_box")
+        return b
+
     def set_arith_mode(self, m):
         self._check(lib().d2pc_set_arith_mode(self._h, m), "d2pc_set_arith_mode")
 
@@ -453,6 +492,10 @@ class Context:
         self._check(lib().d2pc_radius_outlier_device(self._h, d_in, n_frames, n_max, in_stride, d_in_counts or None,
                                                      d_out, out_stride, d_out_counts or None),
                     "d2pc_radius_outlier_device")
+
+    def crop_box_device(self, d_in, n_frames, n_max, in_stride, d_in_counts, d_out, out_stride, d_out_counts):
+        self._check(lib().d2pc_crop_box_device(self._h, d_in, n_frames, n_max, in_stride, d_in_counts or None,
+                                               d_out, out_stride, d_out_counts or None), "d2pc_crop_box_device")
 
     def median_u8_device(self, d_src, w, h, src_step, d_dst, dst_step, ksize):
         self._check(lib().d2pc_median_u8_device(self._h, d_src, w, h, src_step, d_dst, dst_step, ksize),

@@ -26,6 +26,7 @@
 #include <nvtx3/nvToolsExt.h>
 #include <sys/mman.h>
 
+#include "crop_box.h"
 #include "fusion.h"
 #include "median.h"
 #include "radius_outlier.h"
@@ -49,15 +50,17 @@ struct PinBuf {
   size_t cap = 0;
 };
 
-// What the filter mode and the radius outlier stage make of one frame geometry (plan_cloud), decided once per call.
+// What the filter mode, the crop box and the radius outlier stage make of one frame geometry (plan_cloud), decided
+// once per call.
 struct CloudPlan {
   uint64_t n = 0;           // crop points per frame
-  bool compact = false;     // the reproject kernels keep only finite points (CROP_FINITE)
-  bool voxel = false;       // the VOXEL stage runs on the CROP cloud
-  bool ror = false;         // the radius outlier stage runs on the mode's cloud
+  bool compact = false;     // the reproject kernels keep only finite points (CROP_FINITE without the box)
+  bool box = false;         // the crop box runs on the CROP cloud
+  bool voxel = false;       // the VOXEL stage runs on the CROP cloud, or on the box's cloud
+  bool ror = false;         // the radius outlier stage runs on the cloud of the steps before it
   bool counted = false;     // the cloud's size is known only on the device: the kept count decides the bytes
   uint32_t count_words = 1; // count words a slot reads back (Slot::d_count)
-  bool fallback_decides_dense = false;  // VOXEL without the outlier stage: the overflow fallback flag clears is_dense
+  bool fallback_decides_dense = false;  // VOXEL alone: the overflow fallback flag clears is_dense
 };
 
 // The device buffers between a batch's input frames and its cloud: one set per slot, one for the device batch.
@@ -65,7 +68,8 @@ struct StageBufs {
   DevBuf med;      // median-filtered frames
   DevBuf scratch;  // CROP_FINITE tile descriptors (epoch-tagged: zero when allocated, see next_epoch)
   DevBuf tables;   // CROP_FINITE tables
-  DevBuf voxel;    // VOXEL: the CROP clouds, then the stage's keys / indices / sort temp (voxel.h)
+  DevBuf box;      // crop box: the CROP clouds, the counts it hands to VOXEL, then the stage's scratch (crop_box.h)
+  DevBuf voxel;    // VOXEL: its input clouds, then the stage's keys / indices / sort temp (voxel.h)
   DevBuf ror;      // radius outlier stage: the mode's clouds and counts, then the stage's scratch (radius_outlier.h)
 };
 
@@ -110,6 +114,7 @@ struct d2pc_ctx {
   d2pc_voxel_grid voxel;  // D2PC_FILTER_VOXEL parameters (d2pc_set_voxel_grid)
   bool voxel_set = false;
   d2pc_radius_outlier ror;  // the radius outlier stage behind every mode (d2pc_set_radius_outlier; radius 0: off)
+  d2pc_crop_box box;        // the crop box in front of VOXEL and the outlier stage (d2pc_set_crop_box; enabled 0: off)
   // fusion buffers
   DevBuf d_fuse_in[4], d_container, d_combined, d_fused;
   PinBuf h_fused, h_combined;
@@ -253,7 +258,7 @@ void free_pin(PinBuf &b) {
   b = PinBuf{};
 }
 void free_stages(StageBufs &b) {
-  for (DevBuf *d : {&b.med, &b.scratch, &b.tables, &b.voxel, &b.ror}) free_dev(*d);
+  for (DevBuf *d : {&b.med, &b.scratch, &b.tables, &b.box, &b.voxel, &b.ror}) free_dev(*d);
 }
 
 uint64_t crop_points(uint32_t w, uint32_t h, int border) {
@@ -264,12 +269,15 @@ uint64_t crop_points(uint32_t w, uint32_t h, int border) {
 CloudPlan plan_cloud(const d2pc_ctx *ctx, uint32_t w, uint32_t h) {
   CloudPlan p;
   p.n = crop_points(w, h, ctx->cfg.border);
-  p.compact = ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE;
+  p.box = ctx->box.enabled != 0;
+  // the box drops non-finite points itself: CROP_FINITE + box runs the CROP kernels and lets the box compact once
+  p.compact = ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE && !p.box;
   p.voxel = ctx->cfg.filter_mode == D2PC_FILTER_VOXEL;
   p.ror = ctx->ror.radius > 0.0;
-  p.counted = p.compact || p.voxel || p.ror;
+  p.counted = p.compact || p.box || p.voxel || p.ror;
   p.count_words = p.voxel ? 3 : 1;  // the kept count [, the ticket, the VOXEL fallback flag]
-  p.fallback_decides_dense = p.voxel && !p.ror;  // the outlier stage's output is always dense
+  // the box's and the outlier stage's outputs are always dense, so is a VOXEL fallback that copies the box's cloud
+  p.fallback_decides_dense = p.voxel && !p.ror && !p.box;
   return p;
 }
 
@@ -391,6 +399,7 @@ int grow_stages(d2pc_ctx *ctx, StageBufs &b, const CloudPlan &p, const FrameBatc
       {b.med, median ? in.frame_stride * (in.n_frames - 1) + in.step * in.h : 0, false},
       {b.scratch, p.compact ? reproject_scratch_bytes(in.n_frames, in.w, in.h, ctx->cfg.border) : 0, true},
       {b.tables, p.compact ? reproject_table_bytes(in.w, in.h) : 0, false},
+      {b.box, p.box ? crop_box_stage_bytes(in.n_frames, n) : 0, false},
       {b.voxel, p.voxel ? voxel_scratch_bytes(in.n_frames, n) : 0, false},
       {b.ror, p.ror ? ror_stage_bytes(in.n_frames, n) : 0, false},
   };
@@ -411,13 +420,15 @@ uint32_t frames_per_chunk(uint32_t n_frames, uint64_t points_per_frame, uint64_t
   return (uint32_t)std::min<uint64_t>({n_frames, max_frames, by_points});
 }
 
-// The VOXEL stage of a batch whose CROP clouds are in the head of `voxel_scratch` (voxel.h), with the context's grid.
-int enqueue_voxel(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n, const CloudDst &dst, uint32_t *fallback,
-                  void *voxel_scratch, cudaStream_t stream) {
+// The VOXEL stage of a batch whose clouds are in the head of `voxel_scratch` (voxel.h; in_counts null: n points
+// each), with the context's grid.
+int enqueue_voxel(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n, const uint32_t *in_counts, const CloudDst &dst,
+                  uint32_t *fallback, void *voxel_scratch, cudaStream_t stream) {
   const d2pc_voxel_grid &g = ctx->voxel;
   VoxelLaunch V;
   V.n_frames = n_frames;
   V.n = n;
+  V.in_counts = in_counts;
   V.p.inv[0] = 1.0f / g.leaf_x, V.p.inv[1] = 1.0f / g.leaf_y, V.p.inv[2] = 1.0f / g.leaf_z;
   V.p.min_points = g.min_points_per_voxel;
   V.p.limit_field = g.limit_field;
@@ -451,6 +462,29 @@ int enqueue_ror(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n_max, const uint8_t 
   R.scratch = scratch;
   int nl = 0;
   CU(ctx, launch_radius_outlier(R, stream, &nl));
+  ctx->launches += nl;
+  return D2PC_OK;
+}
+
+// The crop box with the context's setting on n_frames clouds (frame f at in + f * in_stride, in_counts[f] points;
+// in_counts null: n_max each).  The launch takes the box by value, so a later d2pc_set_crop_box cannot reach it.
+int enqueue_box(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n_max, const uint8_t *in, size_t in_stride,
+                const uint32_t *in_counts, const CloudDst &dst, void *scratch, cudaStream_t stream) {
+  const d2pc_crop_box &box = ctx->box;
+  CropBoxLaunch B;
+  B.n_frames = n_frames;
+  B.n_max = n_max;
+  B.in = in;
+  B.in_stride = in_stride;
+  B.in_counts = in_counts;
+  for (int a = 0; a < 3; ++a) B.box.mn[a] = box.min_pt[a], B.box.mx[a] = box.max_pt[a];
+  for (int k = 0; k < 12; ++k) B.box.t[k] = box.transform[k];
+  B.out = dst.points;
+  B.out_stride = dst.stride;
+  B.counts = dst.counts;
+  B.scratch = scratch;
+  int nl = 0;
+  CU(ctx, launch_crop_box(B, stream, &nl));
   ctx->launches += nl;
   return D2PC_OK;
 }
@@ -530,22 +564,28 @@ int enqueue_reproject(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, S
   return D2PC_OK;
 }
 
-// Enqueue the plan's stages for one frame batch already on the device: [median] + reproject, then VOXEL, then the
-// radius outlier stage.  The last stage that runs writes `out`; each one before it writes its clouds dense into the
-// next stage's buffer.  fallback: VOXEL's per-frame overflow fallback flags (may be null).
+// Enqueue the plan's stages for one frame batch already on the device: [median] + reproject, then the crop box, then
+// VOXEL, then the radius outlier stage.  The last stage that runs writes `out`; each one before it writes its clouds
+// dense into the head of the next stage's buffer.  fallback: VOXEL's per-frame overflow fallback flags (may be null).
 int enqueue_kernels(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, StageBufs &b, const CloudDst &out,
                     uint32_t *fallback, uint32_t *ticket, cudaStream_t stream) {
   const uint32_t n = (uint32_t)p.n;
   const size_t dense = (size_t)n * 16;
   const RorStage rs = p.ror ? ror_stage(b.ror.p, in.n_frames, n) : RorStage{};
+  const CropBoxStage bs = p.box ? crop_box_stage(b.box.p, in.n_frames, n) : CropBoxStage{};
+  uint8_t *const voxel_in = p.voxel ? reinterpret_cast<uint8_t *>(voxel_crop(b.voxel.p)) : nullptr;
   const CloudDst voxel_dst = p.ror ? CloudDst{rs.clouds, dense, rs.counts} : out;
-  const CloudDst crop_dst =
-      p.voxel ? CloudDst{reinterpret_cast<uint8_t *>(voxel_crop(b.voxel.p)), dense, nullptr} : voxel_dst;
+  const CloudDst box_dst = p.voxel ? CloudDst{voxel_in, dense, bs.counts} : voxel_dst;
+  const CloudDst crop_dst = p.box ? CloudDst{bs.clouds, dense, nullptr} : p.voxel ? CloudDst{voxel_in, dense, nullptr}
+                                                                                   : voxel_dst;
   int rc = enqueue_reproject(ctx, p, in, b, crop_dst, ticket, stream);
-  if (!rc && p.voxel) rc = enqueue_voxel(ctx, in.n_frames, n, voxel_dst, fallback, b.voxel.p, stream);
-  // a CROP cloud has all n points; the other modes' counts are on the device
+  // a CROP cloud has all n points; every later cloud's count is on the device
+  if (!rc && p.box)
+    rc = enqueue_box(ctx, in.n_frames, n, bs.clouds, dense, nullptr, box_dst, bs.scratch, stream);
+  if (!rc && p.voxel)
+    rc = enqueue_voxel(ctx, in.n_frames, n, p.box ? bs.counts : nullptr, voxel_dst, fallback, b.voxel.p, stream);
   if (!rc && p.ror)
-    rc = enqueue_ror(ctx, in.n_frames, n, rs.clouds, dense, p.compact || p.voxel ? rs.counts : nullptr, out,
+    rc = enqueue_ror(ctx, in.n_frames, n, rs.clouds, dense, p.compact || p.box || p.voxel ? rs.counts : nullptr, out,
                      rs.scratch, stream);
   return rc;
 }
@@ -816,6 +856,7 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
   make_qparams(ctx->q, &ctx->Q);
   d2pc_voxel_grid_default(&ctx->voxel);
   d2pc_radius_outlier_default(&ctx->ror);
+  d2pc_crop_box_default(&ctx->box);
 
   if (const char *v = getenv("D2PC_ROWS_PER_UNIT")) ctx->rows_per_unit = atoi(v);
   if (const char *v = getenv("D2PC_CTAS_PER_SM")) ctx->ctas_per_sm = atoi(v);
@@ -925,6 +966,26 @@ int d2pc_set_radius_outlier(d2pc_ctx *ctx, const d2pc_radius_outlier *p) {
 int d2pc_get_radius_outlier(const d2pc_ctx *ctx, d2pc_radius_outlier *p) {
   if (!ctx || !p) return D2PC_ERR_INVALID_ARG;
   *p = ctx->ror;
+  return D2PC_OK;
+}
+void d2pc_crop_box_default(d2pc_crop_box *b) {
+  if (!b) return;
+  memset(b, 0, sizeof(*b));
+  b->struct_size = sizeof(*b);
+  for (int a = 0; a < 3; ++a) b->min_pt[a] = -1.0f, b->max_pt[a] = 1.0f, b->transform[5 * a] = 1.0f;
+}
+int d2pc_set_crop_box(d2pc_ctx *ctx, const d2pc_crop_box *b) {
+  if (!ctx || !b || b->struct_size != sizeof(*b)) return D2PC_ERR_INVALID_ARG;
+  for (int a = 0; a < 3; ++a)  // NaN fails; +-inf bounds make a half-open box
+    if (!(b->min_pt[a] <= b->max_pt[a])) return D2PC_ERR_INVALID_ARG;
+  for (float t : b->transform)
+    if (!std::isfinite(t)) return D2PC_ERR_INVALID_ARG;
+  ctx->box = *b;
+  return D2PC_OK;
+}
+int d2pc_get_crop_box(const d2pc_ctx *ctx, d2pc_crop_box *b) {
+  if (!ctx || !b) return D2PC_ERR_INVALID_ARG;
+  *b = ctx->box;
   return D2PC_OK;
 }
 int d2pc_set_arith_mode(d2pc_ctx *ctx, int m) {
@@ -1153,12 +1214,14 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
   if (p.counted && !d_counts) return D2PC_ERR_INVALID_ARG;
   if (n_frames == 0) return D2PC_OK;  // an empty batch: nothing to launch (and no size below may wrap)
   CU(ctx, cudaSetDevice(ctx->device));
-  // VOXEL and the radius outlier stage: the sort and scan index a batch with int, so a batch of more than
-  // 2^31 - 1 (2^31 - 2) crop points runs in chunks; VOXEL's bounds pass puts the frame on gridDim.y, so a VOXEL
-  // chunk also holds at most 65535 frames
-  const uint32_t chunk = p.voxel || p.ror ? frames_per_chunk(n_frames, n, p.ror ? kRorMaxPoints : 0x7fffffffull,
-                                                             p.voxel ? 65535 : UINT32_MAX)
-                                          : n_frames;
+  // the crop box, VOXEL and the radius outlier stage: the sort and scan index a batch with int, so a batch of more
+  // than 2^31 - 1 (2^31 - 2 with the box or the outlier stage) crop points runs in chunks; VOXEL's bounds pass puts
+  // the frame on gridDim.y, so a VOXEL chunk also holds at most 65535 frames
+  const uint32_t chunk =
+      p.box || p.voxel || p.ror
+          ? frames_per_chunk(n_frames, n, p.box ? kCropBoxMaxPoints : p.ror ? kRorMaxPoints : 0x7fffffffull,
+                             p.voxel ? 65535 : UINT32_MAX)
+          : n_frames;
   FrameBatch in{static_cast<const uint8_t *>(d_in), is_f32, chunk, w, h, step, frame_stride};
   int rc = grow_stages(ctx, ctx->batch, p, in, ctx->s_compute, true);
   if (rc) return rc;
@@ -1173,10 +1236,10 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
   return D2PC_OK;
 }
 
-int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
-                               size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
-                               uint32_t *d_out_counts) {
-  if (!ctx || !d_in || !d_out || !d_out_counts || !(ctx->ror.radius > 0.0)) return D2PC_ERR_INVALID_ARG;
+// The argument rules of the stages that run alone on clouds already on the device (d2pc_radius_outlier_device,
+// d2pc_crop_box_device).
+static int check_cloud_batch(const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
+                             const uint8_t *d_out, size_t out_stride) {
   const uint64_t bytes = (uint64_t)n_max * 16;
   if (bytes > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // per-frame counts and PointCloud2.row_step are uint32
   if (reinterpret_cast<uintptr_t>(d_in) % 16 || reinterpret_cast<uintptr_t>(d_out) % 16 || in_stride % 16 ||
@@ -1188,6 +1251,15 @@ int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_fr
   const uint64_t in_end = in0 + (uint64_t)(n_frames - 1) * in_stride + bytes;
   const uint64_t out_end = out0 + (uint64_t)(n_frames - 1) * out_stride + bytes;
   if (bytes && in0 < out_end && out0 < in_end) return D2PC_ERR_INVALID_ARG;
+  return D2PC_OK;
+}
+
+int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
+                               size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
+                               uint32_t *d_out_counts) {
+  if (!ctx || !d_in || !d_out || !d_out_counts || !(ctx->ror.radius > 0.0)) return D2PC_ERR_INVALID_ARG;
+  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_out, out_stride);
+  if (rc0 || n_frames == 0) return rc0;
   CU(ctx, cudaSetDevice(ctx->device));
   const uint32_t chunk = frames_per_chunk(n_frames, n_max, kRorMaxPoints, UINT32_MAX);
   const size_t need = ror_scratch_bytes(chunk, n_max);
@@ -1200,6 +1272,29 @@ int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_fr
     const uint32_t nf = std::min(chunk, n_frames - f0);
     const int rc = enqueue_ror(ctx, nf, n_max, d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
                                {d_out + f0 * out_stride, out_stride, d_out_counts + f0}, ctx->batch.ror.p,
+                               ctx->s_compute);
+    if (rc) return rc;
+  }
+  return D2PC_OK;
+}
+
+int d2pc_crop_box_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
+                         const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride, uint32_t *d_out_counts) {
+  if (!ctx || !d_in || !d_out || !d_out_counts || !ctx->box.enabled) return D2PC_ERR_INVALID_ARG;
+  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_out, out_stride);
+  if (rc0 || n_frames == 0) return rc0;
+  CU(ctx, cudaSetDevice(ctx->device));
+  const uint32_t chunk = frames_per_chunk(n_frames, n_max, kCropBoxMaxPoints, UINT32_MAX);
+  const size_t need = crop_box_scratch_bytes(chunk, n_max);
+  if (need > ctx->batch.box.cap) {
+    CU(ctx, cudaStreamSynchronize(ctx->s_compute));
+    const int rc = grow_dev(ctx, ctx->batch.box, need);
+    if (rc) return rc;
+  }
+  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
+    const uint32_t nf = std::min(chunk, n_frames - f0);
+    const int rc = enqueue_box(ctx, nf, n_max, d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
+                               {d_out + f0 * out_stride, out_stride, d_out_counts + f0}, ctx->batch.box.p,
                                ctx->s_compute);
     if (rc) return rc;
   }

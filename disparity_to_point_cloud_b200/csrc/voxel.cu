@@ -3,6 +3,8 @@
 // the recipe this file implements; every step there maps onto one stage here:
 //
 //   1. bounds    voxel_bounds_kernel   per-block min / max of the included points of a frame -> partials
+//                                      (positions at or past the frame's input count are excluded like non-finite
+//                                      points; no input counts: n each)
 //                voxel_finish_kernel   one block per frame: partials -> descriptor (min_b, mul, fallback flag)
 //   2. keys      voxel_keys_kernel     (frame << 31 | idx, point index); excluded points sort past every voxel
 //   3. sort      cub::DeviceRadixSort::SortPairs on the key bits in use (stable)
@@ -47,6 +49,13 @@ __device__ __forceinline__ bool included(const float4 &q, const VoxelParams &p) 
   return true;
 }
 
+// the frame's input count (at most n; no counts: n)
+__device__ __forceinline__ uint32_t frame_count(const uint32_t *counts, uint32_t f, uint32_t n) {
+  if (!counts) return n;
+  const uint32_t c = counts[f];
+  return c < n ? c : n;
+}
+
 __device__ __forceinline__ float warp_min(float v) {
   for (int o = 16; o; o >>= 1) v = fminf(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
@@ -72,10 +81,12 @@ __device__ __forceinline__ void block_minmax(float (&v)[6]) {
 
 // grid (blocks_per_frame, n_frames)
 __global__ void __launch_bounds__(kThreads) voxel_bounds_kernel(const float4 *__restrict__ crop, uint32_t n,
+                                                                const uint32_t *__restrict__ in_counts,
                                                                 const VoxelParams p, Partial *__restrict__ partials) {
   const float4 *pts = crop + (size_t)blockIdx.y * n;
+  const uint32_t m = frame_count(in_counts, blockIdx.y, n);
   float v[6] = {FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX};
-  for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < n; i += gridDim.x * kThreads) {
+  for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < m; i += gridDim.x * kThreads) {
     const float4 q = __ldg(pts + i);
     if (!included(q, p)) continue;
     v[0] = fminf(v[0], q.x), v[1] = fminf(v[1], q.y), v[2] = fminf(v[2], q.z);
@@ -127,6 +138,7 @@ __global__ void __launch_bounds__(kThreads) voxel_finish_kernel(const Partial *_
 
 template <typename KeyT>
 __global__ void __launch_bounds__(kThreads) voxel_keys_kernel(const float4 *__restrict__ crop, uint32_t n,
+                                                              const uint32_t *__restrict__ in_counts,
                                                               uint32_t total, const VoxelParams p,
                                                               const Desc *__restrict__ desc, KeyT *__restrict__ keys,
                                                               uint32_t *__restrict__ vals) {
@@ -134,8 +146,8 @@ __global__ void __launch_bounds__(kThreads) voxel_keys_kernel(const float4 *__re
   if (j >= total) return;
   const uint32_t f = j / n, i = j - f * n;
   const Desc d = desc[f];
-  const float4 q = __ldg(crop + j);
   uint32_t idx = kSentinel;
+  const float4 q = i < frame_count(in_counts, f, n) ? __ldg(crop + j) : make_float4(NAN, NAN, NAN, 0.f);
   if (!d.fallback && included(q, p)) {
     const float c[3] = {q.x, q.y, q.z};
     int64_t ijk[3];
@@ -169,6 +181,7 @@ struct HeadFlag {
 
 template <typename KeyT>
 __global__ void __launch_bounds__(kThreads) voxel_centroid_kernel(const float4 *__restrict__ crop, uint32_t n,
+                                                                  const uint32_t *__restrict__ in_counts,
                                                                   uint32_t total, const Desc *__restrict__ desc,
                                                                   const HeadFlag<KeyT> head,
                                                                   const uint32_t *__restrict__ vals,
@@ -181,9 +194,10 @@ __global__ void __launch_bounds__(kThreads) voxel_centroid_kernel(const float4 *
   const uint32_t f = j / n, i = j - f * n, first = f * n;
   float4 *dst = reinterpret_cast<float4 *>(out + (size_t)f * out_stride);
   if (desc[f].fallback) {
-    dst[i] = __ldg(crop + j);
+    const uint32_t m = frame_count(in_counts, f, n);
+    if (i < m) dst[i] = __ldg(crop + j);
     if (i == 0) {
-      counts[f] = n;
+      counts[f] = m;
       if (fallback) fallback[f] = 1;
     }
     return;
@@ -285,10 +299,10 @@ cudaError_t run(const VoxelLaunch &V, cudaStream_t stream, int *launches) {
   void *temp = base + L.temp;
 
   const uint32_t nb = bounds_blocks(V.n_frames, V.n);
-  voxel_bounds_kernel<<<dim3(nb, V.n_frames), kThreads, 0, stream>>>(crop, V.n, V.p, partials);
+  voxel_bounds_kernel<<<dim3(nb, V.n_frames), kThreads, 0, stream>>>(crop, V.n, V.in_counts, V.p, partials);
   voxel_finish_kernel<<<V.n_frames, kThreads, 0, stream>>>(partials, nb, V.p, desc);
   const uint32_t grid = (total + kThreads - 1) / kThreads;
-  voxel_keys_kernel<KeyT><<<grid, kThreads, 0, stream>>>(crop, V.n, total, V.p, desc, keys_in, vals_in);
+  voxel_keys_kernel<KeyT><<<grid, kThreads, 0, stream>>>(crop, V.n, V.in_counts, total, V.p, desc, keys_in, vals_in);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
   size_t tb = L.temp_bytes;
@@ -300,8 +314,8 @@ cudaError_t run(const VoxelLaunch &V, cudaStream_t stream, int *launches) {
   e = cub::DeviceScan::ExclusiveSum(temp, tb, thrust::make_transform_iterator(thrust::counting_iterator<uint32_t>(0), head),
                                     slot, (int)(total + 1), stream);
   if (e != cudaSuccess) return e;
-  voxel_centroid_kernel<KeyT><<<grid, kThreads, 0, stream>>>(crop, V.n, total, desc, head, vals_out, slot, V.out,
-                                                             V.out_stride, V.counts, V.fallback);
+  voxel_centroid_kernel<KeyT><<<grid, kThreads, 0, stream>>>(crop, V.n, V.in_counts, total, desc, head, vals_out, slot,
+                                                             V.out, V.out_stride, V.counts, V.fallback);
   if (launches) *launches = 6;  // four kernels of this file, the sort and the scan (each CUB call counted once)
   return cudaGetLastError();
 }

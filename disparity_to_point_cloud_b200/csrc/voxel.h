@@ -15,9 +15,12 @@ struct VoxelParams {
 };
 
 struct VoxelLaunch {
-  // n_frames CROP clouds of n points each, frame f at voxel_crop(scratch) + f * n (dense, written by the CROP kernels)
+  // n_frames clouds of at most n points each, frame f at voxel_crop(scratch) + f * n (dense, written by the CROP
+  // kernels or the crop box)
   uint32_t n_frames = 0;
   uint32_t n = 0;
+  // per frame (may be null: n each): the points of the frame's cloud; positions at or past it are excluded
+  const uint32_t *in_counts = nullptr;
   VoxelParams p;
   uint8_t *out = nullptr;  // voxel clouds, frame f at out + f * out_stride bytes
   size_t out_stride = 0;

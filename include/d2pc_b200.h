@@ -124,7 +124,7 @@ typedef struct d2pc_cloud {
   uint32_t row_step;   /* 16 * width */
   uint8_t is_bigendian; /* 0 */
   uint8_t is_dense;     /* 0 in CROP mode (cpp:81); 1 in CROP_FINITE; VOXEL: 1, 0 for the overflow fallback;
-                           1 behind the radius outlier stage */
+                           1 behind the crop box or the radius outlier stage */
   uint32_t n_fields;    /* 3 */
   d2pc_point_field fields[3];
 } d2pc_cloud;
@@ -243,6 +243,54 @@ int d2pc_set_radius_outlier(d2pc_ctx *ctx, const d2pc_radius_outlier *p);
 /* The setting last made (d2pc_radius_outlier_default's until then). */
 int d2pc_get_radius_outlier(const d2pc_ctx *ctx, d2pc_radius_outlier *p);
 
+/* ---- crop box (a stage in front of VOXEL and the radius outlier stage) -----------
+ *
+ * Off by default (enabled 0).  With a box enabled, the published cloud is pcl::CropBox<pcl::PointXYZ> with
+ * setTransform only (no setRotation / setTranslation), setNegative(false) and keep_organized false, applied on the
+ * device to the CROP cloud of that frame; VOXEL and the radius outlier stage then run on the box's cloud.  The
+ * recipe, float32 throughout, no FMA contraction:
+ *   1. A point takes part only when x, y and z are all finite (the CROP cloud is not dense, and PCL then skips such
+ *      points).
+ *   2. l = T * p with T = transform (row-major 3x4 [R | t], camera frame -> box frame), each operation rounded:
+ *      lx = ((t00*x + t01*y) + t02*z) + t03, likewise ly (row 1) and lz (row 2).
+ *   3. The point is kept when min_pt[a] <= l[a] <= max_pt[a] on all three axes: the faces are inside the box.
+ *   4. Kept points are copied unchanged -- the original camera-frame coordinates, all 16 bytes -- in input order;
+ *      height 1, width = kept, is_dense 1, row_step = 16 * width.
+ * Composition with the filter mode:
+ *   - CROP + box and CROP_FINITE + box publish the same bytes: the box drops non-finite points anyway, so both run
+ *     the CROP kernels and the box does the one compaction.
+ *   - VOXEL + box is VoxelGrid(CropBox(CROP cloud)): the grid's bounds come from the box's points.  A frame that
+ *     takes VOXEL's overflow fallback publishes the box's cloud with is_dense 1 (all of its points are finite;
+ *     whether PCL's copy in that fallback would set is_dense is not verified here).
+ *   - The radius outlier stage runs on whatever the steps before it produced.
+ * Relation to PCL (CropBox::applyFilter and pcl::transformPoint, PCL 1.8 - 1.12; restated from memory, PCL's source
+ * was not at hand when this was written -- the same footing as DESIGN.md section 0.1 for the OpenCV dispatch):
+ *   - transformPoint computes each row as ((m(i,0)*x + m(i,1)*y) + m(i,2)*z) + m(i,3) in float, which is rule 2.
+ *   - PCL skips the transform when transform_.matrix().isIdentity(), Eigen's fuzzy test (every entry within 1e-5 of
+ *     the identity's for float).  For the exact identity this changes no decision (1*x + 0*y + 0*z + 0 is x up to
+ *     the sign of a zero).  A transform that is within that tolerance but not exactly the identity is applied here,
+ *     and skipped by PCL: the two can then differ for points within about 1e-5 * |p| of a face.
+ *   - PCL rejects a point when l[a] < min_pt[a] or l[a] > max_pt[a], so it would keep a point whose l is NaN.  Such
+ *     an l needs T * p to overflow float (|p| and |T| near 1e38); this library drops that point (rule 3).
+ * With a box enabled every mode is a counted mode, as CROP_FINITE is: BUFFER_TOO_SMALL is reported by d2pc_wait,
+ * the kernel never stores into host memory ("direct_out" does not apply), d2pc_slot_timing's d2h_us covers the
+ * count, and the device batch entries need d_counts.  With enabled 0 nothing of this applies. */
+typedef struct d2pc_crop_box {
+  uint32_t struct_size; /* sizeof(d2pc_crop_box) */
+  int32_t enabled;      /* 0: off (the default) */
+  float min_pt[3];      /* PCL setMin (x, y, z); default -1 */
+  float max_pt[3];      /* PCL setMax; default 1 */
+  float transform[12];  /* row-major 3x4 [R | t], PCL setTransform (camera frame -> box frame); default identity */
+} d2pc_crop_box;
+
+/* enabled 0, min_pt (-1, -1, -1), max_pt (1, 1, 1), the identity transform. */
+void d2pc_crop_box_default(d2pc_crop_box *b);
+/* D2PC_ERR_INVALID_ARG for a NaN bound, min_pt > max_pt on an axis, a non-finite transform entry or a wrong
+ * struct_size; the previous setting is kept then.  +-inf bounds are allowed (a half-open box). */
+int d2pc_set_crop_box(d2pc_ctx *ctx, const d2pc_crop_box *b);
+/* The setting last made (d2pc_crop_box_default's until then). */
+int d2pc_get_crop_box(const d2pc_ctx *ctx, d2pc_crop_box *b);
+
 /* ---- the disparity callback, host buffers (the reference-facing calls) ------ */
 
 /* Whole DisparityCb (src/disparity_to_point_cloud.cpp:46-92) on one mono8
@@ -349,6 +397,14 @@ int d2pc_reproject_mono8_device(d2pc_ctx *ctx, const uint8_t *d_img, uint32_t n_
 int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
                                size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
                                uint32_t *d_out_counts);
+
+/* The crop box alone (the context's d2pc_crop_box, which must be enabled), on clouds already on the device, with the
+ * argument rules of d2pc_radius_outlier_device: frame f's input is d_in + f*in_stride bytes, d_in_counts[f] points
+ * (NULL: n_max each; a count above n_max counts as n_max), its kept points go to d_out + f*out_stride and their
+ * number to d_out_counts[f]; pointers and strides 16-byte aligned, strides >= 16*n_max when n_frames > 1,
+ * n_max*16 < 2^32, no overlap of input and output; batches of more than 2^31 - 2 points run in chunks of frames. */
+int d2pc_crop_box_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
+                         const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride, uint32_t *d_out_counts);
 
 /* cv::medianBlur on CV_8UC1, replicate border (cpp:55-57 with ksize 11,
  * depth_map_fusion.cpp:124 with ksize 3).  ksize odd, 3..15. */

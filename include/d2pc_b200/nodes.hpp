@@ -18,6 +18,7 @@
 //     publisher without subscribers does not serialise either).
 #pragma once
 #include <algorithm>
+#include <cmath>
 #include <cstdio>
 #include <fstream>
 #include <functional>
@@ -140,6 +141,20 @@ inline void check(int status, const char *what, const d2pc_ctx *ctx = nullptr) {
 }
 
 // cv_bridge::toCvCopy(*msg, "mono8") for the encodings this library accepts.
+// [R | t] of the crop box params, row-major 3x4 in float: R = Rz(yaw) Ry(pitch) Rx(roll) evaluated in double,
+// pose = {tx, ty, tz, roll, pitch, yaw}.
+inline void crop_box_transform(const double pose[6], float out[12]) {
+  const double cr = std::cos(pose[3]), sr = std::sin(pose[3]), cp = std::cos(pose[4]), sp = std::sin(pose[4]);
+  const double cy = std::cos(pose[5]), sy = std::sin(pose[5]);
+  const double R[3][3] = {{cy * cp, cy * sp * sr - sy * cr, cy * sp * cr + sy * sr},
+                          {sy * cp, sy * sp * sr + cy * cr, sy * sp * cr - cy * sr},
+                          {-sp, cp * sr, cp * cr}};
+  for (int i = 0; i < 3; ++i) {
+    for (int j = 0; j < 3; ++j) out[4 * i + j] = static_cast<float>(R[i][j]);
+    out[4 * i + 3] = static_cast<float>(pose[i]);
+  }
+}
+
 inline void require_mono8(const sensor_msgs::Image &msg) {
   if (msg.encoding != "mono8" && msg.encoding != "8UC1")
     throw std::invalid_argument("unsupported image encoding '" + msg.encoding + "' (mono8 / 8UC1 only)");
@@ -234,6 +249,31 @@ class Disparity2PCloud {
       r.radius = ror_radius;
       r.min_neighbors = static_cast<uint32_t>(ror_min);
       d2pc_b200::check(d2pc_set_radius_outlier(ctx_, &r), "d2pc_set_radius_outlier", ctx_);
+    }
+    // optional, not in the reference: pcl::CropBox on the device in front of VOXEL and the outlier stage, on when
+    // crop_box_enable != 0.  The box is crop_box_{min,max}_{x,y,z} in a frame given by a translation and
+    // roll / pitch / yaw (crop_box_{tx,ty,tz,roll,pitch,yaw}, radians): this node builds R = Rz(yaw) Ry(pitch) Rx(roll)
+    // in double and rounds [R | t] to the library's float matrix.  That conversion is the node's own; the points are
+    // not moved, so the cloud keeps its frame_id.
+    int box_on = 0;
+    nh_.param<int>("crop_box_enable", box_on, 0);
+    if (box_on) {
+      d2pc_crop_box b;
+      d2pc_crop_box_default(&b);
+      b.enabled = 1;
+      const char *axes[3] = {"x", "y", "z"};
+      for (int a = 0; a < 3; ++a) {
+        double lo = -1.0, hi = 1.0;
+        nh_.param<double>(std::string("crop_box_min_") + axes[a], lo, -1.0);
+        nh_.param<double>(std::string("crop_box_max_") + axes[a], hi, 1.0);
+        b.min_pt[a] = static_cast<float>(lo), b.max_pt[a] = static_cast<float>(hi);
+      }
+      double pose[6];  // tx, ty, tz, roll, pitch, yaw
+      const char *names[6] = {"crop_box_tx", "crop_box_ty", "crop_box_tz", "crop_box_roll", "crop_box_pitch",
+                              "crop_box_yaw"};
+      for (int k = 0; k < 6; ++k) nh_.param<double>(names[k], pose[k], 0.0);
+      d2pc_b200::crop_box_transform(pose, b.transform);
+      d2pc_b200::check(d2pc_set_crop_box(ctx_, &b), "d2pc_set_crop_box", ctx_);
     }
   }
   ~Disparity2PCloud() {

@@ -9,7 +9,9 @@
 #include <sensor_msgs/PointCloud2.h>
 #include <sensor_msgs/image_encodings.h>
 
+#include <cmath>
 #include <cstring>
+#include <string>
 
 #include "d2pc_b200.h"
 
@@ -66,6 +68,43 @@ class Disparity2PCloudGpu {
       if (ror_min < 0 || d2pc_set_radius_outlier(ctx_, &r) != D2PC_OK) {
         ROS_FATAL("radius_outlier_radius %g / radius_outlier_min_neighbors %d: not a valid setting", ror_radius,
                   ror_min);
+        ros::shutdown();
+      }
+    }
+    // optional, not in the reference: pcl::CropBox on the device in front of VOXEL and the outlier stage, on when
+    // crop_box_enable != 0; R = Rz(yaw) Ry(pitch) Rx(roll) in double, rounded with t to the library's float [R | t]
+    // (the node mirror's conversion, include/d2pc_b200/nodes.hpp).  The points are not moved: frame_id stays.
+    int box_on = 0;
+    nh_.param<int>("crop_box_enable", box_on, 0);
+    if (box_on) {
+      d2pc_crop_box b;
+      d2pc_crop_box_default(&b);
+      b.enabled = 1;
+      const char *axes[3] = {"x", "y", "z"};
+      for (int a = 0; a < 3; ++a) {
+        double lo = -1.0, hi = 1.0;
+        nh_.param<double>(std::string("crop_box_min_") + axes[a], lo, -1.0);
+        nh_.param<double>(std::string("crop_box_max_") + axes[a], hi, 1.0);
+        b.min_pt[a] = static_cast<float>(lo), b.max_pt[a] = static_cast<float>(hi);
+      }
+      double t[3], rpy[3];
+      nh_.param<double>("crop_box_tx", t[0], 0.0);
+      nh_.param<double>("crop_box_ty", t[1], 0.0);
+      nh_.param<double>("crop_box_tz", t[2], 0.0);
+      nh_.param<double>("crop_box_roll", rpy[0], 0.0);
+      nh_.param<double>("crop_box_pitch", rpy[1], 0.0);
+      nh_.param<double>("crop_box_yaw", rpy[2], 0.0);
+      const double cr = std::cos(rpy[0]), sr = std::sin(rpy[0]), cp = std::cos(rpy[1]), sp = std::sin(rpy[1]);
+      const double cy = std::cos(rpy[2]), sy = std::sin(rpy[2]);
+      const double R[3][3] = {{cy * cp, cy * sp * sr - sy * cr, cy * sp * cr + sy * sr},
+                              {sy * cp, sy * sp * sr + cy * cr, sy * sp * cr - cy * sr},
+                              {-sp, cp * sr, cp * cr}};
+      for (int i = 0; i < 3; ++i) {
+        for (int j = 0; j < 3; ++j) b.transform[4 * i + j] = static_cast<float>(R[i][j]);
+        b.transform[4 * i + 3] = static_cast<float>(t[i]);
+      }
+      if (d2pc_set_crop_box(ctx_, &b) != D2PC_OK) {
+        ROS_FATAL("crop_box_*: not a valid crop box (min above max, or a non-finite bound or pose)");
         ros::shutdown();
       }
     }
