@@ -39,7 +39,7 @@ using namespace d2pc;
 namespace {
 
 constexpr size_t kAlign = 256;
-inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
+inline size_t round_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 struct DevBuf {
   uint8_t *p = nullptr;
@@ -50,14 +50,17 @@ struct PinBuf {
   size_t cap = 0;
 };
 
+// The filter stages that run on clouds already on the device (cloud_stage.cuh), in the order a plan runs them.
+enum class CloudStage { box, voxel, ror };
+
 // What the filter mode, the crop box and the radius outlier stage make of one frame geometry (plan_cloud), decided
 // once per call.
 struct CloudPlan {
   uint64_t n = 0;           // crop points per frame
   bool compact = false;     // the reproject kernels keep only finite points (CROP_FINITE without the box)
-  bool box = false;         // the crop box runs on the CROP cloud
-  bool voxel = false;       // the VOXEL stage runs on the CROP cloud, or on the box's cloud
-  bool ror = false;         // the radius outlier stage runs on the cloud of the steps before it
+  // the cloud stages that run, in order: the crop box on the CROP cloud, VOXEL, the radius outlier stage
+  CloudStage stages[3];
+  int n_stages = 0;
   bool counted = false;     // the cloud's size is known only on the device: the kept count decides the bytes
   uint32_t count_words = 1; // count words a slot reads back (Slot::d_count)
   bool fallback_decides_dense = false;  // VOXEL alone: the overflow fallback flag clears is_dense
@@ -65,12 +68,11 @@ struct CloudPlan {
 
 // The device buffers between a batch's input frames and its cloud: one set per slot, one for the device batch.
 struct StageBufs {
-  DevBuf med;      // median-filtered frames
-  DevBuf scratch;  // CROP_FINITE tile descriptors (epoch-tagged: zero when allocated, see next_epoch)
-  DevBuf tables;   // CROP_FINITE tables
-  DevBuf box;      // crop box: the CROP clouds, the counts it hands to VOXEL, then the stage's scratch (crop_box.h)
-  DevBuf voxel;    // VOXEL: its input clouds, then the stage's keys / indices / sort temp (voxel.h)
-  DevBuf ror;      // radius outlier stage: the mode's clouds and counts, then the stage's scratch (radius_outlier.h)
+  DevBuf med;       // median-filtered frames
+  DevBuf scratch;   // CROP_FINITE tile descriptors (epoch-tagged: zero when allocated, see next_epoch)
+  DevBuf tables;    // CROP_FINITE tables
+  DevBuf cloud[2];  // the clouds between the steps (dense, frame f at f * n * 16 bytes), then their per-frame counts
+  DevBuf stage;     // the scratch of the cloud stages: they run one after another on one stream, so they share it
 };
 
 struct Slot {
@@ -178,7 +180,7 @@ int grow_dev(d2pc_ctx *ctx, DevBuf &b, size_t bytes, cudaStream_t clear_on = nul
   if (b.p) CU(ctx, cudaFree(b.p));
   b.p = nullptr;
   b.cap = 0;
-  const size_t cap = align_up(bytes, 1 << 16);
+  const size_t cap = round_up(bytes, 1 << 16);
   CU(ctx, cudaMalloc(&b.p, cap));
   if (clear_on) CU(ctx, cudaMemsetAsync(b.p, 0, cap, clear_on));
   b.cap = cap;
@@ -200,10 +202,10 @@ cudaError_t pinned_alloc(void **out, size_t bytes) {
     return v && atoi(v) != 0;
   }();
   if (!thp) return cudaHostAlloc(out, bytes, cudaHostAllocDefault);
-  const size_t huge = (size_t)2 << 20, len = align_up(bytes, huge);
+  const size_t huge = (size_t)2 << 20, len = round_up(bytes, huge);
   void *p = mmap(nullptr, len + huge, PROT_READ | PROT_WRITE, MAP_PRIVATE | MAP_ANONYMOUS, -1, 0);
   if (p == MAP_FAILED) return cudaErrorMemoryAllocation;
-  uint8_t *a = reinterpret_cast<uint8_t *>(align_up(reinterpret_cast<uintptr_t>(p), huge));
+  uint8_t *a = reinterpret_cast<uint8_t *>(round_up(reinterpret_cast<uintptr_t>(p), huge));
   // give back the unaligned head and tail so that munmap(a, len) releases everything
   if (a != p) munmap(p, (size_t)(a - static_cast<uint8_t *>(p)));
   const size_t tail = (static_cast<uint8_t *>(p) + len + huge) - (a + len);
@@ -242,7 +244,7 @@ int grow_pin(d2pc_ctx *ctx, PinBuf &b, size_t bytes) {
   if (b.p) CU(ctx, pinned_free(b.p));
   b.p = nullptr;
   b.cap = 0;
-  const size_t cap = align_up(bytes, 1 << 16);
+  const size_t cap = round_up(bytes, 1 << 16);
   void *p = nullptr;
   CU(ctx, pinned_alloc(&p, cap));
   b.p = static_cast<uint8_t *>(p);
@@ -258,7 +260,7 @@ void free_pin(PinBuf &b) {
   b = PinBuf{};
 }
 void free_stages(StageBufs &b) {
-  for (DevBuf *d : {&b.med, &b.scratch, &b.tables, &b.box, &b.voxel, &b.ror}) free_dev(*d);
+  for (DevBuf *d : {&b.med, &b.scratch, &b.tables, &b.cloud[0], &b.cloud[1], &b.stage}) free_dev(*d);
 }
 
 uint64_t crop_points(uint32_t w, uint32_t h, int border) {
@@ -269,15 +271,17 @@ uint64_t crop_points(uint32_t w, uint32_t h, int border) {
 CloudPlan plan_cloud(const d2pc_ctx *ctx, uint32_t w, uint32_t h) {
   CloudPlan p;
   p.n = crop_points(w, h, ctx->cfg.border);
-  p.box = ctx->box.enabled != 0;
+  const bool box = ctx->box.enabled != 0, voxel = ctx->cfg.filter_mode == D2PC_FILTER_VOXEL,
+             ror = ctx->ror.radius > 0.0;
   // the box drops non-finite points itself: CROP_FINITE + box runs the CROP kernels and lets the box compact once
-  p.compact = ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE && !p.box;
-  p.voxel = ctx->cfg.filter_mode == D2PC_FILTER_VOXEL;
-  p.ror = ctx->ror.radius > 0.0;
-  p.counted = p.compact || p.box || p.voxel || p.ror;
-  p.count_words = p.voxel ? 3 : 1;  // the kept count [, the ticket, the VOXEL fallback flag]
+  p.compact = ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE && !box;
+  if (box) p.stages[p.n_stages++] = CloudStage::box;
+  if (voxel) p.stages[p.n_stages++] = CloudStage::voxel;
+  if (ror) p.stages[p.n_stages++] = CloudStage::ror;
+  p.counted = p.compact || p.n_stages > 0;
+  p.count_words = voxel ? 3 : 1;  // the kept count [, the ticket, the VOXEL fallback flag]
   // the box's and the outlier stage's outputs are always dense, so is a VOXEL fallback that copies the box's cloud
-  p.fallback_decides_dense = p.voxel && !p.ror && !p.box;
+  p.fallback_decides_dense = voxel && !ror && !box;
   return p;
 }
 
@@ -377,12 +381,20 @@ struct FrameBatch {
   size_t step, frame_stride;
 };
 
-// Where a stage writes a batch's clouds: frame f at points + f * stride, its point count at counts[f].
-struct CloudDst {
-  uint8_t *points;
-  size_t stride;
-  uint32_t *counts;
-};
+size_t stage_scratch_bytes(CloudStage st, uint32_t n_frames, uint32_t n) {
+  return st == CloudStage::box     ? crop_box_scratch_bytes(n_frames, n)
+         : st == CloudStage::voxel ? voxel_scratch_bytes(n_frames, n)
+                                   : ror_scratch_bytes(n_frames, n);
+}
+
+// A cloud buffer of StageBufs: n_frames dense clouds of n points, then their per-frame counts.
+size_t cloud_buf_bytes(uint32_t n_frames, uint32_t n) {
+  return align_up((size_t)n_frames * n * 16) + (size_t)n_frames * 4;
+}
+CloudDst cloud_buf(const DevBuf &b, uint32_t n_frames, uint32_t n) {
+  const size_t clouds = align_up((size_t)n_frames * n * 16);
+  return {b.p, (size_t)n * 16, b.p ? reinterpret_cast<uint32_t *>(b.p + clouds) : nullptr};
+}
 
 // Grows a stage-buffer set for batch `in` under plan p.  `stream` is where the set's kernels run; a new CROP_FINITE
 // descriptor buffer is cleared there.  in_use: work queued on `stream` may still use the set, so the stream is
@@ -391,6 +403,9 @@ int grow_stages(d2pc_ctx *ctx, StageBufs &b, const CloudPlan &p, const FrameBatc
                 bool in_use) {
   const uint32_t n = (uint32_t)p.n;
   const bool median = !in.is_f32 && ctx->cfg.median_ksize > 1;
+  const int stages = p.n_stages;
+  size_t scratch = 0;
+  for (int i = 0; i < stages; ++i) scratch = std::max(scratch, stage_scratch_bytes(p.stages[i], in.n_frames, n));
   const struct {
     DevBuf &buf;
     size_t bytes;
@@ -399,9 +414,9 @@ int grow_stages(d2pc_ctx *ctx, StageBufs &b, const CloudPlan &p, const FrameBatc
       {b.med, median ? in.frame_stride * (in.n_frames - 1) + in.step * in.h : 0, false},
       {b.scratch, p.compact ? reproject_scratch_bytes(in.n_frames, in.w, in.h, ctx->cfg.border) : 0, true},
       {b.tables, p.compact ? reproject_table_bytes(in.w, in.h) : 0, false},
-      {b.box, p.box ? crop_box_stage_bytes(in.n_frames, n) : 0, false},
-      {b.voxel, p.voxel ? voxel_scratch_bytes(in.n_frames, n) : 0, false},
-      {b.ror, p.ror ? ror_stage_bytes(in.n_frames, n) : 0, false},
+      {b.cloud[0], stages > 0 ? cloud_buf_bytes(in.n_frames, n) : 0, false},
+      {b.cloud[1], stages > 1 ? cloud_buf_bytes(in.n_frames, n) : 0, false},
+      {b.stage, scratch, false},
   };
   for (const auto &x : need) {
     if (x.bytes <= x.buf.cap) continue;
@@ -413,78 +428,36 @@ int grow_stages(d2pc_ctx *ctx, StageBufs &b, const CloudPlan &p, const FrameBatc
   return D2PC_OK;
 }
 
-// Frames per launch for a stage whose sort and scan index a launch's points with int: at most max_points points (but
-// at least one frame) and max_frames frames.
-uint32_t frames_per_chunk(uint32_t n_frames, uint64_t points_per_frame, uint64_t max_points, uint32_t max_frames) {
-  const uint64_t by_points = std::max<uint64_t>(1, max_points / std::max<uint64_t>(points_per_frame, 1));
-  return (uint32_t)std::min<uint64_t>({n_frames, max_frames, by_points});
+// Frames per launch of the cloud stages: at most kCloudMaxPoints points (but at least one frame).
+uint32_t frames_per_chunk(uint32_t n_frames, uint64_t points_per_frame) {
+  const uint64_t by_points = std::max<uint64_t>(1, kCloudMaxPoints / std::max<uint64_t>(points_per_frame, 1));
+  return (uint32_t)std::min<uint64_t>(n_frames, by_points);
 }
 
-// The VOXEL stage of a batch whose clouds are in the head of `voxel_scratch` (voxel.h; in_counts null: n points
-// each), with the context's grid.
-int enqueue_voxel(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n, const uint32_t *in_counts, const CloudDst &dst,
-                  uint32_t *fallback, void *voxel_scratch, cudaStream_t stream) {
-  const d2pc_voxel_grid &g = ctx->voxel;
-  VoxelLaunch V;
-  V.n_frames = n_frames;
-  V.n = n;
-  V.in_counts = in_counts;
-  V.p.inv[0] = 1.0f / g.leaf_x, V.p.inv[1] = 1.0f / g.leaf_y, V.p.inv[2] = 1.0f / g.leaf_z;
-  V.p.min_points = g.min_points_per_voxel;
-  V.p.limit_field = g.limit_field;
-  V.p.limit_min = g.limit_min, V.p.limit_max = g.limit_max;
-  V.out = dst.points;
-  V.out_stride = dst.stride;
-  V.counts = dst.counts;
-  V.fallback = fallback;
-  V.scratch = voxel_scratch;
+// One cloud stage with the context's setting on a batch of clouds, on `stream`.  The setting travels by value, so a
+// later d2pc_set_* cannot reach a queued launch.  fallback: VOXEL's per-frame overflow fallback flags (may be null).
+int enqueue_stage(d2pc_ctx *ctx, CloudStage st, const CloudSrc &in, const CloudDst &out, uint32_t *fallback,
+                  void *scratch, cudaStream_t stream) {
   int nl = 0;
-  CU(ctx, launch_voxel(V, stream, &nl));
-  ctx->launches += nl;
-  return D2PC_OK;
-}
-
-// The radius outlier stage with the context's setting on n_frames clouds (frame f at in + f * in_stride, in_counts[f]
-// points; in_counts null: n_max each).
-int enqueue_ror(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n_max, const uint8_t *in, size_t in_stride,
-                const uint32_t *in_counts, const CloudDst &dst, void *scratch, cudaStream_t stream) {
-  RorLaunch R;
-  R.n_frames = n_frames;
-  R.n_max = n_max;
-  R.in = in;
-  R.in_stride = in_stride;
-  R.in_counts = in_counts;
-  R.radius = ctx->ror.radius;
-  R.min_neighbors = ctx->ror.min_neighbors;
-  R.out = dst.points;
-  R.out_stride = dst.stride;
-  R.counts = dst.counts;
-  R.scratch = scratch;
-  int nl = 0;
-  CU(ctx, launch_radius_outlier(R, stream, &nl));
-  ctx->launches += nl;
-  return D2PC_OK;
-}
-
-// The crop box with the context's setting on n_frames clouds (frame f at in + f * in_stride, in_counts[f] points;
-// in_counts null: n_max each).  The launch takes the box by value, so a later d2pc_set_crop_box cannot reach it.
-int enqueue_box(d2pc_ctx *ctx, uint32_t n_frames, uint32_t n_max, const uint8_t *in, size_t in_stride,
-                const uint32_t *in_counts, const CloudDst &dst, void *scratch, cudaStream_t stream) {
-  const d2pc_crop_box &box = ctx->box;
-  CropBoxLaunch B;
-  B.n_frames = n_frames;
-  B.n_max = n_max;
-  B.in = in;
-  B.in_stride = in_stride;
-  B.in_counts = in_counts;
-  for (int a = 0; a < 3; ++a) B.box.mn[a] = box.min_pt[a], B.box.mx[a] = box.max_pt[a];
-  for (int k = 0; k < 12; ++k) B.box.t[k] = box.transform[k];
-  B.out = dst.points;
-  B.out_stride = dst.stride;
-  B.counts = dst.counts;
-  B.scratch = scratch;
-  int nl = 0;
-  CU(ctx, launch_crop_box(B, stream, &nl));
+  cudaError_t e;
+  if (st == CloudStage::box) {
+    const d2pc_crop_box &box = ctx->box;
+    CropBoxParams b;
+    for (int a = 0; a < 3; ++a) b.mn[a] = box.min_pt[a], b.mx[a] = box.max_pt[a];
+    for (int k = 0; k < 12; ++k) b.t[k] = box.transform[k];
+    e = launch_crop_box(in, out, b, scratch, stream, &nl);
+  } else if (st == CloudStage::voxel) {
+    const d2pc_voxel_grid &g = ctx->voxel;
+    VoxelParams v;
+    v.inv[0] = 1.0f / g.leaf_x, v.inv[1] = 1.0f / g.leaf_y, v.inv[2] = 1.0f / g.leaf_z;
+    v.min_points = g.min_points_per_voxel;
+    v.limit_field = g.limit_field;
+    v.limit_min = g.limit_min, v.limit_max = g.limit_max;
+    e = launch_voxel(in, out, v, fallback, scratch, stream, &nl);
+  } else {
+    e = launch_radius_outlier(in, out, ctx->ror.radius, ctx->ror.min_neighbors, scratch, stream, &nl);
+  }
+  CU(ctx, e);
   ctx->launches += nl;
   return D2PC_OK;
 }
@@ -564,29 +537,22 @@ int enqueue_reproject(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, S
   return D2PC_OK;
 }
 
-// Enqueue the plan's stages for one frame batch already on the device: [median] + reproject, then the crop box, then
-// VOXEL, then the radius outlier stage.  The last stage that runs writes `out`; each one before it writes its clouds
-// dense into the head of the next stage's buffer.  fallback: VOXEL's per-frame overflow fallback flags (may be null).
+// Enqueue the plan's steps for one frame batch already on the device: [median] + reproject, then each cloud stage
+// in plan order.  The reproject kernels write cloud buffer 0; each stage reads one buffer and writes the other, so
+// its input and output never overlap; the last step writes `out`.  fallback: VOXEL's per-frame overflow fallback
+// flags (may be null).
 int enqueue_kernels(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, StageBufs &b, const CloudDst &out,
                     uint32_t *fallback, uint32_t *ticket, cudaStream_t stream) {
   const uint32_t n = (uint32_t)p.n;
-  const size_t dense = (size_t)n * 16;
-  const RorStage rs = p.ror ? ror_stage(b.ror.p, in.n_frames, n) : RorStage{};
-  const CropBoxStage bs = p.box ? crop_box_stage(b.box.p, in.n_frames, n) : CropBoxStage{};
-  uint8_t *const voxel_in = p.voxel ? reinterpret_cast<uint8_t *>(voxel_crop(b.voxel.p)) : nullptr;
-  const CloudDst voxel_dst = p.ror ? CloudDst{rs.clouds, dense, rs.counts} : out;
-  const CloudDst box_dst = p.voxel ? CloudDst{voxel_in, dense, bs.counts} : voxel_dst;
-  const CloudDst crop_dst = p.box ? CloudDst{bs.clouds, dense, nullptr} : p.voxel ? CloudDst{voxel_in, dense, nullptr}
-                                                                                   : voxel_dst;
-  int rc = enqueue_reproject(ctx, p, in, b, crop_dst, ticket, stream);
-  // a CROP cloud has all n points; every later cloud's count is on the device
-  if (!rc && p.box)
-    rc = enqueue_box(ctx, in.n_frames, n, bs.clouds, dense, nullptr, box_dst, bs.scratch, stream);
-  if (!rc && p.voxel)
-    rc = enqueue_voxel(ctx, in.n_frames, n, p.box ? bs.counts : nullptr, voxel_dst, fallback, b.voxel.p, stream);
-  if (!rc && p.ror)
-    rc = enqueue_ror(ctx, in.n_frames, n, rs.clouds, dense, p.compact || p.box || p.voxel ? rs.counts : nullptr, out,
-                     rs.scratch, stream);
+  const int stages = p.n_stages;
+  const CloudDst buf[2] = {cloud_buf(b.cloud[0], in.n_frames, n), cloud_buf(b.cloud[1], in.n_frames, n)};
+  int rc = enqueue_reproject(ctx, p, in, b, stages ? buf[0] : out, ticket, stream);
+  for (int i = 0; i < stages && !rc; ++i) {
+    const CloudDst &src = buf[i & 1];
+    // a CROP cloud straight from the reproject kernels has all n points; every other cloud's count is on the device
+    const CloudSrc cloud{src.points, src.stride, i > 0 || p.compact ? src.counts : nullptr, in.n_frames, n};
+    rc = enqueue_stage(ctx, p.stages[i], cloud, i + 1 < stages ? buf[(i + 1) & 1] : out, fallback, b.stage.p, stream);
+  }
   return rc;
 }
 
@@ -652,7 +618,7 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   // rows that are already 16-byte multiples stay dense on the device: the H2D copy is then one contiguous DMA.  So do
   // mono8 rows of any width (the callback kernel reads bytes; a 665-wide fused map is then one DMA instead of a
   // pitched 2-D copy); float rows that are not 16-byte multiples keep a 256-byte pitch for the vector loads.
-  const size_t d_pitch = (row_bytes % 16 == 0 || !is_f32) ? row_bytes : align_up(row_bytes, kAlign);
+  const size_t d_pitch = (row_bytes % 16 == 0 || !is_f32) ? row_bytes : round_up(row_bytes, kAlign);
   const CloudPlan p = plan_cloud(ctx, w, h);
   const uint64_t n = p.n;
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // PointCloud2.row_step / width are uint32
@@ -866,7 +832,7 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
   // pre-size the slots when the caller told us the largest frame
   if (c.max_width > 0 && c.max_height > 0) {
     for (auto &s : ctx->slots) {
-      const size_t pitch = align_up((size_t)c.max_width * 4, kAlign);
+      const size_t pitch = round_up((size_t)c.max_width * 4, kAlign);
       const uint64_t np = crop_points(c.max_width, c.max_height, c.border);
       if ((rc = grow_dev(ctx, s.d_in, pitch * c.max_height)) ||
           (rc = grow_dev(ctx, s.stages.med, pitch * c.max_height)) ||
@@ -1214,14 +1180,8 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
   if (p.counted && !d_counts) return D2PC_ERR_INVALID_ARG;
   if (n_frames == 0) return D2PC_OK;  // an empty batch: nothing to launch (and no size below may wrap)
   CU(ctx, cudaSetDevice(ctx->device));
-  // the crop box, VOXEL and the radius outlier stage: the sort and scan index a batch with int, so a batch of more
-  // than 2^31 - 1 (2^31 - 2 with the box or the outlier stage) crop points runs in chunks; VOXEL's bounds pass puts
-  // the frame on gridDim.y, so a VOXEL chunk also holds at most 65535 frames
-  const uint32_t chunk =
-      p.box || p.voxel || p.ror
-          ? frames_per_chunk(n_frames, n, p.box ? kCropBoxMaxPoints : p.ror ? kRorMaxPoints : 0x7fffffffull,
-                             p.voxel ? 65535 : UINT32_MAX)
-          : n_frames;
+  // a batch of more than kCloudMaxPoints crop points runs the cloud stages in chunks
+  const uint32_t chunk = p.n_stages ? frames_per_chunk(n_frames, n) : n_frames;
   FrameBatch in{static_cast<const uint8_t *>(d_in), is_f32, chunk, w, h, step, frame_stride};
   int rc = grow_stages(ctx, ctx->batch, p, in, ctx->s_compute, true);
   if (rc) return rc;
@@ -1254,51 +1214,42 @@ static int check_cloud_batch(const uint8_t *d_in, uint32_t n_frames, uint32_t n_
   return D2PC_OK;
 }
 
-int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
-                               size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
-                               uint32_t *d_out_counts) {
-  if (!ctx || !d_in || !d_out || !d_out_counts || !(ctx->ror.radius > 0.0)) return D2PC_ERR_INVALID_ARG;
+// One cloud stage alone on clouds already on the device (d2pc_radius_outlier_device, d2pc_crop_box_device).
+static int cloud_stage_device(d2pc_ctx *ctx, CloudStage st, bool on, const uint8_t *d_in, uint32_t n_frames,
+                              uint32_t n_max, size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out,
+                              size_t out_stride, uint32_t *d_out_counts) {
+  if (!ctx || !d_in || !d_out || !d_out_counts || !on) return D2PC_ERR_INVALID_ARG;
   const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_out, out_stride);
   if (rc0 || n_frames == 0) return rc0;
   CU(ctx, cudaSetDevice(ctx->device));
-  const uint32_t chunk = frames_per_chunk(n_frames, n_max, kRorMaxPoints, UINT32_MAX);
-  const size_t need = ror_scratch_bytes(chunk, n_max);
-  if (need > ctx->batch.ror.cap) {
+  const uint32_t chunk = frames_per_chunk(n_frames, n_max);
+  const size_t need = stage_scratch_bytes(st, chunk, n_max);
+  if (need > ctx->batch.stage.cap) {
     CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-    const int rc = grow_dev(ctx, ctx->batch.ror, need);
+    const int rc = grow_dev(ctx, ctx->batch.stage, need);
     if (rc) return rc;
   }
   for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
-    const uint32_t nf = std::min(chunk, n_frames - f0);
-    const int rc = enqueue_ror(ctx, nf, n_max, d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
-                               {d_out + f0 * out_stride, out_stride, d_out_counts + f0}, ctx->batch.ror.p,
-                               ctx->s_compute);
+    const CloudSrc in{d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
+                      std::min(chunk, n_frames - f0), n_max};
+    const int rc = enqueue_stage(ctx, st, in, {d_out + f0 * out_stride, out_stride, d_out_counts + f0}, nullptr,
+                                 ctx->batch.stage.p, ctx->s_compute);
     if (rc) return rc;
   }
   return D2PC_OK;
 }
 
+int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
+                               size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
+                               uint32_t *d_out_counts) {
+  return cloud_stage_device(ctx, CloudStage::ror, ctx && ctx->ror.radius > 0.0, d_in, n_frames, n_max, in_stride,
+                            d_in_counts, d_out, out_stride, d_out_counts);
+}
+
 int d2pc_crop_box_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
                          const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride, uint32_t *d_out_counts) {
-  if (!ctx || !d_in || !d_out || !d_out_counts || !ctx->box.enabled) return D2PC_ERR_INVALID_ARG;
-  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_out, out_stride);
-  if (rc0 || n_frames == 0) return rc0;
-  CU(ctx, cudaSetDevice(ctx->device));
-  const uint32_t chunk = frames_per_chunk(n_frames, n_max, kCropBoxMaxPoints, UINT32_MAX);
-  const size_t need = crop_box_scratch_bytes(chunk, n_max);
-  if (need > ctx->batch.box.cap) {
-    CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-    const int rc = grow_dev(ctx, ctx->batch.box, need);
-    if (rc) return rc;
-  }
-  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
-    const uint32_t nf = std::min(chunk, n_frames - f0);
-    const int rc = enqueue_box(ctx, nf, n_max, d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
-                               {d_out + f0 * out_stride, out_stride, d_out_counts + f0}, ctx->batch.box.p,
-                               ctx->s_compute);
-    if (rc) return rc;
-  }
-  return D2PC_OK;
+  return cloud_stage_device(ctx, CloudStage::box, ctx && ctx->box.enabled, d_in, n_frames, n_max, in_stride,
+                            d_in_counts, d_out, out_stride, d_out_counts);
 }
 
 int d2pc_reproject_f32_device(d2pc_ctx *ctx, const float *d_disp, uint32_t n_frames, uint32_t w, uint32_t h,

@@ -3,7 +3,7 @@
 // radius is set, and d2pc_radius_outlier_device.  include/d2pc_b200.h states the recipe; this file finds, for every
 // finite point, whether at least min_neighbors + 1 finite points (itself included) lie within the radius:
 //
-//   1. bounds  ror_bounds_kernel    per-block min / max of the finite points below count[f] -> partials
+//   1. bounds  cloud_bounds_kernel  per-block min / max of the finite points below count[f] -> partials
 //              ror_finish_kernel    one block per frame: partials -> grid (origin, cell size, cells per axis)
 //   2. keys    ror_keys_kernel      (frame, linear cell index) -> point index; non-finite points and positions past
 //                                   the count get the frame's sentinel cell, which sorts after every real cell
@@ -13,8 +13,8 @@
 //                                   the cells x-1..x+1 are one contiguous key range, found by binary search; rule
 //                                   3-4 of the recipe on each point of it, stopping at min_neighbors + 1 -> a flag at
 //                                   the point's input position
-//   6. output  cub::DeviceScan::ExclusiveSum over the flags -> output slots;
-//              ror_scatter_kernel   kept points copied unchanged in input order, and the per-frame counts
+//   6. output  cloud_stage.cuh's compaction over the flags: kept points copied unchanged in input order, and the
+//              per-frame counts
 //
 // Why the 27 cells around a point hold every neighbour (the margin).  Let r' = max(radius, 2^-64) and let the
 // cell size c start at r' * (1 + 2^-10); it only grows.  Take a pair that passes rule 4 with a finite r2 (s <= r2).
@@ -37,16 +37,11 @@
 // requires.  No buffer is read before a kernel of the same launch has written it, so the scratch needs no clearing.
 #include "radius_outlier.h"
 
-#include <cfloat>
 #include <cub/device/device_radix_sort.cuh>
-#include <cub/device/device_scan.cuh>
-#include <thrust/iterator/counting_iterator.h>
-#include <thrust/iterator/transform_iterator.h>
 
 namespace d2pc {
 namespace {
 
-constexpr int kThreads = 256;
 constexpr double kMinCell = 0x1p-64;        // r' = max(radius, kMinCell): see the margin argument above
 constexpr double kMargin = 1.0 + 0x1p-10;   // c >= r' * kMargin
 constexpr double kMaxAxisCells = 0x1p32;    // per-axis cells, padding included
@@ -58,77 +53,20 @@ struct Desc {
   uint64_t dx, dxy;   // cells along x, cells per z layer (padding included)
 };
 
-struct Partial {
-  float mn[3], mx[3], pad[2];
-};
-
 __device__ __forceinline__ bool finite3(const float4 &q) { return isfinite(q.x) && isfinite(q.y) && isfinite(q.z); }
 
-__device__ __forceinline__ uint32_t frame_count(const uint32_t *counts, uint32_t f, uint32_t n_max) {
-  if (!counts) return n_max;
-  const uint32_t c = counts[f];
-  return c < n_max ? c : n_max;
-}
+// the bounds pass's predicate: only finite points span the grid
+struct Finite {
+  __device__ bool operator()(const float4 &q) const { return finite3(q); }
+};
 
-__device__ __forceinline__ const float4 *frame_points(const uint8_t *in, size_t stride, uint32_t f) {
-  return reinterpret_cast<const float4 *>(in + (size_t)f * stride);
-}
-
-// bits of the frame number in a key, and the key of frame f's sentinel cell (all cell bits set)
-__host__ __device__ __forceinline__ int frame_bits(uint32_t n_frames) {
-  int b = 0;
-  while ((1ull << b) < n_frames) ++b;
-  return b;
-}
+// the cell bits of a key with fb frame bits (all set: the frame's sentinel cell), and frame f's bits
 __device__ __forceinline__ uint64_t cell_mask(int fb) { return fb ? (1ull << (64 - fb)) - 1 : ~0ull; }
 __device__ __forceinline__ uint64_t frame_part(uint32_t f, int fb) { return fb ? (uint64_t)f << (64 - fb) : 0ull; }
 
 // the cell coordinate of a finite coordinate (floor(t) + 1 of the margin argument)
 __device__ __forceinline__ uint64_t cell_of(float x, float mn, double ic) {
   return (uint64_t)floor(__dmul_rn(__dsub_rn((double)x, (double)mn), ic)) + 1;
-}
-
-__device__ __forceinline__ float warp_min(float v) {
-  for (int o = 16; o; o >>= 1) v = fminf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
-__device__ __forceinline__ float warp_max(float v) {
-  for (int o = 16; o; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
-  return v;
-}
-
-// min / max of 6 values across the block; the result is valid in thread 0
-__device__ __forceinline__ void block_minmax(float (&v)[6]) {
-  __shared__ float red[kThreads / 32][6];
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  for (int a = 0; a < 3; ++a) v[a] = warp_min(v[a]), v[a + 3] = warp_max(v[a + 3]);
-  if (lane == 0)
-    for (int a = 0; a < 6; ++a) red[warp][a] = v[a];
-  __syncthreads();
-  if (warp == 0) {
-    for (int a = 0; a < 6; ++a) v[a] = lane < kThreads / 32 ? red[lane][a] : (a < 3 ? FLT_MAX : -FLT_MAX);
-    for (int a = 0; a < 3; ++a) v[a] = warp_min(v[a]), v[a + 3] = warp_max(v[a + 3]);
-  }
-}
-
-// grid nb * n_frames blocks, frame f's nb blocks consecutive (the frame number on x: no 65535-frame limit)
-__global__ void __launch_bounds__(kThreads) ror_bounds_kernel(const uint8_t *__restrict__ in, size_t in_stride,
-                                                              const uint32_t *__restrict__ in_counts, uint32_t n_max,
-                                                              uint32_t nb, Partial *__restrict__ partials) {
-  const uint32_t f = blockIdx.x / nb, b = blockIdx.x - f * nb, n = frame_count(in_counts, f, n_max);
-  const float4 *pts = frame_points(in, in_stride, f);
-  float v[6] = {FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX};
-  for (uint32_t i = b * kThreads + threadIdx.x; i < n; i += nb * kThreads) {
-    const float4 q = __ldg(pts + i);
-    if (!finite3(q)) continue;
-    v[0] = fminf(v[0], q.x), v[1] = fminf(v[1], q.y), v[2] = fminf(v[2], q.z);
-    v[3] = fmaxf(v[3], q.x), v[4] = fmaxf(v[4], q.y), v[5] = fmaxf(v[5], q.z);
-  }
-  block_minmax(v);
-  if (threadIdx.x == 0) {
-    Partial &o = partials[blockIdx.x];
-    for (int a = 0; a < 3; ++a) o.mn[a] = v[a], o.mx[a] = v[a + 3];
-  }
 }
 
 // cells per axis D = K + 2 (K holding points, one padding cell on each side) for the frame's bounds v and 1/c;
@@ -146,13 +84,10 @@ __device__ __forceinline__ bool grid_fits(const float (&v)[6], double ic, uint64
 // sentinel's cell index (all bits set) is above every real one.  The bounds are finite floats, so the span is
 // finite and a fit comes before c overflows (<= 1100 doublings from 2^-64); should c reach infinity first anyway,
 // 1/c = 0 makes the frame a single cell, which is correct for any input.
-__global__ void __launch_bounds__(kThreads) ror_finish_kernel(const Partial *__restrict__ partials, uint32_t nb,
-                                                              double radius, int fb, Desc *__restrict__ desc) {
-  const Partial *pp = partials + (size_t)blockIdx.x * nb;
-  float v[6] = {FLT_MAX, FLT_MAX, FLT_MAX, -FLT_MAX, -FLT_MAX, -FLT_MAX};
-  for (uint32_t b = threadIdx.x; b < nb; b += kThreads)
-    for (int a = 0; a < 3; ++a) v[a] = fminf(v[a], pp[b].mn[a]), v[a + 3] = fmaxf(v[a + 3], pp[b].mx[a]);
-  block_minmax(v);
+__global__ void __launch_bounds__(kStageThreads) ror_finish_kernel(const Partial *__restrict__ partials, uint32_t nb,
+                                                                   double radius, int fb, Desc *__restrict__ desc) {
+  float v[6];
+  fold_partials(partials, nb, v);
   if (threadIdx.x != 0) return;
   Desc d = {};
   if (v[0] <= v[3]) {  // at least one finite point (otherwise every key is the sentinel)
@@ -173,16 +108,16 @@ __global__ void __launch_bounds__(kThreads) ror_finish_kernel(const Partial *__r
   desc[blockIdx.x] = d;
 }
 
-__global__ void __launch_bounds__(kThreads) ror_keys_kernel(const uint8_t *__restrict__ in, size_t in_stride,
-                                                            const uint32_t *__restrict__ in_counts, uint32_t n_max,
-                                                            uint32_t total, int fb, const Desc *__restrict__ desc,
-                                                            uint64_t *__restrict__ keys, uint32_t *__restrict__ vals) {
-  const uint32_t j = blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kStageThreads) ror_keys_kernel(const CloudSrc in, uint32_t total, int fb,
+                                                                 const Desc *__restrict__ desc,
+                                                                 uint64_t *__restrict__ keys,
+                                                                 uint32_t *__restrict__ vals) {
+  const uint32_t j = blockIdx.x * kStageThreads + threadIdx.x;
   if (j >= total) return;
-  const uint32_t f = j / n_max, i = j - f * n_max;
+  const uint32_t f = j / in.n_max, i = j - f * in.n_max;
   uint64_t cell = cell_mask(fb);
-  if (i < frame_count(in_counts, f, n_max)) {
-    const float4 q = __ldg(frame_points(in, in_stride, f) + i);
+  if (i < frame_count(in, f)) {
+    const float4 q = __ldg(frame_points(in, f) + i);
     if (finite3(q)) {
       const Desc d = desc[f];
       cell = cell_of(q.x, d.mn[0], d.ic) + cell_of(q.y, d.mn[1], d.ic) * d.dx + cell_of(q.z, d.mn[2], d.ic) * d.dxy;
@@ -192,16 +127,15 @@ __global__ void __launch_bounds__(kThreads) ror_keys_kernel(const uint8_t *__res
   vals[j] = i;
 }
 
-__global__ void __launch_bounds__(kThreads) ror_gather_kernel(const uint8_t *__restrict__ in, size_t in_stride,
-                                                              uint32_t n_max, uint32_t total, int fb,
-                                                              const uint64_t *__restrict__ keys,
-                                                              const uint32_t *__restrict__ vals,
-                                                              float4 *__restrict__ sorted) {
-  const uint32_t j = blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kStageThreads) ror_gather_kernel(const CloudSrc in, uint32_t total, int fb,
+                                                                   const uint64_t *__restrict__ keys,
+                                                                   const uint32_t *__restrict__ vals,
+                                                                   float4 *__restrict__ sorted) {
+  const uint32_t j = blockIdx.x * kStageThreads + threadIdx.x;
   if (j >= total) return;
   const uint64_t mask = cell_mask(fb);
   if ((keys[j] & mask) == mask) return;  // a sentinel: never read
-  sorted[j] = __ldg(frame_points(in, in_stride, j / n_max) + vals[j]);
+  sorted[j] = __ldg(frame_points(in, j / in.n_max) + vals[j]);
 }
 
 // first position in [lo, hi) whose key is >= k
@@ -220,13 +154,13 @@ __device__ __forceinline__ uint32_t lower_bound(const uint64_t *__restrict__ key
 __constant__ int8_t kRowDy[9] = {0, -1, 1, 0, -1, 1, 0, -1, 1};
 __constant__ int8_t kRowDz[9] = {0, 0, 0, -1, -1, -1, 1, 1, 1};
 
-__global__ void __launch_bounds__(kThreads) ror_count_kernel(uint32_t n_max, uint32_t total, int fb, double r2,
-                                                             uint64_t need, const Desc *__restrict__ desc,
-                                                             const uint64_t *__restrict__ keys,
-                                                             const uint32_t *__restrict__ vals,
-                                                             const float4 *__restrict__ sorted,
-                                                             uint8_t *__restrict__ flags) {
-  const uint32_t j = blockIdx.x * kThreads + threadIdx.x;
+__global__ void __launch_bounds__(kStageThreads) ror_count_kernel(uint32_t n_max, uint32_t total, int fb, double r2,
+                                                                  uint64_t need, const Desc *__restrict__ desc,
+                                                                  const uint64_t *__restrict__ keys,
+                                                                  const uint32_t *__restrict__ vals,
+                                                                  const float4 *__restrict__ sorted,
+                                                                  uint8_t *__restrict__ flags) {
+  const uint32_t j = blockIdx.x * kStageThreads + threadIdx.x;
   if (j >= total) return;
   const uint32_t f = j / n_max, s0 = f * n_max, s1 = s0 + n_max;
   const uint64_t mask = cell_mask(fb), key = keys[j], cell = key & mask, fp = key & ~mask;
@@ -251,38 +185,11 @@ __global__ void __launch_bounds__(kThreads) ror_count_kernel(uint32_t n_max, uin
   flags[s0 + vals[j]] = cnt >= need;  // a sentinel position has cnt 0 < need (need >= 1): dropped
 }
 
-// flag of input position j as the scan's uint32 input (0 at j == total: the scan's last slot is the grand total)
-struct FlagAt {
+// the compaction's keep: the flag at position j (0 or 1)
+struct Flagged {
   const uint8_t *flags;
-  uint32_t total;
-  __host__ __device__ uint32_t operator()(uint32_t j) const { return j < total ? flags[j] : 0u; }
+  __device__ uint32_t operator()(const CloudSrc &, uint32_t, uint32_t, uint32_t j) const { return flags[j]; }
 };
-
-__global__ void __launch_bounds__(kThreads) ror_scatter_kernel(const uint8_t *__restrict__ in, size_t in_stride,
-                                                               uint32_t n_max, uint32_t total,
-                                                               const uint8_t *__restrict__ flags,
-                                                               const uint32_t *__restrict__ slot,
-                                                               uint8_t *__restrict__ out, size_t out_stride,
-                                                               uint32_t *__restrict__ counts) {
-  const uint32_t j = blockIdx.x * kThreads + threadIdx.x;
-  if (j >= total) return;
-  const uint32_t f = j / n_max, i = j - f * n_max, first = f * n_max;
-  if (i == 0) counts[f] = slot[first + n_max] - slot[first];
-  if (!flags[j]) return;
-  float4 *dst = reinterpret_cast<float4 *>(out + (size_t)f * out_stride);
-  dst[slot[j] - slot[first]] = __ldg(frame_points(in, in_stride, f) + i);
-}
-
-inline size_t align_up(size_t v) { return (v + 255) / 256 * 256; }
-
-// blocks per frame of the bounds pass: ~8 points per thread, and about kBoundsBlocks blocks over the whole batch
-constexpr uint32_t kBoundsBlocks = 1024;
-uint32_t bounds_blocks(uint32_t n_frames, uint32_t n) {
-  const uint32_t by_size = (n + kThreads * 8 - 1) / (kThreads * 8);
-  const uint32_t by_chip = (kBoundsBlocks + n_frames - 1) / n_frames;
-  const uint32_t b = by_size < by_chip ? by_size : by_chip;
-  return b ? b : 1;
-}
 
 // every buffer of one launch, carved out of the scratch in this order
 struct Layout {
@@ -302,11 +209,10 @@ Layout layout(uint32_t n_frames, uint32_t n_max) {
   L.sorted = o, o += align_up(m * 16);
   L.flags = o, o += align_up(m);
   L.slot = o, o += align_up((m + 1) * 4);
-  size_t sort_bytes = 0, scan_bytes = 0;
+  size_t sort_bytes = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, sort_bytes, (uint64_t *)nullptr, (uint64_t *)nullptr, (uint32_t *)nullptr,
                                   (uint32_t *)nullptr, (int)m, 0, 64);
-  auto flags = thrust::make_transform_iterator(thrust::counting_iterator<uint32_t>(0), FlagAt{nullptr, 0});
-  cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, flags, (uint32_t *)nullptr, (int)(m + 1));
+  const size_t scan_bytes = compaction_temp_bytes<Flagged>(n_frames, n_max);
   L.temp = o;
   L.temp_bytes = sort_bytes > scan_bytes ? sort_bytes : scan_bytes;
   o += align_up(L.temp_bytes);
@@ -318,25 +224,16 @@ Layout layout(uint32_t n_frames, uint32_t n_max) {
 
 size_t ror_scratch_bytes(uint32_t n_frames, uint32_t n_max) { return layout(n_frames, n_max).total; }
 
-size_t ror_stage_bytes(uint32_t n_frames, uint32_t n) {
-  return align_up((size_t)n_frames * n * 16) + align_up((size_t)n_frames * 4) + ror_scratch_bytes(n_frames, n);
-}
-
-RorStage ror_stage(void *buffer, uint32_t n_frames, uint32_t n) {
-  uint8_t *b = static_cast<uint8_t *>(buffer);
-  const size_t clouds = align_up((size_t)n_frames * n * 16);
-  return RorStage{b, reinterpret_cast<uint32_t *>(b + clouds), b + clouds + align_up((size_t)n_frames * 4)};
-}
-
-cudaError_t launch_radius_outlier(const RorLaunch &R, cudaStream_t stream, int *launches) {
+cudaError_t launch_radius_outlier(const CloudSrc &in, const CloudDst &out, double radius, uint32_t min_neighbors,
+                                  void *scratch, cudaStream_t stream, int *launches) {
   if (launches) *launches = 0;
-  if (R.n_frames == 0) return cudaSuccess;
-  if ((uint64_t)R.n_frames * R.n_max > kRorMaxPoints) return cudaErrorInvalidValue;  // the caller splits the batch
-  if (R.n_max == 0) return cudaMemsetAsync(R.counts, 0, R.n_frames * sizeof(uint32_t), stream);
-  const uint32_t total = R.n_frames * R.n_max;
-  const int fb = frame_bits(R.n_frames);
-  const Layout L = layout(R.n_frames, R.n_max);
-  uint8_t *base = static_cast<uint8_t *>(R.scratch);
+  if (in.n_frames == 0) return cudaSuccess;
+  if ((uint64_t)in.n_frames * in.n_max > kCloudMaxPoints) return cudaErrorInvalidValue;  // the caller splits the batch
+  if (in.n_max == 0) return cudaMemsetAsync(out.counts, 0, in.n_frames * sizeof(uint32_t), stream);
+  const uint32_t total = in.n_frames * in.n_max;
+  const int fb = frame_bits(in.n_frames);
+  const Layout L = layout(in.n_frames, in.n_max);
+  uint8_t *base = static_cast<uint8_t *>(scratch);
   Partial *partials = reinterpret_cast<Partial *>(base + L.partials);
   Desc *desc = reinterpret_cast<Desc *>(base + L.desc);
   uint64_t *keys_in = reinterpret_cast<uint64_t *>(base + L.keys_in);
@@ -349,36 +246,28 @@ cudaError_t launch_radius_outlier(const RorLaunch &R, cudaStream_t stream, int *
   void *temp = base + L.temp;
 
   // every launch is checked before anything that reads its output is queued
-  const uint32_t nb = bounds_blocks(R.n_frames, R.n_max);
-  ror_bounds_kernel<<<nb * R.n_frames, kThreads, 0, stream>>>(R.in, R.in_stride, R.in_counts, R.n_max, nb, partials);
+  const uint32_t nb = bounds_blocks(in.n_frames, in.n_max);
+  cloud_bounds_kernel<<<nb * in.n_frames, kStageThreads, 0, stream>>>(in, nb, Finite{}, partials);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return e;
-  ror_finish_kernel<<<R.n_frames, kThreads, 0, stream>>>(partials, nb, R.radius, fb, desc);
+  ror_finish_kernel<<<in.n_frames, kStageThreads, 0, stream>>>(partials, nb, radius, fb, desc);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  const uint32_t grid = (total + kThreads - 1) / kThreads;
-  ror_keys_kernel<<<grid, kThreads, 0, stream>>>(R.in, R.in_stride, R.in_counts, R.n_max, total, fb, desc, keys_in,
-                                                 vals_in);
+  const uint32_t grid = (total + kStageThreads - 1) / kStageThreads;
+  ror_keys_kernel<<<grid, kStageThreads, 0, stream>>>(in, total, fb, desc, keys_in, vals_in);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
   size_t tb = L.temp_bytes;
   e = cub::DeviceRadixSort::SortPairs(temp, tb, keys_in, keys_out, vals_in, vals_out, (int)total, 0, 64, stream);
   if (e != cudaSuccess) return e;
-  ror_gather_kernel<<<grid, kThreads, 0, stream>>>(R.in, R.in_stride, R.n_max, total, fb, keys_out, vals_out, sorted);
+  ror_gather_kernel<<<grid, kStageThreads, 0, stream>>>(in, total, fb, keys_out, vals_out, sorted);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  ror_count_kernel<<<grid, kThreads, 0, stream>>>(R.n_max, total, fb, R.radius * R.radius,
-                                                  (uint64_t)R.min_neighbors + 1, desc, keys_out, vals_out, sorted,
-                                                  flags);
-  e = cudaGetLastError();
-  if (e != cudaSuccess) return e;
-  tb = L.temp_bytes;
-  e = cub::DeviceScan::ExclusiveSum(temp, tb,
-                                    thrust::make_transform_iterator(thrust::counting_iterator<uint32_t>(0),
-                                                                    FlagAt{flags, total}),
-                                    slot, (int)(total + 1), stream);
-  if (e != cudaSuccess) return e;
-  ror_scatter_kernel<<<grid, kThreads, 0, stream>>>(R.in, R.in_stride, R.n_max, total, flags, slot, R.out,
-                                                    R.out_stride, R.counts);
-  if (launches) *launches = 8;  // six kernels of this file, the sort and the scan (each CUB call counted once)
-  return cudaGetLastError();
+  ror_count_kernel<<<grid, kStageThreads, 0, stream>>>(in.n_max, total, fb, radius * radius,
+                                                       (uint64_t)min_neighbors + 1, desc, keys_out, vals_out, sorted,
+                                                       flags);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  e = launch_compaction(in, Flagged{flags}, slot, temp, L.temp_bytes, out, stream);
+  // six kernels of this file and cloud_stage.cuh, the sort and the scan (each CUB call counted once)
+  if (launches && e == cudaSuccess) *launches = 8;
+  return e;
 }
 
 }  // namespace d2pc

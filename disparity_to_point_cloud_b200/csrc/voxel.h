@@ -1,9 +1,8 @@
 // voxel.h -- host-side launcher interface of voxel.cu: pcl::VoxelGrid<pcl::PointXYZ> on the device, applied to
-// the CROP clouds of a frame batch (D2PC_FILTER_VOXEL; the recipe is in include/d2pc_b200.h).
+// the clouds of a frame batch (D2PC_FILTER_VOXEL: the CROP clouds, or the crop box's; the recipe is in
+// include/d2pc_b200.h).  Input, destination and batch limit are cloud_stage.cuh's.
 #pragma once
-#include <cstddef>
-#include <cstdint>
-#include <cuda_runtime.h>
+#include "cloud_stage.cuh"
 
 namespace d2pc {
 
@@ -14,27 +13,12 @@ struct VoxelParams {
   double limit_min, limit_max;
 };
 
-struct VoxelLaunch {
-  // n_frames clouds of at most n points each, frame f at voxel_crop(scratch) + f * n (dense, written by the CROP
-  // kernels or the crop box)
-  uint32_t n_frames = 0;
-  uint32_t n = 0;
-  // per frame (may be null: n each): the points of the frame's cloud; positions at or past it are excluded
-  const uint32_t *in_counts = nullptr;
-  VoxelParams p;
-  uint8_t *out = nullptr;  // voxel clouds, frame f at out + f * out_stride bytes
-  size_t out_stride = 0;
-  uint32_t *counts = nullptr;    // per frame: points written
-  uint32_t *fallback = nullptr;  // per frame (may be null): 1 when the frame took the overflow fallback
-  void *scratch = nullptr;       // voxel_scratch_bytes(n_frames, n)
-};
-
-// Device scratch for one launch (the CROP clouds first, then keys, indices, sort / scan temp storage, descriptors).
-// Sized once per frame geometry; nothing in it needs clearing.
-size_t voxel_scratch_bytes(uint32_t n_frames, uint32_t n);
-// Where the CROP kernels must write the batch's clouds (the head of the scratch).
-inline float *voxel_crop(void *scratch) { return static_cast<float *>(scratch); }
-// n_frames * n < 2^31 (the sort and scan index with int)
-cudaError_t launch_voxel(const VoxelLaunch &L, cudaStream_t stream, int *launches);
+// Device scratch for one launch (keys, indices, sort / scan temp storage, bounds, descriptors).  Sized once per frame
+// geometry; nothing in it needs clearing.
+size_t voxel_scratch_bytes(uint32_t n_frames, uint32_t n_max);
+// The voxel clouds and their per-frame counts into out; positions at or past a frame's input count are excluded.
+// fallback (may be null): per frame, 1 when the frame took the overflow fallback (its output is its input cloud).
+cudaError_t launch_voxel(const CloudSrc &in, const CloudDst &out, const VoxelParams &p, uint32_t *fallback,
+                         void *scratch, cudaStream_t stream, int *launches);
 
 }  // namespace d2pc
