@@ -80,6 +80,11 @@ class CropBox(C.Structure):
                 ("max_pt", C.c_float * 3), ("transform", C.c_float * 12)]
 
 
+class CloudTransform(C.Structure):
+    """d2pc_cloud_transform: pcl::transformPointCloud matrix of the first cloud stage (camera frame -> target frame)."""
+    _fields_ = [("struct_size", C.c_uint32), ("enabled", C.c_int32), ("matrix", C.c_float * 12)]
+
+
 class Timing(C.Structure):
     _fields_ = [("h2d_us", C.c_float), ("kernels_us", C.c_float), ("d2h_us", C.c_float), ("total_us", C.c_float),
                 ("points", C.c_uint64)]
@@ -120,6 +125,11 @@ SYMBOLS = [
     ("d2pc_get_crop_box", C.c_int, [_ctx, C.POINTER(CropBox)]),
     ("d2pc_crop_box_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
                                        C.c_void_p, C.c_size_t, C.c_void_p]),
+    ("d2pc_cloud_transform_default", None, [C.POINTER(CloudTransform)]),
+    ("d2pc_set_cloud_transform", C.c_int, [_ctx, C.POINTER(CloudTransform)]),
+    ("d2pc_get_cloud_transform", C.c_int, [_ctx, C.POINTER(CloudTransform)]),
+    ("d2pc_cloud_transform_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
+                                              C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
     ("d2pc_process_mono8", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_process_f32", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_submit_mono8", C.c_int, [_ctx, C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
@@ -350,6 +360,18 @@ class Context:
         self._check(lib().d2pc_get_radius_outlier(self._h, C.byref(p)), "d2pc_get_radius_outlier")
         return p
 
+    @staticmethod
+    def _affine(m, what) -> np.ndarray:
+        """A 3x4 [A | t], or a 4x4 matrix whose last row is (0, 0, 0, 1), as 12 row-major float32 values."""
+        t = np.asarray(m, np.float32)
+        if t.shape == (4, 4):
+            if not np.array_equal(t[3], np.float32([0, 0, 0, 1])):
+                raise ValueError(f"{what}: the last row of a 4x4 transform must be (0, 0, 0, 1), got {t[3]}")
+            t = t[:3]
+        if t.shape != (3, 4):
+            raise ValueError(f"{what}: transform must be 3x4 or 4x4, got {t.shape}")
+        return t.reshape(12)
+
     def set_crop_box(self, min_pt, max_pt=None, transform=None):
         """pcl::CropBox in front of VOXEL and the outlier stage: keep the points p with min_pt <= T p <= max_pt.
         transform: None (the identity) or the camera -> box transform T as a 3x4 [R | t] or a 4x4 matrix whose last
@@ -363,20 +385,30 @@ class Context:
             b.min_pt[:] = [float(v) for v in np.asarray(min_pt, np.float32).reshape(3)]
             b.max_pt[:] = [float(v) for v in np.asarray(max_pt, np.float32).reshape(3)]
             if transform is not None:
-                t = np.asarray(transform, np.float32)
-                if t.shape == (4, 4):
-                    if not np.array_equal(t[3], np.float32([0, 0, 0, 1])):
-                        raise ValueError(f"set_crop_box: the last row of a 4x4 transform must be (0, 0, 0, 1), got {t[3]}")
-                    t = t[:3]
-                if t.shape != (3, 4):
-                    raise ValueError(f"set_crop_box: transform must be 3x4 or 4x4, got {t.shape}")
-                b.transform[:] = [float(v) for v in t.reshape(12)]
+                b.transform[:] = [float(v) for v in self._affine(transform, "set_crop_box")]
         self._check(lib().d2pc_set_crop_box(self._h, C.byref(b)), "d2pc_set_crop_box")
 
     def get_crop_box(self) -> CropBox:
         b = CropBox()
         self._check(lib().d2pc_get_crop_box(self._h, C.byref(b)), "d2pc_get_crop_box")
         return b
+
+    def set_transform(self, matrix):
+        """pcl::transformPointCloud as the first cloud stage: every finite point p becomes T p (camera frame ->
+        target frame), in front of the crop box, VOXEL and the outlier stage.  matrix: a 3x4 [A | t] or a 4x4 matrix
+        whose last row is (0, 0, 0, 1); None turns the transform off.  A slot uses the setting in force when its frame
+        is submitted."""
+        t = CloudTransform()
+        lib().d2pc_cloud_transform_default(C.byref(t))
+        if matrix is not None:
+            t.enabled = 1
+            t.matrix[:] = [float(v) for v in self._affine(matrix, "set_transform")]
+        self._check(lib().d2pc_set_cloud_transform(self._h, C.byref(t)), "d2pc_set_cloud_transform")
+
+    def get_transform(self) -> CloudTransform:
+        t = CloudTransform()
+        self._check(lib().d2pc_get_cloud_transform(self._h, C.byref(t)), "d2pc_get_cloud_transform")
+        return t
 
     def set_arith_mode(self, m):
         self._check(lib().d2pc_set_arith_mode(self._h, m), "d2pc_set_arith_mode")
@@ -496,6 +528,14 @@ class Context:
     def crop_box_device(self, d_in, n_frames, n_max, in_stride, d_in_counts, d_out, out_stride, d_out_counts):
         self._check(lib().d2pc_crop_box_device(self._h, d_in, n_frames, n_max, in_stride, d_in_counts or None,
                                                d_out, out_stride, d_out_counts or None), "d2pc_crop_box_device")
+
+    def transform_device(self, d_in, n_frames, n_max, in_stride, d_in_counts, d_out, out_stride, d_out_counts=0,
+                         d_transforms=None):
+        """d2pc_cloud_transform_device: d_transforms None applies the context's (enabled) setting, otherwise it is
+        the device address of n_frames row-major 3x4 float32 matrices.  d_out may be d_in (same stride)."""
+        self._check(lib().d2pc_cloud_transform_device(self._h, d_in, n_frames, n_max, in_stride, d_in_counts or None,
+                                                      d_out, out_stride, d_out_counts or None, d_transforms or None),
+                    "d2pc_cloud_transform_device")
 
     def median_u8_device(self, d_src, w, h, src_step, d_dst, dst_step, ksize):
         self._check(lib().d2pc_median_u8_device(self._h, d_src, w, h, src_step, d_dst, dst_step, ksize),

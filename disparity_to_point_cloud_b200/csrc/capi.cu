@@ -26,6 +26,7 @@
 #include <nvtx3/nvToolsExt.h>
 #include <sys/mman.h>
 
+#include "cloud_transform.h"
 #include "crop_box.h"
 #include "fusion.h"
 #include "median.h"
@@ -51,15 +52,15 @@ struct PinBuf {
 };
 
 // The filter stages that run on clouds already on the device (cloud_stage.cuh), in the order a plan runs them.
-enum class CloudStage { box, voxel, ror };
+enum class CloudStage { transform, box, voxel, ror };
 
-// What the filter mode, the crop box and the radius outlier stage make of one frame geometry (plan_cloud), decided
-// once per call.
+// What the filter mode, the cloud transform, the crop box and the radius outlier stage make of one frame geometry
+// (plan_cloud), decided once per call.
 struct CloudPlan {
   uint64_t n = 0;           // crop points per frame
   bool compact = false;     // the reproject kernels keep only finite points (CROP_FINITE without the box)
-  // the cloud stages that run, in order: the crop box on the CROP cloud, VOXEL, the radius outlier stage
-  CloudStage stages[3];
+  // the cloud stages that run, in order: the transform, the crop box on the CROP cloud, VOXEL, the outlier stage
+  CloudStage stages[4];
   int n_stages = 0;
   bool counted = false;     // the cloud's size is known only on the device: the kept count decides the bytes
   uint32_t count_words = 1; // count words a slot reads back (Slot::d_count)
@@ -117,6 +118,7 @@ struct d2pc_ctx {
   bool voxel_set = false;
   d2pc_radius_outlier ror;  // the radius outlier stage behind every mode (d2pc_set_radius_outlier; radius 0: off)
   d2pc_crop_box box;        // the crop box in front of VOXEL and the outlier stage (d2pc_set_crop_box; enabled 0: off)
+  d2pc_cloud_transform xform;  // the first cloud stage (d2pc_set_cloud_transform; enabled 0: off)
   // fusion buffers
   DevBuf d_fuse_in[4], d_container, d_combined, d_fused;
   PinBuf h_fused, h_combined;
@@ -135,8 +137,9 @@ struct d2pc_ctx {
   // CROP clouds written by the kernel straight into the page-locked host buffer (no D2H copy after the kernel; the
   // transfer overlaps the kernel): 0 = the synchronous single-frame mono8 entries only (the median makes that
   // kernel long enough to hide: -6..-8 % per call; a float frame's 5 us kernel hides nothing and SM stores cross
-  // PCIe ~15 % slower than the copy engine, so streams and float frames keep the copy), 1 = every CROP submission,
-  // -1 = never
+  // PCIe ~15 % slower than the copy engine, so streams and float frames keep the copy; so do plans with a cloud
+  // stage after the reproject kernel, the transform: its 1.6 us store kernel hides nothing either), 1 = every CROP
+  // submission, -1 = never
   int direct_out = 0;
   bool timing = false;  // d2pc_set_timing: slot events carry timestamps
   std::vector<std::pair<uintptr_t, bool>> pin_cache;  // host pointer -> pinned (cudaHostAlloc / cudaHostRegister)?
@@ -271,14 +274,16 @@ uint64_t crop_points(uint32_t w, uint32_t h, int border) {
 CloudPlan plan_cloud(const d2pc_ctx *ctx, uint32_t w, uint32_t h) {
   CloudPlan p;
   p.n = crop_points(w, h, ctx->cfg.border);
-  const bool box = ctx->box.enabled != 0, voxel = ctx->cfg.filter_mode == D2PC_FILTER_VOXEL,
-             ror = ctx->ror.radius > 0.0;
+  const bool xform = ctx->xform.enabled != 0, box = ctx->box.enabled != 0,
+             voxel = ctx->cfg.filter_mode == D2PC_FILTER_VOXEL, ror = ctx->ror.radius > 0.0;
   // the box drops non-finite points itself: CROP_FINITE + box runs the CROP kernels and lets the box compact once
   p.compact = ctx->cfg.filter_mode == D2PC_FILTER_CROP_FINITE && !box;
+  if (xform) p.stages[p.n_stages++] = CloudStage::transform;
   if (box) p.stages[p.n_stages++] = CloudStage::box;
   if (voxel) p.stages[p.n_stages++] = CloudStage::voxel;
   if (ror) p.stages[p.n_stages++] = CloudStage::ror;
-  p.counted = p.compact || p.n_stages > 0;
+  // the transform keeps every point: only the stages that change the count make it decide the bytes
+  p.counted = p.compact || box || voxel || ror;
   p.count_words = voxel ? 3 : 1;  // the kept count [, the ticket, the VOXEL fallback flag]
   // the box's and the outlier stage's outputs are always dense, so is a VOXEL fallback that copies the box's cloud
   p.fallback_decides_dense = voxel && !ror && !box;
@@ -382,7 +387,8 @@ struct FrameBatch {
 };
 
 size_t stage_scratch_bytes(CloudStage st, uint32_t n_frames, uint32_t n) {
-  return st == CloudStage::box     ? crop_box_scratch_bytes(n_frames, n)
+  return st == CloudStage::transform ? 0
+         : st == CloudStage::box   ? crop_box_scratch_bytes(n_frames, n)
          : st == CloudStage::voxel ? voxel_scratch_bytes(n_frames, n)
                                    : ror_scratch_bytes(n_frames, n);
 }
@@ -434,13 +440,21 @@ uint32_t frames_per_chunk(uint32_t n_frames, uint64_t points_per_frame) {
   return (uint32_t)std::min<uint64_t>(n_frames, by_points);
 }
 
+CloudTransformParams transform_params(const d2pc_ctx *ctx) {
+  CloudTransformParams t;
+  for (int k = 0; k < 12; ++k) t.m[k] = ctx->xform.matrix[k];
+  return t;
+}
+
 // One cloud stage with the context's setting on a batch of clouds, on `stream`.  The setting travels by value, so a
 // later d2pc_set_* cannot reach a queued launch.  fallback: VOXEL's per-frame overflow fallback flags (may be null).
 int enqueue_stage(d2pc_ctx *ctx, CloudStage st, const CloudSrc &in, const CloudDst &out, uint32_t *fallback,
                   void *scratch, cudaStream_t stream) {
   int nl = 0;
   cudaError_t e;
-  if (st == CloudStage::box) {
+  if (st == CloudStage::transform) {
+    e = launch_cloud_transform(in, out, transform_params(ctx), nullptr, stream, &nl);
+  } else if (st == CloudStage::box) {
     const d2pc_crop_box &box = ctx->box;
     CropBoxParams b;
     for (int a = 0; a < 3; ++a) b.mn[a] = box.min_pt[a], b.mx[a] = box.max_pt[a];
@@ -631,7 +645,8 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   // frame no longer pays kernel + copy back to back (CROP only: a compacted cloud's size is not known up front)
   uint8_t *d_direct = nullptr;
   if (!p.counted && n && !late_copy &&
-      (ctx->direct_out > 0 || (ctx->direct_out == 0 && sync_call && !is_f32 && ctx->cfg.median_ksize > 1)))
+      (ctx->direct_out > 0 ||
+       (ctx->direct_out == 0 && sync_call && !is_f32 && ctx->cfg.median_ksize > 1 && p.n_stages == 0)))
     d_direct = direct_alias(user_pinned ? user_dst : s.h_out.p);
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
   const FrameBatch in{s.d_in.p, is_f32, 1, w, h, d_pitch, d_pitch * h};
@@ -823,6 +838,7 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
   d2pc_voxel_grid_default(&ctx->voxel);
   d2pc_radius_outlier_default(&ctx->ror);
   d2pc_crop_box_default(&ctx->box);
+  d2pc_cloud_transform_default(&ctx->xform);
 
   if (const char *v = getenv("D2PC_ROWS_PER_UNIT")) ctx->rows_per_unit = atoi(v);
   if (const char *v = getenv("D2PC_CTAS_PER_SM")) ctx->ctas_per_sm = atoi(v);
@@ -952,6 +968,24 @@ int d2pc_set_crop_box(d2pc_ctx *ctx, const d2pc_crop_box *b) {
 int d2pc_get_crop_box(const d2pc_ctx *ctx, d2pc_crop_box *b) {
   if (!ctx || !b) return D2PC_ERR_INVALID_ARG;
   *b = ctx->box;
+  return D2PC_OK;
+}
+void d2pc_cloud_transform_default(d2pc_cloud_transform *t) {
+  if (!t) return;
+  memset(t, 0, sizeof(*t));
+  t->struct_size = sizeof(*t);
+  for (int a = 0; a < 3; ++a) t->matrix[5 * a] = 1.0f;
+}
+int d2pc_set_cloud_transform(d2pc_ctx *ctx, const d2pc_cloud_transform *t) {
+  if (!ctx || !t || t->struct_size != sizeof(*t)) return D2PC_ERR_INVALID_ARG;
+  for (float m : t->matrix)
+    if (!std::isfinite(m)) return D2PC_ERR_INVALID_ARG;
+  ctx->xform = *t;
+  return D2PC_OK;
+}
+int d2pc_get_cloud_transform(const d2pc_ctx *ctx, d2pc_cloud_transform *t) {
+  if (!ctx || !t) return D2PC_ERR_INVALID_ARG;
+  *t = ctx->xform;
   return D2PC_OK;
 }
 int d2pc_set_arith_mode(d2pc_ctx *ctx, int m) {
@@ -1197,15 +1231,15 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
 }
 
 // The argument rules of the stages that run alone on clouds already on the device (d2pc_radius_outlier_device,
-// d2pc_crop_box_device).
+// d2pc_crop_box_device, d2pc_cloud_transform_device).  in_place: the output may also be exactly the input.
 static int check_cloud_batch(const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
-                             const uint8_t *d_out, size_t out_stride) {
+                             const uint8_t *d_out, size_t out_stride, bool in_place = false) {
   const uint64_t bytes = (uint64_t)n_max * 16;
   if (bytes > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // per-frame counts and PointCloud2.row_step are uint32
   if (reinterpret_cast<uintptr_t>(d_in) % 16 || reinterpret_cast<uintptr_t>(d_out) % 16 || in_stride % 16 ||
       out_stride % 16 || (n_frames > 1 && (in_stride < bytes || out_stride < bytes)))
     return D2PC_ERR_BAD_DIMS;
-  if (n_frames == 0) return D2PC_OK;
+  if (n_frames == 0 || (in_place && d_in == d_out && in_stride == out_stride)) return D2PC_OK;
   // kept points are copied from the input after every flag is known: the two must not share bytes
   const uintptr_t in0 = reinterpret_cast<uintptr_t>(d_in), out0 = reinterpret_cast<uintptr_t>(d_out);
   const uint64_t in_end = in0 + (uint64_t)(n_frames - 1) * in_stride + bytes;
@@ -1250,6 +1284,27 @@ int d2pc_crop_box_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, 
                          const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride, uint32_t *d_out_counts) {
   return cloud_stage_device(ctx, CloudStage::box, ctx && ctx->box.enabled, d_in, n_frames, n_max, in_stride,
                             d_in_counts, d_out, out_stride, d_out_counts);
+}
+
+int d2pc_cloud_transform_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
+                                size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
+                                uint32_t *d_out_counts, const float *d_transforms) {
+  if (!ctx || !d_in || !d_out || (!d_transforms && !ctx->xform.enabled)) return D2PC_ERR_INVALID_ARG;
+  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_out, out_stride, true);
+  if (rc0 || n_frames == 0) return rc0;
+  CU(ctx, cudaSetDevice(ctx->device));
+  const CloudTransformParams t = transform_params(ctx);
+  const uint32_t chunk = frames_per_chunk(n_frames, n_max);
+  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
+    const CloudSrc in{d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
+                      std::min(chunk, n_frames - f0), n_max};
+    const CloudDst out{d_out + f0 * out_stride, out_stride, d_out_counts ? d_out_counts + f0 : nullptr};
+    int nl = 0;
+    CU(ctx, launch_cloud_transform(in, out, t, d_transforms ? d_transforms + 12 * (size_t)f0 : nullptr, ctx->s_compute,
+                                   &nl));
+    ctx->launches += nl;
+  }
+  return D2PC_OK;
 }
 
 int d2pc_reproject_f32_device(d2pc_ctx *ctx, const float *d_disp, uint32_t n_frames, uint32_t w, uint32_t h,
@@ -1578,8 +1633,9 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
   const uint64_t n = p.n;
   if ((rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
   // a synchronous call: the callback kernel stores the CROP cloud straight into the pinned buffer (see submit_common)
+  const bool direct = ctx->direct_out > 0 || (ctx->direct_out == 0 && p.n_stages == 0);
   uint8_t *const d_direct =
-      !p.counted && n && ctx->direct_out >= 0 && ctx->cfg.median_ksize > 1 ? direct_alias(s.h_out.p) : nullptr;
+      !p.counted && n && direct && ctx->cfg.median_ksize > 1 ? direct_alias(s.h_out.p) : nullptr;
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
   const FrameBatch fused{ctx->d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh};
   if ((rc = grow_stages(ctx, s.stages, p, fused, ctx->s_compute, false)) ||

@@ -23,8 +23,9 @@ struct CloudSrc {
   uint32_t n_max = 0;
 };
 
-// Where a stage writes a batch's clouds: frame f at points + f * stride, its point count at counts[f].  A stage's
-// destination never overlaps its input: kept points are copied after every decision is made.
+// Where a stage writes a batch's clouds: frame f at points + f * stride, its point count at counts[f].  A compacting
+// stage's destination never overlaps its input: kept points are copied after every decision is made.  (The
+// transform, a per-point map, may also write exactly over its input.)
 struct CloudDst {
   uint8_t *points;
   size_t stride;
@@ -53,6 +54,13 @@ __device__ __forceinline__ uint32_t frame_count(const CloudSrc &in, uint32_t f) 
 
 __device__ __forceinline__ const float4 *frame_points(const CloudSrc &in, uint32_t f) {
   return reinterpret_cast<const float4 *>(in.in + (size_t)f * in.in_stride);
+}
+
+// Row a of T * p for a row-major 3x4 [A | t] (t points at the row): ((t[0] * x + t[1] * y) + t[2] * z) + t[3], every
+// operation rounded.  Explicit round-to-nearest intrinsics, because nvcc contracts a * b + c to an FMA by default.
+// The crop box's local coordinates and the transform stage's output both come from here, so the two cannot drift.
+__device__ __forceinline__ float affine_row(const float *t, const float4 &q) {
+  return __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(t[0], q.x), __fmul_rn(t[1], q.y)), __fmul_rn(t[2], q.z)), t[3]);
 }
 
 // ---- per-frame bounds: cloud_bounds_kernel (<= kBoundsBlocks blocks over the batch) -> partials, then

@@ -4,18 +4,12 @@
 // cloud_stage.cuh's order-preserving compaction over it, in two launches: the scan reads the predicate through a
 // transform iterator (no flag array), and the scatter evaluates it again and copies the kept points.
 //
-// The local coordinates are float32 with explicit round-to-nearest intrinsics, because nvcc contracts a * b + c to an
-// FMA by default and the recipe rounds every operation.  No buffer is read before a kernel of the same launch has
-// written it, so the scratch needs no clearing.
+// The local coordinates are cloud_stage.cuh's affine_row, the transform stage's rounding recipe.  No buffer is read
+// before a kernel of the same launch has written it, so the scratch needs no clearing.
 #include "crop_box.h"
 
 namespace d2pc {
 namespace {
-
-// rows a of l = T * p: ((t[a][0] * x + t[a][1] * y) + t[a][2] * z) + t[a][3], every operation rounded
-__device__ __forceinline__ float local(const float *t, const float4 &q) {
-  return __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(t[0], q.x), __fmul_rn(t[1], q.y)), __fmul_rn(t[2], q.z)), t[3]);
-}
 
 // recipe rules 1-3: finite, then min <= l <= max on every axis (a NaN l fails)
 __device__ __forceinline__ bool inside(const float4 &q, const CropBoxParams &b) {
@@ -23,7 +17,7 @@ __device__ __forceinline__ bool inside(const float4 &q, const CropBoxParams &b) 
   bool in = true;
 #pragma unroll
   for (int a = 0; a < 3; ++a) {
-    const float l = local(b.t + 4 * a, q);
+    const float l = affine_row(b.t + 4 * a, q);
     in = in && b.mn[a] <= l && l <= b.mx[a];
   }
   return in;

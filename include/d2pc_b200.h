@@ -124,7 +124,7 @@ typedef struct d2pc_cloud {
   uint32_t row_step;   /* 16 * width */
   uint8_t is_bigendian; /* 0 */
   uint8_t is_dense;     /* 0 in CROP mode (cpp:81); 1 in CROP_FINITE; VOXEL: 1, 0 for the overflow fallback;
-                           1 behind the crop box or the radius outlier stage */
+                           1 behind the crop box or the radius outlier stage; the cloud transform keeps it */
   uint32_t n_fields;    /* 3 */
   d2pc_point_field fields[3];
 } d2pc_cloud;
@@ -263,6 +263,8 @@ int d2pc_get_radius_outlier(const d2pc_ctx *ctx, d2pc_radius_outlier *p);
  *     takes VOXEL's overflow fallback publishes the box's cloud with is_dense 1 (all of its points are finite;
  *     whether PCL's copy in that fallback would set is_dense is not verified here).
  *   - The radius outlier stage runs on whatever the steps before it produced.
+ *   - With a cloud transform enabled (d2pc_set_cloud_transform) the box runs on the transformed cloud: "camera frame"
+ *     above then reads "target frame", and the points it keeps are target-frame points.
  * Relation to PCL (CropBox::applyFilter and pcl::transformPoint, PCL 1.8 - 1.12; restated from memory, PCL's source
  * was not at hand when this was written -- the same footing as DESIGN.md section 0.1 for the OpenCV dispatch):
  *   - transformPoint computes each row as ((m(i,0)*x + m(i,1)*y) + m(i,2)*z) + m(i,3) in float, which is rule 2.
@@ -291,13 +293,60 @@ int d2pc_set_crop_box(d2pc_ctx *ctx, const d2pc_crop_box *b);
 /* The setting last made (d2pc_crop_box_default's until then). */
 int d2pc_get_crop_box(const d2pc_ctx *ctx, d2pc_crop_box *b);
 
+/* ---- cloud transform (the first stage: in front of the crop box, VOXEL and the radius outlier stage) ----------
+ *
+ * Off by default (enabled 0).  With a transform enabled, the published cloud is pcl::transformPointCloud<PointXYZ>
+ * with an affine matrix, applied on the device to the cloud of the filter mode's reproject step (CROP's N points or
+ * CROP_FINITE's compacted ones) before any other stage: reproject -> transform -> crop box -> VOXEL -> outlier stage.
+ * So the crop box's transform maps the TARGET frame to the box frame, VOXEL's grid lies in the target frame, and the
+ * outlier stage sees target-frame points.  The recipe, float32 throughout, no FMA contraction:
+ *   1. A point whose x, y and z are all finite becomes x' = ((m00*x + m01*y) + m02*z) + m03, likewise y' (row 1)
+ *      and z' (row 2), each operation rounded: the crop box's rule 2, one shared device routine.
+ *   2. A point with a non-finite coordinate is copied unchanged, all 16 bytes, NaN payloads included (PCL's
+ *      non-dense branch; for dense input every point is finite and both PCL branches are rule 1).
+ *   3. The fourth word (1.0f) is copied; the point count and the input order are kept.
+ *   4. is_dense is the input's.  A finite point whose T * p overflows is written as computed (+-inf or NaN), as PCL
+ *      writes it, so CROP_FINITE with an extreme transform can publish a non-finite point with is_dense 1.  A NaN
+ *      the arithmetic makes (inf + -inf) is written as 0xFFC00000, the default NaN of x86 SSE arithmetic and so what
+ *      PCL writes on x86-64.
+ * The identity maps every finite coordinate to itself except -0, which becomes +0 (-0 * 1 + 0 * y + ... is +0).
+ * Relation to PCL (transformPointCloud in common/impl/transforms.hpp, PCL 1.8 - 1.12; restated from memory, PCL's
+ * source was not at hand when this was written -- the same footing as DESIGN.md section 0.1 for the OpenCV dispatch):
+ *   - transformPointCloud copies the cloud, then transforms every point if is_dense, otherwise only the points with
+ *     finite x, y and z (rules 1 and 2).
+ *   - PCL >= 1.10 computes a point through detail::Transformer<float>.  Its SSE2 specialisation is believed to form
+ *     each row as x*c0 + (y*c1 + (z*c2 + c3)); its scalar template as ((m0*x + m1*y) + m2*z) + m3, which a compiler
+ *     may contract to FMAs.  PCL 1.8 - 1.9 use Eigen's matrix product.  No single PCL rounding order exists; this
+ *     library uses the scalar template's order without contraction (rule 1), the crop box's order.
+ *   - Measured on three 752x480 S2 scenes (tests/test_oracle_transform.py; yaw 30, pitch 20, roll 10 degrees and a
+ *     translation): the SSE2 order gives a different float on 41 % of the finite points' output coordinates, by at
+ *     most 4 ulp of the row's largest term (a result that cancels towards zero can differ by more of its own ulp).
+ * With a transform and no other cloud stage, CROP stays an uncounted mode (no payload copy in d2pc_wait,
+ * BUFFER_TOO_SMALL at submit, and the device batch entries may pass d_counts NULL); the synchronous mono8 entries then
+ * copy the cloud out of a device buffer instead of storing it into host memory from the kernel ("direct_out" 1
+ * forces the latter).  The setting in force when a frame is submitted is
+ * the one its slot uses: set a frame's pose, submit it, then set the next one. */
+typedef struct d2pc_cloud_transform {
+  uint32_t struct_size; /* sizeof(d2pc_cloud_transform) */
+  int32_t enabled;      /* 0: off (the default) */
+  float matrix[12];     /* row-major 3x4 [A | t], camera frame -> target frame; any finite affine map; default
+                           identity */
+} d2pc_cloud_transform;
+
+/* enabled 0, the identity matrix. */
+void d2pc_cloud_transform_default(d2pc_cloud_transform *t);
+/* D2PC_ERR_INVALID_ARG for a non-finite matrix entry or a wrong struct_size; the previous setting is kept then. */
+int d2pc_set_cloud_transform(d2pc_ctx *ctx, const d2pc_cloud_transform *t);
+/* The setting last made (d2pc_cloud_transform_default's until then). */
+int d2pc_get_cloud_transform(const d2pc_ctx *ctx, d2pc_cloud_transform *t);
+
 /* ---- the disparity callback, host buffers (the reference-facing calls) ------ */
 
 /* Whole DisparityCb (src/disparity_to_point_cloud.cpp:46-92) on one mono8
  * frame in host memory: H2D, median 11, x(1/8), reproject with Q, crop 40,
- * pack {x,y,z,1}, D2H.  Synchronous: `out` is complete on return.  (In CROP mode the kernel of this call stores
- * the points straight into the page-locked destination, so the transfer to the host runs while the kernel does
- * instead of as a copy behind it: tuning key "direct_out".) */
+ * pack {x,y,z,1}, D2H.  Synchronous: `out` is complete on return.  (In CROP mode without a cloud transform the
+ * kernel of this call stores the points straight into the page-locked destination, so the transfer to the host
+ * runs while the kernel does instead of as a copy behind it: tuning key "direct_out".) */
 int d2pc_process_mono8(d2pc_ctx *ctx, const uint8_t *data, uint32_t width, uint32_t height, uint32_t step,
                        d2pc_cloud *out);
 
@@ -405,6 +454,18 @@ int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_fr
  * n_max*16 < 2^32, no overlap of input and output; batches of more than 2^31 - 2 points run in chunks of frames. */
 int d2pc_crop_box_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
                          const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride, uint32_t *d_out_counts);
+
+/* The cloud transform alone, on clouds already on the device, with the argument rules of d2pc_crop_box_device except:
+ *   - d_transforms NULL applies the context's d2pc_cloud_transform, which must be enabled; otherwise frame f uses
+ *     the 12 device floats at d_transforms + 12*f (row-major 3x4 [A | t], finiteness not checked), whatever the
+ *     context's setting;
+ *   - d_out_counts may be NULL; otherwise d_out_counts[f] = frame f's input count (clamped to n_max);
+ *   - the output may be the input exactly (d_out == d_in and out_stride == in_stride, in place, as
+ *     pcl::transformPointCloud(c, c, T) allows); any other overlap is D2PC_ERR_INVALID_ARG.
+ * Positions at or past a frame's count are neither read nor written. */
+int d2pc_cloud_transform_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
+                                size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
+                                uint32_t *d_out_counts, const float *d_transforms);
 
 /* cv::medianBlur on CV_8UC1, replicate border (cpp:55-57 with ksize 11,
  * depth_map_fusion.cpp:124 with ksize 3).  ksize odd, 3..15. */

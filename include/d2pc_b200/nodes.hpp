@@ -49,11 +49,18 @@ class Bus {
     return it == remaps_.end() ? name : it->second;
   }
   void set_param(const std::string &name, double v) { params_[name] = v; }
+  void set_param(const std::string &name, const std::string &v) { str_params_[name] = v; }
   template <typename T>
   bool get_param(const std::string &name, T &out) const {
     auto it = params_.find(name);
     if (it == params_.end()) return false;
     out = static_cast<T>(it->second);
+    return true;
+  }
+  bool get_param(const std::string &name, std::string &out) const {
+    auto it = str_params_.find(name);
+    if (it == str_params_.end()) return false;
+    out = it->second;
     return true;
   }
   template <typename T>
@@ -98,7 +105,8 @@ class Bus {
     return it != image_subs_.end() && !it->second.empty();
   }
 
-  // Reads <remap from= to=/> and <param name= value=/> out of a roslaunch file (launch/*.launch).
+  // Reads <remap from= to=/> and <param name= value=/> out of a roslaunch file (launch/*.launch).  A value that
+  // std::stod reads as a whole (surrounding blanks aside) is a number; any other value is kept as a string.
   bool load_launch_file(const std::string &path) {
     std::ifstream in(path);
     if (!in) return false;
@@ -115,12 +123,26 @@ class Bus {
       if ((*it)[1] == "remap")
         remap(attr(tag, "from"), attr(tag, "to"));
       else
-        set_param(attr(tag, "name"), std::stod(attr(tag, "value")));
+        set_launch_param(attr(tag, "name"), attr(tag, "value"));
     }
     return true;
   }
 
  private:
+  void set_launch_param(const std::string &name, const std::string &value) {
+    size_t used = 0;
+    double v = 0.0;
+    try {
+      v = std::stod(value, &used);
+    } catch (const std::logic_error &) {  // invalid_argument (no number) or out_of_range
+      used = 0;
+    }
+    if (used && value.find_first_not_of(" \t\r\n", used) == std::string::npos)
+      set_param(name, v);
+    else
+      set_param(name, value);
+  }
+
   template <typename Cb>
   struct Sub {
     uint32_t queue_size;
@@ -128,6 +150,7 @@ class Bus {
   };
   std::map<std::string, std::string> remaps_;
   std::map<std::string, double> params_;
+  std::map<std::string, std::string> str_params_;
   std::map<std::string, std::vector<Sub<ImageCb>>> image_subs_;
   std::map<std::string, std::vector<Sub<CloudCb>>> cloud_subs_;
   std::map<std::string, sensor_msgs::PointCloud2> latched_clouds_;
@@ -140,10 +163,9 @@ inline void check(int status, const char *what, const d2pc_ctx *ctx = nullptr) {
                              (ctx ? std::string(" [") + d2pc_last_cuda_error(ctx) + "]" : std::string()));
 }
 
-// cv_bridge::toCvCopy(*msg, "mono8") for the encodings this library accepts.
-// [R | t] of the crop box params, row-major 3x4 in float: R = Rz(yaw) Ry(pitch) Rx(roll) evaluated in double,
-// pose = {tx, ty, tz, roll, pitch, yaw}.
-inline void crop_box_transform(const double pose[6], float out[12]) {
+// [R | t] of a pose param set (the crop box's and the cloud transform's), row-major 3x4 in float:
+// R = Rz(yaw) Ry(pitch) Rx(roll) evaluated in double, pose = {tx, ty, tz, roll, pitch, yaw}.
+inline void pose_matrix(const double pose[6], float out[12]) {
   const double cr = std::cos(pose[3]), sr = std::sin(pose[3]), cp = std::cos(pose[4]), sp = std::sin(pose[4]);
   const double cy = std::cos(pose[5]), sy = std::sin(pose[5]);
   const double R[3][3] = {{cy * cp, cy * sp * sr - sy * cr, cy * sp * cr + sy * sr},
@@ -155,6 +177,15 @@ inline void crop_box_transform(const double pose[6], float out[12]) {
   }
 }
 
+// the six pose params <prefix>{tx,ty,tz,roll,pitch,yaw} (default 0) as a float [R | t]
+inline void pose_param(const Bus &nh, const std::string &prefix, float out[12]) {
+  const char *names[6] = {"tx", "ty", "tz", "roll", "pitch", "yaw"};
+  double pose[6];
+  for (int k = 0; k < 6; ++k) nh.param<double>(prefix + names[k], pose[k], 0.0);
+  pose_matrix(pose, out);
+}
+
+// cv_bridge::toCvCopy(*msg, "mono8") for the encodings this library accepts.
 inline void require_mono8(const sensor_msgs::Image &msg) {
   if (msg.encoding != "mono8" && msg.encoding != "8UC1")
     throw std::invalid_argument("unsupported image encoding '" + msg.encoding + "' (mono8 / 8UC1 only)");
@@ -187,6 +218,7 @@ class Disparity2PCloud {
   sensor_msgs::PointCloud2 output_;
   uint8_t *registered_ = nullptr;
   int border_ = 40;  // cpp:70,72
+  std::string frame_id_ = "/camera_optical_frame";  // cpp:89; transform_target_frame with the transform on
 
   // make output_.data hold `bytes` bytes in page-locked storage without touching bytes it already has
   void reserve_output(size_t bytes) {
@@ -253,8 +285,8 @@ class Disparity2PCloud {
     // optional, not in the reference: pcl::CropBox on the device in front of VOXEL and the outlier stage, on when
     // crop_box_enable != 0.  The box is crop_box_{min,max}_{x,y,z} in a frame given by a translation and
     // roll / pitch / yaw (crop_box_{tx,ty,tz,roll,pitch,yaw}, radians): this node builds R = Rz(yaw) Ry(pitch) Rx(roll)
-    // in double and rounds [R | t] to the library's float matrix.  That conversion is the node's own; the points are
-    // not moved, so the cloud keeps its frame_id.
+    // in double and rounds [R | t] to the library's float matrix.  That conversion is the node's own; the box moves
+    // no point, so it leaves the frame_id alone.
     int box_on = 0;
     nh_.param<int>("crop_box_enable", box_on, 0);
     if (box_on) {
@@ -268,12 +300,22 @@ class Disparity2PCloud {
         nh_.param<double>(std::string("crop_box_max_") + axes[a], hi, 1.0);
         b.min_pt[a] = static_cast<float>(lo), b.max_pt[a] = static_cast<float>(hi);
       }
-      double pose[6];  // tx, ty, tz, roll, pitch, yaw
-      const char *names[6] = {"crop_box_tx", "crop_box_ty", "crop_box_tz", "crop_box_roll", "crop_box_pitch",
-                              "crop_box_yaw"};
-      for (int k = 0; k < 6; ++k) nh_.param<double>(names[k], pose[k], 0.0);
-      d2pc_b200::crop_box_transform(pose, b.transform);
+      d2pc_b200::pose_param(nh_, "crop_box_", b.transform);
       d2pc_b200::check(d2pc_set_crop_box(ctx_, &b), "d2pc_set_crop_box", ctx_);
+    }
+    // optional, not in the reference: pcl_ros::transformPointCloud on the device as the first cloud stage, on when
+    // transform_enable != 0.  transform_{tx,ty,tz,roll,pitch,yaw} is the static camera -> target transform (say a
+    // camera -> body extrinsic), built like the crop box's pose; the crop box then lies in the target frame, and
+    // the published frame_id is transform_target_frame, as pcl_ros::transformPointCloud sets it.
+    int xform_on = 0;
+    nh_.param<int>("transform_enable", xform_on, 0);
+    if (xform_on) {
+      d2pc_cloud_transform t;
+      d2pc_cloud_transform_default(&t);
+      t.enabled = 1;
+      d2pc_b200::pose_param(nh_, "transform_", t.matrix);
+      d2pc_b200::check(d2pc_set_cloud_transform(ctx_, &t), "d2pc_set_cloud_transform", ctx_);
+      nh_.param<std::string>("transform_target_frame", frame_id_, "base_link");
     }
   }
   ~Disparity2PCloud() {
@@ -317,7 +359,7 @@ class Disparity2PCloud {
     // the storage
     output.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
     output.header.stamp = msg->header.stamp;             // cpp:87
-    output.header.frame_id = "/camera_optical_frame";    // cpp:89
+    output.header.frame_id = frame_id_;                  // cpp:89
     nh_.publish(p_cloud_topic_, output);                 // cpp:90
   }
 };

@@ -17,6 +17,27 @@
 
 namespace {
 
+// The six pose params <prefix>{tx,ty,tz,roll,pitch,yaw} (default 0) as the library's float [R | t]:
+// R = Rz(yaw) Ry(pitch) Rx(roll) in double, rounded with t (the node mirror's pose_param, include/d2pc_b200/nodes.hpp).
+void pose_param(ros::NodeHandle &nh, const std::string &prefix, float out[12]) {
+  double t[3], rpy[3];
+  nh.param<double>(prefix + "tx", t[0], 0.0);
+  nh.param<double>(prefix + "ty", t[1], 0.0);
+  nh.param<double>(prefix + "tz", t[2], 0.0);
+  nh.param<double>(prefix + "roll", rpy[0], 0.0);
+  nh.param<double>(prefix + "pitch", rpy[1], 0.0);
+  nh.param<double>(prefix + "yaw", rpy[2], 0.0);
+  const double cr = std::cos(rpy[0]), sr = std::sin(rpy[0]), cp = std::cos(rpy[1]), sp = std::sin(rpy[1]);
+  const double cy = std::cos(rpy[2]), sy = std::sin(rpy[2]);
+  const double R[3][3] = {{cy * cp, cy * sp * sr - sy * cr, cy * sp * cr + sy * sr},
+                          {sy * cp, sy * sp * sr + cy * cr, sy * sp * cr - cy * sr},
+                          {-sp, cp * sr, cp * cr}};
+  for (int i = 0; i < 3; ++i) {
+    for (int j = 0; j < 3; ++j) out[4 * i + j] = static_cast<float>(R[i][j]);
+    out[4 * i + 3] = static_cast<float>(t[i]);
+  }
+}
+
 class Disparity2PCloudGpu {
  public:
   Disparity2PCloudGpu() : nh_("~") {
@@ -72,8 +93,7 @@ class Disparity2PCloudGpu {
       }
     }
     // optional, not in the reference: pcl::CropBox on the device in front of VOXEL and the outlier stage, on when
-    // crop_box_enable != 0; R = Rz(yaw) Ry(pitch) Rx(roll) in double, rounded with t to the library's float [R | t]
-    // (the node mirror's conversion, include/d2pc_b200/nodes.hpp).  The points are not moved: frame_id stays.
+    // crop_box_enable != 0; its pose is crop_box_{tx,ty,tz,roll,pitch,yaw} (pose_param).  The box moves no point.
     int box_on = 0;
     nh_.param<int>("crop_box_enable", box_on, 0);
     if (box_on) {
@@ -87,24 +107,26 @@ class Disparity2PCloudGpu {
         nh_.param<double>(std::string("crop_box_max_") + axes[a], hi, 1.0);
         b.min_pt[a] = static_cast<float>(lo), b.max_pt[a] = static_cast<float>(hi);
       }
-      double t[3], rpy[3];
-      nh_.param<double>("crop_box_tx", t[0], 0.0);
-      nh_.param<double>("crop_box_ty", t[1], 0.0);
-      nh_.param<double>("crop_box_tz", t[2], 0.0);
-      nh_.param<double>("crop_box_roll", rpy[0], 0.0);
-      nh_.param<double>("crop_box_pitch", rpy[1], 0.0);
-      nh_.param<double>("crop_box_yaw", rpy[2], 0.0);
-      const double cr = std::cos(rpy[0]), sr = std::sin(rpy[0]), cp = std::cos(rpy[1]), sp = std::sin(rpy[1]);
-      const double cy = std::cos(rpy[2]), sy = std::sin(rpy[2]);
-      const double R[3][3] = {{cy * cp, cy * sp * sr - sy * cr, cy * sp * cr + sy * sr},
-                              {sy * cp, sy * sp * sr + cy * cr, sy * sp * cr - cy * sr},
-                              {-sp, cp * sr, cp * cr}};
-      for (int i = 0; i < 3; ++i) {
-        for (int j = 0; j < 3; ++j) b.transform[4 * i + j] = static_cast<float>(R[i][j]);
-        b.transform[4 * i + 3] = static_cast<float>(t[i]);
-      }
+      pose_param(nh_, "crop_box_", b.transform);
       if (d2pc_set_crop_box(ctx_, &b) != D2PC_OK) {
         ROS_FATAL("crop_box_*: not a valid crop box (min above max, or a non-finite bound or pose)");
+        ros::shutdown();
+      }
+    }
+    // optional, not in the reference: pcl_ros::transformPointCloud on the device as the first cloud stage, on when
+    // transform_enable != 0.  transform_{tx,ty,tz,roll,pitch,yaw} is a static camera -> target transform (such as a
+    // camera -> body extrinsic; no tf lookup); the crop box then lies in the target frame and the published frame_id
+    // is transform_target_frame, as pcl_ros::transformPointCloud sets it.
+    int xform_on = 0;
+    nh_.param<int>("transform_enable", xform_on, 0);
+    if (xform_on) {
+      d2pc_cloud_transform t;
+      d2pc_cloud_transform_default(&t);
+      t.enabled = 1;
+      pose_param(nh_, "transform_", t.matrix);
+      nh_.param<std::string>("transform_target_frame", frame_id_, "base_link");
+      if (d2pc_set_cloud_transform(ctx_, &t) != D2PC_OK) {
+        ROS_FATAL("transform_*: not a valid transform (a non-finite pose)");
         ros::shutdown();
       }
     }
@@ -158,7 +180,7 @@ class Disparity2PCloudGpu {
     out.is_dense = cloud.is_dense;
     out.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
     out.header.stamp = msg->header.stamp;
-    out.header.frame_id = "/camera_optical_frame";
+    out.header.frame_id = frame_id_;
     pub_.publish(out);
   }
 
@@ -170,6 +192,7 @@ class Disparity2PCloudGpu {
   sensor_msgs::PointCloud2 out_;   // persistent so that its data storage can stay page-locked
   uint8_t *registered_ = nullptr;
   int border_ = 40;
+  std::string frame_id_ = "/camera_optical_frame";  // transform_target_frame with the transform on
 };
 
 }  // namespace

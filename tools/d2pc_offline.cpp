@@ -2,6 +2,9 @@
 //
 //   d2pc_offline wire   <out.bin>
 //       CPU only: serialises a small hand-made PointCloud2 and Image with ros_lite (self-test of the wire code).
+//   d2pc_offline params <launch file> <name>...
+//       CPU only: loads the launch file into a Bus and prints one line per name: "<name> number <value>" (%.17g),
+//       "<name> string <value>" or "<name> missing" (the launch-file loader's number / string rule).
 //   d2pc_offline node1  <launch file> <w> <h> <in.raw> <out.bin> [sec nsec]
 //       BASELINE config 1/2 shape: one mono8 frame published on the node's (remapped) input topic; the
 //       PointCloud2 received on the (remapped) output topic is written in ROS1 wire format.
@@ -72,6 +75,21 @@ int main(int argc, char **argv) {
       auto im2 = ros_lite::deserialize_image(ib.data(), ib.size());
       if (ros_lite::serialize(im2) != ib || im2.encoding != "mono8") throw std::runtime_error("Image round trip differs");
       write_file(argv[2], bytes);
+      return 0;
+    }
+    if (mode == "params" && argc >= 3) {
+      d2pc_b200::Bus bus;
+      if (!bus.load_launch_file(argv[2])) throw std::runtime_error(std::string("cannot read ") + argv[2]);
+      for (int i = 3; i < argc; ++i) {
+        double v = 0.0;
+        std::string str;
+        if (bus.get_param(argv[i], v))
+          std::printf("%s number %.17g\n", argv[i], v);
+        else if (bus.get_param(argv[i], str))
+          std::printf("%s string %s\n", argv[i], str.c_str());
+        else
+          std::printf("%s missing\n", argv[i]);
+      }
       return 0;
     }
     if (mode == "node1" && argc >= 7) {
