@@ -132,7 +132,7 @@ struct d2pc_ctx {
   // tuning / test hooks
   int rows_per_unit = 0, ctas_per_sm = 0, median_strip = 0, median_variant = 0;
   bool force_scalar = false, force_generic = false;
-  int compact_variant = 0, exact_variant = 0, prefetch_dist = 0, zero_numer = 0;
+  int compact_variant = 0, exact_variant = 0, prefetch_dist = 0, zero_numer = 0, crop_load = 0, crop_probe = 0;
   int fuse_median = 0;  // mono8 callback as one fused launch where possible: 0 yes, -1 never (two launches)
   // CROP clouds written by the kernel straight into the page-locked host buffer (no D2H copy after the kernel; the
   // transfer overlaps the kernel): 0 = the synchronous single-frame mono8 entries only (the median makes that
@@ -509,6 +509,8 @@ int enqueue_reproject(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, S
   L.exact_variant = ctx->exact_variant;
   L.zero_numer = ctx->zero_numer;
   L.prefetch_dist = ctx->prefetch_dist;
+  L.crop_load = ctx->crop_load;
+  L.crop_probe = ctx->crop_probe != 0;
   if (!in.is_f32 && c.median_ksize > 1) {
     // cpp:55-57: only crop pixels are consumed downstream, so only those medians are produced
     // (the replicate border is still the image edge, which matters when border < ksize/2).
@@ -842,6 +844,7 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
 
   if (const char *v = getenv("D2PC_ROWS_PER_UNIT")) ctx->rows_per_unit = atoi(v);
   if (const char *v = getenv("D2PC_CTAS_PER_SM")) ctx->ctas_per_sm = atoi(v);
+  if (const char *v = getenv("D2PC_CROP_LOAD")) ctx->crop_load = atoi(v);
   if (const char *v = getenv("D2PC_MEDIAN_STRIP")) ctx->median_strip = atoi(v);
   if (const char *v = getenv("D2PC_EXACT_VARIANT")) ctx->exact_variant = atoi(v);
 
@@ -1008,6 +1011,8 @@ int d2pc_set_tuning(d2pc_ctx *ctx, const char *key, int value) {
   else if (k == "fuse_median") ctx->fuse_median = value;
   else if (k == "direct_out") ctx->direct_out = value;
   else if (k == "prefetch_dist") ctx->prefetch_dist = value;
+  else if (k == "crop_load") ctx->crop_load = value;
+  else if (k == "crop_probe") ctx->crop_probe = value;
   else if (k == "median_ksize") {
     if (value < 1 || value > 15 || !(value & 1)) return D2PC_ERR_INVALID_ARG;
     ctx->cfg.median_ksize = value;

@@ -28,6 +28,9 @@
 //   their measurements are kept in DESIGN.md.)
 #include "reproject.h"
 
+#include <cuda.h>
+#include <cudaTypedefs.h>
+
 #include <algorithm>
 #include <cmath>
 
@@ -62,6 +65,8 @@ __device__ __forceinline__ uint32_t fastdiv(uint32_t n, FastDiv f) {
 }
 
 struct ReprojArgs {
+  CUtensorMap tmap;  // CROP kernel, TMA form: crop columns x crop rows x frames of the input
+  bool tma;
   const uint8_t *in;
   size_t step, frame_stride;
   float4 *out;
@@ -86,7 +91,9 @@ struct ReprojArgs {
 // M: Markstein quotients.  Z: kMathRect0 for a calibration whose principal point column is an image column (X is
 // exactly 0 there): zero numerators stay on the straight-line path instead of taking the exact function -- 4-25 %
 // faster for such a Q, 2-4 % slower for any other (a few more instructions per pixel), hence chosen on the host.
-enum { kMathRect0 = 0, kMathRectW = 1, kMathGeneric = 2, kMathFast = 3, kMathRect0M = 4, kMathRect0Z = 5 };
+// Probe: no arithmetic, the CROP kernels store {d, d, d, 1} -- the traffic of the reprojection alone (test hook that
+// measures the memory ceiling of the CROP kernels' access pattern).
+enum { kMathRect0 = 0, kMathRectW = 1, kMathGeneric = 2, kMathFast = 3, kMathRect0M = 4, kMathRect0Z = 5, kMathProbe = 6 };
 #define D2PC_IS_RECT(m) ((m) == kMathRect0 || (m) == kMathRectW || (m) == kMathRect0M || (m) == kMathRect0Z)
 #define D2PC_IS_GUARD(m) ((m) == kMathRect0 || (m) == kMathRect0Z)
 
@@ -199,6 +206,9 @@ __device__ __forceinline__ void points_of4(const QParams &Q, const double (&xd)[
       for (int k = 0; k < 4; ++k)
         if (slow[k]) p[k] = reproject_exact_slow(Q.q, u0 + 32 * k, v, d[k]);
     }
+  } else if constexpr (kMath == kMathProbe) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) p[k] = make_float4(d[k], d[k], d[k], 1.0f);
   } else {
 #pragma unroll
     for (int k = 0; k < 4; ++k) p[k] = reproject_fast(Q.qf, u0 + 32 * k, v, d[k]);
@@ -268,22 +278,101 @@ __device__ __forceinline__ float4 point_of(const QParams &Q, int u, int v, float
 }
 
 // ---------------------------------------------------------------------------
-// CROP kernel
+// CROP kernels
 // ---------------------------------------------------------------------------
+// What both CROP kernels (LDG rows below, TMA boxes further down) hold per work unit: column constants live in
+// registers for the whole unit; row constants are computed by one lane per row and broadcast by shuffle.
+template <int kMath>
+struct CropCols {
+  double xd[4];
+  uint32_t xslow;
+  double yd_lane;  // row constant of crop row r_base + lane
+  double gcx[kMath == kMathGeneric ? 4 : 1][4];  // generic exact path: q[4i] * u of each of the lane's columns
+};
+
+template <int kMath>
+__device__ __forceinline__ void crop_cols_init(CropCols<kMath> &c, const ReprojArgs &a, int c_base, int r_base,
+                                               int lane) {
+  const QParams &Q = a.Q;
+  c.xslow = 0;
+  c.yd_lane = 0.0;
+  if constexpr (D2PC_IS_RECT(kMath)) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      c.xd[k] = rect_axis_const(a.border + c_base + 32 * k + lane, Q.q03);
+      c.xslow |= rect_axis_slow_t<kMath == kMathRect0Z>(c.xd[k]) ? (1u << k) : 0u;
+      if constexpr (kMath == kMathRect0Z) c.xslow |= rect_axis_zero(c.xd[k]) ? (16u << k) : 0u;
+    }
+    if (Q.zd_slow) c.xslow = 0xfu;
+    c.yd_lane = rect_axis_const(a.border + r_base + lane, Q.q13);
+  } else {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) c.xd[k] = 0.0;
+  }
+  if constexpr (kMath == kMathGeneric) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      const double du = (double)(a.border + c_base + 32 * k + lane);
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        c.gcx[k][i] = __dmul_rn(Q.q[4 * i], du);
+        asm volatile("" : "+d"(c.gcx[k][i]));  // keep the products in registers: ptxas would recompute them per pixel
+      }
+    }
+  }
+}
+
+// The four points of crop row r_base + r of the unit, lane L owning columns L, L+32, L+64, L+96.
+template <int kMath>
+__device__ __forceinline__ void crop_row_points(const ReprojArgs &a, const CropCols<kMath> &c, int c_base, int r_base,
+                                                int r, int lane, const float (&d)[4], float4 (&p)[4]) {
+  const QParams &Q = a.Q;
+  double yd = 0.0;
+  uint32_t yslow = 0;
+  if constexpr (D2PC_IS_RECT(kMath)) {
+    yd = __shfl_sync(0xffffffffu, c.yd_lane, r);
+    yslow = rect_axis_slow_t<kMath == kMathRect0Z>(yd) ? 1u : 0u;
+    if constexpr (kMath == kMathRect0Z) yslow |= rect_axis_zero(yd) ? 2u : 0u;
+  }
+  if constexpr (kMath == kMathGeneric) {
+    const int v = a.border + r_base + r, u0 = a.border + c_base + lane;
+    const double dv = (double)v;
+    double gry[4];
+#pragma unroll
+    for (int i = 0; i < 4; ++i) gry[i] = __dmul_rn(Q.q[4 * i + 1], dv);
+    bool slow[4];
+#pragma unroll
+    for (int k = 0; k < 4; ++k) p[k] = reproject_exact_generic_hoisted(Q.q, c.gcx[k], gry, d[k], slow[k]);
+    if (__builtin_expect(slow[0] || slow[1] || slow[2] || slow[3], 0)) {
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        if (slow[k]) p[k] = reproject_exact_slow(Q.q, u0 + 32 * k, v, d[k]);
+    }
+  } else {
+    points_of4<kMath>(Q, c.xd, yd, c.xslow, yslow, a.border + c_base + lane, a.border + r_base + r, d, p);
+  }
+}
+
+// Unit -> (frame, row block, segment) of the CROP kernels.
+__device__ __forceinline__ void crop_unit(const ReprojArgs &a, uint32_t unit, uint32_t &f, int &rb, int &seg) {
+  f = fastdiv(unit, a.div_upf);
+  const uint32_t rem = unit - f * a.units_per_frame;
+  rb = (int)fastdiv(rem, a.div_nseg);
+  seg = (int)rem - rb * a.n_seg;
+}
+
 template <typename InT, bool kVec, int kMath, int kMinBlocks>
 __global__ void __launch_bounds__(kThreads, kMinBlocks) reproject_crop_kernel(const __grid_constant__ ReprojArgs a) {
   __shared__ __align__(16) float stage[kWarpsPerCta][2][kSegCols];
   const int lane = threadIdx.x & 31;
   const int wic = threadIdx.x >> 5;
-  const QParams &Q = a.Q;
 
   // one work unit (128 crop columns x rows_per_unit crop rows) per warp; the hardware CTA scheduler balances
   const uint32_t unit = blockIdx.x * kWarpsPerCta + wic;
   if (unit >= a.total_units) return;
-  const uint32_t f = fastdiv(unit, a.div_upf);
-  const uint32_t rem = unit - f * a.units_per_frame;
-  const int rb = (int)fastdiv(rem, a.div_nseg);
-  const int seg = rem - rb * a.n_seg;
+  uint32_t f;
+  int rb, seg;
+  crop_unit(a, unit, f, rb, seg);
   const int c_base = seg * kSegCols;
   const int r_base = rb * a.rows_per_unit;
   const int rows = min(a.rows_per_unit, a.ch - r_base);
@@ -293,9 +382,9 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) reproject_crop_kernel(co
     if (a.prefetch_dist > 0 && lane < a.rows_per_unit) {
       const uint32_t u2 = unit + (uint32_t)a.prefetch_dist;  // total_units < 2^31 and the distance is clamped: no wrap
       if (u2 < a.total_units) {
-        const uint32_t f2 = fastdiv(u2, a.div_upf);
-        const uint32_t rem2 = u2 - f2 * a.units_per_frame;
-        const int rb2 = (int)fastdiv(rem2, a.div_nseg), seg2 = rem2 - rb2 * a.n_seg;
+        uint32_t f2;
+        int rb2, seg2;
+        crop_unit(a, u2, f2, rb2, seg2);
         const int row2 = rb2 * a.rows_per_unit + lane;
         const int cols2 = min(kSegCols, ((a.cw - seg2 * kSegCols) + 3) & ~3);
         if (row2 < a.ch)
@@ -308,36 +397,8 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) reproject_crop_kernel(co
     }
   }
 
-  // column constants live in registers for the whole unit; row constants are computed by one lane per row
-  double xd[4];
-  uint32_t xslow = 0;
-  double yd_lane = 0.0;
-  if constexpr (D2PC_IS_RECT(kMath)) {
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      xd[k] = rect_axis_const(a.border + c_base + 32 * k + lane, Q.q03);
-      xslow |= rect_axis_slow_t<kMath == kMathRect0Z>(xd[k]) ? (1u << k) : 0u;
-      if constexpr (kMath == kMathRect0Z) xslow |= rect_axis_zero(xd[k]) ? (16u << k) : 0u;
-    }
-    if (Q.zd_slow) xslow = 0xfu;
-    yd_lane = rect_axis_const(a.border + r_base + lane, Q.q13);
-  } else {
-#pragma unroll
-    for (int k = 0; k < 4; ++k) xd[k] = 0.0;
-  }
-  // generic exact path: the four products q[4i] * u of each of the lane's four columns, for the whole unit
-  double gcx[kMath == kMathGeneric ? 4 : 1][4];
-  if constexpr (kMath == kMathGeneric) {
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const double du = (double)(a.border + c_base + 32 * k + lane);
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        gcx[k][i] = __dmul_rn(Q.q[4 * i], du);
-        asm volatile("" : "+d"(gcx[k][i]));  // keep the products in registers: ptxas would recompute them per pixel
-      }
-    }
-  }
+  CropCols<kMath> cols;
+  crop_cols_init(cols, a, c_base, r_base, lane);
 
   const uint8_t *in_row = a.in + (size_t)f * a.frame_stride + (size_t)(a.border + r_base) * a.step;
   float4 *out_row = a.out + (size_t)f * a.out_frame_stride + (size_t)r_base * a.cw;
@@ -374,31 +435,8 @@ __global__ void __launch_bounds__(kThreads, kMinBlocks) reproject_crop_kernel(co
 #pragma unroll
     for (int j = 0; j < 2; ++j) {
       if (r + j >= rows) break;
-      double yd = 0.0;
-      uint32_t yslow = 0;
-      if constexpr (D2PC_IS_RECT(kMath)) {
-        yd = __shfl_sync(0xffffffffu, yd_lane, r + j);
-        yslow = rect_axis_slow_t<kMath == kMathRect0Z>(yd) ? 1u : 0u;
-        if constexpr (kMath == kMathRect0Z) yslow |= rect_axis_zero(yd) ? 2u : 0u;
-      }
       float4 p[4];
-      if constexpr (kMath == kMathGeneric) {
-        const int v = a.border + r_base + r + j, u0 = a.border + c_base + lane;
-        const double dv = (double)v;
-        double gry[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) gry[i] = __dmul_rn(Q.q[4 * i + 1], dv);
-        bool slow[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) p[k] = reproject_exact_generic_hoisted(Q.q, gcx[k], gry, dd[j][k], slow[k]);
-        if (__builtin_expect(slow[0] || slow[1] || slow[2] || slow[3], 0)) {
-#pragma unroll
-          for (int k = 0; k < 4; ++k)
-            if (slow[k]) p[k] = reproject_exact_slow(Q.q, u0 + 32 * k, v, dd[j][k]);
-        }
-      } else {
-        points_of4<kMath>(Q, xd, yd, xslow, yslow, a.border + c_base + lane, a.border + r_base + r + j, dd[j], p);
-      }
+      crop_row_points<kMath>(a, cols, c_base, r_base, r + j, lane, dd[j], p);
       float4 *o = out_row + (size_t)j * a.cw + c_base + lane;
 #pragma unroll
       for (int k = 0; k < 4; ++k)
@@ -953,6 +991,92 @@ __global__ void __launch_bounds__(kW * 32, kMinB) reproject_compact_band_kernel(
 }
 
 
+// ---------------------------------------------------------------------------
+// CROP kernel, TMA form (aligned float rows, kR = 4 / 6 / 8 rows per unit)
+// ---------------------------------------------------------------------------
+// Same work units and 512-byte point stores as reproject_crop_kernel.  One lane per warp loads the unit's whole
+// 128 x kR box into shared memory with one cp.async.bulk.tensor over a 3-D map (crop columns x crop rows x frames,
+// encoded on the host, zero-filled past the crop edge) and issues one cp.async.bulk.prefetch.tensor.L2 for the
+// unit prefetch_dist ahead.  Lanes then read their strided columns straight from the box: no per-row load,
+// transpose or __syncwarp.  Full units (all but the last segment of a row and the last row block of a frame) run
+// without row or column tests.
+template <int kMath, int kMinBlocks, int kR>
+__global__ void __launch_bounds__(kThreads, kMinBlocks) reproject_crop_tma_kernel(const __grid_constant__ ReprojArgs a) {
+  __shared__ __align__(128) float box[kWarpsPerCta][kR * kSegCols];
+  __shared__ __align__(8) unsigned long long bar[kWarpsPerCta];
+  const int lane = threadIdx.x & 31;
+  const int wic = threadIdx.x >> 5;
+  const uint32_t unit = blockIdx.x * kWarpsPerCta + wic;
+  if (unit >= a.total_units) return;
+  uint32_t f;
+  int rb, seg;
+  crop_unit(a, unit, f, rb, seg);
+  const int c_base = seg * kSegCols;
+  const int r_base = rb * kR;
+  const uint64_t tmap = reinterpret_cast<uint64_t>(&a.tmap);
+  if (lane == 0) {
+    mbar_init(&bar[wic], 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    mbar_arrive_expect_tx(&bar[wic], kR * kSegCols * 4);  // out-of-bounds elements count too (zero-filled)
+    asm volatile(
+        "cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], "
+        "[%5];" ::"r"(smem_u32(box[wic])),
+        "l"(tmap), "r"(c_base), "r"(r_base), "r"((int)f), "r"(smem_u32(&bar[wic]))
+        : "memory");
+    const uint32_t u2 = unit + (uint32_t)a.prefetch_dist;  // total_units < 2^31 and the distance is clamped: no wrap
+    if (a.prefetch_dist > 0 && u2 < a.total_units) {
+      uint32_t f2;
+      int rb2, seg2;
+      crop_unit(a, u2, f2, rb2, seg2);
+      asm volatile("cp.async.bulk.prefetch.tensor.3d.L2.global.tile [%0, {%1, %2, %3}];" ::"l"(tmap),
+                   "r"(seg2 * kSegCols), "r"(rb2 * kR), "r"((int)f2)
+                   : "memory");
+    }
+  }
+  CropCols<kMath> cols;
+  crop_cols_init(cols, a, c_base, r_base, lane);
+  __syncwarp();  // the barrier is initialised before any lane waits on it
+  mbar_wait(&bar[wic], 0);
+
+  const float *bx = box[wic] + lane;
+  // one 64-bit frame base, 32-bit offsets inside the frame (cw * ch < 2^31 where this kernel runs)
+  float4 *o = a.out + (size_t)f * a.out_frame_stride + (uint32_t)(r_base * a.cw + c_base + lane);
+  if (r_base + kR <= a.ch && c_base + kSegCols <= a.cw) {
+#pragma unroll
+    for (int r = 0; r < kR; ++r, o += a.cw) {
+      float d[4];
+#pragma unroll
+      for (int k = 0; k < 4; ++k) d[k] = bx[r * kSegCols + 32 * k];
+      float4 p[4];
+      crop_row_points<kMath>(a, cols, c_base, r_base, r, lane, d, p);
+#pragma unroll
+      for (int k = 0; k < 4; ++k) st_stream_f4(o + 32 * k, p[k]);
+    }
+  } else {
+    const int rows = min(kR, a.ch - r_base);
+#pragma unroll 1
+    for (int r = 0; r < rows; ++r, o += a.cw) {
+      float d[4];
+#pragma unroll
+      for (int k = 0; k < 4; ++k) d[k] = bx[r * kSegCols + 32 * k];
+      float4 p[4];
+      crop_row_points<kMath>(a, cols, c_base, r_base, r, lane, d, p);
+#pragma unroll
+      for (int k = 0; k < 4; ++k)
+        if (c_base + 32 * k + lane < a.cw) st_stream_f4(o + 32 * k, p[k]);
+    }
+  }
+}
+
+template <int kMath, int kMinBlocks>
+void launch_crop_tma(const ReprojArgs &a, int grid, cudaStream_t s) {
+  switch (a.rows_per_unit) {
+    case 4: reproject_crop_tma_kernel<kMath, kMinBlocks, 4><<<grid, kThreads, 0, s>>>(a); break;
+    case 6: reproject_crop_tma_kernel<kMath, kMinBlocks, 6><<<grid, kThreads, 0, s>>>(a); break;
+    default: reproject_crop_tma_kernel<kMath, kMinBlocks, 8><<<grid, kThreads, 0, s>>>(a); break;
+  }
+}
+
 template <typename K>
 cudaError_t launch_compact(K kernel, const ReprojArgs &a, int grid, cudaStream_t s) {
   // 52 KB of dynamic shared memory needs the opt-in on every instantiation (and on every device)
@@ -964,7 +1088,19 @@ cudaError_t launch_compact(K kernel, const ReprojArgs &a, int grid, cudaStream_t
 
 template <typename InT, int kMath>
 cudaError_t launch_typed(const ReprojArgs &a, bool vec, bool compact, int grid, int min_blocks, cudaStream_t s) {
+  if constexpr (sizeof(InT) == 4) {
+    if (a.tma) {
+      switch (min_blocks) {
+        case 4: launch_crop_tma<kMath, 4>(a, grid, s); break;
+        case 6: launch_crop_tma<kMath, 6>(a, grid, s); break;
+        case 8: launch_crop_tma<kMath, 8>(a, grid, s); break;
+        default: launch_crop_tma<kMath, 7>(a, grid, s); break;
+      }
+      return cudaGetLastError();
+    }
+  }
   if (compact) {
+    if constexpr (kMath == kMathProbe) return cudaErrorInvalidValue;  // a CROP-kernel hook only
     if constexpr (D2PC_IS_GUARD(kMath)) {
       if (a.d_sure_bits != 0 && a.band_rows > 0) {  // band kernel
         constexpr bool kZN = kMath == kMathRect0Z;
@@ -980,8 +1116,9 @@ cudaError_t launch_typed(const ReprojArgs &a, bool vec, bool compact, int grid, 
         return cudaGetLastError();
       }
     }
-    return vec ? launch_compact(reproject_compact_kernel<InT, true, kMath>, a, grid, s)
-               : launch_compact(reproject_compact_kernel<InT, false, kMath>, a, grid, s);
+    if constexpr (kMath != kMathProbe)
+      return vec ? launch_compact(reproject_compact_kernel<InT, true, kMath>, a, grid, s)
+                 : launch_compact(reproject_compact_kernel<InT, false, kMath>, a, grid, s);
   } else if (vec) {
     switch (min_blocks) {  // 128-thread CTAs: 4 -> <=128 regs, 6 -> 80, 7 -> 72, 8 -> 64
       case 4: reproject_crop_kernel<InT, true, kMath, 4><<<grid, kThreads, 0, s>>>(a); break;
@@ -1077,6 +1214,29 @@ bool reproject_fuses_with_median(const ReprojectLaunch &L, bool *zero_numer) {
   return D2PC_IS_GUARD(math);
 }
 
+// 3-D tiled map of the crop region (columns x rows x frames, 4-byte elements) with a 128 x rows x 1 box.
+// cuTensorMapEncodeTiled comes through the runtime's driver entry point, so the library links no libcuda.
+static bool encode_crop_map(CUtensorMap *m, const ReprojectLaunch &L, long cw, long ch, int rows) {
+  static const PFN_cuTensorMapEncodeTiled_v12000 encode = [] {
+    void *fn = nullptr;
+    cudaDriverEntryPointQueryResult q;
+    return cudaGetDriverEntryPointByVersion("cuTensorMapEncodeTiled", &fn, 12000, cudaEnableDefault, &q) ==
+                       cudaSuccess &&
+                   q == cudaDriverEntryPointSuccess
+               ? reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(fn)
+               : nullptr;
+  }();
+  if (!encode) return false;
+  const cuuint64_t dims[3] = {(cuuint64_t)cw, (cuuint64_t)ch, (cuuint64_t)L.n_frames};
+  // a lone frame's stride is never stepped over; any valid one will do
+  const cuuint64_t strides[2] = {(cuuint64_t)L.step, L.n_frames > 1 ? (cuuint64_t)L.frame_stride : (cuuint64_t)L.step * ch};
+  const cuuint32_t box[3] = {(cuuint32_t)kSegCols, (cuuint32_t)rows, 1u}, elem[3] = {1u, 1u, 1u};
+  const uint8_t *base = static_cast<const uint8_t *>(L.in) + (size_t)L.border * L.step + (size_t)L.border * 4;
+  return encode(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<uint8_t *>(base), dims, strides, box, elem,
+                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+}
+
 cudaError_t launch_reproject(const ReprojectLaunch &L, cudaStream_t stream, int *launches) {
   const long cw = (long)L.width - 2L * L.border, ch = (long)L.height - 2L * L.border;
   if (launches) *launches = 0;
@@ -1112,7 +1272,7 @@ cudaError_t launch_reproject(const ReprojectLaunch &L, cudaStream_t stream, int 
                    (L.frame_stride % valign == 0) && ((size_t)L.border * esz % valign == 0) &&
                    (cw % 4 == 0 || L.border >= 3) && !L.force_scalar;
 
-  const int math = select_math(L);
+  int math = select_math(L);
   const bool compact = L.compact;
 
   int grid;
@@ -1186,8 +1346,11 @@ cudaError_t launch_reproject(const ReprojectLaunch &L, cudaStream_t stream, int 
       if (launches) *launches += 1;
     }
   } else {
-    // rows per unit: large units amortise the per-unit constants, small ones spread a lone frame over the chip
-    int rb = L.rows_per_unit > 0 ? L.rows_per_unit : 8;
+    // rows per unit: large units amortise the per-unit constants, small ones spread a lone frame over the chip.
+    // TMA boxes make a unit's fixed cost small enough that 4-row units win under the sustained power cap as well
+    // (4K x 16, 320 launches: 369 us against 375 at 8 rows; the per-row loads want 8: 381 against 390).
+    const bool tma_rows = vec && L.in_is_f32 && L.crop_load == 0;
+    int rb = L.rows_per_unit > 0 ? L.rows_per_unit : (tma_rows ? 4 : 8);
     const uint64_t want_units = (uint64_t)L.sm_count * 32;
     while (rb > 2 && (uint64_t)a.n_seg * ((ch + rb - 1) / rb) * L.n_frames < want_units) rb >>= 1;
     if (rb > 32) rb = 32;
@@ -1204,6 +1367,13 @@ cudaError_t launch_reproject(const ReprojectLaunch &L, cudaStream_t stream, int 
     grid = (int)((total + kWarpsPerCta - 1) / kWarpsPerCta);
     // L2 prefetch distance in units (~4100 units are in flight; measured plateau 256-2048)
     a.prefetch_dist = L.prefetch_dist < 0 ? 0 : (L.prefetch_dist > 0 ? std::min(L.prefetch_dist, 1 << 24) : 512);
+    // TMA box loads where the map can describe the rows (the LDG kernel serves every other case)
+    a.tma = tma_rows && (rb == 4 || rb == 6 || rb == 8) &&
+            (uint64_t)cw * (uint64_t)ch < (1ull << 31) && encode_crop_map(&a.tmap, L, cw, ch, rb);
+  }
+  if (L.crop_probe && !compact) {
+    if (!L.in_is_f32) return cudaErrorInvalidValue;
+    math = kMathProbe;
   }
   // the generic exact path keeps 16 column products in registers: 4 CTAs per SM (<= 128 registers).  The others:
   // 6 CTAs (80 registers) beat 7 (72, more spills) by 0.5 % in every sustained and burst A/B of round 2
@@ -1221,6 +1391,7 @@ cudaError_t launch_reproject(const ReprojectLaunch &L, cudaStream_t stream, int 
     default: return launch_typed<T, kMathFast>(a, vec, compact, grid, min_blocks, stream);    \
   }
   if (L.in_is_f32) {
+    if (math == kMathProbe) return launch_typed<float, kMathProbe>(a, vec, compact, grid, min_blocks, stream);
     D2PC_DISPATCH(float)
   } else {
     D2PC_DISPATCH(uint8_t)

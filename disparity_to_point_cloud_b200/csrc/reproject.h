@@ -51,6 +51,8 @@ struct ReprojectLaunch {
                                // 1 = park-then-compact for every Q (test hook for the fallback)
   int prefetch_dist = 0;       // L2 prefetch distance: CROP kernel in work units, band kernel in tiles
                                // (0 = automatic, < 0 = off)
+  int crop_load = 0;           // CROP kernel input: 0 = TMA boxes where the rows allow, 1 = per-row LDG always
+  bool crop_probe = false;     // CROP kernel stores {d, d, d, 1} without arithmetic (traffic probe, f32 only)
 };
 
 void make_qparams(const double q[16], QParams *out);

@@ -565,6 +565,9 @@ size_t d2pc_serialize_pointcloud2(const d2pc_ctx *ctx, const d2pc_cloud *cloud, 
  *             histogram for every size),
  *             "compact_variant" (0 auto: band kernel where Q allows; 1 park kernel for every Q),
  *             "prefetch_dist" (L2 prefetch distance in work units / tiles; 0 automatic, < 0 off),
+ *             "crop_load" (CROP kernel input: 0 TMA box loads where the rows allow, 1 per-row vector loads),
+ *             "crop_probe" (1: the CROP kernel stores {d, d, d, 1} instead of points -- a measurement hook that
+ *             moves the kernel's traffic without its arithmetic; float input only),
  *             "exact_variant" (0 guarded multiply, 1 Markstein), "zero_numer" (kernel variant that keeps an
  *             exactly-zero X numerator column straight-line: 0 when Q has such a column, 1 always, -1 never),
  *             "fuse_median" (mono8 callback: 0 one fused median + reproject launch where Q allows, -1 always two),
