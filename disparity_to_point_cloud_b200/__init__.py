@@ -85,6 +85,33 @@ class CloudTransform(C.Structure):
     _fields_ = [("struct_size", C.c_uint32), ("enabled", C.c_int32), ("matrix", C.c_float * 12)]
 
 
+class LaserScanParams(C.Structure):
+    """d2pc_laser_scan_params: pointcloud_to_laserscan's parameters of the scan output (and keep_cloud)."""
+    _fields_ = [("struct_size", C.c_uint32), ("enabled", C.c_int32), ("min_height", C.c_double),
+                ("max_height", C.c_double), ("angle_min", C.c_double), ("angle_max", C.c_double),
+                ("angle_increment", C.c_double), ("scan_time", C.c_double), ("range_min", C.c_double),
+                ("range_max", C.c_double), ("use_inf", C.c_int32), ("inf_epsilon", C.c_double),
+                ("keep_cloud", C.c_int32)]
+
+
+class LaserScan(C.Structure):
+    """d2pc_laser_scan: the message fields of a scan and its library-owned ranges."""
+    _fields_ = [("angle_min", C.c_float), ("angle_max", C.c_float), ("angle_increment", C.c_float),
+                ("time_increment", C.c_float), ("scan_time", C.c_float), ("range_min", C.c_float),
+                ("range_max", C.c_float), ("n_ranges", C.c_uint32), ("ranges", C.POINTER(C.c_float))]
+
+    FIELDS = ("angle_min", "angle_max", "angle_increment", "time_increment", "scan_time", "range_min", "range_max")
+
+    def fields(self) -> dict:
+        return {k: getattr(self, k) for k in self.FIELDS}
+
+    def ranges_array(self) -> np.ndarray:
+        """A copy of the ranges (float32)."""
+        if self.n_ranges == 0:
+            return np.empty(0, np.float32)
+        return np.ctypeslib.as_array(self.ranges, shape=(self.n_ranges,)).copy()
+
+
 class Timing(C.Structure):
     _fields_ = [("h2d_us", C.c_float), ("kernels_us", C.c_float), ("d2h_us", C.c_float), ("total_us", C.c_float),
                 ("points", C.c_uint64)]
@@ -130,6 +157,13 @@ SYMBOLS = [
     ("d2pc_get_cloud_transform", C.c_int, [_ctx, C.POINTER(CloudTransform)]),
     ("d2pc_cloud_transform_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
                                               C.c_void_p, C.c_size_t, C.c_void_p, C.c_void_p]),
+    ("d2pc_laser_scan_params_default", None, [C.POINTER(LaserScanParams)]),
+    ("d2pc_set_laser_scan", C.c_int, [_ctx, C.POINTER(LaserScanParams)]),
+    ("d2pc_get_laser_scan", C.c_int, [_ctx, C.POINTER(LaserScanParams)]),
+    ("d2pc_laser_scan_ranges", C.c_int, [C.POINTER(LaserScanParams), _u32p]),
+    ("d2pc_last_scan", C.c_int, [_ctx, C.POINTER(LaserScan)]),
+    ("d2pc_laser_scan_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
+                                         C.c_void_p, C.c_size_t]),
     ("d2pc_process_mono8", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_process_f32", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_submit_mono8", C.c_int, [_ctx, C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
@@ -182,6 +216,8 @@ SYMBOLS = [
                                              C.c_uint32, C.c_uint32, C.c_int, CLOUD_SINK, C.c_void_p]),
     ("d2pc_serialize_pointcloud2", C.c_size_t, [_ctx, C.POINTER(Cloud), C.c_uint32, C.c_uint32, C.c_uint32,
                                                 C.c_void_p, C.c_size_t]),
+    ("d2pc_serialize_laserscan", C.c_size_t, [_ctx, C.POINTER(LaserScan), C.c_uint32, C.c_uint32, C.c_uint32,
+                                              C.c_void_p, C.c_size_t]),
     ("d2pc_set_tuning", C.c_int, [_ctx, C.c_char_p, C.c_int]),
     ("d2pc_strerror", C.c_char_p, [C.c_int]),
     ("d2pc_last_cuda_error", C.c_char_p, [_ctx]),
@@ -228,6 +264,27 @@ def q_from_intrinsics(fx=714.24, fy=713.5, cx=376.0, cy=240.0, baseline=0.09, re
     if rc:
         raise D2pcError(rc, "d2pc_q_from_intrinsics")
     return q.reshape(4, 4)
+
+
+def laser_scan_params(**params) -> LaserScanParams:
+    """d2pc_laser_scan_params_default with `params` (any field of LaserScanParams) set on top; enabled defaults to 1."""
+    p = LaserScanParams()
+    lib().d2pc_laser_scan_params_default(C.byref(p))
+    p.enabled = 1
+    for k, v in params.items():
+        if k not in {f[0] for f in LaserScanParams._fields_} or k == "struct_size":
+            raise ValueError(f"laser_scan_params: unknown parameter {k!r}")
+        setattr(p, k, v)
+    return p
+
+
+def laser_scan_ranges(**params) -> int:
+    """The number of ranges pointcloud_to_laserscan makes for these params (d2pc_laser_scan_ranges)."""
+    n = C.c_uint32()
+    rc = lib().d2pc_laser_scan_ranges(C.byref(laser_scan_params(**params)), C.byref(n))
+    if rc:
+        raise D2pcError(rc, "d2pc_laser_scan_ranges")
+    return int(n.value)
 
 
 class PinnedArray:
@@ -409,6 +466,42 @@ class Context:
         t = CloudTransform()
         self._check(lib().d2pc_get_cloud_transform(self._h, C.byref(t)), "d2pc_get_cloud_transform")
         return t
+
+    def set_laser_scan(self, enabled: bool = True, **params):
+        """pointcloud_to_laserscan as an output next to the cloud: the scan of every cloud a host entry publishes,
+        read with last_scan().  params: any field of LaserScanParams (the nodelet's ten params and keep_cloud);
+        set_laser_scan(False) turns it off."""
+        p = laser_scan_params(**params)
+        p.enabled = 1 if enabled else 0
+        self._check(lib().d2pc_set_laser_scan(self._h, C.byref(p)), "d2pc_set_laser_scan")
+
+    def get_laser_scan(self) -> LaserScanParams:
+        p = LaserScanParams()
+        self._check(lib().d2pc_get_laser_scan(self._h, C.byref(p)), "d2pc_get_laser_scan")
+        return p
+
+    def last_scan_raw(self) -> LaserScan:
+        """d2pc_last_scan as it is (its ranges point into library memory)."""
+        s = LaserScan()
+        self._check(lib().d2pc_last_scan(self._h, C.byref(s)), "d2pc_last_scan")
+        return s
+
+    def last_scan(self):
+        """The scan of the cloud last returned: (dict of the seven float fields, float32 ranges)."""
+        s = self.last_scan_raw()
+        return s.fields(), s.ranges_array()
+
+    def laser_scan_device(self, d_in, n_frames, n_max, in_stride, d_in_counts, d_ranges, ranges_stride):
+        """d2pc_laser_scan_device: the context's (enabled) scan of clouds on the device, frame f's ranges at
+        d_ranges + f * ranges_stride bytes."""
+        self._check(lib().d2pc_laser_scan_device(self._h, d_in, n_frames, n_max, in_stride, d_in_counts or None,
+                                                 d_ranges, ranges_stride), "d2pc_laser_scan_device")
+
+    def serialize_laserscan(self, scan: LaserScan, seq=0, sec=0, nsec=0) -> bytes:
+        need = lib().d2pc_serialize_laserscan(self._h, C.byref(scan), seq, sec, nsec, None, 0)
+        buf = (C.c_uint8 * need)()
+        lib().d2pc_serialize_laserscan(self._h, C.byref(scan), seq, sec, nsec, buf, need)
+        return bytes(buf)
 
     def set_arith_mode(self, m):
         self._check(lib().d2pc_set_arith_mode(self._h, m), "d2pc_set_arith_mode")

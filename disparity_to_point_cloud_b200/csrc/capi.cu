@@ -13,6 +13,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <cfloat>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -29,6 +30,7 @@
 #include "cloud_transform.h"
 #include "crop_box.h"
 #include "fusion.h"
+#include "laser_scan.h"
 #include "median.h"
 #include "radius_outlier.h"
 #include "reproject.h"
@@ -54,6 +56,14 @@ struct PinBuf {
 // The filter stages that run on clouds already on the device (cloud_stage.cuh), in the order a plan runs them.
 enum class CloudStage { transform, box, voxel, ror };
 
+// The laser scan of a plan (d2pc_set_laser_scan), derived once per setting and carried by value into each submission.
+struct ScanPlan {
+  bool on = false;
+  bool keep_cloud = true;  // false: only the ranges leave the device
+  LaserScanParams p{};
+  d2pc_laser_scan msg{};   // the message fields (ranges unset)
+};
+
 // What the filter mode, the cloud transform, the crop box and the radius outlier stage make of one frame geometry
 // (plan_cloud), decided once per call.
 struct CloudPlan {
@@ -65,6 +75,7 @@ struct CloudPlan {
   bool counted = false;     // the cloud's size is known only on the device: the kept count decides the bytes
   uint32_t count_words = 1; // count words a slot reads back (Slot::d_count)
   bool fallback_decides_dense = false;  // VOXEL alone: the overflow fallback flag clears is_dense
+  ScanPlan scan;                        // the host entries' laser scan (add_scan)
 };
 
 // The device buffers between a batch's input frames and its cloud: one set per slot, one for the device batch.
@@ -82,6 +93,8 @@ struct Slot {
   StageBufs stages;
   // fusion pipeline (d2pc_submit_fusion): the four input frames, the two preprocessed scores, merge outputs
   DevBuf d_fuse_in[4], d_pre[2], d_container, d_combined, d_fused;
+  DevBuf d_ranges;  // the laser scan of the pending submission (ScanPlan), and its host copy
+  PinBuf h_ranges;
   uint32_t *d_count = nullptr;  // [0] = kept points, [1] = compaction ticket, [2] = VOXEL overflow fallback taken
   uint32_t *h_count = nullptr;  // pinned
   cudaEvent_t ev_h2d = nullptr, ev_kernel = nullptr, ev_d2h = nullptr;
@@ -119,6 +132,10 @@ struct d2pc_ctx {
   d2pc_radius_outlier ror;  // the radius outlier stage behind every mode (d2pc_set_radius_outlier; radius 0: off)
   d2pc_crop_box box;        // the crop box in front of VOXEL and the outlier stage (d2pc_set_crop_box; enabled 0: off)
   d2pc_cloud_transform xform;  // the first cloud stage (d2pc_set_cloud_transform; enabled 0: off)
+  d2pc_laser_scan_params scan;  // the laser scan output (d2pc_set_laser_scan; enabled 0: off)
+  ScanPlan scan_plan;           // derived from `scan`
+  d2pc_laser_scan last_scan{};  // d2pc_last_scan: the scan of the cloud last returned
+  bool last_scan_on = false;
   // fusion buffers
   DevBuf d_fuse_in[4], d_container, d_combined, d_fused;
   PinBuf h_fused, h_combined;
@@ -290,8 +307,52 @@ CloudPlan plan_cloud(const d2pc_ctx *ctx, uint32_t w, uint32_t h) {
   return p;
 }
 
-// a cloud's size: all crop points, or the count the device kept
-uint64_t kept_points(const CloudPlan &p, const uint32_t *h_count) { return p.counted && p.n ? h_count[0] : p.n; }
+// The host entries' laser scan: the context's setting, when it is on.
+void add_scan(const d2pc_ctx *ctx, CloudPlan &p) {
+  if (ctx->scan.enabled) p.scan = ctx->scan_plan;
+}
+// the cloud leaves the device (with the scan on and keep_cloud 0 only the ranges do)
+bool cloud_out(const CloudPlan &p) { return !p.scan.on || p.scan.keep_cloud; }
+
+// A scan setting checked (d2pc_set_laser_scan's rules) and derived.
+int scan_plan_of(const d2pc_laser_scan_params *q, ScanPlan *out) {
+  if (!q || q->struct_size != sizeof(*q)) return D2PC_ERR_INVALID_ARG;
+  for (double v : {q->angle_min, q->angle_max, q->angle_increment, q->range_min, q->range_max})
+    if (!std::isfinite(v)) return D2PC_ERR_INVALID_ARG;
+  if (std::isnan(q->min_height) || std::isnan(q->max_height)) return D2PC_ERR_INVALID_ARG;
+  if (!(q->range_min >= 0.0) || !(q->range_max >= q->range_min) || !(q->inf_epsilon >= 0.0) ||
+      !std::isfinite(q->inf_epsilon))
+    return D2PC_ERR_INVALID_ARG;
+  ScanPlan s;
+  d2pc_laser_scan &m = s.msg;
+  m.angle_min = (float)q->angle_min, m.angle_max = (float)q->angle_max;
+  m.angle_increment = (float)q->angle_increment;
+  m.time_increment = 0.0f, m.scan_time = (float)q->scan_time;
+  m.range_min = (float)q->range_min, m.range_max = (float)q->range_max;
+  if (!(m.angle_increment > 0.0f) || !(m.angle_min <= m.angle_max)) return D2PC_ERR_INVALID_ARG;
+  // the reference's size, in float arithmetic from the message's fields
+  const float span = m.angle_max - m.angle_min;
+  const float nf = ceilf(span / m.angle_increment);
+  if (!(nf <= (float)(1u << 20))) return D2PC_ERR_INVALID_ARG;
+  m.n_ranges = (uint32_t)nf;
+  const float init = q->use_inf ? INFINITY : (float)((double)m.range_max + q->inf_epsilon);
+  s.on = q->enabled != 0;
+  s.keep_cloud = q->keep_cloud != 0;
+  LaserScanParams &p = s.p;
+  p.min_height = q->min_height, p.max_height = q->max_height;
+  p.range_min = q->range_min, p.range_max = q->range_max;
+  p.angle_min = (double)m.angle_min, p.angle_max = (double)m.angle_max, p.angle_increment = (double)m.angle_increment;
+  p.n = m.n_ranges;
+  memcpy(&p.init_bits, &init, 4);
+  *out = s;
+  return D2PC_OK;
+}
+
+// a cloud's size: all crop points, or the count the device kept (0 when only the scan leaves the device)
+uint64_t kept_points(const CloudPlan &p, const uint32_t *h_count) {
+  if (!cloud_out(p)) return 0;
+  return p.counted && p.n ? h_count[0] : p.n;
+}
 // a cloud's is_dense: 0 in CROP mode (cpp:81); 1 for a counted cloud, except a VOXEL frame that took the overflow
 // fallback
 bool cloud_is_dense(const CloudPlan &p, const uint32_t *h_count) {
@@ -556,9 +617,10 @@ int enqueue_reproject(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, S
 // Enqueue the plan's steps for one frame batch already on the device: [median] + reproject, then each cloud stage
 // in plan order.  The reproject kernels write cloud buffer 0; each stage reads one buffer and writes the other, so
 // its input and output never overlap; the last step writes `out`.  fallback: VOXEL's per-frame overflow fallback
-// flags (may be null).
+// flags (may be null).  ranges: with the plan's scan on, the scan of `out` is the last step and writes each frame's
+// ranges there (frame f at f * 4 * n bytes).
 int enqueue_kernels(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, StageBufs &b, const CloudDst &out,
-                    uint32_t *fallback, uint32_t *ticket, cudaStream_t stream) {
+                    uint32_t *fallback, uint32_t *ticket, cudaStream_t stream, float *ranges = nullptr) {
   const uint32_t n = (uint32_t)p.n;
   const int stages = p.n_stages;
   const CloudDst buf[2] = {cloud_buf(b.cloud[0], in.n_frames, n), cloud_buf(b.cloud[1], in.n_frames, n)};
@@ -569,7 +631,13 @@ int enqueue_kernels(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, Sta
     const CloudSrc cloud{src.points, src.stride, i > 0 || p.compact ? src.counts : nullptr, in.n_frames, n};
     rc = enqueue_stage(ctx, p.stages[i], cloud, i + 1 < stages ? buf[(i + 1) & 1] : out, fallback, b.stage.p, stream);
   }
-  return rc;
+  if (rc || !p.scan.on || !ranges) return rc;
+  // an uncounted plan's cloud has all n points in every frame
+  const CloudSrc cloud{out.points, out.stride, p.counted ? out.counts : nullptr, in.n_frames, n};
+  int nl = 0;
+  CU(ctx, launch_laser_scan(cloud, p.scan.p, ranges, (size_t)p.scan.p.n * 4, stream, &nl));
+  ctx->launches += nl;
+  return D2PC_OK;
 }
 
 int check_frame(const d2pc_ctx *ctx, const void *data, uint32_t w, uint32_t h, size_t step, int esz) {
@@ -599,14 +667,19 @@ uint8_t *direct_alias(void *host) {
 }
 
 // A slot's D2H (stream 3), behind its kernels: the count words when the count decides the bytes (the payload copy is
-// issued in d2pc_wait), else the whole cloud into dst.
+// issued in d2pc_wait), else the whole cloud into dst (dst null: the cloud leaves elsewhere, or not at all); then the
+// scan's ranges.
 int enqueue_readback(d2pc_ctx *ctx, Slot &s, const CloudPlan &p, uint8_t *dst) {
   CU(ctx, cudaStreamWaitEvent(ctx->s_d2h, s.ev_kernel, 0));
-  if (p.counted)
-    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, p.count_words * sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                            ctx->s_d2h));
-  else if (p.n)
-    CU(ctx, cudaMemcpyAsync(dst, s.d_out.p, p.n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
+  if (dst && cloud_out(p)) {
+    if (p.counted)
+      CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, p.count_words * sizeof(uint32_t), cudaMemcpyDeviceToHost,
+                              ctx->s_d2h));
+    else if (p.n)
+      CU(ctx, cudaMemcpyAsync(dst, s.d_out.p, p.n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
+  }
+  if (p.scan.on && p.scan.p.n)
+    CU(ctx, cudaMemcpyAsync(s.h_ranges.p, s.d_ranges.p, (size_t)p.scan.p.n * 4, cudaMemcpyDeviceToHost, ctx->s_d2h));
   CU(ctx, cudaEventRecord(s.ev_d2h, ctx->s_d2h));
   return D2PC_OK;
 }
@@ -635,18 +708,24 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   // mono8 rows of any width (the callback kernel reads bytes; a 665-wide fused map is then one DMA instead of a
   // pitched 2-D copy); float rows that are not 16-byte multiples keep a 256-byte pitch for the vector loads.
   const size_t d_pitch = (row_bytes % 16 == 0 || !is_f32) ? row_bytes : round_up(row_bytes, kAlign);
-  const CloudPlan p = plan_cloud(ctx, w, h);
+  CloudPlan p = plan_cloud(ctx, w, h);
+  add_scan(ctx, p);
   const uint64_t n = p.n;
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // PointCloud2.row_step / width are uint32
-  if (user_dst && !p.counted && user_cap < n * 16) return D2PC_ERR_BUFFER_TOO_SMALL;
+  const bool out_cloud = cloud_out(p);
+  if (user_dst && !p.counted && out_cloud && user_cap < n * 16) return D2PC_ERR_BUFFER_TOO_SMALL;
   const bool user_pinned = user_dst && reinterpret_cast<uintptr_t>(user_dst) % 16 == 0 && lookup_pinned(ctx, user_dst);
   if ((rc = grow_dev(ctx, s.d_in, d_pitch * h))) return rc;
-  const bool late_copy = sync_call && user_dst && !user_pinned && !p.counted && n;
-  if (!user_pinned && !late_copy && (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
+  const bool late_copy = sync_call && user_dst && !user_pinned && !p.counted && n && out_cloud;
+  if (!user_pinned && !late_copy && out_cloud && (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
+  if (p.scan.on && ((rc = grow_dev(ctx, s.d_ranges, (size_t)p.scan.p.n * 4)) ||
+                    (rc = grow_pin(ctx, s.h_ranges, (size_t)p.scan.p.n * 4))))
+    return rc;
   // direct output: the kernel's point stores go over PCIe into the page-locked destination while it runs, so a lone
-  // frame no longer pays kernel + copy back to back (CROP only: a compacted cloud's size is not known up front)
+  // frame no longer pays kernel + copy back to back (CROP only: a compacted cloud's size is not known up front; not
+  // with the scan, which reads the cloud on the device)
   uint8_t *d_direct = nullptr;
-  if (!p.counted && n && !late_copy &&
+  if (!p.counted && n && !late_copy && !p.scan.on &&
       (ctx->direct_out > 0 ||
        (ctx->direct_out == 0 && sync_call && !is_f32 && ctx->cfg.median_ksize > 1 && p.n_stages == 0)))
     d_direct = direct_alias(user_pinned ? user_dst : s.h_out.p);
@@ -687,19 +766,20 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   {
     NvtxRange nvtx_k("d2pc kernels");
     rc = enqueue_kernels(ctx, p, in, s.stages, {d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count},
-                         s.d_count + 2, s.d_count + 1, ctx->s_compute);
+                         s.d_count + 2, s.d_count + 1, ctx->s_compute, reinterpret_cast<float *>(s.d_ranges.p));
   }
   if (rc) return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, ctx->s_compute));
 
   NvtxRange nvtx_d2h("d2pc D2H");
-  if (d_direct || late_copy) {
+  if ((d_direct || late_copy) && !p.scan.on) {
     // the cloud is already in host memory when the kernel ends (direct output), or leaves the device in d2pc_wait
     // (pageable destination of a synchronous call): the slot completes on the compute stream
     CU(ctx, cudaEventRecord(s.ev_d2h, ctx->s_compute));
   } else {
     // a page-locked caller buffer receives the cloud by DMA directly; a pageable one is filled from h_out in wait
-    if ((rc = enqueue_readback(ctx, s, p, user_pinned ? user_dst : s.h_out.p))) return rc;
+    // (a late copy with the scan on: only the ranges here)
+    if ((rc = enqueue_readback(ctx, s, p, late_copy ? nullptr : user_pinned ? user_dst : s.h_out.p))) return rc;
   }
   arm_slot(s, p, user_dst, user_cap, user_pinned, late_copy);
   return D2PC_OK;
@@ -841,6 +921,8 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
   d2pc_radius_outlier_default(&ctx->ror);
   d2pc_crop_box_default(&ctx->box);
   d2pc_cloud_transform_default(&ctx->xform);
+  d2pc_laser_scan_params_default(&ctx->scan);
+  scan_plan_of(&ctx->scan, &ctx->scan_plan);
 
   if (const char *v = getenv("D2PC_ROWS_PER_UNIT")) ctx->rows_per_unit = atoi(v);
   if (const char *v = getenv("D2PC_CTAS_PER_SM")) ctx->ctas_per_sm = atoi(v);
@@ -870,7 +952,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
   cudaDeviceSynchronize();
   for (auto &s : ctx->slots) {
     free_pin(s.h_in), free_pin(s.h_out);
-    free_dev(s.d_in), free_dev(s.d_out), free_stages(s.stages);
+    free_dev(s.d_in), free_dev(s.d_out), free_stages(s.stages), free_dev(s.d_ranges), free_pin(s.h_ranges);
     for (auto &b : s.d_fuse_in) free_dev(b);
     free_dev(s.d_pre[0]), free_dev(s.d_pre[1]), free_dev(s.d_container), free_dev(s.d_combined), free_dev(s.d_fused);
     if (s.d_count) cudaFree(s.d_count);
@@ -991,6 +1073,44 @@ int d2pc_get_cloud_transform(const d2pc_ctx *ctx, d2pc_cloud_transform *t) {
   *t = ctx->xform;
   return D2PC_OK;
 }
+void d2pc_laser_scan_params_default(d2pc_laser_scan_params *p) {
+  if (!p) return;
+  memset(p, 0, sizeof(*p));
+  p->struct_size = sizeof(*p);
+  p->min_height = DBL_MIN, p->max_height = DBL_MAX;
+  p->angle_min = -M_PI, p->angle_max = M_PI, p->angle_increment = M_PI / 180.0;
+  p->scan_time = 1.0 / 30.0;
+  p->range_min = 0.0, p->range_max = DBL_MAX;
+  p->use_inf = 1, p->inf_epsilon = 1.0;
+  p->keep_cloud = 1;
+}
+int d2pc_set_laser_scan(d2pc_ctx *ctx, const d2pc_laser_scan_params *p) {
+  if (!ctx) return D2PC_ERR_INVALID_ARG;
+  ScanPlan s;
+  const int rc = scan_plan_of(p, &s);
+  if (rc) return rc;
+  ctx->scan = *p;
+  ctx->scan_plan = s;
+  return D2PC_OK;
+}
+int d2pc_get_laser_scan(const d2pc_ctx *ctx, d2pc_laser_scan_params *p) {
+  if (!ctx || !p) return D2PC_ERR_INVALID_ARG;
+  *p = ctx->scan;
+  return D2PC_OK;
+}
+int d2pc_laser_scan_ranges(const d2pc_laser_scan_params *p, uint32_t *n) {
+  ScanPlan s;
+  const int rc = n ? scan_plan_of(p, &s) : D2PC_ERR_INVALID_ARG;
+  if (rc) return rc;
+  *n = s.msg.n_ranges;
+  return D2PC_OK;
+}
+int d2pc_last_scan(const d2pc_ctx *ctx, d2pc_laser_scan *out) {
+  if (!ctx || !out) return D2PC_ERR_INVALID_ARG;
+  if (!ctx->last_scan_on) return D2PC_ERR_NOT_READY;
+  *out = ctx->last_scan;
+  return D2PC_OK;
+}
 int d2pc_set_arith_mode(d2pc_ctx *ctx, int m) {
   if (!ctx || m < 0 || m > 1) return D2PC_ERR_INVALID_ARG;
   ctx->cfg.arith_mode = m;
@@ -1045,6 +1165,13 @@ int d2pc_submit_f32(d2pc_ctx *ctx, int slot, const float *disp, uint32_t w, uint
   return submit_common(ctx, slot, disp, w, h, step, true);
 }
 
+// d2pc_last_scan's answer from now on: the scan of the cloud just returned, whose ranges are in `ranges`.
+static void note_scan(d2pc_ctx *ctx, const ScanPlan &scan, const PinBuf &ranges) {
+  ctx->last_scan_on = scan.on;
+  ctx->last_scan = scan.msg;
+  ctx->last_scan.ranges = reinterpret_cast<const float *>(ranges.p);
+}
+
 int d2pc_wait(d2pc_ctx *ctx, int slot, d2pc_cloud *out) {
   if (!ctx || slot < 0 || slot >= (int)ctx->slots.size()) return D2PC_ERR_INVALID_ARG;
   Slot &s = ctx->slots[slot];
@@ -1054,6 +1181,7 @@ int d2pc_wait(d2pc_ctx *ctx, int slot, d2pc_cloud *out) {
   const uint64_t n = kept_points(s.plan, s.h_count);
   if (s.plan.counted && s.user_dst && s.user_cap < n * 16) {
     s.pending = false;
+    ctx->last_scan_on = false;  // no cloud is returned, so there is no last scan either
     return D2PC_ERR_BUFFER_TOO_SMALL;
   }
   // a counted cloud and a late copy leave the device here: the copy is synchronous anyway, so it goes straight to
@@ -1068,7 +1196,11 @@ int d2pc_wait(d2pc_ctx *ctx, int slot, d2pc_cloud *out) {
   s.late_copy = false;
   s.pending = false;
   if (ctx->cfg.verbose) printf("Cloud size: %llu\n", (unsigned long long)n);  // cpp:82
-  if (out) fill_cloud(ctx, s.user_dst ? s.user_dst : s.h_out.p, n, cloud_is_dense(s.plan, s.h_count), out);
+  if (out) {
+    if (cloud_out(s.plan)) fill_cloud(ctx, s.user_dst ? s.user_dst : s.h_out.p, n, cloud_is_dense(s.plan, s.h_count), out);
+    else fill_cloud(ctx, nullptr, 0, true, out);
+  }
+  note_scan(ctx, s.plan.scan, s.h_ranges);
   return D2PC_OK;
 }
 
@@ -1307,6 +1439,33 @@ int d2pc_cloud_transform_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_f
     int nl = 0;
     CU(ctx, launch_cloud_transform(in, out, t, d_transforms ? d_transforms + 12 * (size_t)f0 : nullptr, ctx->s_compute,
                                    &nl));
+    ctx->launches += nl;
+  }
+  return D2PC_OK;
+}
+
+int d2pc_laser_scan_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
+                           const uint32_t *d_in_counts, float *d_ranges, size_t ranges_stride) {
+  if (!ctx || !d_in || !d_ranges || !ctx->scan.enabled) return D2PC_ERR_INVALID_ARG;
+  const LaserScanParams &p = ctx->scan_plan.p;
+  const uint64_t bytes = (uint64_t)n_max * 16, rbytes = (uint64_t)p.n * 4;
+  if (bytes > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // the argument rules of the other cloud stages
+  if (reinterpret_cast<uintptr_t>(d_in) % 16 || in_stride % 16 || reinterpret_cast<uintptr_t>(d_ranges) % 4 ||
+      ranges_stride % 4 || (n_frames > 1 && (in_stride < bytes || ranges_stride < rbytes)))
+    return D2PC_ERR_BAD_DIMS;
+  if (n_frames == 0 || p.n == 0) return D2PC_OK;
+  const uintptr_t in0 = reinterpret_cast<uintptr_t>(d_in), out0 = reinterpret_cast<uintptr_t>(d_ranges);
+  const uint64_t in_end = in0 + (uint64_t)(n_frames - 1) * in_stride + bytes;
+  const uint64_t out_end = out0 + (uint64_t)(n_frames - 1) * ranges_stride + rbytes;
+  if (bytes && in0 < out_end && out0 < in_end) return D2PC_ERR_INVALID_ARG;
+  CU(ctx, cudaSetDevice(ctx->device));
+  const uint32_t chunk = frames_per_chunk(n_frames, n_max);
+  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
+    const CloudSrc in{d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
+                      std::min(chunk, n_frames - f0), n_max};
+    int nl = 0;
+    CU(ctx, launch_laser_scan(in, p, reinterpret_cast<float *>(reinterpret_cast<uint8_t *>(d_ranges) + f0 * ranges_stride),
+                              ranges_stride, ctx->s_compute, &nl));
     ctx->launches += nl;
   }
   return D2PC_OK;
@@ -1634,20 +1793,26 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
   Slot &s = ctx->slots[0];
   if ((rc = slot_wait_idle(ctx, s))) return rc;
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
-  const CloudPlan p = plan_cloud(ctx, fw, fh);
+  CloudPlan p = plan_cloud(ctx, fw, fh);
+  add_scan(ctx, p);
   const uint64_t n = p.n;
-  if ((rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
+  if (cloud_out(p) && (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
+  if (p.scan.on && ((rc = grow_dev(ctx, s.d_ranges, (size_t)p.scan.p.n * 4)) ||
+                    (rc = grow_pin(ctx, s.h_ranges, (size_t)p.scan.p.n * 4))))
+    return rc;
   // a synchronous call: the callback kernel stores the CROP cloud straight into the pinned buffer (see submit_common)
-  const bool direct = ctx->direct_out > 0 || (ctx->direct_out == 0 && p.n_stages == 0);
+  const bool direct = !p.scan.on && (ctx->direct_out > 0 || (ctx->direct_out == 0 && p.n_stages == 0));
   uint8_t *const d_direct =
       !p.counted && n && direct && ctx->cfg.median_ksize > 1 ? direct_alias(s.h_out.p) : nullptr;
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
   const FrameBatch fused{ctx->d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh};
   if ((rc = grow_stages(ctx, s.stages, p, fused, ctx->s_compute, false)) ||
       (rc = enqueue_kernels(ctx, p, fused, s.stages, {d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count},
-                            s.d_count + 2, s.d_count + 1, ctx->s_compute)))
+                            s.d_count + 2, s.d_count + 1, ctx->s_compute, reinterpret_cast<float *>(s.d_ranges.p))))
     return rc;
-  if (p.counted) {
+  if (p.scan.on && p.scan.p.n)
+    CU(ctx, cudaMemcpyAsync(s.h_ranges.p, s.d_ranges.p, (size_t)p.scan.p.n * 4, cudaMemcpyDeviceToHost, ctx->s_compute));
+  if (p.counted && cloud_out(p)) {
     CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, p.count_words * sizeof(uint32_t), cudaMemcpyDeviceToHost,
                             ctx->s_compute));
     CU(ctx, cudaStreamSynchronize(ctx->s_compute));
@@ -1657,7 +1822,9 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
     CU(ctx, cudaMemcpyAsync(s.h_out.p, s.d_out.p, kept * 16, cudaMemcpyDeviceToHost, ctx->s_compute));
   CU(ctx, cudaStreamSynchronize(ctx->s_compute));
   if (ctx->cfg.verbose) printf("Cloud size: %llu\n", (unsigned long long)kept);
-  fill_cloud(ctx, s.h_out.p, kept, cloud_is_dense(p, s.h_count), out);
+  if (cloud_out(p)) fill_cloud(ctx, s.h_out.p, kept, cloud_is_dense(p, s.h_count), out);
+  else fill_cloud(ctx, nullptr, 0, true, out);
+  note_scan(ctx, p.scan, s.h_ranges);
   return D2PC_OK;
 }
 
@@ -1680,8 +1847,12 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
   // (mono8 frames of any width: the fusion kernels read bytes, and a pitched 2-D copy is the slow way in)
   const size_t pitch = w, frame_bytes = (size_t)w * h, nn = (size_t)g.n * g.n;
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
-  const CloudPlan p = plan_cloud(ctx, fw, fh);
+  CloudPlan p = plan_cloud(ctx, fw, fh);
+  add_scan(ctx, p);
   const uint64_t n = p.n;
+  if (p.scan.on && ((rc = grow_dev(ctx, s.d_ranges, (size_t)p.scan.p.n * 4)) ||
+                    (rc = grow_pin(ctx, s.h_ranges, (size_t)p.scan.p.n * 4))))
+    return rc;
   // the four input frames of a set live in one allocation, so that a contiguous pinned set is one DMA
   if ((rc = grow_dev(ctx, s.d_fuse_in[0], 4 * pitch * h))) return rc;
   uint8_t *const fin[4] = {s.d_fuse_in[0].p, s.d_fuse_in[0].p + pitch * h, s.d_fuse_in[0].p + 2 * pitch * h,
@@ -1734,7 +1905,7 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
                              nullptr, preprocess_scores != 0, &s.d_container, sk)))
     return rc;
   if ((rc = enqueue_kernels(ctx, p, fused, s.stages, {s.d_out.p, n * 16 + 16, s.d_count}, s.d_count + 2,
-                            s.d_count + 1, sk)))
+                            s.d_count + 1, sk, reinterpret_cast<float *>(s.d_ranges.p))))
     return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, sk));
   if ((rc = enqueue_readback(ctx, s, p, s.h_out.p))) return rc;
@@ -1805,6 +1976,37 @@ size_t d2pc_serialize_pointcloud2(const d2pc_ctx *ctx, const d2pc_cloud *cloud, 
   u32(cloud->point_step), u32(cloud->row_step);
   u32((uint32_t)data_len), bytes(cloud->data, data_len);
   *p++ = cloud->is_dense;
+  return need;
+}
+
+size_t d2pc_serialize_laserscan(const d2pc_ctx *ctx, const d2pc_laser_scan *scan, uint32_t seq, uint32_t sec,
+                                uint32_t nsec, uint8_t *out, size_t cap) {
+  if (!ctx || !scan || (scan->n_ranges && !scan->ranges)) return 0;
+  // std_msgs/Header, then the sensor_msgs/LaserScan members in declaration order: seven float32, ranges and
+  // intensities as length-prefixed float32 arrays (intensities empty)
+  const char *fid = ctx->cfg.frame_id;
+  const uint32_t fid_len = (uint32_t)strlen(fid);
+  const size_t need = 12 + 4 + fid_len + 7 * 4 + 4 + (size_t)scan->n_ranges * 4 + 4;
+  if (!out || cap < need) return need;
+  uint8_t *p = out;
+  auto u32 = [&](uint32_t v) {
+    memcpy(p, &v, 4);
+    p += 4;
+  };
+  auto f32 = [&](float v) {
+    memcpy(p, &v, 4);
+    p += 4;
+  };
+  u32(seq), u32(sec), u32(nsec);
+  u32(fid_len);
+  memcpy(p, fid, fid_len);
+  p += fid_len;
+  f32(scan->angle_min), f32(scan->angle_max), f32(scan->angle_increment), f32(scan->time_increment);
+  f32(scan->scan_time), f32(scan->range_min), f32(scan->range_max);
+  u32(scan->n_ranges);
+  if (scan->n_ranges) memcpy(p, scan->ranges, (size_t)scan->n_ranges * 4);
+  p += (size_t)scan->n_ranges * 4;
+  u32(0);
   return need;
 }
 

@@ -340,6 +340,93 @@ int d2pc_set_cloud_transform(d2pc_ctx *ctx, const d2pc_cloud_transform *t);
 /* The setting last made (d2pc_cloud_transform_default's until then). */
 int d2pc_get_cloud_transform(const d2pc_ctx *ctx, d2pc_cloud_transform *t);
 
+/* ---- laser scan (an output next to the cloud: pointcloud_to_laserscan on the device) -------------------------------
+ *
+ * Off by default (enabled 0).  With the scan on, every host entry point that publishes a cloud (the process_* and
+ * *_into calls, submit / d2pc_wait, d2pc_process_stream, the fusion entries) also produces the sensor_msgs/LaserScan
+ * that pointcloud_to_laserscan would publish for exactly that cloud: after the transform, the crop box, VOXEL and the
+ * outlier stage, in the cloud's frame (the target frame with the cloud transform on: the scan needs a z-up frame).
+ * d2pc_last_scan returns it.  The d2pc_reproject_*_device batch entries make no scan; d2pc_laser_scan_device makes one
+ * of clouds already on the device.
+ * Reference: PointCloudToLaserScanNodelet::cloudCb, pointcloud_to_laserscan ROS1 1.4.x, restated from memory (its
+ * source was not at hand when this was written -- the same footing as DESIGN.md section 0.1 for the OpenCV dispatch).
+ * The recipe:
+ *   - message fields: angle_min_f, angle_max_f, angle_increment_f, scan_time, range_min, range_max are the double
+ *     params rounded to float; time_increment 0; no intensities.
+ *   - n = (uint32)ceilf((angle_max_f - angle_min_f) / angle_increment_f), float arithmetic (the reference computes it
+ *     from the message's float fields).
+ *   - every range starts at init = +inf when use_inf, otherwise (float)((double)range_max_f + inf_epsilon).
+ *   - per point, in this order:
+ *       1. skip if x, y or z is NaN (only NaN: +-inf goes on, as std::isnan lets it);
+ *       2. skip if (double)z > max_height or (double)z < min_height;
+ *       3. r = range(x, y); skip if r < range_min or r > range_max (the double params, not the float fields);
+ *       4. a = angle(y, x); skip if a < (double)angle_min_f or a > (double)angle_max_f;
+ *       5. k = (int)((a - (double)angle_min_f) / (double)angle_increment_f), double arithmetic, truncated;
+ *       6. skip if k >= n.  The reference writes past its vector there (a point exactly on angle_max when the span
+ *          is a whole number of increments); this library drops the point.
+ *   - ranges[k] = min(init, min over the bin's points of (float)r).
+ *     This is the reference's sequential `if (range < ranges[k]) ranges[k] = range` in every point order: with m the
+ *     current float value, r < m implies (float)r <= m and r >= m implies (float)r >= m (rounding is monotone and m
+ *     is a float), so every step sets m = min(m, (float)r), and a min does not depend on the order.  Every value is
+ *     >= 0 (r is a square root, init >= 0 by the checks below), so the device takes the min on the floats' bits.
+ *   - range and angle are the library's own (csrc/scan_math.h, one source for the kernel and the C reference):
+ *     range = sqrt((double)x*x + (double)y*y) (exact products, one rounded add, a correctly rounded sqrt) and angle a
+ *     double atan2 built from IEEE add, sub, mul, div, sqrt and fma only, within 1 ulp for float inputs.  glibc's
+ *     hypot and atan2 are within 1 ulp too; the two can pick a different bin or range only for a point within a few
+ *     ulp of a bin edge, an angle limit or a range limit (tests/test_oracle_laser_scan.py measures it).
+ *   - Defaults follow the nodelet as recalled, unverified: min_height DBL_MIN and max_height DBL_MAX (so z <= 0 is
+ *     dropped), angles -pi, pi, pi/180 (n = 360), scan_time 1/30, range_min 0, range_max DBL_MAX, use_inf 1,
+ *     inf_epsilon 1.
+ * keep_cloud 1 (the default): both outputs; the cloud's bytes, timing spans and BUFFER_TOO_SMALL rules are what they
+ * are with the scan off.  keep_cloud 0: the cloud never leaves the device -- no payload copy, no count read-back, only
+ * the ranges are copied; d2pc_wait returns a cloud of width 0, data NULL, is_dense 1, and a *_into destination is
+ * neither written nor checked against cap.  The ranges' copy runs on the D2H stream behind the kernels, so
+ * d2pc_slot_timing's d2h_us covers it.  Plans with the scan never store the cloud from the kernel into host memory
+ * ("direct_out").  The setting in force when a frame is submitted is the one its slot uses. */
+typedef struct d2pc_laser_scan_params {
+  uint32_t struct_size; /* sizeof(d2pc_laser_scan_params) */
+  int32_t enabled;      /* 0: off (the default) */
+  double min_height, max_height;                 /* DBL_MIN, DBL_MAX; not NaN (+-inf allowed) */
+  double angle_min, angle_max, angle_increment;  /* -pi, pi, pi/180; finite */
+  double scan_time;                              /* 1/30 */
+  double range_min, range_max;                   /* 0, DBL_MAX; finite, 0 <= range_min <= range_max */
+  int32_t use_inf;                               /* 1 */
+  double inf_epsilon;                            /* 1; finite, >= 0 */
+  int32_t keep_cloud;                            /* 1: the cloud is produced as well; 0: only the scan leaves */
+} d2pc_laser_scan_params;
+
+/* A scan: the message fields and the ranges.  `ranges` is library-owned pinned host memory, valid until the next call
+ * that uses the same pipeline slot (inside a stream sink: until the sink returns). */
+typedef struct d2pc_laser_scan {
+  float angle_min, angle_max, angle_increment, time_increment, scan_time, range_min, range_max;
+  uint32_t n_ranges;
+  const float *ranges;
+} d2pc_laser_scan;
+
+/* enabled 0, keep_cloud 1, the nodelet's defaults above. */
+void d2pc_laser_scan_params_default(d2pc_laser_scan_params *p);
+/* D2PC_ERR_INVALID_ARG, keeping the previous setting, for: a non-finite angle or range param; angle_increment_f <= 0
+ * or angle_min_f > angle_max_f; range_min < 0, range_max < range_min or inf_epsilon < 0 (NaN included); a NaN height;
+ * more than 2^20 ranges; a wrong struct_size. */
+int d2pc_set_laser_scan(d2pc_ctx *ctx, const d2pc_laser_scan_params *p);
+/* The setting last made (d2pc_laser_scan_params_default's until then). */
+int d2pc_get_laser_scan(const d2pc_ctx *ctx, d2pc_laser_scan_params *p);
+/* n for these params, with the recipe's float formula (the other checks of d2pc_set_laser_scan apply as well). */
+int d2pc_laser_scan_ranges(const d2pc_laser_scan_params *p, uint32_t *n);
+/* The scan of the cloud this context last returned (d2pc_wait, the synchronous process_* / *_into and
+ * d2pc_fuse_then_process; inside a stream sink, the cloud handed to it).  D2PC_ERR_NOT_READY when the scan was off
+ * for that submission, when no cloud has been returned yet, or after a d2pc_wait that returned
+ * D2PC_ERR_BUFFER_TOO_SMALL (no cloud was returned then). */
+int d2pc_last_scan(const d2pc_ctx *ctx, d2pc_laser_scan *out);
+/* The scan alone (the context's setting, which must be enabled) of clouds already on the device, with the argument
+ * rules of d2pc_crop_box_device for the input: frame f's input is d_in + f*in_stride bytes, d_in_counts[f] points
+ * (NULL: n_max each; a count above n_max counts as n_max), pointers and strides 16-byte aligned, in_stride >= 16*n_max
+ * when n_frames > 1, n_max*16 < 2^32, batches of more than 2^31 - 2 points run in chunks of frames.  Frame f's n
+ * ranges go to d_ranges + f*ranges_stride bytes: d_ranges and ranges_stride 4-byte aligned, ranges_stride >= 4*n when
+ * n_frames > 1, no overlap with the input (D2PC_ERR_INVALID_ARG). */
+int d2pc_laser_scan_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
+                           const uint32_t *d_in_counts, float *d_ranges, size_t ranges_stride);
+
 /* ---- the disparity callback, host buffers (the reference-facing calls) ------ */
 
 /* Whole DisparityCb (src/disparity_to_point_cloud.cpp:46-92) on one mono8
@@ -556,6 +643,9 @@ int d2pc_process_fusion_stream(d2pc_ctx *ctx, const uint8_t *sets, uint64_t n_se
  * byte count (write happens only if cap suffices; pass NULL/0 to size). */
 size_t d2pc_serialize_pointcloud2(const d2pc_ctx *ctx, const d2pc_cloud *cloud, uint32_t seq, uint32_t stamp_sec,
                                   uint32_t stamp_nsec, uint8_t *out, size_t cap);
+/* sensor_msgs/LaserScan with header {seq, stamp, cfg.frame_id} and empty intensities; same return rule. */
+size_t d2pc_serialize_laserscan(const d2pc_ctx *ctx, const d2pc_laser_scan *scan, uint32_t seq, uint32_t stamp_sec,
+                                uint32_t stamp_nsec, uint8_t *out, size_t cap);
 
 /* ---- diagnostics ---------------------------------------------------------------- */
 

@@ -41,6 +41,7 @@ class Bus {
  public:
   using ImageCb = std::function<void(const sensor_msgs::ImageConstPtr &)>;
   using CloudCb = std::function<void(const sensor_msgs::PointCloud2 &)>;
+  using ScanCb = std::function<void(const sensor_msgs::LaserScan &)>;
 
   // <remap from="/disparity" to="/throttled_depth_map"/>
   void remap(const std::string &from, const std::string &to) { remaps_[from] = to; }
@@ -77,6 +78,9 @@ class Bus {
     auto it = latched_clouds_.find(t);  // a latched publisher re-delivers its last message to late subscribers
     if (it != latched_clouds_.end()) cb(it->second);
   }
+  void subscribe_scan(const std::string &topic, uint32_t queue_size, ScanCb cb) {
+    scan_subs_[resolve(topic)].push_back({queue_size, std::move(cb)});
+  }
   struct Advertised {
     std::string topic;
     uint32_t queue_size;
@@ -97,6 +101,11 @@ class Bus {
       if (a.topic == resolved_topic && a.latch) latched_clouds_[resolved_topic] = msg;
     auto it = cloud_subs_.find(resolved_topic);
     if (it != cloud_subs_.end())
+      for (auto &s : it->second) s.cb(msg);
+  }
+  void publish(const std::string &resolved_topic, const sensor_msgs::LaserScan &msg) {
+    auto it = scan_subs_.find(resolved_topic);
+    if (it != scan_subs_.end())
       for (auto &s : it->second) s.cb(msg);
   }
   const std::vector<Advertised> &advertised() const { return advertised_; }
@@ -153,6 +162,7 @@ class Bus {
   std::map<std::string, std::string> str_params_;
   std::map<std::string, std::vector<Sub<ImageCb>>> image_subs_;
   std::map<std::string, std::vector<Sub<CloudCb>>> cloud_subs_;
+  std::map<std::string, std::vector<Sub<ScanCb>>> scan_subs_;
   std::map<std::string, sensor_msgs::PointCloud2> latched_clouds_;
   std::vector<Advertised> advertised_;
 };
@@ -219,6 +229,9 @@ class Disparity2PCloud {
   uint8_t *registered_ = nullptr;
   int border_ = 40;  // cpp:70,72
   std::string frame_id_ = "/camera_optical_frame";  // cpp:89; transform_target_frame with the transform on
+  std::string p_scan_topic_;  // "/scan" when scan_enable != 0
+  bool publish_cloud_ = true;  // false with scan_keep_cloud 0: only /scan is published
+  sensor_msgs::LaserScan scan_;
 
   // make output_.data hold `bytes` bytes in page-locked storage without touching bytes it already has
   void reserve_output(size_t bytes) {
@@ -317,6 +330,32 @@ class Disparity2PCloud {
       d2pc_b200::check(d2pc_set_cloud_transform(ctx_, &t), "d2pc_set_cloud_transform", ctx_);
       nh_.param<std::string>("transform_target_frame", frame_id_, "base_link");
     }
+    // optional, not in the reference: pointcloud_to_laserscan on the device, published on /scan with the cloud's
+    // header, on when scan_enable != 0.  scan_<param> are the nodelet's ten params (min_height, max_height,
+    // angle_min, angle_max, angle_increment, scan_time, range_min, range_max, use_inf, inf_epsilon) with its defaults;
+    // scan_keep_cloud 0 leaves the cloud on the device and /point_cloud unpublished.  The scan needs a z-up frame:
+    // set the transform params.
+    int scan_on = 0;
+    nh_.param<int>("scan_enable", scan_on, 0);
+    if (scan_on) {
+      d2pc_laser_scan_params s;
+      d2pc_laser_scan_params_default(&s);
+      s.enabled = 1;
+      nh_.param<double>("scan_min_height", s.min_height, s.min_height);
+      nh_.param<double>("scan_max_height", s.max_height, s.max_height);
+      nh_.param<double>("scan_angle_min", s.angle_min, s.angle_min);
+      nh_.param<double>("scan_angle_max", s.angle_max, s.angle_max);
+      nh_.param<double>("scan_angle_increment", s.angle_increment, s.angle_increment);
+      nh_.param<double>("scan_scan_time", s.scan_time, s.scan_time);
+      nh_.param<double>("scan_range_min", s.range_min, s.range_min);
+      nh_.param<double>("scan_range_max", s.range_max, s.range_max);
+      nh_.param<int>("scan_use_inf", s.use_inf, s.use_inf);
+      nh_.param<double>("scan_inf_epsilon", s.inf_epsilon, s.inf_epsilon);
+      nh_.param<int>("scan_keep_cloud", s.keep_cloud, 1);
+      d2pc_b200::check(d2pc_set_laser_scan(ctx_, &s), "d2pc_set_laser_scan", ctx_);
+      publish_cloud_ = s.keep_cloud != 0;
+      p_scan_topic_ = nh_.advertise("/scan", 1);
+    }
   }
   ~Disparity2PCloud() {
     d2pc_destroy(ctx_);  // waits for the device: nothing writes into output_ any more
@@ -332,7 +371,7 @@ class Disparity2PCloud {
   void DisparityCb(const sensor_msgs::ImageConstPtr &msg) {
     d2pc_b200::require_mono8(*msg);
     const long cw = static_cast<long>(msg->width) - 2L * border_, ch = static_cast<long>(msg->height) - 2L * border_;
-    reserve_output(cw > 0 && ch > 0 ? static_cast<size_t>(cw) * static_cast<size_t>(ch) * 16 : 0);
+    reserve_output(publish_cloud_ && cw > 0 && ch > 0 ? static_cast<size_t>(cw) * static_cast<size_t>(ch) * 16 : 0);
     d2pc_cloud cloud;
     uint8_t dummy[16];
     uint8_t *dst = output_.data.empty() ? dummy : output_.data.data();
@@ -360,7 +399,16 @@ class Disparity2PCloud {
     output.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
     output.header.stamp = msg->header.stamp;             // cpp:87
     output.header.frame_id = frame_id_;                  // cpp:89
-    nh_.publish(p_cloud_topic_, output);                 // cpp:90
+    if (publish_cloud_) nh_.publish(p_cloud_topic_, output);  // cpp:90
+    if (p_scan_topic_.empty()) return;
+    d2pc_laser_scan s;
+    d2pc_b200::check(d2pc_last_scan(ctx_, &s), "d2pc_last_scan", ctx_);
+    scan_.header = output.header;
+    scan_.angle_min = s.angle_min, scan_.angle_max = s.angle_max, scan_.angle_increment = s.angle_increment;
+    scan_.time_increment = s.time_increment, scan_.scan_time = s.scan_time;
+    scan_.range_min = s.range_min, scan_.range_max = s.range_max;
+    scan_.ranges.assign(s.ranges, s.ranges + s.n_ranges);
+    nh_.publish(p_scan_topic_, scan_);
   }
 };
 

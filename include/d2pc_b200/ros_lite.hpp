@@ -1,7 +1,8 @@
 // ros_lite.hpp -- the handful of ROS1 message types the two nodes exchange, as plain structs with the ROS1
 // wire (de)serialisation, so the node classes in nodes.hpp compile and run without a ROS installation.
 // Field order and types follow the message definitions the reference uses:
-//   std_msgs/Header, sensor_msgs/Image, sensor_msgs/PointField, sensor_msgs/PointCloud2
+//   std_msgs/Header, sensor_msgs/Image, sensor_msgs/PointField, sensor_msgs/PointCloud2, and sensor_msgs/LaserScan
+//   (pointcloud_to_laserscan's output, which the point cloud node can publish next to its cloud)
 //   (src/disparity_to_point_cloud.cpp:46-92, src/depth_map_fusion.cpp:46-136).
 // With a real ROS1 the ros1_shim/ sources use the genuine sensor_msgs types instead; the layouts are identical.
 #pragma once
@@ -55,6 +56,13 @@ struct PointCloud2 {
   uint8_t is_dense = 0;
 };
 
+struct LaserScan {
+  Header header;
+  float angle_min = 0, angle_max = 0, angle_increment = 0, time_increment = 0, scan_time = 0, range_min = 0,
+        range_max = 0;
+  std::vector<float> ranges, intensities;
+};
+
 }  // namespace sensor_msgs
 
 // ---- ROS1 serialisation: little endian, strings and arrays prefixed by a uint32 length --------------------
@@ -74,6 +82,15 @@ class Writer {
   void bytes(const std::vector<uint8_t> &d) {
     u32(static_cast<uint32_t>(d.size()));
     buf.insert(buf.end(), d.begin(), d.end());
+  }
+  void f32(float v) {
+    uint8_t b[4];
+    std::memcpy(b, &v, 4);
+    buf.insert(buf.end(), b, b + 4);
+  }
+  void floats(const std::vector<float> &d) {
+    u32(static_cast<uint32_t>(d.size()));
+    for (float v : d) f32(v);
   }
   void header(const Header &h) {
     u32(h.seq), u32(h.stamp.sec), u32(h.stamp.nsec), str(h.frame_id);
@@ -106,6 +123,19 @@ class Reader {
     need(n);
     std::vector<uint8_t> d(p_, p_ + n);
     p_ += n;
+    return d;
+  }
+  float f32() {
+    const uint32_t b = u32();
+    float v;
+    std::memcpy(&v, &b, 4);
+    return v;
+  }
+  std::vector<float> floats() {
+    const uint32_t n = u32();
+    need(static_cast<size_t>(n) * 4);
+    std::vector<float> d(n);
+    for (auto &v : d) v = f32();
     return d;
   }
   Header header() {
@@ -157,6 +187,22 @@ inline sensor_msgs::PointCloud2 deserialize_pointcloud2(const uint8_t *p, size_t
     m.fields.push_back(f);
   }
   m.is_bigendian = r.u8(), m.point_step = r.u32(), m.row_step = r.u32(), m.data = r.bytes(), m.is_dense = r.u8();
+  return m;
+}
+inline std::vector<uint8_t> serialize(const sensor_msgs::LaserScan &m) {
+  Writer w;
+  w.header(m.header);
+  w.f32(m.angle_min), w.f32(m.angle_max), w.f32(m.angle_increment), w.f32(m.time_increment), w.f32(m.scan_time);
+  w.f32(m.range_min), w.f32(m.range_max), w.floats(m.ranges), w.floats(m.intensities);
+  return std::move(w.buf);
+}
+inline sensor_msgs::LaserScan deserialize_laserscan(const uint8_t *p, size_t n) {
+  Reader r(p, n);
+  sensor_msgs::LaserScan m;
+  m.header = r.header();
+  m.angle_min = r.f32(), m.angle_max = r.f32(), m.angle_increment = r.f32(), m.time_increment = r.f32();
+  m.scan_time = r.f32(), m.range_min = r.f32(), m.range_max = r.f32();
+  m.ranges = r.floats(), m.intensities = r.floats();
   return m;
 }
 

@@ -6,6 +6,7 @@
 // launch/d2pcloud.launch works unchanged.
 #include <ros/ros.h>
 #include <sensor_msgs/Image.h>
+#include <sensor_msgs/LaserScan.h>
 #include <sensor_msgs/PointCloud2.h>
 #include <sensor_msgs/image_encodings.h>
 
@@ -130,6 +131,37 @@ class Disparity2PCloudGpu {
         ros::shutdown();
       }
     }
+    // optional, not in the reference: pointcloud_to_laserscan on the device, published on /scan with the cloud's
+    // header, on when scan_enable != 0.  scan_<param> are the nodelet's ten params with its defaults; scan_keep_cloud
+    // 0 leaves the cloud on the device and /point_cloud unpublished.  The scan needs a z-up frame: set transform_*.
+    int scan_on = 0;
+    nh_.param<int>("scan_enable", scan_on, 0);
+    if (scan_on) {
+      d2pc_laser_scan_params s;
+      d2pc_laser_scan_params_default(&s);
+      s.enabled = 1;
+      nh_.param<double>("scan_min_height", s.min_height, s.min_height);
+      nh_.param<double>("scan_max_height", s.max_height, s.max_height);
+      nh_.param<double>("scan_angle_min", s.angle_min, s.angle_min);
+      nh_.param<double>("scan_angle_max", s.angle_max, s.angle_max);
+      nh_.param<double>("scan_angle_increment", s.angle_increment, s.angle_increment);
+      nh_.param<double>("scan_scan_time", s.scan_time, s.scan_time);
+      nh_.param<double>("scan_range_min", s.range_min, s.range_min);
+      nh_.param<double>("scan_range_max", s.range_max, s.range_max);
+      int use_inf = s.use_inf, keep = 1;
+      nh_.param<int>("scan_use_inf", use_inf, use_inf);
+      nh_.param<double>("scan_inf_epsilon", s.inf_epsilon, s.inf_epsilon);
+      nh_.param<int>("scan_keep_cloud", keep, 1);
+      s.use_inf = use_inf, s.keep_cloud = keep;
+      if (d2pc_set_laser_scan(ctx_, &s) != D2PC_OK) {
+        ROS_FATAL("scan_*: not a valid laser scan setting");
+        ros::shutdown();
+      } else {
+        publish_cloud_ = keep != 0;
+        scan_pub_ = nh_.advertise<sensor_msgs::LaserScan>("/scan", 1);
+        scan_on_ = true;
+      }
+    }
   }
   ~Disparity2PCloudGpu() {
     d2pc_destroy(ctx_);
@@ -145,7 +177,7 @@ class Disparity2PCloudGpu {
     // the cloud is DMA'd straight into the message's (page-locked) data vector: no counterpart of the
     // pcl::toROSMsg memcpy (reference cpp:84-85)
     const long cw = static_cast<long>(msg->width) - 2L * border_, ch = static_cast<long>(msg->height) - 2L * border_;
-    const size_t bytes = cw > 0 && ch > 0 ? static_cast<size_t>(cw) * static_cast<size_t>(ch) * 16 : 0;
+    const size_t bytes = publish_cloud_ && cw > 0 && ch > 0 ? static_cast<size_t>(cw) * static_cast<size_t>(ch) * 16 : 0;
     sensor_msgs::PointCloud2 &out = out_;
     if (out.data.capacity() < bytes || out.data.data() != registered_) {
       if (registered_) d2pc_host_unregister(registered_);
@@ -181,13 +213,24 @@ class Disparity2PCloudGpu {
     out.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
     out.header.stamp = msg->header.stamp;
     out.header.frame_id = frame_id_;
-    pub_.publish(out);
+    if (publish_cloud_) pub_.publish(out);
+    if (!scan_on_) return;
+    d2pc_laser_scan s;
+    if (d2pc_last_scan(ctx_, &s) != D2PC_OK) return;
+    scan_.header = out.header;
+    scan_.angle_min = s.angle_min, scan_.angle_max = s.angle_max, scan_.angle_increment = s.angle_increment;
+    scan_.time_increment = s.time_increment, scan_.scan_time = s.scan_time;
+    scan_.range_min = s.range_min, scan_.range_max = s.range_max;
+    scan_.ranges.assign(s.ranges, s.ranges + s.n_ranges);
+    scan_pub_.publish(scan_);
   }
 
  private:
   ros::NodeHandle nh_;
   ros::Subscriber sub_;
-  ros::Publisher pub_;
+  ros::Publisher pub_, scan_pub_;
+  bool scan_on_ = false, publish_cloud_ = true;  // scan_enable, scan_keep_cloud
+  sensor_msgs::LaserScan scan_;
   d2pc_ctx *ctx_ = nullptr;
   sensor_msgs::PointCloud2 out_;   // persistent so that its data storage can stay page-locked
   uint8_t *registered_ = nullptr;

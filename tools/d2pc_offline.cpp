@@ -8,6 +8,9 @@
 //   d2pc_offline node1  <launch file> <w> <h> <in.raw> <out.bin> [sec nsec]
 //       BASELINE config 1/2 shape: one mono8 frame published on the node's (remapped) input topic; the
 //       PointCloud2 received on the (remapped) output topic is written in ROS1 wire format.
+//   d2pc_offline node1scan <launch file> <w> <h> <in.raw> <cloud.bin> <scan.bin>
+//       node1 with the /scan subscriber too (scan_enable in the launch file): the PointCloud2 (an empty file when
+//       none was published) and the LaserScan in ROS1 wire format.
 //   d2pc_offline fusion <fusion launch> <w> <h> <d1.raw> <d2.raw> <s1.raw> <s2.raw> <fused.bin> [<cloud.bin> [<debug dir>]]
 //       BASELINE config 5 shape: four mono8 frames into DepthMapFusion; the fused Image is written, and when
 //       <cloud.bin> is given it is also fed to a Disparity2PCloud node whose /disparity is remapped to
@@ -74,7 +77,29 @@ int main(int argc, char **argv) {
       auto ib = ros_lite::serialize(im);
       auto im2 = ros_lite::deserialize_image(ib.data(), ib.size());
       if (ros_lite::serialize(im2) != ib || im2.encoding != "mono8") throw std::runtime_error("Image round trip differs");
+      sm::LaserScan sc;
+      sc.header = c.header;
+      sc.angle_min = -1.5f, sc.angle_max = 1.5f, sc.angle_increment = 0.75f, sc.scan_time = 0.25f, sc.range_max = 9.f;
+      sc.ranges = {1.f, 2.f, 3.f, 4.f};
+      auto sb = ros_lite::serialize(sc);
+      auto sc2 = ros_lite::deserialize_laserscan(sb.data(), sb.size());
+      if (ros_lite::serialize(sc2) != sb || sb.size() != 16 + 21 + 28 + 4 + 16 + 4)
+        throw std::runtime_error("LaserScan round trip differs");
       write_file(argv[2], bytes);
+      return 0;
+    }
+    if (mode == "node1scan" && argc == 8) {
+      const uint32_t w = (uint32_t)std::atoi(argv[3]), h = (uint32_t)std::atoi(argv[4]);
+      d2pc_b200::Bus bus;
+      if (!bus.load_launch_file(argv[2])) throw std::runtime_error(std::string("cannot read ") + argv[2]);
+      d2pc::Disparity2PCloud node(bus);
+      std::vector<uint8_t> cloud, scan;
+      bus.subscribe_cloud("/point_cloud", 1, [&](const sm::PointCloud2 &c) { cloud = ros_lite::serialize(c); });
+      bus.subscribe_scan("/scan", 1, [&](const sm::LaserScan &s) { scan = ros_lite::serialize(s); });
+      bus.publish(bus.resolve("/disparity"), make_image(read_file(argv[5], (size_t)w * h), w, h, 3, 4));
+      if (scan.empty()) throw std::runtime_error("no scan was published");
+      write_file(argv[6], cloud);
+      write_file(argv[7], scan);
       return 0;
     }
     if (mode == "params" && argc >= 3) {
