@@ -94,6 +94,23 @@ class LaserScanParams(C.Structure):
                 ("keep_cloud", C.c_int32)]
 
 
+class OccupancyParams(C.Structure):
+    """d2pc_occupancy_params: octomap_server's parameters of the occupancy map (and keep_cloud)."""
+    _fields_ = [("struct_size", C.c_uint32), ("enabled", C.c_int32), ("resolution", C.c_double),
+                ("prob_hit", C.c_double), ("prob_miss", C.c_double), ("clamp_min", C.c_double),
+                ("clamp_max", C.c_double), ("occupancy_thres", C.c_double), ("max_range", C.c_double),
+                ("max_bricks", C.c_uint32), ("keep_cloud", C.c_int32)]
+
+
+class OccupancyInfo(C.Structure):
+    """d2pc_occupancy_info: the map's counters (d2pc_occupancy_stats)."""
+    _fields_ = [("frames_inserted", C.c_uint64), ("frames_dropped", C.c_uint64), ("known_voxels", C.c_uint64),
+                ("occupied_voxels", C.c_uint64), ("bricks_used", C.c_uint64), ("bricks_capacity", C.c_uint64)]
+
+    def as_dict(self) -> dict:
+        return {f[0]: int(getattr(self, f[0])) for f in self._fields_}
+
+
 class LaserScan(C.Structure):
     """d2pc_laser_scan: the message fields of a scan and its library-owned ranges."""
     _fields_ = [("angle_min", C.c_float), ("angle_max", C.c_float), ("angle_increment", C.c_float),
@@ -164,6 +181,15 @@ SYMBOLS = [
     ("d2pc_last_scan", C.c_int, [_ctx, C.POINTER(LaserScan)]),
     ("d2pc_laser_scan_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
                                          C.c_void_p, C.c_size_t]),
+    ("d2pc_occupancy_params_default", None, [C.POINTER(OccupancyParams)]),
+    ("d2pc_set_occupancy", C.c_int, [_ctx, C.POINTER(OccupancyParams)]),
+    ("d2pc_get_occupancy", C.c_int, [_ctx, C.POINTER(OccupancyParams)]),
+    ("d2pc_occupancy_reset", C.c_int, [_ctx]),
+    ("d2pc_occupancy_stats", C.c_int, [_ctx, C.POINTER(OccupancyInfo)]),
+    ("d2pc_occupancy_centers", C.c_int, [_ctx, C.c_void_p, C.c_size_t, C.POINTER(Cloud)]),
+    ("d2pc_occupancy_voxels", C.c_int, [_ctx, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
+    ("d2pc_occupancy_insert_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
+                                               C.c_void_p]),
     ("d2pc_process_mono8", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_process_f32", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_submit_mono8", C.c_int, [_ctx, C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
@@ -274,6 +300,18 @@ def laser_scan_params(**params) -> LaserScanParams:
     for k, v in params.items():
         if k not in {f[0] for f in LaserScanParams._fields_} or k == "struct_size":
             raise ValueError(f"laser_scan_params: unknown parameter {k!r}")
+        setattr(p, k, v)
+    return p
+
+
+def occupancy_params(**params) -> OccupancyParams:
+    """d2pc_occupancy_params_default with `params` (any field of OccupancyParams) set on top; enabled defaults to 1."""
+    p = OccupancyParams()
+    lib().d2pc_occupancy_params_default(C.byref(p))
+    p.enabled = 1
+    for k, v in params.items():
+        if k not in {f[0] for f in OccupancyParams._fields_} or k == "struct_size":
+            raise ValueError(f"occupancy_params: unknown parameter {k!r}")
         setattr(p, k, v)
     return p
 
@@ -502,6 +540,63 @@ class Context:
         buf = (C.c_uint8 * need)()
         lib().d2pc_serialize_laserscan(self._h, C.byref(scan), seq, sec, nsec, buf, need)
         return bytes(buf)
+
+    def set_occupancy(self, enabled: bool = True, **params):
+        """octomap_server's insertScan as a map the context keeps on the device, updated by every cloud a host entry
+        publishes.  params: any field of OccupancyParams; set_occupancy(False) stops updates and keeps the map."""
+        p = occupancy_params(**params)
+        p.enabled = 1 if enabled else 0
+        self._check(lib().d2pc_set_occupancy(self._h, C.byref(p)), "d2pc_set_occupancy")
+
+    def get_occupancy(self) -> OccupancyParams:
+        p = OccupancyParams()
+        self._check(lib().d2pc_get_occupancy(self._h, C.byref(p)), "d2pc_get_occupancy")
+        return p
+
+    def occupancy_reset(self):
+        self._check(lib().d2pc_occupancy_reset(self._h), "d2pc_occupancy_reset")
+
+    def occupancy_stats(self) -> dict:
+        s = OccupancyInfo()
+        self._check(lib().d2pc_occupancy_stats(self._h, C.byref(s)), "d2pc_occupancy_stats")
+        return s.as_dict()
+
+    def occupancy_centers(self) -> np.ndarray:
+        """The centres of the occupied voxels in Morton order, an (n, 4) float32 array of PointXYZ {x, y, z, 1}."""
+        cl = Cloud()
+        rc = lib().d2pc_occupancy_centers(self._h, None, 0, C.byref(cl))
+        if rc not in (0, -9):
+            self._check(rc, "d2pc_occupancy_centers")
+        while True:
+            out = np.empty((max(int(cl.width), 1), 4), np.float32)
+            rc = lib().d2pc_occupancy_centers(self._h, out.ctypes.data, out.nbytes, C.byref(cl))
+            if rc != -9:  # the map may have grown in between (frames still in flight): size again
+                break
+        self._check(rc, "d2pc_occupancy_centers")
+        return out[: cl.width]
+
+    def occupancy_voxels(self):
+        """Every known voxel in Morton order: keys as an (n, 3) uint16 array (kx, ky, kz) and float32 log-odds."""
+        n = C.c_uint64()
+        rc = lib().d2pc_occupancy_voxels(self._h, None, None, 0, C.byref(n))
+        while True:
+            if rc not in (0, -9):
+                self._check(rc, "d2pc_occupancy_voxels")
+            keys, lo = np.empty(max(n.value, 1), np.uint64), np.empty(max(n.value, 1), np.float32)
+            rc = lib().d2pc_occupancy_voxels(self._h, keys.ctypes.data, lo.ctypes.data, keys.size, C.byref(n))
+            if rc != -9:
+                break
+        self._check(rc, "d2pc_occupancy_voxels")
+        keys, lo = keys[: n.value], lo[: n.value]
+        k3 = np.stack([(keys >> np.uint64(16 * a)) & np.uint64(0xFFFF) for a in range(3)], axis=1).astype(np.uint16)
+        return k3, lo
+
+    def occupancy_insert_device(self, d_in, n_frames, n_max, in_stride, d_in_counts, origins):
+        """d2pc_occupancy_insert_device: clouds on the device into the map, frame f from origins[f] (host, (n, 3))."""
+        o = np.ascontiguousarray(origins, np.float32).reshape(-1)
+        assert o.size >= 3 * n_frames
+        self._check(lib().d2pc_occupancy_insert_device(self._h, d_in, n_frames, n_max, in_stride, d_in_counts or None,
+                                                       o.ctypes.data), "d2pc_occupancy_insert_device")
 
     def set_arith_mode(self, m):
         self._check(lib().d2pc_set_arith_mode(self._h, m), "d2pc_set_arith_mode")

@@ -32,6 +32,7 @@
 #include "fusion.h"
 #include "laser_scan.h"
 #include "median.h"
+#include "occupancy.h"
 #include "radius_outlier.h"
 #include "reproject.h"
 #include "score.h"
@@ -64,6 +65,14 @@ struct ScanPlan {
   d2pc_laser_scan msg{};   // the message fields (ranges unset)
 };
 
+// The occupancy map update of a plan (d2pc_set_occupancy): the setting and the sensor origin in force at submission,
+// carried by value (the epoch is given when the step is enqueued).
+struct MapPlan {
+  bool on = false;
+  bool keep_cloud = true;  // false: the cloud stays on the device
+  MapUpdate u{};
+};
+
 // What the filter mode, the cloud transform, the crop box and the radius outlier stage make of one frame geometry
 // (plan_cloud), decided once per call.
 struct CloudPlan {
@@ -76,6 +85,7 @@ struct CloudPlan {
   uint32_t count_words = 1; // count words a slot reads back (Slot::d_count)
   bool fallback_decides_dense = false;  // VOXEL alone: the overflow fallback flag clears is_dense
   ScanPlan scan;                        // the host entries' laser scan (add_scan)
+  MapPlan map;                          // the host entries' occupancy map update (add_map)
 };
 
 // The device buffers between a batch's input frames and its cloud: one set per slot, one for the device batch.
@@ -99,6 +109,8 @@ struct Slot {
   uint32_t *h_count = nullptr;  // pinned
   cudaEvent_t ev_h2d = nullptr, ev_kernel = nullptr, ev_d2h = nullptr;
   cudaEvent_t ev_start = nullptr;  // recorded in front of the H2D copy when per-call timing is on (d2pc_set_timing)
+  cudaEvent_t ev_map = nullptr;    // the map step of the last submission has read the slot's cloud
+  bool map_pending = false;
   bool timed = false;              // the last submission on this slot recorded all four events with timing
   cudaStream_t s_kern = nullptr;  // fusion pipeline: this slot's own kernel stream (small kernels of consecutive sets overlap)
   bool pending = false;
@@ -136,6 +148,13 @@ struct d2pc_ctx {
   ScanPlan scan_plan;           // derived from `scan`
   d2pc_laser_scan last_scan{};  // d2pc_last_scan: the scan of the cloud last returned
   bool last_scan_on = false;
+  d2pc_occupancy_params occ;  // the occupancy map (d2pc_set_occupancy; enabled 0: no updates)
+  DevBuf map_mem;             // the map's table (allocated on first use, cleared then)
+  MapTable map;               // carved from map_mem
+  uint32_t map_epoch = 0;     // of the last frame inserted (marks are tagged with it)
+  DevBuf map_tmp, map_out, map_n;  // export scratch, output staging and counters
+  cudaStream_t s_map = nullptr;    // every map step and export, in submission order
+  cudaEvent_t ev_map_in = nullptr; // orders d2pc_occupancy_insert_device behind the compute stream
   // fusion buffers
   DevBuf d_fuse_in[4], d_container, d_combined, d_fused;
   PinBuf h_fused, h_combined;
@@ -311,8 +330,29 @@ CloudPlan plan_cloud(const d2pc_ctx *ctx, uint32_t w, uint32_t h) {
 void add_scan(const d2pc_ctx *ctx, CloudPlan &p) {
   if (ctx->scan.enabled) p.scan = ctx->scan_plan;
 }
-// the cloud leaves the device (with the scan on and keep_cloud 0 only the ranges do)
-bool cloud_out(const CloudPlan &p) { return !p.scan.on || p.scan.keep_cloud; }
+// The host entries' map update: the context's setting, when it is on, from the cloud transform's translation.
+float log_odds(double p) { return (float)log(p / (1.0 - p)); }
+MapUpdate map_update(const d2pc_ctx *ctx, const float origin[3]) {
+  const d2pc_occupancy_params &q = ctx->occ;
+  MapUpdate u{};
+  for (int a = 0; a < 3; ++a) u.origin[a] = origin[a];
+  u.res = q.resolution, u.rf = 1.0 / q.resolution, u.max_range = q.max_range;
+  u.hit = log_odds(q.prob_hit), u.miss = log_odds(q.prob_miss);
+  u.clamp_min = log_odds(q.clamp_min), u.clamp_max = log_odds(q.clamp_max);
+  return u;
+}
+void add_map(const d2pc_ctx *ctx, CloudPlan &p) {
+  if (!ctx->occ.enabled) return;
+  const float *m = ctx->xform.matrix;
+  const float zero[3] = {0.0f, 0.0f, 0.0f}, t[3] = {m[3], m[7], m[11]};
+  p.map.on = true;
+  p.map.keep_cloud = ctx->occ.keep_cloud != 0;
+  p.map.u = map_update(ctx, ctx->xform.enabled ? t : zero);
+}
+// the cloud leaves the device unless an enabled scan or an enabled map keeps it there (keep_cloud 0)
+bool cloud_out(const CloudPlan &p) {
+  return (!p.scan.on || p.scan.keep_cloud) && (!p.map.on || p.map.keep_cloud);
+}
 
 // A scan setting checked (d2pc_set_laser_scan's rules) and derived.
 int scan_plan_of(const d2pc_laser_scan_params *q, ScanPlan *out) {
@@ -653,6 +693,51 @@ int slot_wait_idle(d2pc_ctx *ctx, Slot &s) {
     CU(ctx, cudaEventSynchronize(s.ev_d2h));
     s.pending = false;
   }
+  if (s.map_pending) {  // the map step still reads the slot's cloud
+    CU(ctx, cudaEventSynchronize(s.ev_map));
+    s.map_pending = false;
+  }
+  return D2PC_OK;
+}
+
+// The map's table, allocated and cleared on s_map on first use (and after a change of max_bricks).
+int map_ready(d2pc_ctx *ctx) {
+  if (ctx->map_mem.p) return D2PC_OK;
+  const int rc = grow_dev(ctx, ctx->map_mem, map_table_bytes(ctx->occ.max_bricks));
+  if (rc) return rc;
+  ctx->map = map_table_carve(ctx->map_mem.p, ctx->occ.max_bricks);
+  CU(ctx, map_clear(ctx->map, true, ctx->s_map));
+  ctx->map_epoch = 0;
+  return D2PC_OK;
+}
+
+// One frame into the map on s_map, after `after` (the kernels that wrote the cloud).  The epoch wraps as next_epoch's
+// does: every mark and slot epoch is cleared with s_map idle.
+int enqueue_map(d2pc_ctx *ctx, MapUpdate u, const CloudSrc &cloud, cudaEvent_t after) {
+  int rc = map_ready(ctx);
+  if (rc) return rc;
+  if (++ctx->map_epoch >= (1u << 30)) {
+    ctx->map_epoch = 1;
+    CU(ctx, cudaStreamSynchronize(ctx->s_map));
+    CU(ctx, cudaMemsetAsync(ctx->map.marks, 0, (size_t)ctx->map.cap * 512 * 4, ctx->s_map));
+    CU(ctx, cudaMemsetAsync(ctx->map.slot_epoch, 0, (size_t)ctx->map.cap * 4, ctx->s_map));
+  }
+  u.epoch = ctx->map_epoch;
+  if (after) CU(ctx, cudaStreamWaitEvent(ctx->s_map, after, 0));
+  int nl = 0;
+  CU(ctx, launch_map_insert(cloud, ctx->map, u, ctx->sm_count, ctx->s_map, &nl));
+  ctx->launches += nl;
+  return D2PC_OK;
+}
+
+// A slot's map step: its cloud `out` (all n points, or the count the device kept), behind ev_kernel.
+int enqueue_slot_map(d2pc_ctx *ctx, Slot &s, const CloudPlan &p, const CloudDst &out) {
+  if (!p.map.on) return D2PC_OK;
+  const CloudSrc cloud{out.points, out.stride, p.counted ? out.counts : nullptr, 1, (uint32_t)p.n};
+  const int rc = enqueue_map(ctx, p.map.u, cloud, s.ev_kernel);
+  if (rc) return rc;
+  CU(ctx, cudaEventRecord(s.ev_map, ctx->s_map));
+  s.map_pending = true;
   return D2PC_OK;
 }
 
@@ -710,6 +795,7 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   const size_t d_pitch = (row_bytes % 16 == 0 || !is_f32) ? row_bytes : round_up(row_bytes, kAlign);
   CloudPlan p = plan_cloud(ctx, w, h);
   add_scan(ctx, p);
+  add_map(ctx, p);
   const uint64_t n = p.n;
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // PointCloud2.row_step / width are uint32
   const bool out_cloud = cloud_out(p);
@@ -723,9 +809,9 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
     return rc;
   // direct output: the kernel's point stores go over PCIe into the page-locked destination while it runs, so a lone
   // frame no longer pays kernel + copy back to back (CROP only: a compacted cloud's size is not known up front; not
-  // with the scan, which reads the cloud on the device)
+  // with the scan or the map, which read the cloud on the device)
   uint8_t *d_direct = nullptr;
-  if (!p.counted && n && !late_copy && !p.scan.on &&
+  if (!p.counted && n && !late_copy && !p.scan.on && !p.map.on &&
       (ctx->direct_out > 0 ||
        (ctx->direct_out == 0 && sync_call && !is_f32 && ctx->cfg.median_ksize > 1 && p.n_stages == 0)))
     d_direct = direct_alias(user_pinned ? user_dst : s.h_out.p);
@@ -770,6 +856,7 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
   }
   if (rc) return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, ctx->s_compute));
+  if ((rc = enqueue_slot_map(ctx, s, p, {s.d_out.p, n * 16 + 16, s.d_count}))) return rc;
 
   NvtxRange nvtx_d2h("d2pc D2H");
   if ((d_direct || late_copy) && !p.scan.on) {
@@ -900,7 +987,9 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
   if (cudaStreamCreateWithFlags(&ctx->s_h2d, cudaStreamNonBlocking) != cudaSuccess ||
       cudaStreamCreateWithFlags(&ctx->s_compute, cudaStreamNonBlocking) != cudaSuccess ||
       cudaStreamCreateWithFlags(&ctx->s_d2h, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaEventCreateWithFlags(&ctx->ev_fuse, cudaEventDisableTiming) != cudaSuccess)
+      cudaEventCreateWithFlags(&ctx->ev_fuse, cudaEventDisableTiming) != cudaSuccess ||
+      cudaStreamCreateWithFlags(&ctx->s_map, cudaStreamNonBlocking) != cudaSuccess ||
+      cudaEventCreateWithFlags(&ctx->ev_map_in, cudaEventDisableTiming) != cudaSuccess)
     return fail(D2PC_ERR_CUDA);
   if (cudaMalloc(&ctx->d_ticket, 64) != cudaSuccess) return fail(D2PC_ERR_NOMEM);
   ctx->slots.resize(c.n_slots);
@@ -908,6 +997,7 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
     if (cudaEventCreateWithFlags(&s.ev_h2d, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&s.ev_kernel, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&s.ev_d2h, cudaEventDisableTiming) != cudaSuccess ||
+        cudaEventCreateWithFlags(&s.ev_map, cudaEventDisableTiming) != cudaSuccess ||
         cudaStreamCreateWithFlags(&s.s_kern, cudaStreamNonBlocking) != cudaSuccess)
       return fail(D2PC_ERR_CUDA);
     if (cudaMalloc(&s.d_count, 64) != cudaSuccess) return fail(D2PC_ERR_NOMEM);
@@ -923,6 +1013,7 @@ int d2pc_create(const d2pc_config *cfg, int device, d2pc_ctx **out) {
   d2pc_cloud_transform_default(&ctx->xform);
   d2pc_laser_scan_params_default(&ctx->scan);
   scan_plan_of(&ctx->scan, &ctx->scan_plan);
+  d2pc_occupancy_params_default(&ctx->occ);
 
   if (const char *v = getenv("D2PC_ROWS_PER_UNIT")) ctx->rows_per_unit = atoi(v);
   if (const char *v = getenv("D2PC_CTAS_PER_SM")) ctx->ctas_per_sm = atoi(v);
@@ -961,6 +1052,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
     if (s.ev_kernel) cudaEventDestroy(s.ev_kernel);
     if (s.ev_d2h) cudaEventDestroy(s.ev_d2h);
     if (s.ev_start) cudaEventDestroy(s.ev_start);
+    if (s.ev_map) cudaEventDestroy(s.ev_map);
     if (s.s_kern) cudaStreamDestroy(s.s_kern);
   }
   free_stages(ctx->batch);
@@ -971,6 +1063,9 @@ void d2pc_destroy(d2pc_ctx *ctx) {
   free_pin(ctx->h_score[0]), free_pin(ctx->h_score[1]);
   free_dev(ctx->d_color_in), free_dev(ctx->d_color_out), free_dev(ctx->d_color_lut), free_pin(ctx->h_color);
   free_pin(ctx->h_stage);
+  free_dev(ctx->map_mem), free_dev(ctx->map_tmp), free_dev(ctx->map_out), free_dev(ctx->map_n);
+  if (ctx->ev_map_in) cudaEventDestroy(ctx->ev_map_in);
+  if (ctx->s_map) cudaStreamDestroy(ctx->s_map);
   if (ctx->d_ticket) cudaFree(ctx->d_ticket);
   if (ctx->ev_fuse) cudaEventDestroy(ctx->ev_fuse);
   if (ctx->s_h2d) cudaStreamDestroy(ctx->s_h2d);
@@ -1111,6 +1206,129 @@ int d2pc_last_scan(const d2pc_ctx *ctx, d2pc_laser_scan *out) {
   *out = ctx->last_scan;
   return D2PC_OK;
 }
+void d2pc_occupancy_params_default(d2pc_occupancy_params *p) {
+  if (!p) return;
+  memset(p, 0, sizeof(*p));
+  p->struct_size = sizeof(*p);
+  p->resolution = 0.05;
+  p->prob_hit = 0.7, p->prob_miss = 0.4;
+  p->clamp_min = 0.12, p->clamp_max = 0.97;
+  p->occupancy_thres = 0.5;
+  p->max_range = -1.0;
+  p->max_bricks = 1u << 18;
+  p->keep_cloud = 1;
+}
+int d2pc_set_occupancy(d2pc_ctx *ctx, const d2pc_occupancy_params *p) {
+  if (!ctx || !p || p->struct_size != sizeof(*p)) return D2PC_ERR_INVALID_ARG;
+  if (!(std::isfinite(p->resolution) && p->resolution > 0.0)) return D2PC_ERR_INVALID_ARG;
+  for (double v : {p->prob_hit, p->prob_miss, p->clamp_min, p->clamp_max, p->occupancy_thres})
+    if (!(v > 0.0 && v < 1.0)) return D2PC_ERR_INVALID_ARG;
+  if (!(p->prob_hit >= 0.5) || !(p->prob_miss <= 0.5) || !(p->clamp_min <= p->clamp_max)) return D2PC_ERR_INVALID_ARG;
+  if (std::isnan(p->max_range) || p->max_bricks == 0 || p->max_bricks > (1u << 26)) return D2PC_ERR_INVALID_ARG;
+  CU(ctx, cudaSetDevice(ctx->device));
+  if (ctx->map_mem.p && p->max_bricks != ctx->occ.max_bricks) {
+    // a new table: every frame submitted so far is done with the old one, which goes (map_ready makes the new one)
+    CU(ctx, cudaStreamSynchronize(ctx->s_map));
+    free_dev(ctx->map_mem);
+  } else if (ctx->map_mem.p && p->resolution != ctx->occ.resolution) {
+    CU(ctx, map_clear(ctx->map, false, ctx->s_map));
+  }
+  ctx->occ = *p;
+  return D2PC_OK;
+}
+int d2pc_get_occupancy(const d2pc_ctx *ctx, d2pc_occupancy_params *p) {
+  if (!ctx || !p) return D2PC_ERR_INVALID_ARG;
+  *p = ctx->occ;
+  return D2PC_OK;
+}
+int d2pc_occupancy_reset(d2pc_ctx *ctx) {
+  if (!ctx) return D2PC_ERR_INVALID_ARG;
+  CU(ctx, cudaSetDevice(ctx->device));
+  if (ctx->map_mem.p) CU(ctx, map_clear(ctx->map, false, ctx->s_map));
+  return D2PC_OK;
+}
+
+// The number of exported voxels (all known, or the occupied ones), read back with s_map idle.
+static int map_export_count(d2pc_ctx *ctx, bool occupied_only, uint32_t *n) {
+  *n = 0;
+  if (!ctx->map_mem.p) return D2PC_OK;  // no frame since the table was made: nothing is known
+  const int rc = grow_dev(ctx, ctx->map_n, 16);
+  if (rc) return rc;
+  CU(ctx, map_count(ctx->map, occupied_only, log_odds(ctx->occ.occupancy_thres), reinterpret_cast<uint32_t *>(ctx->map_n.p),
+                    ctx->s_map));
+  CU(ctx, cudaMemcpyAsync(n, ctx->map_n.p, 4, cudaMemcpyDeviceToHost, ctx->s_map));
+  CU(ctx, cudaStreamSynchronize(ctx->s_map));
+  return D2PC_OK;
+}
+
+// The exported voxels sorted into ctx->map_out: n float4 centres, or n packed keys then n log-odds.
+static int map_export_run(d2pc_ctx *ctx, bool centres, uint32_t n) {
+  int rc;
+  const size_t out_bytes = centres ? (size_t)n * 16 : align_up((size_t)n * 8) + (size_t)n * 4;
+  if ((rc = grow_dev(ctx, ctx->map_tmp, map_export_temp_bytes(n))) || (rc = grow_dev(ctx, ctx->map_out, out_bytes)))
+    return rc;
+  uint8_t *o = ctx->map_out.p;
+  CU(ctx, map_export(ctx->map, centres, log_odds(ctx->occ.occupancy_thres), ctx->occ.resolution, n, ctx->map_tmp.p,
+                     reinterpret_cast<uint32_t *>(ctx->map_n.p) + 1, centres ? reinterpret_cast<float4 *>(o) : nullptr,
+                     centres ? nullptr : reinterpret_cast<unsigned long long *>(o),
+                     centres ? nullptr : reinterpret_cast<float *>(o + align_up((size_t)n * 8)), ctx->s_map));
+  return D2PC_OK;
+}
+
+int d2pc_occupancy_stats(d2pc_ctx *ctx, d2pc_occupancy_info *out) {
+  if (!ctx || !out) return D2PC_ERR_INVALID_ARG;
+  CU(ctx, cudaSetDevice(ctx->device));
+  memset(out, 0, sizeof(*out));
+  uint32_t known = 0, occupied = 0, ctr[4] = {0, 0, 0, 0};
+  unsigned long long frames[2] = {0, 0};
+  int rc;
+  if ((rc = map_export_count(ctx, false, &known)) || (rc = map_export_count(ctx, true, &occupied))) return rc;
+  out->bricks_capacity = ctx->occ.max_bricks;
+  if (!ctx->map_mem.p) return D2PC_OK;
+  CU(ctx, cudaMemcpyAsync(ctr, ctx->map.ctr, sizeof(ctr), cudaMemcpyDeviceToHost, ctx->s_map));
+  CU(ctx, cudaMemcpyAsync(frames, ctx->map.frames, sizeof(frames), cudaMemcpyDeviceToHost, ctx->s_map));
+  CU(ctx, cudaStreamSynchronize(ctx->s_map));
+  out->frames_inserted = frames[0], out->frames_dropped = frames[1];
+  out->known_voxels = known, out->occupied_voxels = occupied;
+  out->bricks_used = ctr[0];
+  return D2PC_OK;
+}
+
+int d2pc_occupancy_centers(d2pc_ctx *ctx, uint8_t *dst, size_t cap, d2pc_cloud *out) {
+  if (!ctx || !out) return D2PC_ERR_INVALID_ARG;
+  CU(ctx, cudaSetDevice(ctx->device));
+  uint32_t n = 0;
+  int rc = map_export_count(ctx, true, &n);
+  if (rc) return rc;
+  if (cap < (size_t)n * 16 || (n && !dst)) {
+    fill_cloud(ctx, nullptr, n, true, out);
+    return D2PC_ERR_BUFFER_TOO_SMALL;
+  }
+  if (n && (rc = map_export_run(ctx, true, n))) return rc;
+  if (n) CU(ctx, cudaMemcpyAsync(dst, ctx->map_out.p, (size_t)n * 16, cudaMemcpyDeviceToHost, ctx->s_map));
+  CU(ctx, cudaStreamSynchronize(ctx->s_map));
+  fill_cloud(ctx, dst, n, true, out);
+  return D2PC_OK;
+}
+
+int d2pc_occupancy_voxels(d2pc_ctx *ctx, uint64_t *keys, float *log_odds_out, uint64_t cap, uint64_t *n_out) {
+  if (!ctx || !n_out) return D2PC_ERR_INVALID_ARG;
+  CU(ctx, cudaSetDevice(ctx->device));
+  uint32_t n = 0;
+  int rc = map_export_count(ctx, false, &n);
+  if (rc) return rc;
+  *n_out = n;
+  if (cap < n || (n && (!keys || !log_odds_out))) return D2PC_ERR_BUFFER_TOO_SMALL;
+  if (n && (rc = map_export_run(ctx, false, n))) return rc;
+  if (n) {
+    CU(ctx, cudaMemcpyAsync(keys, ctx->map_out.p, (size_t)n * 8, cudaMemcpyDeviceToHost, ctx->s_map));
+    CU(ctx, cudaMemcpyAsync(log_odds_out, ctx->map_out.p + align_up((size_t)n * 8), (size_t)n * 4,
+                            cudaMemcpyDeviceToHost, ctx->s_map));
+  }
+  CU(ctx, cudaStreamSynchronize(ctx->s_map));
+  return D2PC_OK;
+}
+
 int d2pc_set_arith_mode(d2pc_ctx *ctx, int m) {
   if (!ctx || m < 0 || m > 1) return D2PC_ERR_INVALID_ARG;
   ctx->cfg.arith_mode = m;
@@ -1471,6 +1689,25 @@ int d2pc_laser_scan_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames
   return D2PC_OK;
 }
 
+int d2pc_occupancy_insert_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
+                                 size_t in_stride, const uint32_t *d_in_counts, const float *origins) {
+  if (!ctx || !d_in || !origins || !ctx->occ.enabled) return D2PC_ERR_INVALID_ARG;
+  const uint64_t bytes = (uint64_t)n_max * 16;
+  if (bytes > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // the argument rules of the other cloud stages
+  if (reinterpret_cast<uintptr_t>(d_in) % 16 || in_stride % 16 || (n_frames > 1 && in_stride < bytes))
+    return D2PC_ERR_BAD_DIMS;
+  if (n_frames == 0) return D2PC_OK;
+  CU(ctx, cudaSetDevice(ctx->device));
+  CU(ctx, cudaEventRecord(ctx->ev_map_in, ctx->s_compute));
+  // one frame per map step: a frame of at most 2^28 points is always within kCloudMaxPoints, so no chunk spans frames
+  for (uint32_t f = 0; f < n_frames; ++f) {
+    const CloudSrc in{d_in + (size_t)f * in_stride, in_stride, d_in_counts ? d_in_counts + f : nullptr, 1, n_max};
+    const int rc = enqueue_map(ctx, map_update(ctx, origins + 3 * (size_t)f), in, f == 0 ? ctx->ev_map_in : nullptr);
+    if (rc) return rc;
+  }
+  return D2PC_OK;
+}
+
 int d2pc_reproject_f32_device(d2pc_ctx *ctx, const float *d_disp, uint32_t n_frames, uint32_t w, uint32_t h,
                               size_t step, size_t frame_stride, uint8_t *d_points, size_t points_stride,
                               uint32_t *d_counts) {
@@ -1515,6 +1752,7 @@ int d2pc_sync(d2pc_ctx *ctx) {
   for (auto &s : ctx->slots)
     if (s.s_kern) CU(ctx, cudaStreamSynchronize(s.s_kern));
   CU(ctx, cudaStreamSynchronize(ctx->s_d2h));
+  CU(ctx, cudaStreamSynchronize(ctx->s_map));
   return D2PC_OK;
 }
 uint64_t d2pc_launch_count(const d2pc_ctx *ctx) { return ctx ? ctx->launches : 0; }
@@ -1795,13 +2033,14 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
   CloudPlan p = plan_cloud(ctx, fw, fh);
   add_scan(ctx, p);
+  add_map(ctx, p);
   const uint64_t n = p.n;
   if (cloud_out(p) && (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
   if (p.scan.on && ((rc = grow_dev(ctx, s.d_ranges, (size_t)p.scan.p.n * 4)) ||
                     (rc = grow_pin(ctx, s.h_ranges, (size_t)p.scan.p.n * 4))))
     return rc;
   // a synchronous call: the callback kernel stores the CROP cloud straight into the pinned buffer (see submit_common)
-  const bool direct = !p.scan.on && (ctx->direct_out > 0 || (ctx->direct_out == 0 && p.n_stages == 0));
+  const bool direct = !p.scan.on && !p.map.on && (ctx->direct_out > 0 || (ctx->direct_out == 0 && p.n_stages == 0));
   uint8_t *const d_direct =
       !p.counted && n && direct && ctx->cfg.median_ksize > 1 ? direct_alias(s.h_out.p) : nullptr;
   if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
@@ -1810,6 +2049,10 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
       (rc = enqueue_kernels(ctx, p, fused, s.stages, {d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count},
                             s.d_count + 2, s.d_count + 1, ctx->s_compute, reinterpret_cast<float *>(s.d_ranges.p))))
     return rc;
+  if (p.map.on) {
+    CU(ctx, cudaEventRecord(s.ev_kernel, ctx->s_compute));
+    if ((rc = enqueue_slot_map(ctx, s, p, {s.d_out.p, n * 16 + 16, s.d_count}))) return rc;
+  }
   if (p.scan.on && p.scan.p.n)
     CU(ctx, cudaMemcpyAsync(s.h_ranges.p, s.d_ranges.p, (size_t)p.scan.p.n * 4, cudaMemcpyDeviceToHost, ctx->s_compute));
   if (p.counted && cloud_out(p)) {
@@ -1849,6 +2092,7 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
   CloudPlan p = plan_cloud(ctx, fw, fh);
   add_scan(ctx, p);
+  add_map(ctx, p);
   const uint64_t n = p.n;
   if (p.scan.on && ((rc = grow_dev(ctx, s.d_ranges, (size_t)p.scan.p.n * 4)) ||
                     (rc = grow_pin(ctx, s.h_ranges, (size_t)p.scan.p.n * 4))))
@@ -1908,6 +2152,8 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
                             s.d_count + 1, sk, reinterpret_cast<float *>(s.d_ranges.p))))
     return rc;
   CU(ctx, cudaEventRecord(s.ev_kernel, sk));
+  // the map step runs on s_map behind this slot's kernel stream, so fusion slots update the map in submission order
+  if ((rc = enqueue_slot_map(ctx, s, p, {s.d_out.p, n * 16 + 16, s.d_count}))) return rc;
   if ((rc = enqueue_readback(ctx, s, p, s.h_out.p))) return rc;
   arm_slot(s, p, nullptr, 0, false, false);
   return D2PC_OK;

@@ -1,0 +1,58 @@
+// occupancy.h -- host-side launcher interface of occupancy.cu: the device occupancy map (octomap_server's insertScan
+// on a depth-16 OcTree, the recipe is in include/d2pc_b200.h) and its export.  Input is cloud_stage.cuh's.
+#pragma once
+#include "cloud_stage.cuh"
+
+namespace d2pc {
+
+// A hash of 8x8x8-voxel bricks, open addressing on the brick key (key >> 3 per axis, packed 16 bits per axis).  Slot s
+// owns its brick's storage: 512 float log-odds, a 512-bit known mask and 512 epoch-tagged mark words, so a brick
+// needs no allocator.  All of it lives in one device allocation (map_table_bytes / map_table_carve).
+struct MapTable {
+  unsigned long long *keys = nullptr;  // cap slots, kMapEmpty when free
+  float *log_odds = nullptr;           // cap * 512
+  uint32_t *known = nullptr;           // cap * 16 mask words: bit i of word w is voxel 32 w + i
+  uint32_t *marks = nullptr;           // cap * 512: epoch * 4 + 3 (hit) or + 2 (miss), monotone within an epoch range
+  uint32_t *slot_epoch = nullptr;      // cap: the last epoch that touched the slot
+  uint32_t *touched = nullptr;         // cap: the slots touched in the current epoch
+  uint32_t *ctr = nullptr;             // [0] bricks created, [1] overflow flag, [2] touched slots
+  unsigned long long *frames = nullptr;  // [0] frames applied, [1] frames dropped (overflow)
+  uint32_t cap = 0;         // slots: a power of two, at least 2 * max_bricks
+  uint32_t max_bricks = 0;  // bricks a frame may bring the map to
+};
+
+constexpr unsigned long long kMapEmpty = ~0ull;
+
+// One frame's update, decided on the host and carried by value into its launches.
+struct MapUpdate {
+  float origin[3];     // the sensor origin
+  double res, rf;      // resolution and 1.0 / resolution
+  double max_range;    // < 0: unlimited
+  float hit, miss;     // log-odds updates
+  float clamp_min, clamp_max;
+  uint32_t epoch;      // 1 .. 2^30 - 1
+};
+
+// Slots of the table for max_bricks, and the bytes of its allocation (256-byte aligned parts).
+uint32_t map_table_cap(uint32_t max_bricks);
+size_t map_table_bytes(uint32_t max_bricks);
+MapTable map_table_carve(uint8_t *base, uint32_t max_bricks);
+
+// The empty map (keys, known masks, counters).  marks_too: also every mark and slot epoch (the epoch wrapped).
+cudaError_t map_clear(const MapTable &t, bool marks_too, cudaStream_t stream);
+
+// One frame into the map: mark (every point's ray and endpoint), apply (the touched slots; nothing on overflow) and
+// finish (frame counters, flags cleared): three launches.  `in` holds exactly one frame.
+cudaError_t launch_map_insert(const CloudSrc &in, const MapTable &t, const MapUpdate &u, int sm_count,
+                              cudaStream_t stream, int *launches);
+
+// Export.  map_count: the known voxels (occupied_only: those with log-odds >= occ_thres) into *d_n.  map_export:
+// the same voxels sorted by Morton code into centres (float4 {x, y, z, 1}) or (packed key, log-odds); temp holds
+// map_export_temp_bytes(n).
+cudaError_t map_count(const MapTable &t, bool occupied_only, float occ_thres, uint32_t *d_n, cudaStream_t stream);
+size_t map_export_temp_bytes(uint32_t n);
+cudaError_t map_export(const MapTable &t, bool occupied_only, float occ_thres, double res, uint32_t n, void *temp,
+                       uint32_t *d_pos, float4 *centres, unsigned long long *keys, float *log_odds,
+                       cudaStream_t stream);
+
+}  // namespace d2pc

@@ -427,6 +427,117 @@ int d2pc_last_scan(const d2pc_ctx *ctx, d2pc_laser_scan *out);
 int d2pc_laser_scan_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
                            const uint32_t *d_in_counts, float *d_ranges, size_t ranges_stride);
 
+/* ---- occupancy map (octomap_server's insertScan on the device, updated by every published cloud) -------------------
+ *
+ * Off by default (enabled 0).  With the map on, every host entry point that publishes a cloud (the process_* and
+ * *_into calls, submit / d2pc_wait, d2pc_process_stream, d2pc_submit_fusion, d2pc_process_fusion_stream and
+ * d2pc_fuse_then_process) also inserts exactly that cloud -- after the transform, the crop box, VOXEL and the outlier
+ * stage, in the cloud's frame -- into one occupancy map the context keeps on the device.  The d2pc_reproject_*_device
+ * batches do not update it; d2pc_occupancy_insert_device inserts clouds already on the device.
+ * Reference: OctomapServer::insertScan (octomap_server) with filter_ground off and compress_map off, on an
+ * octomap::OcTree of depth 16, restated from memory (neither octomap's nor octomap_server's source was at hand when
+ * this was written -- the footing of the laser scan above).  The recipe:
+ *   - origin: o = the cloud transform's translation (m03, m13, m23) when the transform is on, else (0, 0, 0); a float
+ *     point3d.
+ *   - a point with a non-finite x, y or z is skipped (the pass-through filters drop NaN; coordToKey of +-inf is
+ *     undefined).
+ *   - keys: per axis k = (int)floor(res_factor * (double)c) + 32768 with res_factor = 1.0 / resolution (double); valid
+ *     only when 0 <= k < 65536 (coordToKeyChecked).  A key's centre is ((double)(k - 32768) + 0.5) * resolution.
+ *   - range test: d = (p - o).norm(): float subtracts, the sum of squares ((x*x + y*y) + z*z) in float with no FMA,
+ *     widened to double, a double sqrt.
+ *       - max_range < 0 or d <= max_range: the free cells of computeRayKeys(o, p) join the frame's free set, and
+ *         key(p) joins its occupied set when valid;
+ *       - otherwise e = o + normalized(p - o) * (float)max_range (octomath's float normalize: each component divided
+ *         by (float)norm), and the free cells of computeRayKeys(o, e) join the free set; no occupied cell.
+ *   - computeRayKeys(o, e), Amanatides & Woo in 3-D:
+ *       1. empty when either key is invalid or the two keys are equal;
+ *       2. otherwise the ray starts with the origin's key;
+ *       3. length = (float)norm(e - o), dir = (e - o) / length in float;
+ *       4. per axis: step = sign(dir); tMax = (centre(k_o) + (double)(float)(step * res * 0.5) - (double)o) /
+ *          (double)dir and tDelta = res / fabs(dir), in double; DBL_MAX for both when dir is 0;
+ *       5. loop: the axis of the least tMax with strict < in octomap's nesting (tMax0 < tMax1 ? (tMax0 < tMax2 ? 0 : 2)
+ *          : (tMax1 < tMax2 ? 1 : 2)); step the key (uint16) and add tDelta; stop when the key equals the end key (not
+ *          added) or when min(tMax) > length; otherwise add the key.
+ *     csrc/map_math.h holds this math once for the kernels and the C reference.
+ *   - update, after every point of the frame: each key of the free set that is not in the occupied set gets one miss,
+ *     each key of the occupied set one hit.  A key is updated once per frame, so the order within a frame does not
+ *     matter.
+ *   - updateNode(key, update): a known voxel that is already >= clamp_max under an update >= 0, or <= clamp_min under
+ *     an update <= 0, is left as it is (the early abort -- it matters when the clamp bounds change between frames);
+ *     otherwise value = value + update in float (a new voxel starts at 0), then clamped to [clamp_min, clamp_max].
+ *   - log-odds: prob_hit, prob_miss, clamp_min, clamp_max and occupancy_thres are probabilities, each converted on the
+ *     host as octomap does, (float)log(p / (1 - p)).  A voxel is occupied when log_odds >= occ_thres_log.
+ * What rests on recollection and is not verified against the sources: the float / double mix of the DDA (float
+ * direction and length, double tMax and tDelta, the float cast of the half-voxel offset); octomath's normalize and
+ * norm as float sums; the early abort; that a new voxel starts at log-odds 0; that the max-range branch adds no cell
+ * for e itself (some octomap_server versions also mark key(e) free); octomap_server's param names and defaults
+ * (resolution 0.05, sensor_model/hit 0.7, /miss 0.4, /min 0.12, /max 0.97, occupancy 0.5 as the OcTree default,
+ * sensor_model/max_range -1).
+ * Export: the known voxels in Morton order (bits interleaved z, y, x from bit 15 down), which is octomap's leaf
+ * iterator order at full depth.  d2pc_occupancy_centers is then what octomap_server publishes on
+ * octomap_point_cloud_centers with compress_map off, byte for byte: {(float)centre(kx), (float)centre(ky),
+ * (float)centre(kz), 1.0f} per occupied voxel.  octomap merges eight equal siblings into one coarser leaf when it
+ * prunes (compress_map on, and as recalled also inside updateNode); it would then publish one coarser point for a
+ * uniform octant where this library publishes the eight full-depth voxels with the same value.
+ * The device map: a hash of 8x8x8-voxel bricks (max_bricks of them; the table has 2 * max_bricks slots rounded up to a
+ * power of two, each about 4.2 KB).  A frame that would take the map past max_bricks bricks is dropped as a whole: the
+ * known map stays bit for bit what it was and d2pc_occupancy_stats counts the drop.  Bricks made by a dropped frame stay
+ * unknown (invisible to the export) but count as used.
+ * Ordering: updates follow submission order (fusion slots too); the map step of a slot reads its cloud before the slot
+ * can be reused.  A d2pc_wait that returns D2PC_ERR_BUFFER_TOO_SMALL has still updated the map.  Plans with the map
+ * never store the cloud from the kernel into host memory ("direct_out").
+ * keep_cloud: the cloud leaves the device unless an enabled scan or an enabled map says keep_cloud 0; then the host
+ * entries return a cloud of width 0, data NULL, is_dense 1 (the laser scan's rules above). */
+typedef struct d2pc_occupancy_params {
+  uint32_t struct_size; /* sizeof(d2pc_occupancy_params) */
+  int32_t enabled;      /* 0: off (the default); the map stays readable */
+  double resolution;    /* 0.05 (m); finite, > 0.  A change clears the map */
+  double prob_hit, prob_miss;     /* 0.7, 0.4; in (0, 1), hit >= 0.5 >= miss */
+  double clamp_min, clamp_max;    /* 0.12, 0.97; in (0, 1), min <= max */
+  double occupancy_thres;         /* 0.5; in (0, 1): the export's occupied test */
+  double max_range;               /* -1 (m): negative means unlimited; not NaN */
+  uint32_t max_bricks;            /* 262144 (about 2.2 GB of device memory); >= 1, <= 2^26.  A change clears the map */
+  int32_t keep_cloud;             /* 1: the cloud is produced as well; 0: it stays on the device */
+} d2pc_occupancy_params;
+
+/* Counters of the map (d2pc_occupancy_stats). */
+typedef struct d2pc_occupancy_info {
+  uint64_t frames_inserted; /* frames applied since the map was last cleared */
+  uint64_t frames_dropped;  /* frames dropped because the map would pass max_bricks */
+  uint64_t known_voxels, occupied_voxels;
+  uint64_t bricks_used, bricks_capacity;
+} d2pc_occupancy_info;
+
+/* enabled 0, keep_cloud 1, octomap_server's defaults above. */
+void d2pc_occupancy_params_default(d2pc_occupancy_params *p);
+/* D2PC_ERR_INVALID_ARG, keeping the previous setting, for: a resolution that is not finite and > 0; a probability
+ * outside (0, 1); prob_hit < 0.5 or prob_miss > 0.5; clamp_min > clamp_max; a NaN max_range; max_bricks 0 or above
+ * 2^26; a wrong struct_size.  A change of resolution or max_bricks clears the map (every frame submitted before the
+ * call); every other field travels by value into each submission, like the transform's pose. */
+int d2pc_set_occupancy(d2pc_ctx *ctx, const d2pc_occupancy_params *p);
+/* The setting last made (d2pc_occupancy_params_default's until then). */
+int d2pc_get_occupancy(const d2pc_ctx *ctx, d2pc_occupancy_params *p);
+/* Clears the map: every frame submitted before the call is gone, frames submitted after it are inserted. */
+int d2pc_occupancy_reset(d2pc_ctx *ctx);
+/* Synchronous; reflects every frame submitted before the call. */
+int d2pc_occupancy_stats(d2pc_ctx *ctx, d2pc_occupancy_info *out);
+/* The centres of the occupied voxels (log_odds >= the current occupancy_thres) as a PointCloud2 of 16-byte PointXYZ
+ * {x, y, z, 1.0f} in Morton order, written to dst (cap bytes); *out describes it (is_dense 1, data = dst).
+ * Synchronous; reflects every frame submitted before the call.  D2PC_ERR_BUFFER_TOO_SMALL when cap < 16 * n, with
+ * out->width = n and out->data NULL. */
+int d2pc_occupancy_centers(d2pc_ctx *ctx, uint8_t *dst, size_t cap, d2pc_cloud *out);
+/* Every known voxel in Morton order: keys[i] = kx | ky << 16 | kz << 32 and its log-odds.  *n = the number of known
+ * voxels; D2PC_ERR_BUFFER_TOO_SMALL when cap < *n (nothing written).  Synchronous, like d2pc_occupancy_centers. */
+int d2pc_occupancy_voxels(d2pc_ctx *ctx, uint64_t *keys, float *log_odds, uint64_t cap, uint64_t *n);
+/* Inserts clouds already on the device, frame f (in order) from the host origin origins[3f .. 3f+2], with the
+ * context's setting, which must be enabled.  The input follows d2pc_crop_box_device's rules: frame f at d_in +
+ * f*in_stride bytes, d_in_counts[f] points (NULL: n_max each; above n_max counts as n_max), pointers and strides
+ * 16-byte aligned, in_stride >= 16*n_max when n_frames > 1, n_max*16 < 2^32, batches of more than 2^31 - 2 points run
+ * in chunks of frames.  Asynchronous: the map step runs after the work queued on the compute stream
+ * (d2pc_compute_stream) and after every earlier map update; d2pc_sync waits for it. */
+int d2pc_occupancy_insert_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
+                                 size_t in_stride, const uint32_t *d_in_counts, const float *origins);
+
 /* ---- the disparity callback, host buffers (the reference-facing calls) ------ */
 
 /* Whole DisparityCb (src/disparity_to_point_cloud.cpp:46-92) on one mono8

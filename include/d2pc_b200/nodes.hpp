@@ -230,8 +230,10 @@ class Disparity2PCloud {
   int border_ = 40;  // cpp:70,72
   std::string frame_id_ = "/camera_optical_frame";  // cpp:89; transform_target_frame with the transform on
   std::string p_scan_topic_;  // "/scan" when scan_enable != 0
-  bool publish_cloud_ = true;  // false with scan_keep_cloud 0: only /scan is published
+  bool publish_cloud_ = true;  // false with scan_keep_cloud 0 or map_keep_cloud 0: /point_cloud is not published
   sensor_msgs::LaserScan scan_;
+  std::string p_map_topic_;  // "/octomap_point_cloud_centers" when map_enable != 0
+  sensor_msgs::PointCloud2 centres_;
 
   // make output_.data hold `bytes` bytes in page-locked storage without touching bytes it already has
   void reserve_output(size_t bytes) {
@@ -356,6 +358,33 @@ class Disparity2PCloud {
       publish_cloud_ = s.keep_cloud != 0;
       p_scan_topic_ = nh_.advertise("/scan", 1);
     }
+    // optional, not in the reference: octomap_server's insertScan on the device, every published cloud inserted into
+    // one occupancy map, whose occupied voxel centres go out on /octomap_point_cloud_centers with the cloud's header
+    // after each frame; on when map_enable != 0.  map_resolution, map_sensor_model_{hit,miss,min,max},
+    // map_occupancy_thres and map_max_range are octomap_server's resolution, sensor_model/* and occupancy params with
+    // its defaults; map_max_bricks sizes the device map; map_keep_cloud 0 leaves the cloud on the device and
+    // /point_cloud unpublished.  The sensor origin is the transform's translation: set the transform params.
+    int map_on = 0;
+    nh_.param<int>("map_enable", map_on, 0);
+    if (map_on) {
+      d2pc_occupancy_params o;
+      d2pc_occupancy_params_default(&o);
+      o.enabled = 1;
+      int bricks = static_cast<int>(o.max_bricks);
+      nh_.param<double>("map_resolution", o.resolution, o.resolution);
+      nh_.param<double>("map_sensor_model_hit", o.prob_hit, o.prob_hit);
+      nh_.param<double>("map_sensor_model_miss", o.prob_miss, o.prob_miss);
+      nh_.param<double>("map_sensor_model_min", o.clamp_min, o.clamp_min);
+      nh_.param<double>("map_sensor_model_max", o.clamp_max, o.clamp_max);
+      nh_.param<double>("map_occupancy_thres", o.occupancy_thres, o.occupancy_thres);
+      nh_.param<double>("map_max_range", o.max_range, o.max_range);
+      nh_.param<int>("map_max_bricks", bricks, bricks);
+      nh_.param<int>("map_keep_cloud", o.keep_cloud, 1);
+      o.max_bricks = bricks > 0 ? static_cast<uint32_t>(bricks) : 0u;  // 0 is refused
+      d2pc_b200::check(d2pc_set_occupancy(ctx_, &o), "d2pc_set_occupancy", ctx_);
+      publish_cloud_ = publish_cloud_ && o.keep_cloud != 0;
+      p_map_topic_ = nh_.advertise("/octomap_point_cloud_centers", 1);
+    }
   }
   ~Disparity2PCloud() {
     d2pc_destroy(ctx_);  // waits for the device: nothing writes into output_ any more
@@ -379,36 +408,54 @@ class Disparity2PCloud {
                                              output_.data.size(), &cloud),
                      "d2pc_process_mono8_into", ctx_);
     sensor_msgs::PointCloud2 &output = output_;  // pcl::toROSMsg(*cloud, output), cpp:84-85 -- the bytes are already there
-    output.height = cloud.height;
-    output.width = cloud.width;
-    output.fields.clear();
+    // CROP_FINITE / VOXEL / the radius outlier stage keep fewer points than the crop holds: shrink the view, never
+    // the storage
+    describe(cloud, output);
+    output.header.stamp = msg->header.stamp;             // cpp:87
+    output.header.frame_id = frame_id_;                  // cpp:89
+    if (publish_cloud_) nh_.publish(p_cloud_topic_, output);  // cpp:90
+    if (!p_scan_topic_.empty()) {
+      d2pc_laser_scan s;
+      d2pc_b200::check(d2pc_last_scan(ctx_, &s), "d2pc_last_scan", ctx_);
+      scan_.header = output.header;
+      scan_.angle_min = s.angle_min, scan_.angle_max = s.angle_max, scan_.angle_increment = s.angle_increment;
+      scan_.time_increment = s.time_increment, scan_.scan_time = s.scan_time;
+      scan_.range_min = s.range_min, scan_.range_max = s.range_max;
+      scan_.ranges.assign(s.ranges, s.ranges + s.n_ranges);
+      nh_.publish(p_scan_topic_, scan_);
+    }
+    if (!p_map_topic_.empty()) {
+      // the map's occupied voxel centres after this frame (octomap_server's octomap_point_cloud_centers)
+      d2pc_cloud c;
+      int rc = d2pc_occupancy_centers(ctx_, centres_.data.data(), centres_.data.size(), &c);
+      if (rc == D2PC_ERR_BUFFER_TOO_SMALL) {
+        centres_.data.resize(static_cast<size_t>(c.width) * 16);
+        rc = d2pc_occupancy_centers(ctx_, centres_.data.data(), centres_.data.size(), &c);
+      }
+      d2pc_b200::check(rc, "d2pc_occupancy_centers", ctx_);
+      describe(c, centres_);
+      centres_.header = output.header;
+      nh_.publish(p_map_topic_, centres_);
+    }
+  }
+  // a PointCloud2's fields from the library's d2pc_cloud; data keeps its storage and shows the cloud's bytes
+  static void describe(const d2pc_cloud &cloud, sensor_msgs::PointCloud2 &m) {
+    m.height = cloud.height;
+    m.width = cloud.width;
+    m.fields.clear();
     for (uint32_t i = 0; i < cloud.n_fields; ++i) {
       sensor_msgs::PointField f;
       f.name = cloud.fields[i].name;
       f.offset = cloud.fields[i].offset;
       f.datatype = cloud.fields[i].datatype;
       f.count = cloud.fields[i].count;
-      output.fields.push_back(f);
+      m.fields.push_back(f);
     }
-    output.is_bigendian = cloud.is_bigendian;
-    output.point_step = cloud.point_step;
-    output.row_step = cloud.row_step;
-    output.is_dense = cloud.is_dense;
-    // CROP_FINITE / VOXEL / the radius outlier stage keep fewer points than the crop holds: shrink the view, never
-    // the storage
-    output.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
-    output.header.stamp = msg->header.stamp;             // cpp:87
-    output.header.frame_id = frame_id_;                  // cpp:89
-    if (publish_cloud_) nh_.publish(p_cloud_topic_, output);  // cpp:90
-    if (p_scan_topic_.empty()) return;
-    d2pc_laser_scan s;
-    d2pc_b200::check(d2pc_last_scan(ctx_, &s), "d2pc_last_scan", ctx_);
-    scan_.header = output.header;
-    scan_.angle_min = s.angle_min, scan_.angle_max = s.angle_max, scan_.angle_increment = s.angle_increment;
-    scan_.time_increment = s.time_increment, scan_.scan_time = s.scan_time;
-    scan_.range_min = s.range_min, scan_.range_max = s.range_max;
-    scan_.ranges.assign(s.ranges, s.ranges + s.n_ranges);
-    nh_.publish(p_scan_topic_, scan_);
+    m.is_bigendian = cloud.is_bigendian;
+    m.point_step = cloud.point_step;
+    m.row_step = cloud.row_step;
+    m.is_dense = cloud.is_dense;
+    m.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
   }
 };
 

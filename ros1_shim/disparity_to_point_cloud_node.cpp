@@ -162,6 +162,38 @@ class Disparity2PCloudGpu {
         scan_on_ = true;
       }
     }
+    // optional, not in the reference: octomap_server's insertScan on the device; the occupied voxel centres go out
+    // on /octomap_point_cloud_centers with the cloud's header after each frame, on when map_enable != 0.  The params
+    // are octomap_server's with its defaults (map_resolution, map_sensor_model_{hit,miss,min,max},
+    // map_occupancy_thres, map_max_range), map_max_bricks and map_keep_cloud (0: /point_cloud is not published).
+    // The sensor origin is the transform's translation: set transform_*.
+    int map_on = 0;
+    nh_.param<int>("map_enable", map_on, 0);
+    if (map_on) {
+      d2pc_occupancy_params o;
+      d2pc_occupancy_params_default(&o);
+      o.enabled = 1;
+      int bricks = static_cast<int>(o.max_bricks), keep = 1;
+      nh_.param<double>("map_resolution", o.resolution, o.resolution);
+      nh_.param<double>("map_sensor_model_hit", o.prob_hit, o.prob_hit);
+      nh_.param<double>("map_sensor_model_miss", o.prob_miss, o.prob_miss);
+      nh_.param<double>("map_sensor_model_min", o.clamp_min, o.clamp_min);
+      nh_.param<double>("map_sensor_model_max", o.clamp_max, o.clamp_max);
+      nh_.param<double>("map_occupancy_thres", o.occupancy_thres, o.occupancy_thres);
+      nh_.param<double>("map_max_range", o.max_range, o.max_range);
+      nh_.param<int>("map_max_bricks", bricks, bricks);
+      nh_.param<int>("map_keep_cloud", keep, 1);
+      o.max_bricks = bricks > 0 ? static_cast<uint32_t>(bricks) : 0u;  // 0 is refused
+      o.keep_cloud = keep;
+      if (d2pc_set_occupancy(ctx_, &o) != D2PC_OK) {
+        ROS_FATAL("map_*: not a valid occupancy map setting");
+        ros::shutdown();
+      } else {
+        publish_cloud_ = publish_cloud_ && keep != 0;
+        map_pub_ = nh_.advertise<sensor_msgs::PointCloud2>("/octomap_point_cloud_centers", 1);
+        map_on_ = true;
+      }
+    }
   }
   ~Disparity2PCloudGpu() {
     d2pc_destroy(ctx_);
@@ -197,39 +229,61 @@ class Disparity2PCloudGpu {
       ROS_ERROR("d2pc_process_mono8_into: %s (%s)", d2pc_strerror(rc), d2pc_last_cuda_error(ctx_));
       return;
     }
-    out.height = cloud.height;
-    out.width = cloud.width;
-    out.fields.resize(cloud.n_fields);
-    for (uint32_t i = 0; i < cloud.n_fields; ++i) {
-      out.fields[i].name = cloud.fields[i].name;
-      out.fields[i].offset = cloud.fields[i].offset;
-      out.fields[i].datatype = cloud.fields[i].datatype;
-      out.fields[i].count = cloud.fields[i].count;
-    }
-    out.is_bigendian = cloud.is_bigendian;
-    out.point_step = cloud.point_step;
-    out.row_step = cloud.row_step;
-    out.is_dense = cloud.is_dense;
-    out.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
+    describe(cloud, out);
     out.header.stamp = msg->header.stamp;
     out.header.frame_id = frame_id_;
     if (publish_cloud_) pub_.publish(out);
-    if (!scan_on_) return;
     d2pc_laser_scan s;
-    if (d2pc_last_scan(ctx_, &s) != D2PC_OK) return;
-    scan_.header = out.header;
-    scan_.angle_min = s.angle_min, scan_.angle_max = s.angle_max, scan_.angle_increment = s.angle_increment;
-    scan_.time_increment = s.time_increment, scan_.scan_time = s.scan_time;
-    scan_.range_min = s.range_min, scan_.range_max = s.range_max;
-    scan_.ranges.assign(s.ranges, s.ranges + s.n_ranges);
-    scan_pub_.publish(scan_);
+    if (scan_on_ && d2pc_last_scan(ctx_, &s) == D2PC_OK) {
+      scan_.header = out.header;
+      scan_.angle_min = s.angle_min, scan_.angle_max = s.angle_max, scan_.angle_increment = s.angle_increment;
+      scan_.time_increment = s.time_increment, scan_.scan_time = s.scan_time;
+      scan_.range_min = s.range_min, scan_.range_max = s.range_max;
+      scan_.ranges.assign(s.ranges, s.ranges + s.n_ranges);
+      scan_pub_.publish(scan_);
+    }
+    if (!map_on_) return;
+    // the map's occupied voxel centres after this frame (octomap_server's octomap_point_cloud_centers)
+    d2pc_cloud c;
+    int mrc = d2pc_occupancy_centers(ctx_, centres_.data.data(), centres_.data.size(), &c);
+    if (mrc == D2PC_ERR_BUFFER_TOO_SMALL) {
+      centres_.data.resize(static_cast<size_t>(c.width) * 16);
+      mrc = d2pc_occupancy_centers(ctx_, centres_.data.data(), centres_.data.size(), &c);
+    }
+    if (mrc != D2PC_OK) {
+      ROS_ERROR("d2pc_occupancy_centers: %s (%s)", d2pc_strerror(mrc), d2pc_last_cuda_error(ctx_));
+      return;
+    }
+    describe(c, centres_);
+    centres_.header = out.header;
+    map_pub_.publish(centres_);
+  }
+
+  // a PointCloud2's fields from the library's d2pc_cloud; data keeps its storage and shows the cloud's bytes
+  static void describe(const d2pc_cloud &cloud, sensor_msgs::PointCloud2 &m) {
+    m.height = cloud.height;
+    m.width = cloud.width;
+    m.fields.resize(cloud.n_fields);
+    for (uint32_t i = 0; i < cloud.n_fields; ++i) {
+      m.fields[i].name = cloud.fields[i].name;
+      m.fields[i].offset = cloud.fields[i].offset;
+      m.fields[i].datatype = cloud.fields[i].datatype;
+      m.fields[i].count = cloud.fields[i].count;
+    }
+    m.is_bigendian = cloud.is_bigendian;
+    m.point_step = cloud.point_step;
+    m.row_step = cloud.row_step;
+    m.is_dense = cloud.is_dense;
+    m.data.resize(static_cast<size_t>(cloud.row_step) * cloud.height);
   }
 
  private:
   ros::NodeHandle nh_;
   ros::Subscriber sub_;
-  ros::Publisher pub_, scan_pub_;
-  bool scan_on_ = false, publish_cloud_ = true;  // scan_enable, scan_keep_cloud
+  ros::Publisher pub_, scan_pub_, map_pub_;
+  bool scan_on_ = false, map_on_ = false;  // scan_enable, map_enable
+  bool publish_cloud_ = true;              // scan_keep_cloud and map_keep_cloud
+  sensor_msgs::PointCloud2 centres_;       // /octomap_point_cloud_centers
   sensor_msgs::LaserScan scan_;
   d2pc_ctx *ctx_ = nullptr;
   sensor_msgs::PointCloud2 out_;   // persistent so that its data storage can stay page-locked

@@ -11,6 +11,9 @@
 //   d2pc_offline node1scan <launch file> <w> <h> <in.raw> <cloud.bin> <scan.bin>
 //       node1 with the /scan subscriber too (scan_enable in the launch file): the PointCloud2 (an empty file when
 //       none was published) and the LaserScan in ROS1 wire format.
+//   d2pc_offline node1map <launch file> <w> <h> <cloud.bin> <centres.bin> <in.raw> [<in.raw> ...]
+//       node1 with the map on (map_enable in the launch file), one frame per <in.raw> stamped (3 + i, 4): the last
+//       PointCloud2 (an empty file when none was published) and the last /octomap_point_cloud_centers cloud.
 //   d2pc_offline fusion <fusion launch> <w> <h> <d1.raw> <d2.raw> <s1.raw> <s2.raw> <fused.bin> [<cloud.bin> [<debug dir>]]
 //       BASELINE config 5 shape: four mono8 frames into DepthMapFusion; the fused Image is written, and when
 //       <cloud.bin> is given it is also fed to a Disparity2PCloud node whose /disparity is remapped to
@@ -100,6 +103,25 @@ int main(int argc, char **argv) {
       if (scan.empty()) throw std::runtime_error("no scan was published");
       write_file(argv[6], cloud);
       write_file(argv[7], scan);
+      return 0;
+    }
+    if (mode == "node1map" && argc >= 8) {
+      const uint32_t w = (uint32_t)std::atoi(argv[3]), h = (uint32_t)std::atoi(argv[4]);
+      d2pc_b200::Bus bus;
+      if (!bus.load_launch_file(argv[2])) throw std::runtime_error(std::string("cannot read ") + argv[2]);
+      d2pc::Disparity2PCloud node(bus);
+      std::vector<uint8_t> cloud, centres;
+      int n_centres = 0;
+      bus.subscribe_cloud("/point_cloud", 1, [&](const sm::PointCloud2 &c) { cloud = ros_lite::serialize(c); });
+      bus.subscribe_cloud("/octomap_point_cloud_centers", 1, [&](const sm::PointCloud2 &c) {
+        centres = ros_lite::serialize(c);
+        ++n_centres;
+      });
+      for (int i = 7; i < argc; ++i)  // frame i - 7 stamped (3 + i - 7, 4)
+        bus.publish(bus.resolve("/disparity"), make_image(read_file(argv[i], (size_t)w * h), w, h, 3 + (i - 7), 4));
+      if (n_centres != argc - 7) throw std::runtime_error("not one centres cloud per frame");
+      write_file(argv[5], cloud);
+      write_file(argv[6], centres);
       return 0;
     }
     if (mode == "params" && argc >= 3) {
