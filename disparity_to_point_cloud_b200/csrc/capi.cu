@@ -97,6 +97,21 @@ struct StageBufs {
   DevBuf stage;     // the scratch of the cloud stages: they run one after another on one stream, so they share it
 };
 
+// One cloud submission on a slot.  The caller fills the first five fields; submit_front decides the rest.
+struct Submission {
+  uint8_t *user_dst;    // the caller's destination (d2pc_*_into); nullptr = the slot's h_out
+  size_t user_cap;
+  bool sync_call;       // the caller waits for this cloud right away (d2pc_process_*, d2pc_fuse_then_process)
+  bool mono8;
+  cudaStream_t stream;  // where the slot's kernels run: s_compute, or a fusion slot's own s_kern
+  CloudPlan p;
+  bool user_pinned;
+  // synchronous call into a PAGEABLE caller buffer: no D2H at submit; d2pc_wait copies device -> caller directly
+  // (driver-staged in chunks: 280 vs 346 us for a 752x480 cloud against D2H into pinned memory + memcpy)
+  bool late_copy;
+  uint8_t *d_direct;    // the device alias the kernels store the cloud into (direct output); nullptr = s.d_out
+};
+
 struct Slot {
   PinBuf h_in, h_out;
   DevBuf d_in, d_out;
@@ -114,14 +129,7 @@ struct Slot {
   bool timed = false;              // the last submission on this slot recorded all four events with timing
   cudaStream_t s_kern = nullptr;  // fusion pipeline: this slot's own kernel stream (small kernels of consecutive sets overlap)
   bool pending = false;
-  CloudPlan plan;  // of the pending submission
-  // caller-supplied destination of this submission (d2pc_submit_*_into); nullptr = library-owned h_out
-  uint8_t *user_dst = nullptr;
-  size_t user_cap = 0;
-  bool user_pinned = false;
-  // synchronous call into a PAGEABLE caller buffer: no D2H at submit; d2pc_wait copies device -> caller directly
-  // (driver-staged in chunks: 280 vs 346 us for a 752x480 cloud against D2H into pinned memory + memcpy)
-  bool late_copy = false;
+  Submission sub{};  // the pending submission (the last one armed)
 };
 
 }  // namespace
@@ -541,6 +549,19 @@ uint32_t frames_per_chunk(uint32_t n_frames, uint64_t points_per_frame) {
   return (uint32_t)std::min<uint64_t>(n_frames, by_points);
 }
 
+// A batch of clouds on the device in frames_per_chunk chunks: fn(f0, chunk) for the chunk of frames f0, f0 + 1, ...
+template <class Fn>
+int for_each_chunk(const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride, const uint32_t *d_in_counts,
+                   Fn fn) {
+  const uint32_t chunk = frames_per_chunk(n_frames, n_max);
+  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
+    const int rc = fn(f0, CloudSrc{d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
+                                   std::min(chunk, n_frames - f0), n_max});
+    if (rc) return rc;
+  }
+  return D2PC_OK;
+}
+
 CloudTransformParams transform_params(const d2pc_ctx *ctx) {
   CloudTransformParams t;
   for (int k = 0; k < 12; ++k) t.m[k] = ctx->xform.matrix[k];
@@ -660,7 +681,7 @@ int enqueue_reproject(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, S
 // flags (may be null).  ranges: with the plan's scan on, the scan of `out` is the last step and writes each frame's
 // ranges there (frame f at f * 4 * n bytes).
 int enqueue_kernels(d2pc_ctx *ctx, const CloudPlan &p, const FrameBatch &in, StageBufs &b, const CloudDst &out,
-                    uint32_t *fallback, uint32_t *ticket, cudaStream_t stream, float *ranges = nullptr) {
+                    uint32_t *fallback, uint32_t *ticket, cudaStream_t stream, float *ranges) {
   const uint32_t n = (uint32_t)p.n;
   const int stages = p.n_stages;
   const CloudDst buf[2] = {cloud_buf(b.cloud[0], in.n_frames, n), cloud_buf(b.cloud[1], in.n_frames, n)};
@@ -769,55 +790,89 @@ int enqueue_readback(d2pc_ctx *ctx, Slot &s, const CloudPlan &p, uint8_t *dst) {
   return D2PC_OK;
 }
 
-void arm_slot(Slot &s, const CloudPlan &p, uint8_t *user_dst, size_t user_cap, bool user_pinned, bool late_copy) {
-  s.pending = true;
-  s.plan = p;
-  s.user_dst = user_dst, s.user_cap = user_cap, s.user_pinned = user_pinned;
-  s.late_copy = late_copy;
-}
-
-int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_t h, uint32_t step, bool is_f32,
-                  uint8_t *user_dst = nullptr, size_t user_cap = 0, bool sync_call = false) {
-  if (!ctx || slot < 0 || slot >= (int)ctx->slots.size()) return D2PC_ERR_INVALID_ARG;
-  const int esz = is_f32 ? 4 : 1;
-  int rc = check_frame(ctx, data, w, h, step, esz);
-  if (rc) return rc;
+// What every slot submission does before its input reaches the device: the plan for a w x h frame, its checks, and
+// the slot's output buffers.  Nothing is allocated or read before the checks.
+int submit_front(d2pc_ctx *ctx, Slot &s, uint32_t w, uint32_t h, Submission &sub) {
   CU(ctx, cudaSetDevice(ctx->device));
-  Slot &s = ctx->slots[slot];
-  rc = slot_wait_idle(ctx, s);
+  int rc = slot_wait_idle(ctx, s);
   if (rc) return rc;
-  NvtxRange nvtx_submit(is_f32 ? "d2pc submit f32" : "d2pc submit mono8");
-
-  const size_t row_bytes = (size_t)w * esz;
-  // rows that are already 16-byte multiples stay dense on the device: the H2D copy is then one contiguous DMA.  So do
-  // mono8 rows of any width (the callback kernel reads bytes; a 665-wide fused map is then one DMA instead of a
-  // pitched 2-D copy); float rows that are not 16-byte multiples keep a 256-byte pitch for the vector loads.
-  const size_t d_pitch = (row_bytes % 16 == 0 || !is_f32) ? row_bytes : round_up(row_bytes, kAlign);
-  CloudPlan p = plan_cloud(ctx, w, h);
+  CloudPlan &p = sub.p;
+  p = plan_cloud(ctx, w, h);
   add_scan(ctx, p);
   add_map(ctx, p);
   const uint64_t n = p.n;
   if (n * 16 > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // PointCloud2.row_step / width are uint32
   const bool out_cloud = cloud_out(p);
-  if (user_dst && !p.counted && out_cloud && user_cap < n * 16) return D2PC_ERR_BUFFER_TOO_SMALL;
-  const bool user_pinned = user_dst && reinterpret_cast<uintptr_t>(user_dst) % 16 == 0 && lookup_pinned(ctx, user_dst);
-  if ((rc = grow_dev(ctx, s.d_in, d_pitch * h))) return rc;
-  const bool late_copy = sync_call && user_dst && !user_pinned && !p.counted && n && out_cloud;
-  if (!user_pinned && !late_copy && out_cloud && (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
+  uint8_t *const dst = sub.user_dst;
+  if (dst && !p.counted && out_cloud && sub.user_cap < n * 16) return D2PC_ERR_BUFFER_TOO_SMALL;
+  sub.user_pinned = dst && reinterpret_cast<uintptr_t>(dst) % 16 == 0 && lookup_pinned(ctx, dst);
+  sub.late_copy = sub.sync_call && dst && !sub.user_pinned && !p.counted && n && out_cloud;
+  if (!sub.user_pinned && !sub.late_copy && out_cloud && (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
   if (p.scan.on && ((rc = grow_dev(ctx, s.d_ranges, (size_t)p.scan.p.n * 4)) ||
                     (rc = grow_pin(ctx, s.h_ranges, (size_t)p.scan.p.n * 4))))
     return rc;
   // direct output: the kernel's point stores go over PCIe into the page-locked destination while it runs, so a lone
   // frame no longer pays kernel + copy back to back (CROP only: a compacted cloud's size is not known up front; not
   // with the scan or the map, which read the cloud on the device)
-  uint8_t *d_direct = nullptr;
-  if (!p.counted && n && !late_copy && !p.scan.on && !p.map.on &&
+  sub.d_direct = nullptr;
+  if (!p.counted && n && !sub.late_copy && !p.scan.on && !p.map.on &&
       (ctx->direct_out > 0 ||
-       (ctx->direct_out == 0 && sync_call && !is_f32 && ctx->cfg.median_ksize > 1 && p.n_stages == 0)))
-    d_direct = direct_alias(user_pinned ? user_dst : s.h_out.p);
-  if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
-  const FrameBatch in{s.d_in.p, is_f32, 1, w, h, d_pitch, d_pitch * h};
-  if ((rc = grow_stages(ctx, s.stages, p, in, ctx->s_compute, false))) return rc;
+       (ctx->direct_out == 0 && sub.sync_call && sub.mono8 && ctx->cfg.median_ksize > 1 && p.n_stages == 0)))
+    sub.d_direct = direct_alias(sub.user_pinned ? dst : s.h_out.p);
+  if (!sub.d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
+  return D2PC_OK;
+}
+
+// What every slot submission does once its input frame `in` is on the device, or queued to be, ahead of sub.stream:
+// the plan's kernels, the map step, the cloud's way to the host, and the slot armed for d2pc_wait.
+int submit_back(d2pc_ctx *ctx, Slot &s, const FrameBatch &in, const Submission &sub) {
+  const CloudPlan &p = sub.p;
+  const uint64_t n = p.n;
+  int rc;
+  {
+    NvtxRange nvtx_k("d2pc kernels");
+    if ((rc = grow_stages(ctx, s.stages, p, in, sub.stream, false)) ||
+        (rc = enqueue_kernels(ctx, p, in, s.stages, {sub.d_direct ? sub.d_direct : s.d_out.p, n * 16 + 16, s.d_count},
+                              s.d_count + 2, s.d_count + 1, sub.stream, reinterpret_cast<float *>(s.d_ranges.p))))
+      return rc;
+  }
+  CU(ctx, cudaEventRecord(s.ev_kernel, sub.stream));
+  // the map step runs on s_map behind ev_kernel, so every slot updates the map in submission order
+  if ((rc = enqueue_slot_map(ctx, s, p, {s.d_out.p, n * 16 + 16, s.d_count}))) return rc;
+
+  NvtxRange nvtx_d2h("d2pc D2H");
+  if ((sub.d_direct || sub.late_copy) && !p.scan.on) {
+    // the cloud is already in host memory when the kernel ends (direct output), or leaves the device in d2pc_wait
+    // (pageable destination of a synchronous call): the slot completes on its kernel stream
+    CU(ctx, cudaEventRecord(s.ev_d2h, sub.stream));
+  } else {
+    // a page-locked caller buffer receives the cloud by DMA directly; a pageable one is filled from h_out in wait
+    // (a late copy with the scan on: only the ranges here)
+    uint8_t *const dst = sub.late_copy ? nullptr : sub.user_pinned ? sub.user_dst : s.h_out.p;
+    if ((rc = enqueue_readback(ctx, s, p, dst))) return rc;
+  }
+  s.pending = true;
+  s.sub = sub;
+  return D2PC_OK;
+}
+
+int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_t h, uint32_t step, bool is_f32,
+                  uint8_t *user_dst, size_t user_cap, bool sync_call) {
+  if (!ctx || slot < 0 || slot >= (int)ctx->slots.size()) return D2PC_ERR_INVALID_ARG;
+  const int esz = is_f32 ? 4 : 1;
+  int rc = check_frame(ctx, data, w, h, step, esz);
+  if (rc) return rc;
+  Slot &s = ctx->slots[slot];
+  NvtxRange nvtx_submit(is_f32 ? "d2pc submit f32" : "d2pc submit mono8");
+  Submission sub{user_dst, user_cap, sync_call, !is_f32, ctx->s_compute};
+  if ((rc = submit_front(ctx, s, w, h, sub))) return rc;
+
+  const size_t row_bytes = (size_t)w * esz;
+  // rows that are already 16-byte multiples stay dense on the device: the H2D copy is then one contiguous DMA.  So do
+  // mono8 rows of any width (the callback kernel reads bytes; a 665-wide fused map is then one DMA instead of a
+  // pitched 2-D copy); float rows that are not 16-byte multiples keep a 256-byte pitch for the vector loads.
+  const size_t d_pitch = (row_bytes % 16 == 0 || !is_f32) ? row_bytes : round_up(row_bytes, kAlign);
+  if ((rc = grow_dev(ctx, s.d_in, d_pitch * h))) return rc;
 
   // ---- H2D (stream 1).  Pinned caller memory is DMA'd in place; pageable memory is staged.
   const void *src = data;
@@ -849,26 +904,29 @@ int submit_common(d2pc_ctx *ctx, int slot, const void *data, uint32_t w, uint32_
 
   // ---- kernels (stream 2)
   CU(ctx, cudaStreamWaitEvent(ctx->s_compute, s.ev_h2d, 0));
-  {
-    NvtxRange nvtx_k("d2pc kernels");
-    rc = enqueue_kernels(ctx, p, in, s.stages, {d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count},
-                         s.d_count + 2, s.d_count + 1, ctx->s_compute, reinterpret_cast<float *>(s.d_ranges.p));
-  }
-  if (rc) return rc;
-  CU(ctx, cudaEventRecord(s.ev_kernel, ctx->s_compute));
-  if ((rc = enqueue_slot_map(ctx, s, p, {s.d_out.p, n * 16 + 16, s.d_count}))) return rc;
+  return submit_back(ctx, s, {s.d_in.p, is_f32, 1, w, h, d_pitch, d_pitch * h}, sub);
+}
 
-  NvtxRange nvtx_d2h("d2pc D2H");
-  if ((d_direct || late_copy) && !p.scan.on) {
-    // the cloud is already in host memory when the kernel ends (direct output), or leaves the device in d2pc_wait
-    // (pageable destination of a synchronous call): the slot completes on the compute stream
-    CU(ctx, cudaEventRecord(s.ev_d2h, ctx->s_compute));
-  } else {
-    // a page-locked caller buffer receives the cloud by DMA directly; a pageable one is filled from h_out in wait
-    // (a late copy with the scan on: only the ranges here)
-    if ((rc = enqueue_readback(ctx, s, p, late_copy ? nullptr : user_pinned ? user_dst : s.h_out.p))) return rc;
+// A stream of n items over the slots: item i is read from base + (i % ring_len) * stride (ring_len 0: no wrap) and
+// submitted with submit(item, slot) while a slot is free -- the H2D of item i+2, the kernels of i+1 and the D2H of i
+// overlap on the three streams -- then the oldest is waited on and handed to the sink, in submission order.
+template <class Submit>
+int run_ring(d2pc_ctx *ctx, const uint8_t *base, uint64_t n, size_t stride, uint64_t ring_len, Submit submit,
+             d2pc_cloud_sink sink, void *user) {
+  const uint64_t ns = ctx->slots.size();
+  d2pc_cloud cloud;
+  uint64_t submitted = 0, retired = 0;
+  while (retired < n) {
+    while (submitted < n && submitted - retired < ns) {
+      const int rc = submit(base + (ring_len ? submitted % ring_len : submitted) * stride, (int)(submitted % ns));
+      if (rc) return rc;
+      ++submitted;
+    }
+    const int rc = d2pc_wait(ctx, (int)(retired % ns), &cloud);
+    if (rc) return rc;
+    if (sink) sink(user, retired, &cloud);
+    ++retired;
   }
-  arm_slot(s, p, user_dst, user_cap, user_pinned, late_copy);
   return D2PC_OK;
 }
 
@@ -1377,17 +1435,10 @@ int d2pc_set_tuning(d2pc_ctx *ctx, const char *key, int value) {
 // host-buffer entry points
 // ---------------------------------------------------------------------------
 int d2pc_submit_mono8(d2pc_ctx *ctx, int slot, const uint8_t *data, uint32_t w, uint32_t h, uint32_t step) {
-  return submit_common(ctx, slot, data, w, h, step, false);
+  return submit_common(ctx, slot, data, w, h, step, false, nullptr, 0, false);
 }
 int d2pc_submit_f32(d2pc_ctx *ctx, int slot, const float *disp, uint32_t w, uint32_t h, uint32_t step) {
-  return submit_common(ctx, slot, disp, w, h, step, true);
-}
-
-// d2pc_last_scan's answer from now on: the scan of the cloud just returned, whose ranges are in `ranges`.
-static void note_scan(d2pc_ctx *ctx, const ScanPlan &scan, const PinBuf &ranges) {
-  ctx->last_scan_on = scan.on;
-  ctx->last_scan = scan.msg;
-  ctx->last_scan.ranges = reinterpret_cast<const float *>(ranges.p);
+  return submit_common(ctx, slot, disp, w, h, step, true, nullptr, 0, false);
 }
 
 int d2pc_wait(d2pc_ctx *ctx, int slot, d2pc_cloud *out) {
@@ -1396,41 +1447,46 @@ int d2pc_wait(d2pc_ctx *ctx, int slot, d2pc_cloud *out) {
   if (!s.pending) return D2PC_ERR_NOT_READY;
   CU(ctx, cudaSetDevice(ctx->device));
   CU(ctx, cudaEventSynchronize(s.ev_d2h));
-  const uint64_t n = kept_points(s.plan, s.h_count);
-  if (s.plan.counted && s.user_dst && s.user_cap < n * 16) {
+  const Submission &sub = s.sub;
+  const CloudPlan &p = sub.p;
+  const uint64_t n = kept_points(p, s.h_count);
+  if (p.counted && sub.user_dst && sub.user_cap < n * 16) {
     s.pending = false;
     ctx->last_scan_on = false;  // no cloud is returned, so there is no last scan either
     return D2PC_ERR_BUFFER_TOO_SMALL;
   }
   // a counted cloud and a late copy leave the device here: the copy is synchronous anyway, so it goes straight to
   // the caller's buffer, page-locked or not
-  const bool copy_here = s.plan.counted || s.late_copy;
+  const bool copy_here = p.counted || sub.late_copy;
+  uint8_t *const dst = sub.user_dst ? sub.user_dst : s.h_out.p;
   if (copy_here && n) {
-    CU(ctx, cudaMemcpyAsync(s.user_dst ? s.user_dst : s.h_out.p, s.d_out.p, n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CU(ctx, cudaMemcpyAsync(dst, s.d_out.p, n * 16, cudaMemcpyDeviceToHost, ctx->s_d2h));
     CU(ctx, cudaStreamSynchronize(ctx->s_d2h));
   }
   // otherwise a page-locked caller buffer already holds the cloud; a pageable one is filled from h_out
-  if (s.user_dst && !s.user_pinned && !copy_here && n) memcpy(s.user_dst, s.h_out.p, n * 16);
-  s.late_copy = false;
+  if (sub.user_dst && !sub.user_pinned && !copy_here && n) memcpy(sub.user_dst, s.h_out.p, n * 16);
   s.pending = false;
   if (ctx->cfg.verbose) printf("Cloud size: %llu\n", (unsigned long long)n);  // cpp:82
   if (out) {
-    if (cloud_out(s.plan)) fill_cloud(ctx, s.user_dst ? s.user_dst : s.h_out.p, n, cloud_is_dense(s.plan, s.h_count), out);
+    if (cloud_out(p)) fill_cloud(ctx, dst, n, cloud_is_dense(p, s.h_count), out);
     else fill_cloud(ctx, nullptr, 0, true, out);
   }
-  note_scan(ctx, s.plan.scan, s.h_ranges);
+  // d2pc_last_scan's answer from now on: the scan of the cloud just returned
+  ctx->last_scan_on = p.scan.on;
+  ctx->last_scan = p.scan.msg;
+  ctx->last_scan.ranges = reinterpret_cast<const float *>(s.h_ranges.p);
   return D2PC_OK;
 }
 
 int d2pc_submit_mono8_into(d2pc_ctx *ctx, int slot, const uint8_t *data, uint32_t w, uint32_t h, uint32_t step,
                            uint8_t *dst, size_t cap) {
   if (!dst) return D2PC_ERR_INVALID_ARG;
-  return submit_common(ctx, slot, data, w, h, step, false, dst, cap);
+  return submit_common(ctx, slot, data, w, h, step, false, dst, cap, false);
 }
 int d2pc_submit_f32_into(d2pc_ctx *ctx, int slot, const float *disp, uint32_t w, uint32_t h, uint32_t step,
                          uint8_t *dst, size_t cap) {
   if (!dst) return D2PC_ERR_INVALID_ARG;
-  return submit_common(ctx, slot, disp, w, h, step, true, dst, cap);
+  return submit_common(ctx, slot, disp, w, h, step, true, dst, cap, false);
 }
 int d2pc_process_mono8_into(d2pc_ctx *ctx, const uint8_t *data, uint32_t w, uint32_t h, uint32_t step, uint8_t *dst,
                             size_t cap, d2pc_cloud *out) {
@@ -1487,7 +1543,7 @@ int d2pc_slot_timing(d2pc_ctx *ctx, int slot, d2pc_timing *out) {
   CU(ctx, cudaEventElapsedTime(&d2h, s.ev_kernel, s.ev_d2h));
   CU(ctx, cudaEventElapsedTime(&tot, s.ev_start, s.ev_d2h));
   out->h2d_us = h2d * 1e3f, out->kernels_us = ker * 1e3f, out->d2h_us = d2h * 1e3f, out->total_us = tot * 1e3f;
-  out->points = kept_points(s.plan, s.h_count);
+  out->points = kept_points(s.sub.p, s.h_count);
   return D2PC_OK;
 }
 
@@ -1529,26 +1585,10 @@ int d2pc_host_unregister(void *ptr) {
 int d2pc_process_stream(d2pc_ctx *ctx, const void *frames, uint64_t n_frames, size_t frame_stride, uint64_t ring_len,
                         int is_f32, uint32_t w, uint32_t h, uint32_t step, d2pc_cloud_sink sink, void *user) {
   if (!ctx || (!frames && n_frames)) return D2PC_ERR_INVALID_ARG;
-  const uint64_t ns = ctx->slots.size();
-  const uint8_t *base = static_cast<const uint8_t *>(frames);
-  d2pc_cloud cloud;
-  uint64_t submitted = 0, retired = 0;
-  while (retired < n_frames) {
-    // keep every slot busy: H2D of frame i+2, kernels of i+1 and D2H of i overlap on the three streams
-    while (submitted < n_frames && submitted - retired < ns) {
-      const uint8_t *f = base + (ring_len ? submitted % ring_len : submitted) * frame_stride;
-      const int slot = (int)(submitted % ns);
-      const int rc = is_f32 ? d2pc_submit_f32(ctx, slot, reinterpret_cast<const float *>(f), w, h, step)
-                            : d2pc_submit_mono8(ctx, slot, f, w, h, step);
-      if (rc) return rc;
-      ++submitted;
-    }
-    const int rc = d2pc_wait(ctx, (int)(retired % ns), &cloud);
-    if (rc) return rc;
-    if (sink) sink(user, retired, &cloud);
-    ++retired;
-  }
-  return D2PC_OK;
+  auto submit = [&](const uint8_t *f, int slot) {
+    return submit_common(ctx, slot, f, w, h, step, is_f32 != 0, nullptr, 0, false);
+  };
+  return run_ring(ctx, static_cast<const uint8_t *>(frames), n_frames, frame_stride, ring_len, submit, sink, user);
 }
 
 // ---------------------------------------------------------------------------
@@ -1579,26 +1619,29 @@ static int reproject_device_common(d2pc_ctx *ctx, const void *d_in, bool is_f32,
     in.n_frames = std::min(chunk, n_frames - f0);
     if ((rc = enqueue_kernels(ctx, p, in, ctx->batch,
                               {d_points + f0 * points_stride, points_stride, d_counts ? d_counts + f0 : nullptr},
-                              nullptr, ctx->d_ticket, ctx->s_compute)))
+                              nullptr, ctx->d_ticket, ctx->s_compute, nullptr)))
       return rc;
   }
   return D2PC_OK;
 }
 
-// The argument rules of the stages that run alone on clouds already on the device (d2pc_radius_outlier_device,
-// d2pc_crop_box_device, d2pc_cloud_transform_device).  in_place: the output may also be exactly the input.
+// The argument rules of the stages that run alone on clouds already on the device: n_frames clouds of n_max points
+// at d_in, in_stride bytes apart, and per frame out_bytes of output at d_out, out_stride bytes apart, both
+// out_align-aligned (16 for a cloud, 4 for laser-scan ranges; no output: null, 0, 0, 1).  in_place: the output may
+// also be exactly the input.
 static int check_cloud_batch(const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
-                             const uint8_t *d_out, size_t out_stride, bool in_place = false) {
+                             const void *d_out, size_t out_stride, uint64_t out_bytes, size_t out_align,
+                             bool in_place) {
   const uint64_t bytes = (uint64_t)n_max * 16;
   if (bytes > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // per-frame counts and PointCloud2.row_step are uint32
-  if (reinterpret_cast<uintptr_t>(d_in) % 16 || reinterpret_cast<uintptr_t>(d_out) % 16 || in_stride % 16 ||
-      out_stride % 16 || (n_frames > 1 && (in_stride < bytes || out_stride < bytes)))
+  if (reinterpret_cast<uintptr_t>(d_in) % 16 || in_stride % 16 || reinterpret_cast<uintptr_t>(d_out) % out_align ||
+      out_stride % out_align || (n_frames > 1 && (in_stride < bytes || out_stride < out_bytes)))
     return D2PC_ERR_BAD_DIMS;
-  if (n_frames == 0 || (in_place && d_in == d_out && in_stride == out_stride)) return D2PC_OK;
+  if (n_frames == 0 || out_bytes == 0 || (in_place && d_in == d_out && in_stride == out_stride)) return D2PC_OK;
   // kept points are copied from the input after every flag is known: the two must not share bytes
   const uintptr_t in0 = reinterpret_cast<uintptr_t>(d_in), out0 = reinterpret_cast<uintptr_t>(d_out);
   const uint64_t in_end = in0 + (uint64_t)(n_frames - 1) * in_stride + bytes;
-  const uint64_t out_end = out0 + (uint64_t)(n_frames - 1) * out_stride + bytes;
+  const uint64_t out_end = out0 + (uint64_t)(n_frames - 1) * out_stride + out_bytes;
   if (bytes && in0 < out_end && out0 < in_end) return D2PC_ERR_INVALID_ARG;
   return D2PC_OK;
 }
@@ -1608,24 +1651,19 @@ static int cloud_stage_device(d2pc_ctx *ctx, CloudStage st, bool on, const uint8
                               uint32_t n_max, size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out,
                               size_t out_stride, uint32_t *d_out_counts) {
   if (!ctx || !d_in || !d_out || !d_out_counts || !on) return D2PC_ERR_INVALID_ARG;
-  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_out, out_stride);
+  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_out, out_stride, (uint64_t)n_max * 16, 16, false);
   if (rc0 || n_frames == 0) return rc0;
   CU(ctx, cudaSetDevice(ctx->device));
-  const uint32_t chunk = frames_per_chunk(n_frames, n_max);
-  const size_t need = stage_scratch_bytes(st, chunk, n_max);
+  const size_t need = stage_scratch_bytes(st, frames_per_chunk(n_frames, n_max), n_max);
   if (need > ctx->batch.stage.cap) {
     CU(ctx, cudaStreamSynchronize(ctx->s_compute));
     const int rc = grow_dev(ctx, ctx->batch.stage, need);
     if (rc) return rc;
   }
-  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
-    const CloudSrc in{d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
-                      std::min(chunk, n_frames - f0), n_max};
-    const int rc = enqueue_stage(ctx, st, in, {d_out + f0 * out_stride, out_stride, d_out_counts + f0}, nullptr,
-                                 ctx->batch.stage.p, ctx->s_compute);
-    if (rc) return rc;
-  }
-  return D2PC_OK;
+  return for_each_chunk(d_in, n_frames, n_max, in_stride, d_in_counts, [&](uint32_t f0, const CloudSrc &in) -> int {
+    return enqueue_stage(ctx, st, in, {d_out + f0 * out_stride, out_stride, d_out_counts + f0}, nullptr,
+                         ctx->batch.stage.p, ctx->s_compute);
+  });
 }
 
 int d2pc_radius_outlier_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
@@ -1645,58 +1683,42 @@ int d2pc_cloud_transform_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_f
                                 size_t in_stride, const uint32_t *d_in_counts, uint8_t *d_out, size_t out_stride,
                                 uint32_t *d_out_counts, const float *d_transforms) {
   if (!ctx || !d_in || !d_out || (!d_transforms && !ctx->xform.enabled)) return D2PC_ERR_INVALID_ARG;
-  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_out, out_stride, true);
+  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_out, out_stride, (uint64_t)n_max * 16, 16, true);
   if (rc0 || n_frames == 0) return rc0;
   CU(ctx, cudaSetDevice(ctx->device));
   const CloudTransformParams t = transform_params(ctx);
-  const uint32_t chunk = frames_per_chunk(n_frames, n_max);
-  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
-    const CloudSrc in{d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
-                      std::min(chunk, n_frames - f0), n_max};
+  return for_each_chunk(d_in, n_frames, n_max, in_stride, d_in_counts, [&](uint32_t f0, const CloudSrc &in) -> int {
     const CloudDst out{d_out + f0 * out_stride, out_stride, d_out_counts ? d_out_counts + f0 : nullptr};
     int nl = 0;
     CU(ctx, launch_cloud_transform(in, out, t, d_transforms ? d_transforms + 12 * (size_t)f0 : nullptr, ctx->s_compute,
                                    &nl));
     ctx->launches += nl;
-  }
-  return D2PC_OK;
+    return D2PC_OK;
+  });
 }
 
 int d2pc_laser_scan_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max, size_t in_stride,
                            const uint32_t *d_in_counts, float *d_ranges, size_t ranges_stride) {
   if (!ctx || !d_in || !d_ranges || !ctx->scan.enabled) return D2PC_ERR_INVALID_ARG;
   const LaserScanParams &p = ctx->scan_plan.p;
-  const uint64_t bytes = (uint64_t)n_max * 16, rbytes = (uint64_t)p.n * 4;
-  if (bytes > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // the argument rules of the other cloud stages
-  if (reinterpret_cast<uintptr_t>(d_in) % 16 || in_stride % 16 || reinterpret_cast<uintptr_t>(d_ranges) % 4 ||
-      ranges_stride % 4 || (n_frames > 1 && (in_stride < bytes || ranges_stride < rbytes)))
-    return D2PC_ERR_BAD_DIMS;
-  if (n_frames == 0 || p.n == 0) return D2PC_OK;
-  const uintptr_t in0 = reinterpret_cast<uintptr_t>(d_in), out0 = reinterpret_cast<uintptr_t>(d_ranges);
-  const uint64_t in_end = in0 + (uint64_t)(n_frames - 1) * in_stride + bytes;
-  const uint64_t out_end = out0 + (uint64_t)(n_frames - 1) * ranges_stride + rbytes;
-  if (bytes && in0 < out_end && out0 < in_end) return D2PC_ERR_INVALID_ARG;
+  const uint64_t rbytes = (uint64_t)p.n * 4;
+  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, d_ranges, ranges_stride, rbytes, 4, false);
+  if (rc0 || n_frames == 0 || p.n == 0) return rc0;
   CU(ctx, cudaSetDevice(ctx->device));
-  const uint32_t chunk = frames_per_chunk(n_frames, n_max);
-  for (uint32_t f0 = 0; f0 < n_frames; f0 += chunk) {
-    const CloudSrc in{d_in + f0 * in_stride, in_stride, d_in_counts ? d_in_counts + f0 : nullptr,
-                      std::min(chunk, n_frames - f0), n_max};
+  return for_each_chunk(d_in, n_frames, n_max, in_stride, d_in_counts, [&](uint32_t f0, const CloudSrc &in) -> int {
     int nl = 0;
     CU(ctx, launch_laser_scan(in, p, reinterpret_cast<float *>(reinterpret_cast<uint8_t *>(d_ranges) + f0 * ranges_stride),
                               ranges_stride, ctx->s_compute, &nl));
     ctx->launches += nl;
-  }
-  return D2PC_OK;
+    return D2PC_OK;
+  });
 }
 
 int d2pc_occupancy_insert_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
                                  size_t in_stride, const uint32_t *d_in_counts, const float *origins) {
   if (!ctx || !d_in || !origins || !ctx->occ.enabled) return D2PC_ERR_INVALID_ARG;
-  const uint64_t bytes = (uint64_t)n_max * 16;
-  if (bytes > 0xffffffffull) return D2PC_ERR_BAD_DIMS;  // the argument rules of the other cloud stages
-  if (reinterpret_cast<uintptr_t>(d_in) % 16 || in_stride % 16 || (n_frames > 1 && in_stride < bytes))
-    return D2PC_ERR_BAD_DIMS;
-  if (n_frames == 0) return D2PC_OK;
+  const int rc0 = check_cloud_batch(d_in, n_frames, n_max, in_stride, nullptr, 0, 0, 1, false);
+  if (rc0 || n_frames == 0) return rc0;
   CU(ctx, cudaSetDevice(ctx->device));
   CU(ctx, cudaEventRecord(ctx->ev_map_in, ctx->s_compute));
   // one frame per map step: a frame of at most 2^28 points is always within kCloudMaxPoints, so no chunk spans frames
@@ -2023,52 +2045,23 @@ int d2pc_fuse_then_process(d2pc_ctx *ctx, const uint8_t *d1, const uint8_t *d2, 
                            uint32_t w, uint32_t h, uint32_t step, d2pc_cloud *out) {
   if (!ctx || !d1 || !d2 || !s1 || !s2 || !out) return D2PC_ERR_INVALID_ARG;
   if (w == 0 || h == 0 || step < w) return D2PC_ERR_BAD_DIMS;
-  const uint8_t *in[4] = {d1, d2, s1, s2};
+  const d2pc_config &c = ctx->cfg;
   FuseGeometry g;
-  int rc = fuse_upload_and_run(ctx, in, w, h, step, &g);
-  if (rc) return rc;
-  // the fused map stays on the device and enters DisparityCb's mono8 path there (cpp:55-85)
-  Slot &s = ctx->slots[0];
-  if ((rc = slot_wait_idle(ctx, s))) return rc;
+  if (!fuse_geometry((int)w, (int)h, c.offset_x, c.offset_y, c.fuse_crop_left, c.fuse_crop_right, c.fuse_crop_top,
+                     c.fuse_crop_bottom, &g))
+    return D2PC_ERR_GEOMETRY;
+  // a synchronous mono8 submission on slot 0 whose frame is the fused map: it stays on the device and enters
+  // DisparityCb's mono8 path there (cpp:55-85); there is no H2D of it to time
   const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
-  CloudPlan p = plan_cloud(ctx, fw, fh);
-  add_scan(ctx, p);
-  add_map(ctx, p);
-  const uint64_t n = p.n;
-  if (cloud_out(p) && (rc = grow_pin(ctx, s.h_out, n * 16 + 16))) return rc;
-  if (p.scan.on && ((rc = grow_dev(ctx, s.d_ranges, (size_t)p.scan.p.n * 4)) ||
-                    (rc = grow_pin(ctx, s.h_ranges, (size_t)p.scan.p.n * 4))))
+  Slot &s = ctx->slots[0];
+  s.timed = false;
+  Submission sub{nullptr, 0, true, true, ctx->s_compute};
+  const uint8_t *in[4] = {d1, d2, s1, s2};
+  int rc;
+  if ((rc = submit_front(ctx, s, fw, fh, sub)) || (rc = fuse_upload_and_run(ctx, in, w, h, step, nullptr)) ||
+      (rc = submit_back(ctx, s, {ctx->d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh}, sub)))
     return rc;
-  // a synchronous call: the callback kernel stores the CROP cloud straight into the pinned buffer (see submit_common)
-  const bool direct = !p.scan.on && !p.map.on && (ctx->direct_out > 0 || (ctx->direct_out == 0 && p.n_stages == 0));
-  uint8_t *const d_direct =
-      !p.counted && n && direct && ctx->cfg.median_ksize > 1 ? direct_alias(s.h_out.p) : nullptr;
-  if (!d_direct && (rc = grow_dev(ctx, s.d_out, n * 16 + 16))) return rc;
-  const FrameBatch fused{ctx->d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh};
-  if ((rc = grow_stages(ctx, s.stages, p, fused, ctx->s_compute, false)) ||
-      (rc = enqueue_kernels(ctx, p, fused, s.stages, {d_direct ? d_direct : s.d_out.p, n * 16 + 16, s.d_count},
-                            s.d_count + 2, s.d_count + 1, ctx->s_compute, reinterpret_cast<float *>(s.d_ranges.p))))
-    return rc;
-  if (p.map.on) {
-    CU(ctx, cudaEventRecord(s.ev_kernel, ctx->s_compute));
-    if ((rc = enqueue_slot_map(ctx, s, p, {s.d_out.p, n * 16 + 16, s.d_count}))) return rc;
-  }
-  if (p.scan.on && p.scan.p.n)
-    CU(ctx, cudaMemcpyAsync(s.h_ranges.p, s.d_ranges.p, (size_t)p.scan.p.n * 4, cudaMemcpyDeviceToHost, ctx->s_compute));
-  if (p.counted && cloud_out(p)) {
-    CU(ctx, cudaMemcpyAsync(s.h_count, s.d_count, p.count_words * sizeof(uint32_t), cudaMemcpyDeviceToHost,
-                            ctx->s_compute));
-    CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-  }
-  const uint64_t kept = kept_points(p, s.h_count);
-  if (kept && !d_direct)
-    CU(ctx, cudaMemcpyAsync(s.h_out.p, s.d_out.p, kept * 16, cudaMemcpyDeviceToHost, ctx->s_compute));
-  CU(ctx, cudaStreamSynchronize(ctx->s_compute));
-  if (ctx->cfg.verbose) printf("Cloud size: %llu\n", (unsigned long long)kept);
-  if (cloud_out(p)) fill_cloud(ctx, s.h_out.p, kept, cloud_is_dense(p, s.h_count), out);
-  else fill_cloud(ctx, nullptr, 0, true, out);
-  note_scan(ctx, p.scan, s.h_ranges);
-  return D2PC_OK;
+  return d2pc_wait(ctx, 0, out);
 }
 
 // ---- the whole fusion node + DisparityCb per frame set, on the slot pipeline ------------------------------------
@@ -2081,35 +2074,25 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
   if (!fuse_geometry((int)w, (int)h, c.offset_x, c.offset_y, c.fuse_crop_left, c.fuse_crop_right, c.fuse_crop_top,
                      c.fuse_crop_bottom, &g))
     return D2PC_ERR_GEOMETRY;
-  CU(ctx, cudaSetDevice(ctx->device));
   Slot &s = ctx->slots[slot];
-  int rc = slot_wait_idle(ctx, s);
+  NvtxRange nvtx_submit("d2pc submit fusion set");
+  const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
+  Submission sub{nullptr, 0, false, true, s.s_kern};
+  int rc = submit_front(ctx, s, fw, fh, sub);
   if (rc) return rc;
   // rows that are 16-byte multiples stay dense on the device, so a frame (or a whole contiguous set) is one 1-D DMA:
   // four pitched 2-D copies per set ran at 43 GB/s and bounded the stream at 6.6 k sets/s (one 1-D copy: 9.2 k)
   // (mono8 frames of any width: the fusion kernels read bytes, and a pitched 2-D copy is the slow way in)
   const size_t pitch = w, frame_bytes = (size_t)w * h, nn = (size_t)g.n * g.n;
-  const uint32_t fw = (uint32_t)g.out_w, fh = (uint32_t)g.out_h;
-  CloudPlan p = plan_cloud(ctx, fw, fh);
-  add_scan(ctx, p);
-  add_map(ctx, p);
-  const uint64_t n = p.n;
-  if (p.scan.on && ((rc = grow_dev(ctx, s.d_ranges, (size_t)p.scan.p.n * 4)) ||
-                    (rc = grow_pin(ctx, s.h_ranges, (size_t)p.scan.p.n * 4))))
-    return rc;
   // the four input frames of a set live in one allocation, so that a contiguous pinned set is one DMA
   if ((rc = grow_dev(ctx, s.d_fuse_in[0], 4 * pitch * h))) return rc;
   uint8_t *const fin[4] = {s.d_fuse_in[0].p, s.d_fuse_in[0].p + pitch * h, s.d_fuse_in[0].p + 2 * pitch * h,
                            s.d_fuse_in[0].p + 3 * pitch * h};
   if ((rc = grow_dev(ctx, s.d_pre[0], nn)) || (rc = grow_dev(ctx, s.d_pre[1], nn)) ||
       (rc = grow_dev(ctx, s.d_container, (size_t)g.nc * g.nc)) || (rc = grow_dev(ctx, s.d_combined, nn)) ||
-      (rc = grow_dev(ctx, s.d_fused, (size_t)fw * fh)) || (rc = grow_dev(ctx, s.d_out, n * 16 + 16)) ||
-      (rc = grow_pin(ctx, s.h_out, n * 16 + 16)))
+      (rc = grow_dev(ctx, s.d_fused, (size_t)fw * fh)))
     return rc;
-  const FrameBatch fused{s.d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh};
-  if ((rc = grow_stages(ctx, s.stages, p, fused, s.s_kern, false))) return rc;
 
-  NvtxRange nvtx_submit("d2pc submit fusion set");
   s.timed = ctx->timing && s.ev_start;
   if (s.timed) CU(ctx, cudaEventRecord(s.ev_start, ctx->s_h2d));
   // ---- H2D (stream 1): pinned caller frames are DMA'd in place, pageable ones are staged
@@ -2148,39 +2131,18 @@ int d2pc_submit_fusion(d2pc_ctx *ctx, int slot, const uint8_t *d1, const uint8_t
   if ((rc = fuse_device_impl(ctx, fin[0], fin[1], sc1, sc2, w, h, pitch, s.d_fused.p, s.d_combined.p,
                              nullptr, preprocess_scores != 0, &s.d_container, sk)))
     return rc;
-  if ((rc = enqueue_kernels(ctx, p, fused, s.stages, {s.d_out.p, n * 16 + 16, s.d_count}, s.d_count + 2,
-                            s.d_count + 1, sk, reinterpret_cast<float *>(s.d_ranges.p))))
-    return rc;
-  CU(ctx, cudaEventRecord(s.ev_kernel, sk));
-  // the map step runs on s_map behind this slot's kernel stream, so fusion slots update the map in submission order
-  if ((rc = enqueue_slot_map(ctx, s, p, {s.d_out.p, n * 16 + 16, s.d_count}))) return rc;
-  if ((rc = enqueue_readback(ctx, s, p, s.h_out.p))) return rc;
-  arm_slot(s, p, nullptr, 0, false, false);
-  return D2PC_OK;
+  return submit_back(ctx, s, {s.d_fused.p, false, 1, fw, fh, fw, (size_t)fw * fh}, sub);
 }
 
 int d2pc_process_fusion_stream(d2pc_ctx *ctx, const uint8_t *sets, uint64_t n_sets, size_t set_stride, uint64_t ring_len,
                                uint32_t w, uint32_t h, uint32_t step, int preprocess_scores, d2pc_cloud_sink sink,
                                void *user) {
   if (!ctx || (!sets && n_sets)) return D2PC_ERR_INVALID_ARG;
-  const uint64_t ns = ctx->slots.size();
   const size_t fb = (size_t)step * h;
-  d2pc_cloud cloud;
-  uint64_t submitted = 0, retired = 0;
-  while (retired < n_sets) {
-    while (submitted < n_sets && submitted - retired < ns) {
-      const uint8_t *f = sets + (ring_len ? submitted % ring_len : submitted) * set_stride;
-      const int rc = d2pc_submit_fusion(ctx, (int)(submitted % ns), f, f + fb, f + 2 * fb, f + 3 * fb, w, h, step,
-                                        preprocess_scores);
-      if (rc) return rc;
-      ++submitted;
-    }
-    const int rc = d2pc_wait(ctx, (int)(retired % ns), &cloud);
-    if (rc) return rc;
-    if (sink) sink(user, retired, &cloud);
-    ++retired;
-  }
-  return D2PC_OK;
+  auto submit = [&](const uint8_t *f, int slot) {
+    return d2pc_submit_fusion(ctx, slot, f, f + fb, f + 2 * fb, f + 3 * fb, w, h, step, preprocess_scores);
+  };
+  return run_ring(ctx, sets, n_sets, set_stride, ring_len, submit, sink, user);
 }
 
 // ---------------------------------------------------------------------------

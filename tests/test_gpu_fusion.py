@@ -105,6 +105,7 @@ def test_alternate_rules(ctx, rule):
 
 
 def test_bad_geometry_is_an_error(ctx):
+    import ctypes as C
     import disparity_to_point_cloud_b200 as d2pc
     ctx.set_tuning("offset_y", 400)
     try:
@@ -113,6 +114,12 @@ def test_bad_geometry_is_an_error(ctx):
         assert e.value.status == -7
     finally:
         ctx.set_tuning("offset_y", 15)
+    # 20000 x 20000 frames fuse into a 19865^2-point cloud, more bytes than PointCloud2's uint32 row_step holds: both
+    # slot entries refuse it before they read an input (all four pointers name one 64-byte buffer) or allocate
+    tiny = np.zeros(64, np.uint8)
+    p = tiny.ctypes.data
+    assert d2pc.lib().d2pc_submit_fusion(ctx._h, 0, p, p, p, p, 20000, 20000, 20000, 1) == -3
+    assert d2pc.lib().d2pc_fuse_then_process(ctx._h, p, p, p, p, 20000, 20000, 20000, C.byref(d2pc.Cloud())) == -3
 
 
 def _expected_cloud(crop, mode):

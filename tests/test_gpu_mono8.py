@@ -255,7 +255,8 @@ def test_caller_supplied_destination(ctx, q):
 def test_direct_output_modes(ctx, q, direct):
     """direct_out: a CROP cloud is written by the kernel straight into the page-locked host buffer (no D2H copy
     behind the kernel): 0 = synchronous single-frame mono8 entries only (default), 1 = every CROP submission (float
-    frames, slots, streams), -1 = never.  Same bytes in every mode, every destination kind, nothing written past the cloud."""
+    frames, slots, streams, fusion sets), -1 = never.  Same bytes in every mode, every destination kind, nothing written
+    past the cloud."""
     import disparity_to_point_cloud_b200 as d2pc
     ctx.set_tuning("direct_out", direct)
     pin = reg = None
@@ -293,6 +294,16 @@ def test_direct_output_modes(ctx, q, direct):
         for i in (0, 3, 5):
             assert_same_bits(clouds[i], oracle.disparity_cb_mono8(frames.array[i], q), f"stream frame {i}")
         frames.free()
+        # fusion sets on a slot and in a stream: DisparityCb on the fused map (the context's offsets are 0, 0)
+        rng = np.random.default_rng(88)
+        sets = np.stack([np.stack([synth.s2_scene(h, w, 96 + i), synth.s2_scene(h, w, 98 + i),
+                                   rng.integers(0, 256, (h, w), dtype=np.uint8),
+                                   rng.integers(0, 256, (h, w), dtype=np.uint8)]) for i in range(2)])
+        fused = [oracle.disparity_cb_mono8(oracle.fuse(*sets[i], 0, 0)[0], q) for i in range(2)]
+        ctx.submit_fusion(2, *sets[1], preprocess_scores=False)
+        assert_same_bits(ctx.wait(2), fused[1], "fusion slot")
+        for i, c in enumerate(ctx.process_fusion_stream(sets, preprocess_scores=False, n_sets=5)):
+            assert_same_bits(c, fused[i % 2], f"fusion stream set {i}")
         ctx.set_tuning("fuse_median", -1)
         assert_same_bits(ctx.process_mono8(img), want, "two-launch callback")
         ctx.set_tuning("fuse_median", 0)
