@@ -111,6 +111,12 @@ class OccupancyInfo(C.Structure):
         return {f[0]: int(getattr(self, f[0])) for f in self._fields_}
 
 
+class Octomap(C.Structure):
+    """d2pc_octomap: octomap_msgs/Octomap data in library-owned memory."""
+    _fields_ = [("data", C.POINTER(C.c_uint8)), ("size", C.c_uint64), ("resolution", C.c_double),
+                ("binary", C.c_int32)]
+
+
 class LaserScan(C.Structure):
     """d2pc_laser_scan: the message fields of a scan and its library-owned ranges."""
     _fields_ = [("angle_min", C.c_float), ("angle_max", C.c_float), ("angle_increment", C.c_float),
@@ -190,6 +196,7 @@ SYMBOLS = [
     ("d2pc_occupancy_voxels", C.c_int, [_ctx, C.c_void_p, C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)]),
     ("d2pc_occupancy_insert_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
                                                C.c_void_p]),
+    ("d2pc_occupancy_octomap", C.c_int, [_ctx, C.c_int, C.POINTER(Octomap)]),
     ("d2pc_process_mono8", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_process_f32", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_submit_mono8", C.c_int, [_ctx, C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
@@ -590,6 +597,12 @@ class Context:
         keys, lo = keys[: n.value], lo[: n.value]
         k3 = np.stack([(keys >> np.uint64(16 * a)) & np.uint64(0xFFFF) for a in range(3)], axis=1).astype(np.uint16)
         return k3, lo
+
+    def occupancy_octomap(self, binary: bool = False) -> bytes:
+        """The map as octomap_msgs/Octomap data (octomap_server's /octomap_full, or /octomap_binary with binary)."""
+        m = Octomap()
+        self._check(lib().d2pc_occupancy_octomap(self._h, 1 if binary else 0, C.byref(m)), "d2pc_occupancy_octomap")
+        return C.string_at(m.data, m.size) if m.size else b""
 
     def occupancy_insert_device(self, d_in, n_frames, n_max, in_stride, d_in_counts, origins):
         """d2pc_occupancy_insert_device: clouds on the device into the map, frame f from origins[f] (host, (n, 3))."""

@@ -161,6 +161,7 @@ struct d2pc_ctx {
   MapTable map;               // carved from map_mem
   uint32_t map_epoch = 0;     // of the last frame inserted (marks are tagged with it)
   DevBuf map_tmp, map_out, map_n;  // export scratch, output staging and counters
+  PinBuf octomap;                  // d2pc_occupancy_octomap's data, valid until the next call
   cudaStream_t s_map = nullptr;    // every map step and export, in submission order
   cudaEvent_t ev_map_in = nullptr; // orders d2pc_occupancy_insert_device behind the compute stream
   // fusion buffers
@@ -1122,6 +1123,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
   free_dev(ctx->d_color_in), free_dev(ctx->d_color_out), free_dev(ctx->d_color_lut), free_pin(ctx->h_color);
   free_pin(ctx->h_stage);
   free_dev(ctx->map_mem), free_dev(ctx->map_tmp), free_dev(ctx->map_out), free_dev(ctx->map_n);
+  free_pin(ctx->octomap);
   if (ctx->ev_map_in) cudaEventDestroy(ctx->ev_map_in);
   if (ctx->s_map) cudaStreamDestroy(ctx->s_map);
   if (ctx->d_ticket) cudaFree(ctx->d_ticket);
@@ -1384,6 +1386,42 @@ int d2pc_occupancy_voxels(d2pc_ctx *ctx, uint64_t *keys, float *log_odds_out, ui
                             cudaMemcpyDeviceToHost, ctx->s_map));
   }
   CU(ctx, cudaStreamSynchronize(ctx->s_map));
+  return D2PC_OK;
+}
+
+int d2pc_occupancy_octomap(d2pc_ctx *ctx, int binary, d2pc_octomap *out) {
+  if (!ctx || !out || binary < 0 || binary > 1) return D2PC_ERR_INVALID_ARG;
+  CU(ctx, cudaSetDevice(ctx->device));
+  uint32_t n = 0;
+  int rc = map_export_count(ctx, false, &n);
+  if (rc) return rc;
+  unsigned long long records = 0;
+  if (n) {
+    if ((rc = grow_dev(ctx, ctx->map_tmp, octomap_temp_bytes(n)))) return rc;
+    CU(ctx, octomap_plan(ctx->map, n, binary, ctx->map_tmp.p, reinterpret_cast<uint32_t *>(ctx->map_n.p) + 1,
+                         &records, ctx->s_map));
+    CU(ctx, cudaStreamSynchronize(ctx->s_map));  // the size of the stream sizes the result
+  }
+  const size_t bytes = records * (binary ? 2 : 5);
+  if (bytes && (rc = grow_dev(ctx, ctx->map_out, octomap_out_bytes(records, binary)))) return rc;
+  if (bytes > ctx->octomap.cap) {
+    // a new buffer before the old one goes, so a failed allocation leaves the last result as it was
+    void *p = nullptr;
+    const size_t cap = round_up(bytes, 1 << 16);
+    CU(ctx, pinned_alloc(&p, cap));
+    free_pin(ctx->octomap);
+    ctx->octomap.p = static_cast<uint8_t *>(p), ctx->octomap.cap = cap;
+  }
+  if (bytes) {
+    CU(ctx, octomap_emit(ctx->map, n, binary, log_odds(ctx->occ.occupancy_thres), ctx->map_tmp.p, records,
+                         ctx->map_out.p, ctx->s_map));
+    CU(ctx, cudaMemcpyAsync(ctx->octomap.p, ctx->map_out.p, bytes, cudaMemcpyDeviceToHost, ctx->s_map));
+    CU(ctx, cudaStreamSynchronize(ctx->s_map));
+  }
+  out->data = bytes ? ctx->octomap.p : nullptr;
+  out->size = bytes;
+  out->resolution = ctx->occ.resolution;
+  out->binary = binary;
   return D2PC_OK;
 }
 

@@ -15,7 +15,9 @@
 //          abort and clamp; nothing at all when the overflow flag is set, so a dropped frame leaves the known map as
 //          it was.
 //   finish one thread: counts the frame as applied or dropped and clears the flag and the touched count.
+// The export sorts the known voxels by Morton code (map_sort); the octomap serialization below builds the tree on it.
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 #include "map_math.h"
 #include "occupancy.h"
@@ -289,10 +291,8 @@ size_t map_export_temp_bytes(uint32_t n) {
   return 2 * align_up((size_t)n * 8) + 2 * align_up((size_t)n * 4) + cub_sort_bytes(n);
 }
 
-cudaError_t map_export(const MapTable &t, bool occupied_only, float occ_thres, double res, uint32_t n, void *temp,
-                       uint32_t *d_pos, float4 *centres, unsigned long long *keys, float *log_odds,
-                       cudaStream_t stream) {
-  if (n == 0) return cudaSuccess;
+cudaError_t map_sort(const MapTable &t, bool occupied_only, float occ_thres, uint32_t n, void *temp, uint32_t *d_pos,
+                     const unsigned long long **morton, const uint32_t **vals, cudaStream_t stream) {
   uint8_t *p = static_cast<uint8_t *>(temp);
   auto *m0 = reinterpret_cast<unsigned long long *>(p);
   auto *m1 = reinterpret_cast<unsigned long long *>(p + align_up((size_t)n * 8));
@@ -300,16 +300,261 @@ cudaError_t map_export(const MapTable &t, bool occupied_only, float occ_thres, d
   auto *v1 = reinterpret_cast<uint32_t *>(p + 2 * align_up((size_t)n * 8) + align_up((size_t)n * 4));
   void *sort_temp = p + 2 * align_up((size_t)n * 8) + 2 * align_up((size_t)n * 4);
   size_t sort_bytes = cub_sort_bytes(n);
+  *morton = m1;
+  *vals = v1;
   cudaError_t e = cudaMemsetAsync(d_pos, 0, 4, stream);
   if (e != cudaSuccess) return e;
   const uint32_t grid = t.cap < 4096 ? t.cap : 4096;
   map_gather_kernel<<<grid, kApplyThreads, 0, stream>>>(t, occupied_only, occ_thres, d_pos, m0, v0);
   if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  if ((e = cub::DeviceRadixSort::SortPairs(sort_temp, sort_bytes, m0, m1, v0, v1, (int)n, 0, 48, stream)) !=
-      cudaSuccess)
-    return e;
-  map_write_kernel<<<(n + kStageThreads - 1) / kStageThreads, kStageThreads, 0, stream>>>(m1, v1, n, res, centres,
+  return cub::DeviceRadixSort::SortPairs(sort_temp, sort_bytes, m0, m1, v0, v1, (int)n, 0, 48, stream);
+}
+
+cudaError_t map_export(const MapTable &t, bool occupied_only, float occ_thres, double res, uint32_t n, void *temp,
+                       uint32_t *d_pos, float4 *centres, unsigned long long *keys, float *log_odds,
+                       cudaStream_t stream) {
+  if (n == 0) return cudaSuccess;
+  const unsigned long long *m;
+  const uint32_t *v;
+  cudaError_t e = map_sort(t, occupied_only, occ_thres, n, temp, d_pos, &m, &v, stream);
+  if (e != cudaSuccess) return e;
+  map_write_kernel<<<(n + kStageThreads - 1) / kStageThreads, kStageThreads, 0, stream>>>(m, v, n, res, centres,
                                                                                           keys, log_odds);
+  return cudaGetLastError();
+}
+
+// ---- octomap_msgs/Octomap serialization (the recipe is in include/d2pc_b200.h)
+//
+// From the known voxels sorted by Morton code (map_sort), with n voxels, s_i the first level at which voxel i starts
+// a node (0 for i = 0, else 1 + the leading equal 3-bit digits of m_i and m_{i-1}) and lambda_i the shallowest leaf
+// level on its path, voxel i writes the nodes of levels s_i .. lambda_i (full) or s_i .. lambda_i - 1 (binary, inner
+// nodes only), none when lambda_i < s_i (it lies inside a leaf an earlier voxel wrote).  Node (L, i), started by voxel
+// i, is record off_i + L - s_i in either format, so a voxel's records are consecutive and pre-order is voxel order.
+//   octo_flags  runs d_i = (v_i != v_{i-1}) and s_i
+//   (scan)      D = inclusive sum of d: v is constant on [a, b] iff D_a == D_b
+//   octo_levels lambda_i: node (L, i) is full when the codes at both ends of its 8^(16-L) aligned range are present,
+//               and a leaf when full and constant; leaf(L) implies leaf(L + 1), so lambda is found from level 16 up.
+//               Writes the record count of the format
+//   (scan)      off over n + 1 counts: off_n is the total, the one value the host waits for
+//   octo_link   per writing voxel: the parent record of its first node (a binary search for the parent's first
+//               voxel unless i starts the parent too), then each of its nodes ORs its child bit (full) or its 2-bit
+//               code (binary) into its parent's record in the output; the binary stream is complete here
+//   octo_max    full only, levels 16 .. 1: each node of the level atomicMax'es its value into its parent's
+//   octo_emit   full only: the 4 value bytes of every record
+namespace {
+
+constexpr int kOctoThreads = 256;
+
+__device__ __forceinline__ uint32_t ordered(uint32_t f) { return f ^ ((f >> 31) ? 0xffffffffu : 0x80000000u); }
+__device__ __forceinline__ uint32_t unordered(uint32_t o) { return o ^ ((o >> 31) ? 0x80000000u : 0xffffffffu); }
+__device__ __forceinline__ uint32_t level_of(uint16_t sl) { return sl & 0xff; }      // s
+__device__ __forceinline__ uint32_t leaf_of(uint16_t sl) { return sl >> 8; }         // lambda
+__device__ __forceinline__ uint32_t digit(unsigned long long m, uint32_t level) {   // child index of node (level)
+  return (uint32_t)(m >> (3 * (16 - level))) & 7u;
+}
+
+__global__ void __launch_bounds__(kOctoThreads) octo_flags_kernel(const unsigned long long *__restrict__ m,
+                                                                  const uint32_t *__restrict__ v, uint32_t n,
+                                                                  uint32_t *d, uint16_t *sl) {
+  const uint32_t i = blockIdx.x * kOctoThreads + threadIdx.x;
+  if (i >= n) return;
+  uint32_t s = 0, diff = 0;
+  if (i > 0) {
+    const int h = 63 - __clzll((long long)(m[i] ^ m[i - 1]));  // codes are distinct
+    s = 16 - h / 3;
+    diff = v[i] != v[i - 1];
+  }
+  d[i] = diff;
+  sl[i] = (uint16_t)s;
+}
+
+__global__ void __launch_bounds__(kOctoThreads) octo_levels_kernel(const unsigned long long *__restrict__ m,
+                                                                   const uint32_t *__restrict__ D, uint32_t n,
+                                                                   bool binary, uint16_t *sl,
+                                                                   unsigned long long *cnt) {
+  const uint32_t i = blockIdx.x * kOctoThreads + threadIdx.x;
+  if (i > n) return;
+  if (i == n) {
+    cnt[n] = 0;
+    return;
+  }
+  const unsigned long long mi = m[i];
+  uint32_t lam = 16;
+  for (int L = 15; L >= 0; --L) {
+    const unsigned long long size = 1ull << (3 * (16 - L)), off = mi & (size - 1);
+    if (size > n || off > i) break;
+    const unsigned long long a = i - off, b = a + size - 1;
+    if (b >= n || m[a] != mi - off || m[b] != mi - off + size - 1 || D[a] != D[b]) break;
+    lam = (uint32_t)L;
+  }
+  const uint32_t s = level_of(sl[i]);
+  sl[i] = (uint16_t)(s | (lam << 8));
+  cnt[i] = lam < s ? 0 : lam - s + (binary ? 0 : 1);
+}
+
+// The record of node (level, voxel p), p its first voxel.
+__device__ __forceinline__ unsigned long long record(const unsigned long long *off, const uint16_t *sl, uint32_t p,
+                                                     uint32_t level) {
+  return off[p] + level - level_of(sl[p]);
+}
+
+// ORs `bits` into byte `at` of the output (the word that holds it: the other bytes are left as they are).
+__device__ __forceinline__ void or_byte(uint8_t *out, unsigned long long at, uint32_t bits) {
+  atomicOr(reinterpret_cast<uint32_t *>(out + (at & ~3ull)), bits << (8 * (at & 3)));
+}
+
+__global__ void __launch_bounds__(kOctoThreads) octo_link_kernel(const unsigned long long *__restrict__ m,
+                                                                 const uint32_t *__restrict__ v,
+                                                                 const uint16_t *__restrict__ sl,
+                                                                 const unsigned long long *__restrict__ off,
+                                                                 uint32_t n, bool binary, float occ_thres,
+                                                                 unsigned long long *up, uint8_t *out) {
+  const uint32_t i = blockIdx.x * kOctoThreads + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t s = level_of(sl[i]), lam = leaf_of(sl[i]);
+  if (lam < s) return;
+  const unsigned long long mi = m[i], r0 = off[i];
+  if (s > 0) {
+    // the parent (level s - 1) started at an earlier voxel: the first one whose code has the parent's prefix
+    const uint32_t P = s - 1;
+    const unsigned long long base = mi & ~((1ull << (3 * (16 - P))) - 1);
+    uint32_t lo = (mi - base) > i ? 0 : (uint32_t)(i - (mi - base)), hi = i - 1;
+    while (lo < hi) {
+      const uint32_t mid = lo + (hi - lo) / 2;
+      if (m[mid] < base) lo = mid + 1;
+      else hi = mid;
+    }
+    up[i] = record(off, sl, lo, P);
+  }
+  const float val = __uint_as_float(v[i]);
+  for (uint32_t L = s > 0 ? s : 1; L <= lam; ++L) {
+    const unsigned long long parent = L == s ? up[i] : r0 + (L - 1 - s);
+    const uint32_t c = digit(mi, L);
+    if (binary) {
+      const uint32_t code = L < lam ? 3u : (val >= occ_thres ? 2u : 1u);
+      const uint32_t bits = code << (2 * c);  // a little-endian uint16: children 0-3 in byte 0, 4-7 in byte 1
+      if (bits & 0xff) or_byte(out, 2 * parent, bits & 0xff);
+      if (bits >> 8) or_byte(out, 2 * parent + 1, bits >> 8);
+    } else {
+      or_byte(out, 5 * parent + 4, 1u << c);
+    }
+  }
+}
+
+// level L's nodes into their parents' values (vmax holds ordered floats, 0 below every value)
+__global__ void __launch_bounds__(kOctoThreads) octo_max_kernel(const uint32_t *__restrict__ v,
+                                                                const uint16_t *__restrict__ sl,
+                                                                const unsigned long long *__restrict__ off,
+                                                                const unsigned long long *__restrict__ up, uint32_t n,
+                                                                uint32_t L, uint32_t *vmax) {
+  const uint32_t i = blockIdx.x * kOctoThreads + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t s = level_of(sl[i]), lam = leaf_of(sl[i]);
+  if (L < s || L > lam) return;
+  const unsigned long long r = off[i] + (L - s);
+  const uint32_t val = L == lam ? ordered(v[i]) : vmax[r];
+  atomicMax(vmax + (L == s ? up[i] : r - 1), val);
+}
+
+__global__ void __launch_bounds__(kOctoThreads) octo_emit_kernel(const uint32_t *__restrict__ v,
+                                                                 const uint16_t *__restrict__ sl,
+                                                                 const unsigned long long *__restrict__ off,
+                                                                 const uint32_t *__restrict__ vmax, uint32_t n,
+                                                                 uint8_t *out) {
+  const uint32_t i = blockIdx.x * kOctoThreads + threadIdx.x;
+  if (i >= n) return;
+  const uint32_t s = level_of(sl[i]), lam = leaf_of(sl[i]);
+  for (uint32_t L = s; L <= lam; ++L) {
+    const unsigned long long r = off[i] + (L - s);
+    const uint32_t f = L == lam ? v[i] : unordered(vmax[r]);
+    uint8_t *p = out + 5 * r;
+    p[0] = (uint8_t)f, p[1] = (uint8_t)(f >> 8), p[2] = (uint8_t)(f >> 16), p[3] = (uint8_t)(f >> 24);
+  }
+}
+
+size_t cub_sum_bytes(uint32_t n) {
+  size_t a = 0, b = 0;
+  cub::DeviceScan::InclusiveSum(nullptr, a, (const uint32_t *)nullptr, (uint32_t *)nullptr, (int)n);
+  cub::DeviceScan::ExclusiveSum(nullptr, b, (const unsigned long long *)nullptr, (unsigned long long *)nullptr,
+                                (int)n + 1);
+  return a > b ? a : b;
+}
+
+// the parts of the octomap scratch behind map_sort's
+struct OctoTemp {
+  uint32_t *d, *D;
+  uint16_t *sl;
+  unsigned long long *cnt, *off, *up;
+  void *scan;
+  size_t scan_bytes;
+};
+OctoTemp octo_temp(void *temp, uint32_t n) {
+  uint8_t *p = static_cast<uint8_t *>(temp) + align_up(map_export_temp_bytes(n));  // CUB's part is not aligned
+  OctoTemp o;
+  auto take = [&](size_t bytes) {
+    uint8_t *q = p;
+    p += align_up(bytes);
+    return q;
+  };
+  o.d = reinterpret_cast<uint32_t *>(take((size_t)n * 4));
+  o.D = reinterpret_cast<uint32_t *>(take((size_t)n * 4));
+  o.sl = reinterpret_cast<uint16_t *>(take((size_t)n * 2));
+  o.cnt = reinterpret_cast<unsigned long long *>(take(((size_t)n + 1) * 8));
+  o.off = reinterpret_cast<unsigned long long *>(take(((size_t)n + 1) * 8));
+  o.up = o.cnt;  // the counts are dead once scanned
+  o.scan_bytes = cub_sum_bytes(n);
+  o.scan = take(o.scan_bytes);
+  return o;
+}
+
+}  // namespace
+
+size_t octomap_temp_bytes(uint32_t n) {
+  return align_up(map_export_temp_bytes(n)) + 2 * align_up((size_t)n * 4) + align_up((size_t)n * 2) +
+         2 * align_up(((size_t)n + 1) * 8) + align_up(cub_sum_bytes(n));
+}
+
+cudaError_t octomap_plan(const MapTable &t, uint32_t n, bool binary, void *temp, uint32_t *d_pos,
+                         unsigned long long *records, cudaStream_t stream) {
+  const unsigned long long *m;
+  const uint32_t *v;
+  OctoTemp o = octo_temp(temp, n);
+  cudaError_t e = map_sort(t, false, 0.0f, n, temp, d_pos, &m, &v, stream);
+  if (e != cudaSuccess) return e;
+  const uint32_t grid = (n + kOctoThreads - 1) / kOctoThreads, grid1 = n / kOctoThreads + 1;
+  octo_flags_kernel<<<grid, kOctoThreads, 0, stream>>>(m, v, n, o.d, o.sl);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  if ((e = cub::DeviceScan::InclusiveSum(o.scan, o.scan_bytes, o.d, o.D, (int)n, stream)) != cudaSuccess) return e;
+  octo_levels_kernel<<<grid1, kOctoThreads, 0, stream>>>(m, o.D, n, binary, o.sl, o.cnt);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  if ((e = cub::DeviceScan::ExclusiveSum(o.scan, o.scan_bytes, o.cnt, o.off, (int)n + 1, stream)) != cudaSuccess)
+    return e;
+  return cudaMemcpyAsync(records, o.off + n, 8, cudaMemcpyDeviceToHost, stream);
+}
+
+size_t octomap_out_bytes(unsigned long long records, bool binary) {
+  return binary ? align_up(records * 2 + 4) : align_up(records * 5 + 4) + align_up(records * 4);
+}
+
+cudaError_t octomap_emit(const MapTable &t, uint32_t n, bool binary, float occ_thres, void *temp,
+                         unsigned long long records, uint8_t *out, cudaStream_t stream) {
+  const OctoTemp o = octo_temp(temp, n);
+  const unsigned long long *m = reinterpret_cast<const unsigned long long *>(static_cast<uint8_t *>(temp) +
+                                                                             align_up((size_t)n * 8));
+  const uint32_t *v = reinterpret_cast<const uint32_t *>(static_cast<uint8_t *>(temp) + 2 * align_up((size_t)n * 8) +
+                                                         align_up((size_t)n * 4));
+  const size_t bytes = binary ? records * 2 : records * 5;
+  uint32_t *vmax = binary ? nullptr : reinterpret_cast<uint32_t *>(out + align_up(bytes + 4));
+  cudaError_t e = cudaMemsetAsync(out, 0, bytes, stream);
+  if (e != cudaSuccess) return e;
+  if (vmax && (e = cudaMemsetAsync(vmax, 0, records * 4, stream)) != cudaSuccess) return e;
+  const uint32_t grid = (n + kOctoThreads - 1) / kOctoThreads;
+  octo_link_kernel<<<grid, kOctoThreads, 0, stream>>>(m, v, o.sl, o.off, n, binary, occ_thres, o.up, out);
+  if (!binary) {
+    for (uint32_t L = 16; L >= 1; --L)
+      octo_max_kernel<<<grid, kOctoThreads, 0, stream>>>(v, o.sl, o.off, o.up, n, L, vmax);
+    octo_emit_kernel<<<grid, kOctoThreads, 0, stream>>>(v, o.sl, o.off, vmax, n, out);
+  }
   return cudaGetLastError();
 }
 

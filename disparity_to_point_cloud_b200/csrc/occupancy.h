@@ -54,5 +54,20 @@ size_t map_export_temp_bytes(uint32_t n);
 cudaError_t map_export(const MapTable &t, bool occupied_only, float occ_thres, double res, uint32_t n, void *temp,
                        uint32_t *d_pos, float4 *centres, unsigned long long *keys, float *log_odds,
                        cudaStream_t stream);
+// The first step of map_export: the voxels gathered and sorted by Morton code inside temp (*morton, *vals).
+cudaError_t map_sort(const MapTable &t, bool occupied_only, float occ_thres, uint32_t n, void *temp, uint32_t *d_pos,
+                     const unsigned long long **morton, const uint32_t **vals, cudaStream_t stream);
+
+// octomap_msgs/Octomap data of the n known voxels (> 0) in two steps on one temp of octomap_temp_bytes(n), both
+// asynchronous on `stream`.  octomap_plan: sorts the voxels and places the tree's records (full: every written node,
+// 5 bytes; binary: every written inner node, 2 bytes), their count into the host's *records.  octomap_emit, once
+// *records is there: the stream into out, which holds octomap_out_bytes(records, binary), the data in its first
+// records * 5 (or * 2) bytes.
+size_t octomap_temp_bytes(uint32_t n);
+cudaError_t octomap_plan(const MapTable &t, uint32_t n, bool binary, void *temp, uint32_t *d_pos,
+                         unsigned long long *records, cudaStream_t stream);
+size_t octomap_out_bytes(unsigned long long records, bool binary);
+cudaError_t octomap_emit(const MapTable &t, uint32_t n, bool binary, float occ_thres, void *temp,
+                         unsigned long long records, uint8_t *out, cudaStream_t stream);
 
 }  // namespace d2pc

@@ -478,7 +478,8 @@ int d2pc_laser_scan_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames
  * octomap_point_cloud_centers with compress_map off, byte for byte: {(float)centre(kx), (float)centre(ky),
  * (float)centre(kz), 1.0f} per occupied voxel.  octomap merges eight equal siblings into one coarser leaf when it
  * prunes (compress_map on, and as recalled also inside updateNode); it would then publish one coarser point for a
- * uniform octant where this library publishes the eight full-depth voxels with the same value.
+ * uniform octant where this library publishes the eight full-depth voxels with the same value.  d2pc_occupancy_centers
+ * stays per full-depth voxel; d2pc_occupancy_octomap below follows updateNode's pruning.
  * The device map: a hash of 8x8x8-voxel bricks (max_bricks of them; the table has 2 * max_bricks slots rounded up to a
  * power of two, each about 4.2 KB).  A frame that would take the map past max_bricks bricks is dropped as a whole: the
  * known map stays bit for bit what it was and d2pc_occupancy_stats counts the drop.  Bricks made by a dropped frame stay
@@ -537,6 +538,55 @@ int d2pc_occupancy_voxels(d2pc_ctx *ctx, uint64_t *keys, float *log_odds, uint64
  * (d2pc_compute_stream) and after every earlier map update; d2pc_sync waits for it. */
 int d2pc_occupancy_insert_device(d2pc_ctx *ctx, const uint8_t *d_in, uint32_t n_frames, uint32_t n_max,
                                  size_t in_stride, const uint32_t *d_in_counts, const float *origins);
+
+/* ---- the map as octomap_msgs/Octomap (octomap_server's /octomap_full and /octomap_binary) ----------------------------
+ *
+ * Reference: octomap_msgs::fullMapToMsg / binaryMapToMsg of the OcTree octomap_server keeps, restated from memory like
+ * the recipe above.  The recipe:
+ *   1. tree shape: OccupancyOcTreeBase::updateNode with lazy_eval false (as insertScan calls it) prunes on its way
+ *      back up every update path: pruneNode collapses a node when isNodeCollapsible holds (all 8 children exist, none
+ *      has children, every child's value == child 0's, a float compare), otherwise updateOccupancyChildren sets the
+ *      node to the max of its existing children's log-odds.  Updating a key under a pruned leaf first expands it (8
+ *      children with the parent's value).
+ *   2. consequence: after any sequence of updates the tree is a function of the known full-depth voxels alone.  A
+ *      level-L node (L = 0 the root, 16 a voxel) exists iff some known voxel has its top L Morton digits; it is a leaf
+ *      iff L = 16, or all 8^(16-L) voxels under it are known with equal log-odds; it is written iff no proper ancestor
+ *      is a leaf; its value is the max log-odds of the voxels under it.  (Every ancestor on an update path is
+ *      re-checked bottom-up and nodes off the path do not change, so maximal pruning is an invariant; pruning is
+ *      lossless and expanding restores equal children, so each voxel's value is the flat map's.  Log-odds are never
+ *      NaN and never -0.0 -- logodds(0.5) is +0 and a new voxel starts at +0 -- so == and bit equality agree.)
+ *      tests/test_oracle_octomap_msg.py checks this against a pointer tree that restates updateNode literally.
+ *   3. child index at level L: x_bit | y_bit << 1 | z_bit << 2 of key bit 15 - L, the Morton digit the export sorts
+ *      by, so pre-order is Morton order, parent before child.
+ *   4. full (fullMapToMsg -> OcTree::writeData -> writeNodesRecurs): pre-order over the written nodes; each writes its
+ *      float value (4 bytes, little endian), then one byte of std::bitset<8> child-exists mask (bit i = child i; 0 for
+ *      a leaf), then its children in index order.  An empty tree writes 0 bytes.
+ *   5. binary (binaryMapToMsg -> the const writeBinaryData, so no toMaxLikelihood or prune -> writeBinaryNode): each
+ *      written inner node writes 2 bytes in pre-order, children 0-3 then 4-7, child i in the 2 bits at 2i (of its
+ *      byte): 0 unknown, 1 free leaf (octomap's "10": bit 2i set), 2 occupied leaf (log-odds >= occ_thres_log of the
+ *      current occupancy_thres), 3 has children.  The recursion visits only children with children; the root is
+ *      always written as an inner node.  An empty map writes 0 bytes.
+ *   6. message: id "OcTree", resolution as float64, binary 0 / 1, data the bytes above without the .ot file header.
+ * What rests on recollection and is not verified against the sources: all of items 1, 4, 5 and 6 -- that updateNode
+ * prunes with lazy_eval false, isNodeCollapsible's three conditions and its float ==, updateOccupancyChildren's max,
+ * expandNode's copies, writeNodesRecurs' value-then-mask layout, writeBinaryNode's bit pairs and its skip of leaf
+ * children, that binaryMapToMsg neither converts to maximum likelihood nor prunes, and the message's id and fields.
+ * On the device: the known voxels are sorted as for d2pc_occupancy_voxels, then every node's first voxel, leaf level
+ * and record offset come from two scans, and one thread per voxel writes the nodes that voxel starts
+ * (csrc/occupancy.cu).  The library does this work only when this call is made. */
+typedef struct d2pc_octomap {
+  const uint8_t *data; /* page-locked memory the library owns: valid until the next call on the context or
+                          d2pc_destroy; NULL when size is 0 */
+  uint64_t size;       /* bytes of data */
+  double resolution;   /* the map's resolution (m) */
+  int32_t binary;      /* 0: octomap_full's data, 1: octomap_binary's */
+} d2pc_octomap;
+
+/* The map serialized as octomap_msgs/Octomap data: binary 0 the full format, 1 the binary format (recipe above).
+ * Synchronous; reflects every frame submitted before the call, like d2pc_occupancy_centers.  An empty map gives size 0
+ * and D2PC_OK.  D2PC_ERR_INVALID_ARG for binary outside {0, 1}; D2PC_ERR_NOMEM when a host or device allocation fails,
+ * leaving the map and the previous result as they were. */
+int d2pc_occupancy_octomap(d2pc_ctx *ctx, int binary, d2pc_octomap *out);
 
 /* ---- the disparity callback, host buffers (the reference-facing calls) ------ */
 

@@ -20,6 +20,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdio>
+#include <cstring>
 #include <fstream>
 #include <functional>
 #include <map>
@@ -42,6 +43,7 @@ class Bus {
   using ImageCb = std::function<void(const sensor_msgs::ImageConstPtr &)>;
   using CloudCb = std::function<void(const sensor_msgs::PointCloud2 &)>;
   using ScanCb = std::function<void(const sensor_msgs::LaserScan &)>;
+  using OctomapCb = std::function<void(const ros_lite::octomap_msgs::Octomap &)>;
 
   // <remap from="/disparity" to="/throttled_depth_map"/>
   void remap(const std::string &from, const std::string &to) { remaps_[from] = to; }
@@ -81,6 +83,9 @@ class Bus {
   void subscribe_scan(const std::string &topic, uint32_t queue_size, ScanCb cb) {
     scan_subs_[resolve(topic)].push_back({queue_size, std::move(cb)});
   }
+  void subscribe_octomap(const std::string &topic, uint32_t queue_size, OctomapCb cb) {
+    octomap_subs_[resolve(topic)].push_back({queue_size, std::move(cb)});
+  }
   struct Advertised {
     std::string topic;
     uint32_t queue_size;
@@ -108,10 +113,16 @@ class Bus {
     if (it != scan_subs_.end())
       for (auto &s : it->second) s.cb(msg);
   }
+  void publish(const std::string &resolved_topic, const ros_lite::octomap_msgs::Octomap &msg) {
+    auto it = octomap_subs_.find(resolved_topic);
+    if (it != octomap_subs_.end())
+      for (auto &s : it->second) s.cb(msg);
+  }
   const std::vector<Advertised> &advertised() const { return advertised_; }
   bool has_subscribers(const std::string &resolved_topic) const {  // ros::Publisher::getNumSubscribers() > 0
     auto it = image_subs_.find(resolved_topic);
-    return it != image_subs_.end() && !it->second.empty();
+    auto ot = octomap_subs_.find(resolved_topic);
+    return (it != image_subs_.end() && !it->second.empty()) || (ot != octomap_subs_.end() && !ot->second.empty());
   }
 
   // Reads <remap from= to=/> and <param name= value=/> out of a roslaunch file (launch/*.launch).  A value that
@@ -163,6 +174,7 @@ class Bus {
   std::map<std::string, std::vector<Sub<ImageCb>>> image_subs_;
   std::map<std::string, std::vector<Sub<CloudCb>>> cloud_subs_;
   std::map<std::string, std::vector<Sub<ScanCb>>> scan_subs_;
+  std::map<std::string, std::vector<Sub<OctomapCb>>> octomap_subs_;
   std::map<std::string, sensor_msgs::PointCloud2> latched_clouds_;
   std::vector<Advertised> advertised_;
 };
@@ -234,6 +246,8 @@ class Disparity2PCloud {
   sensor_msgs::LaserScan scan_;
   std::string p_map_topic_;  // "/octomap_point_cloud_centers" when map_enable != 0
   sensor_msgs::PointCloud2 centres_;
+  std::string p_octomap_topic_[2];  // "/octomap_full", "/octomap_binary" when map_enable != 0
+  ros_lite::octomap_msgs::Octomap octomap_;
 
   // make output_.data hold `bytes` bytes in page-locked storage without touching bytes it already has
   void reserve_output(size_t bytes) {
@@ -364,6 +378,8 @@ class Disparity2PCloud {
     // map_occupancy_thres and map_max_range are octomap_server's resolution, sensor_model/* and occupancy params with
     // its defaults; map_max_bricks sizes the device map; map_keep_cloud 0 leaves the cloud on the device and
     // /point_cloud unpublished.  The sensor origin is the transform's translation: set the transform params.
+    // The map also goes out as octomap_msgs/Octomap on /octomap_full and /octomap_binary (octomap_server with
+    // latch false), each serialized only while somebody subscribes to it.
     int map_on = 0;
     nh_.param<int>("map_enable", map_on, 0);
     if (map_on) {
@@ -384,6 +400,8 @@ class Disparity2PCloud {
       d2pc_b200::check(d2pc_set_occupancy(ctx_, &o), "d2pc_set_occupancy", ctx_);
       publish_cloud_ = publish_cloud_ && o.keep_cloud != 0;
       p_map_topic_ = nh_.advertise("/octomap_point_cloud_centers", 1);
+      p_octomap_topic_[0] = nh_.advertise("/octomap_full", 1);
+      p_octomap_topic_[1] = nh_.advertise("/octomap_binary", 1);
     }
   }
   ~Disparity2PCloud() {
@@ -436,6 +454,18 @@ class Disparity2PCloud {
       describe(c, centres_);
       centres_.header = output.header;
       nh_.publish(p_map_topic_, centres_);
+      for (int binary = 0; binary < 2; ++binary) {
+        if (!nh_.has_subscribers(p_octomap_topic_[binary])) continue;
+        d2pc_octomap m;
+        d2pc_b200::check(d2pc_occupancy_octomap(ctx_, binary, &m), "d2pc_occupancy_octomap", ctx_);
+        octomap_.header = output.header;
+        octomap_.binary = static_cast<uint8_t>(binary);
+        octomap_.id = "OcTree";
+        octomap_.resolution = m.resolution;
+        octomap_.data.resize(m.size);
+        if (m.size) std::memcpy(octomap_.data.data(), m.data, m.size);
+        nh_.publish(p_octomap_topic_[binary], octomap_);
+      }
     }
   }
   // a PointCloud2's fields from the library's d2pc_cloud; data keeps its storage and shows the cloud's bytes

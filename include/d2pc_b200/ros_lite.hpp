@@ -2,7 +2,8 @@
 // wire (de)serialisation, so the node classes in nodes.hpp compile and run without a ROS installation.
 // Field order and types follow the message definitions the reference uses:
 //   std_msgs/Header, sensor_msgs/Image, sensor_msgs/PointField, sensor_msgs/PointCloud2, and sensor_msgs/LaserScan
-//   (pointcloud_to_laserscan's output, which the point cloud node can publish next to its cloud)
+//   (pointcloud_to_laserscan's output, which the point cloud node can publish next to its cloud), and
+//   octomap_msgs/Octomap (octomap_server's /octomap_full and /octomap_binary, published next to it with the map on)
 //   (src/disparity_to_point_cloud.cpp:46-92, src/depth_map_fusion.cpp:46-136).
 // With a real ROS1 the ros1_shim/ sources use the genuine sensor_msgs types instead; the layouts are identical.
 #pragma once
@@ -65,6 +66,18 @@ struct LaserScan {
 
 }  // namespace sensor_msgs
 
+namespace octomap_msgs {
+
+struct Octomap {
+  Header header;
+  uint8_t binary = 0;  // bool
+  std::string id;
+  double resolution = 0;
+  std::vector<int8_t> data;
+};
+
+}  // namespace octomap_msgs
+
 // ---- ROS1 serialisation: little endian, strings and arrays prefixed by a uint32 length --------------------
 class Writer {
  public:
@@ -91,6 +104,16 @@ class Writer {
   void floats(const std::vector<float> &d) {
     u32(static_cast<uint32_t>(d.size()));
     for (float v : d) f32(v);
+  }
+  void f64(double v) {
+    uint8_t b[8];
+    std::memcpy(b, &v, 8);
+    buf.insert(buf.end(), b, b + 8);
+  }
+  void int8s(const std::vector<int8_t> &d) {
+    u32(static_cast<uint32_t>(d.size()));
+    const uint8_t *p = reinterpret_cast<const uint8_t *>(d.data());
+    buf.insert(buf.end(), p, p + d.size());
   }
   void header(const Header &h) {
     u32(h.seq), u32(h.stamp.sec), u32(h.stamp.nsec), str(h.frame_id);
@@ -136,6 +159,21 @@ class Reader {
     need(static_cast<size_t>(n) * 4);
     std::vector<float> d(n);
     for (auto &v : d) v = f32();
+    return d;
+  }
+  double f64() {
+    need(8);
+    double v;
+    std::memcpy(&v, p_, 8);
+    p_ += 8;
+    return v;
+  }
+  std::vector<int8_t> int8s() {
+    const uint32_t n = u32();
+    need(n);
+    std::vector<int8_t> d(n);
+    if (n) std::memcpy(d.data(), p_, n);
+    p_ += n;
     return d;
   }
   Header header() {
@@ -203,6 +241,19 @@ inline sensor_msgs::LaserScan deserialize_laserscan(const uint8_t *p, size_t n) 
   m.angle_min = r.f32(), m.angle_max = r.f32(), m.angle_increment = r.f32(), m.time_increment = r.f32();
   m.scan_time = r.f32(), m.range_min = r.f32(), m.range_max = r.f32();
   m.ranges = r.floats(), m.intensities = r.floats();
+  return m;
+}
+inline std::vector<uint8_t> serialize(const octomap_msgs::Octomap &m) {
+  Writer w;
+  w.header(m.header);
+  w.u8(m.binary), w.str(m.id), w.f64(m.resolution), w.int8s(m.data);
+  return std::move(w.buf);
+}
+inline octomap_msgs::Octomap deserialize_octomap(const uint8_t *p, size_t n) {
+  Reader r(p, n);
+  octomap_msgs::Octomap m;
+  m.header = r.header();
+  m.binary = r.u8(), m.id = r.str(), m.resolution = r.f64(), m.data = r.int8s();
   return m;
 }
 

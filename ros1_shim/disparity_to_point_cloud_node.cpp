@@ -4,6 +4,7 @@
 // Topic names, queue sizes, the (accidentally) latched publisher, parameter names and defaults follow
 // include/disparity_to_point_cloud/disparity_to_point_cloud.hpp:75-106 of the reference, so
 // launch/d2pcloud.launch works unchanged.
+#include <octomap_msgs/Octomap.h>
 #include <ros/ros.h>
 #include <sensor_msgs/Image.h>
 #include <sensor_msgs/LaserScan.h>
@@ -166,7 +167,9 @@ class Disparity2PCloudGpu {
     // on /octomap_point_cloud_centers with the cloud's header after each frame, on when map_enable != 0.  The params
     // are octomap_server's with its defaults (map_resolution, map_sensor_model_{hit,miss,min,max},
     // map_occupancy_thres, map_max_range), map_max_bricks and map_keep_cloud (0: /point_cloud is not published).
-    // The sensor origin is the transform's translation: set transform_*.
+    // The sensor origin is the transform's translation: set transform_*.  The map also goes out as
+    // octomap_msgs/Octomap on /octomap_full and /octomap_binary (octomap_server with latch false), each serialized
+    // only while somebody subscribes to it.
     int map_on = 0;
     nh_.param<int>("map_enable", map_on, 0);
     if (map_on) {
@@ -191,6 +194,8 @@ class Disparity2PCloudGpu {
       } else {
         publish_cloud_ = publish_cloud_ && keep != 0;
         map_pub_ = nh_.advertise<sensor_msgs::PointCloud2>("/octomap_point_cloud_centers", 1);
+        octomap_pub_[0] = nh_.advertise<octomap_msgs::Octomap>("/octomap_full", 1);
+        octomap_pub_[1] = nh_.advertise<octomap_msgs::Octomap>("/octomap_binary", 1);
         map_on_ = true;
       }
     }
@@ -257,6 +262,22 @@ class Disparity2PCloudGpu {
     describe(c, centres_);
     centres_.header = out.header;
     map_pub_.publish(centres_);
+    for (int binary = 0; binary < 2; ++binary) {
+      if (octomap_pub_[binary].getNumSubscribers() == 0) continue;
+      d2pc_octomap m;
+      const int orc = d2pc_occupancy_octomap(ctx_, binary, &m);
+      if (orc != D2PC_OK) {
+        ROS_ERROR("d2pc_occupancy_octomap: %s (%s)", d2pc_strerror(orc), d2pc_last_cuda_error(ctx_));
+        return;
+      }
+      octomap_.header = out.header;
+      octomap_.binary = binary != 0;
+      octomap_.id = "OcTree";
+      octomap_.resolution = m.resolution;
+      octomap_.data.resize(m.size);
+      if (m.size) std::memcpy(octomap_.data.data(), m.data, m.size);
+      octomap_pub_[binary].publish(octomap_);
+    }
   }
 
   // a PointCloud2's fields from the library's d2pc_cloud; data keeps its storage and shows the cloud's bytes
@@ -281,6 +302,8 @@ class Disparity2PCloudGpu {
   ros::NodeHandle nh_;
   ros::Subscriber sub_;
   ros::Publisher pub_, scan_pub_, map_pub_;
+  ros::Publisher octomap_pub_[2];          // /octomap_full, /octomap_binary
+  octomap_msgs::Octomap octomap_;
   bool scan_on_ = false, map_on_ = false;  // scan_enable, map_enable
   bool publish_cloud_ = true;              // scan_keep_cloud and map_keep_cloud
   sensor_msgs::PointCloud2 centres_;       // /octomap_point_cloud_centers

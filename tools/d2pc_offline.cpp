@@ -2,6 +2,8 @@
 //
 //   d2pc_offline wire   <out.bin>
 //       CPU only: serialises a small hand-made PointCloud2 and Image with ros_lite (self-test of the wire code).
+//   d2pc_offline wire-octomap <out.bin>
+//       CPU only: a small hand-made octomap_msgs/Octomap through ros_lite's serialize / deserialize; its wire bytes.
 //   d2pc_offline params <launch file> <name>...
 //       CPU only: loads the launch file into a Bus and prints one line per name: "<name> number <value>" (%.17g),
 //       "<name> string <value>" or "<name> missing" (the launch-file loader's number / string rule).
@@ -14,6 +16,10 @@
 //   d2pc_offline node1map <launch file> <w> <h> <cloud.bin> <centres.bin> <in.raw> [<in.raw> ...]
 //       node1 with the map on (map_enable in the launch file), one frame per <in.raw> stamped (3 + i, 4): the last
 //       PointCloud2 (an empty file when none was published) and the last /octomap_point_cloud_centers cloud.
+//   d2pc_offline node1octomap <launch file> <w> <h> <cloud.bin> <centres.bin> <full.bin> <binary.bin> <in.raw>...
+//       node1map with /octomap_full and /octomap_binary subscribed too: the last message of each (an empty file when
+//       none was published); a path of "-" leaves that topic without a subscriber.  With map_enable 0 in the launch file nothing is subscribed but /point_cloud, and the
+//       harness fails if the node advertised any octomap topic.
 //   d2pc_offline fusion <fusion launch> <w> <h> <d1.raw> <d2.raw> <s1.raw> <s2.raw> <fused.bin> [<cloud.bin> [<debug dir>]]
 //       BASELINE config 5 shape: four mono8 frames into DepthMapFusion; the fused Image is written, and when
 //       <cloud.bin> is given it is also fed to a Disparity2PCloud node whose /disparity is remapped to
@@ -122,6 +128,48 @@ int main(int argc, char **argv) {
       if (n_centres != argc - 7) throw std::runtime_error("not one centres cloud per frame");
       write_file(argv[5], cloud);
       write_file(argv[6], centres);
+      return 0;
+    }
+    if (mode == "wire-octomap" && argc == 3) {
+      ros_lite::octomap_msgs::Octomap m;
+      m.header.seq = 7, m.header.stamp.sec = 11, m.header.stamp.nsec = 13, m.header.frame_id = "/map";
+      m.binary = 1, m.id = "OcTree", m.resolution = 0.05;
+      m.data = {0, -128, 0x3F, -1, 1};
+      auto bytes = ros_lite::serialize(m);
+      auto back = ros_lite::deserialize_octomap(bytes.data(), bytes.size());
+      if (ros_lite::serialize(back) != bytes || back.id != "OcTree" || back.data.size() != 5)
+        throw std::runtime_error("Octomap round trip differs");
+      write_file(argv[2], bytes);
+      return 0;
+    }
+    if (mode == "node1octomap" && argc >= 10) {
+      const uint32_t w = (uint32_t)std::atoi(argv[3]), h = (uint32_t)std::atoi(argv[4]);
+      d2pc_b200::Bus bus;
+      if (!bus.load_launch_file(argv[2])) throw std::runtime_error(std::string("cannot read ") + argv[2]);
+      d2pc::Disparity2PCloud node(bus);
+      bool map_on = false;
+      for (const auto &a : bus.advertised()) map_on = map_on || a.topic == "/octomap_point_cloud_centers";
+      std::vector<uint8_t> cloud, centres, full, binary;
+      bus.subscribe_cloud("/point_cloud", 1, [&](const sm::PointCloud2 &c) { cloud = ros_lite::serialize(c); });
+      if (map_on) {
+        bus.subscribe_cloud("/octomap_point_cloud_centers", 1,
+                            [&](const sm::PointCloud2 &c) { centres = ros_lite::serialize(c); });
+        if (std::string(argv[7]) != "-")
+          bus.subscribe_octomap("/octomap_full", 1,
+                                [&](const ros_lite::octomap_msgs::Octomap &m) { full = ros_lite::serialize(m); });
+        if (std::string(argv[8]) != "-")
+          bus.subscribe_octomap("/octomap_binary", 1,
+                                [&](const ros_lite::octomap_msgs::Octomap &m) { binary = ros_lite::serialize(m); });
+      } else {
+        for (const auto &a : bus.advertised())
+          if (a.topic.find("octomap") != std::string::npos) throw std::runtime_error("map off, " + a.topic + " advertised");
+      }
+      for (int i = 9; i < argc; ++i)  // frame i - 9 stamped (3 + i - 9, 4)
+        bus.publish(bus.resolve("/disparity"), make_image(read_file(argv[i], (size_t)w * h), w, h, 3 + (i - 9), 4));
+      write_file(argv[5], cloud);
+      write_file(argv[6], centres);
+      if (std::string(argv[7]) != "-") write_file(argv[7], full);
+      if (std::string(argv[8]) != "-") write_file(argv[8], binary);
       return 0;
     }
     if (mode == "params" && argc >= 3) {
