@@ -10,6 +10,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import sys
 
 import numpy as np
 
@@ -117,6 +118,18 @@ class Octomap(C.Structure):
                 ("binary", C.c_int32)]
 
 
+class ProjectedMapParams(C.Structure):
+    """d2pc_projected_map_params: octomap_server's parameters of the projected 2-D map."""
+    _fields_ = [("struct_size", C.c_uint32), ("occupancy_min_z", C.c_double), ("occupancy_max_z", C.c_double),
+                ("min_x_size", C.c_double), ("min_y_size", C.c_double)]
+
+
+class GridMap(C.Structure):
+    """d2pc_grid_map: nav_msgs/OccupancyGrid's info and its cells in library-owned memory."""
+    _fields_ = [("data", C.POINTER(C.c_int8)), ("width", C.c_uint32), ("height", C.c_uint32),
+                ("resolution", C.c_float), ("origin_x", C.c_double), ("origin_y", C.c_double)]
+
+
 class LaserScan(C.Structure):
     """d2pc_laser_scan: the message fields of a scan and its library-owned ranges."""
     _fields_ = [("angle_min", C.c_float), ("angle_max", C.c_float), ("angle_increment", C.c_float),
@@ -197,6 +210,8 @@ SYMBOLS = [
     ("d2pc_occupancy_insert_device", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_size_t, C.c_void_p,
                                                C.c_void_p]),
     ("d2pc_occupancy_octomap", C.c_int, [_ctx, C.c_int, C.POINTER(Octomap)]),
+    ("d2pc_projected_map_params_default", None, [C.POINTER(ProjectedMapParams)]),
+    ("d2pc_occupancy_projected_map", C.c_int, [_ctx, C.POINTER(ProjectedMapParams), C.POINTER(GridMap)]),
     ("d2pc_process_mono8", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_process_f32", C.c_int, [_ctx, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.POINTER(Cloud)]),
     ("d2pc_submit_mono8", C.c_int, [_ctx, C.c_int, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32]),
@@ -603,6 +618,21 @@ class Context:
         m = Octomap()
         self._check(lib().d2pc_occupancy_octomap(self._h, 1 if binary else 0, C.byref(m)), "d2pc_occupancy_octomap")
         return C.string_at(m.data, m.size) if m.size else b""
+
+    def occupancy_projected_map(self, occupancy_min_z: float = -sys.float_info.max,
+                                occupancy_max_z: float = sys.float_info.max, min_x_size: float = 0.0,
+                                min_y_size: float = 0.0):
+        """The map projected to 2-D (octomap_server's /projected_map): (cells, resolution, (origin_x, origin_y)) with
+        cells a (height, width) int8 copy of -1 / 0 / 100, row y, column x; (0, 0) for an empty map."""
+        p = ProjectedMapParams()
+        lib().d2pc_projected_map_params_default(C.byref(p))
+        p.occupancy_min_z, p.occupancy_max_z = occupancy_min_z, occupancy_max_z
+        p.min_x_size, p.min_y_size = min_x_size, min_y_size
+        g = GridMap()
+        self._check(lib().d2pc_occupancy_projected_map(self._h, C.byref(p), C.byref(g)), "d2pc_occupancy_projected_map")
+        n = g.width * g.height
+        cells = (np.ctypeslib.as_array(g.data, (n,)).copy() if n else np.zeros(0, np.int8)).reshape(g.height, g.width)
+        return cells, float(g.resolution), (float(g.origin_x), float(g.origin_y))
 
     def occupancy_insert_device(self, d_in, n_frames, n_max, in_stride, d_in_counts, origins):
         """d2pc_occupancy_insert_device: clouds on the device into the map, frame f from origins[f] (host, (n, 3))."""

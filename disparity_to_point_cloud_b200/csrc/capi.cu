@@ -162,6 +162,7 @@ struct d2pc_ctx {
   uint32_t map_epoch = 0;     // of the last frame inserted (marks are tagged with it)
   DevBuf map_tmp, map_out, map_n;  // export scratch, output staging and counters
   PinBuf octomap;                  // d2pc_occupancy_octomap's data, valid until the next call
+  PinBuf projmap;                  // d2pc_occupancy_projected_map's cells, valid until the next call
   cudaStream_t s_map = nullptr;    // every map step and export, in submission order
   cudaEvent_t ev_map_in = nullptr; // orders d2pc_occupancy_insert_device behind the compute stream
   // fusion buffers
@@ -1123,7 +1124,7 @@ void d2pc_destroy(d2pc_ctx *ctx) {
   free_dev(ctx->d_color_in), free_dev(ctx->d_color_out), free_dev(ctx->d_color_lut), free_pin(ctx->h_color);
   free_pin(ctx->h_stage);
   free_dev(ctx->map_mem), free_dev(ctx->map_tmp), free_dev(ctx->map_out), free_dev(ctx->map_n);
-  free_pin(ctx->octomap);
+  free_pin(ctx->octomap), free_pin(ctx->projmap);
   if (ctx->ev_map_in) cudaEventDestroy(ctx->ev_map_in);
   if (ctx->s_map) cudaStreamDestroy(ctx->s_map);
   if (ctx->d_ticket) cudaFree(ctx->d_ticket);
@@ -1422,6 +1423,54 @@ int d2pc_occupancy_octomap(d2pc_ctx *ctx, int binary, d2pc_octomap *out) {
   out->size = bytes;
   out->resolution = ctx->occ.resolution;
   out->binary = binary;
+  return D2PC_OK;
+}
+
+void d2pc_projected_map_params_default(d2pc_projected_map_params *p) {
+  if (!p) return;
+  memset(p, 0, sizeof(*p));
+  p->struct_size = sizeof(*p);
+  p->occupancy_min_z = -DBL_MAX, p->occupancy_max_z = DBL_MAX;
+}
+
+int d2pc_occupancy_projected_map(d2pc_ctx *ctx, const d2pc_projected_map_params *p, d2pc_grid_map *out) {
+  if (!ctx || !p || !out || p->struct_size != sizeof(*p)) return D2PC_ERR_INVALID_ARG;
+  if (std::isnan(p->occupancy_min_z) || std::isnan(p->occupancy_max_z)) return D2PC_ERR_INVALID_ARG;
+  for (double v : {p->min_x_size, p->min_y_size})
+    if (!(std::isfinite(v) && v >= 0.0)) return D2PC_ERR_INVALID_ARG;
+  CU(ctx, cudaSetDevice(ctx->device));
+  uint32_t n = 0;
+  int rc = map_export_count(ctx, false, &n);
+  if (rc) return rc;
+  const double res = ctx->occ.resolution;
+  ProjGrid g{};
+  size_t bytes = 0;
+  if (n) {
+    if ((rc = grow_dev(ctx, ctx->map_tmp, octomap_temp_bytes(n))) || (rc = grow_dev(ctx, ctx->map_n, 64))) return rc;
+    unsigned long long ext[6];
+    CU(ctx, projmap_extent(ctx->map, n, res, ctx->map_tmp.p, reinterpret_cast<uint32_t *>(ctx->map_n.p) + 1,
+                           reinterpret_cast<unsigned long long *>(ctx->map_n.p + 16), ext, ctx->s_map));
+    CU(ctx, cudaStreamSynchronize(ctx->s_map));  // the tree's extent sizes the grid
+    if (!projmap_grid(ext, res, p->min_x_size, p->min_y_size, &g)) return D2PC_ERR_BAD_DIMS;
+    bytes = (size_t)g.width * g.height;
+    if ((rc = grow_dev(ctx, ctx->map_out, projmap_cells_bytes(g)))) return rc;
+    if (bytes > ctx->projmap.cap) {
+      // a new buffer before the old one goes, so a failed allocation leaves the last result as it was
+      void *q = nullptr;
+      const size_t cap = round_up(bytes, 1 << 16);
+      CU(ctx, pinned_alloc(&q, cap));
+      free_pin(ctx->projmap);
+      ctx->projmap.p = static_cast<uint8_t *>(q), ctx->projmap.cap = cap;
+    }
+    CU(ctx, projmap_fill(ctx->map, n, res, p->occupancy_min_z, p->occupancy_max_z,
+                         log_odds(ctx->occ.occupancy_thres), ctx->map_tmp.p, g, ctx->map_out.p, ctx->s_map));
+    CU(ctx, cudaMemcpyAsync(ctx->projmap.p, ctx->map_out.p, bytes, cudaMemcpyDeviceToHost, ctx->s_map));
+    CU(ctx, cudaStreamSynchronize(ctx->s_map));
+  }
+  out->data = bytes ? reinterpret_cast<const int8_t *>(ctx->projmap.p) : nullptr;
+  out->width = g.width, out->height = g.height;
+  out->resolution = (float)res;
+  out->origin_x = g.origin[0], out->origin_y = g.origin[1];
   return D2PC_OK;
 }
 

@@ -9,6 +9,7 @@
  *   d2pc_map_key(rf, c, &k)   k = (int)floor(rf * (double)c) + 32768, valid only when 0 <= k < 65536
  *                             (OcTreeBaseImpl::coordToKeyChecked, rf = 1.0 / resolution in double).
  *   d2pc_map_centre(k, res)   ((double)(k - 32768) + 0.5) * res (keyToCoord at full depth).
+ *   d2pc_map_node_size / d2pc_map_node_centre   getNodeSize(depth) and keyToCoord(k, depth) of a coarser node.
  *   d2pc_map_norm(x, y, z)    sqrt((double)((x*x + y*y) + z*z)): float products and sums, no FMA, a double sqrt
  *                             (octomath Vector3::norm).
  *   d2pc_map_ray_begin/next   OcTreeBaseImpl::computeRayKeys step by step: begin yields the origin's key, each next
@@ -69,6 +70,20 @@ D2PC_MM_FN int d2pc_map_key3(double rf, float x, float y, float z, uint16_t k[3]
 
 D2PC_MM_FN double d2pc_map_centre(uint16_t k, double res) {
   return D2PC_MM_DMUL(D2PC_MM_DADD((double)((int)k - 32768), 0.5), res);
+}
+
+/* OcTreeBaseImpl::getNodeSize(depth): res * (double)(1 << (16 - depth)), depth 0 (the root) .. 16 (a voxel) */
+D2PC_MM_FN double d2pc_map_node_size(uint32_t depth, double res) {
+  return D2PC_MM_DMUL(res, (double)(1u << (16u - depth)));
+}
+
+/* OcTreeBaseImpl::keyToCoord(k, depth): the centre of the depth-`depth` node that holds key k (any key inside the
+ * node gives the same floor).  0 at the root, d2pc_map_centre at full depth. */
+D2PC_MM_FN double d2pc_map_node_centre(uint16_t k, uint32_t depth, double res) {
+  if (depth == 0) return 0.0;
+  if (depth == 16) return d2pc_map_centre(k, res);
+  const double q = floor(D2PC_MM_DDIV(D2PC_MM_DSUB((double)k, 32768.0), (double)(1u << (16u - depth))));
+  return D2PC_MM_DMUL(D2PC_MM_DADD(q, 0.5), d2pc_map_node_size(depth, res));
 }
 
 D2PC_MM_FN double d2pc_map_norm(float x, float y, float z) {

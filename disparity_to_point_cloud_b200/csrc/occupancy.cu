@@ -15,7 +15,10 @@
 //          abort and clamp; nothing at all when the overflow flag is set, so a dropped frame leaves the known map as
 //          it was.
 //   finish one thread: counts the frame as applied or dropped and clears the flag and the touched count.
-// The export sorts the known voxels by Morton code (map_sort); the octomap serialization below builds the tree on it.
+// The export sorts the known voxels by Morton code (map_sort); the octomap serialization below builds the tree on it,
+// and the projected 2-D map after it reads each voxel's leaf level from the same front.
+#include <cstring>
+
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -507,6 +510,29 @@ OctoTemp octo_temp(void *temp, uint32_t n) {
   return o;
 }
 
+// map_sort's output inside temp
+void sorted_of(const void *temp, uint32_t n, const unsigned long long **m, const uint32_t **v) {
+  const uint8_t *p = static_cast<const uint8_t *>(temp);
+  *m = reinterpret_cast<const unsigned long long *>(p + align_up((size_t)n * 8));
+  *v = reinterpret_cast<const uint32_t *>(p + 2 * align_up((size_t)n * 8) + align_up((size_t)n * 4));
+}
+
+// The front the octomap export and the projected map share: the voxels sorted (map_sort), then each voxel's first
+// and leaf level in o.sl and the record count of `binary` in o.cnt (octo_flags, the inclusive scan, octo_levels).
+cudaError_t octo_front(const MapTable &t, uint32_t n, bool binary, void *temp, uint32_t *d_pos, OctoTemp o,
+                       cudaStream_t stream) {
+  const unsigned long long *m;
+  const uint32_t *v;
+  cudaError_t e = map_sort(t, false, 0.0f, n, temp, d_pos, &m, &v, stream);
+  if (e != cudaSuccess) return e;
+  const uint32_t grid = (n + kOctoThreads - 1) / kOctoThreads, grid1 = n / kOctoThreads + 1;
+  octo_flags_kernel<<<grid, kOctoThreads, 0, stream>>>(m, v, n, o.d, o.sl);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  if ((e = cub::DeviceScan::InclusiveSum(o.scan, o.scan_bytes, o.d, o.D, (int)n, stream)) != cudaSuccess) return e;
+  octo_levels_kernel<<<grid1, kOctoThreads, 0, stream>>>(m, o.D, n, binary, o.sl, o.cnt);
+  return cudaGetLastError();
+}
+
 }  // namespace
 
 size_t octomap_temp_bytes(uint32_t n) {
@@ -516,17 +542,9 @@ size_t octomap_temp_bytes(uint32_t n) {
 
 cudaError_t octomap_plan(const MapTable &t, uint32_t n, bool binary, void *temp, uint32_t *d_pos,
                          unsigned long long *records, cudaStream_t stream) {
-  const unsigned long long *m;
-  const uint32_t *v;
   OctoTemp o = octo_temp(temp, n);
-  cudaError_t e = map_sort(t, false, 0.0f, n, temp, d_pos, &m, &v, stream);
+  cudaError_t e = octo_front(t, n, binary, temp, d_pos, o, stream);
   if (e != cudaSuccess) return e;
-  const uint32_t grid = (n + kOctoThreads - 1) / kOctoThreads, grid1 = n / kOctoThreads + 1;
-  octo_flags_kernel<<<grid, kOctoThreads, 0, stream>>>(m, v, n, o.d, o.sl);
-  if ((e = cudaGetLastError()) != cudaSuccess) return e;
-  if ((e = cub::DeviceScan::InclusiveSum(o.scan, o.scan_bytes, o.d, o.D, (int)n, stream)) != cudaSuccess) return e;
-  octo_levels_kernel<<<grid1, kOctoThreads, 0, stream>>>(m, o.D, n, binary, o.sl, o.cnt);
-  if ((e = cudaGetLastError()) != cudaSuccess) return e;
   if ((e = cub::DeviceScan::ExclusiveSum(o.scan, o.scan_bytes, o.cnt, o.off, (int)n + 1, stream)) != cudaSuccess)
     return e;
   return cudaMemcpyAsync(records, o.off + n, 8, cudaMemcpyDeviceToHost, stream);
@@ -539,10 +557,9 @@ size_t octomap_out_bytes(unsigned long long records, bool binary) {
 cudaError_t octomap_emit(const MapTable &t, uint32_t n, bool binary, float occ_thres, void *temp,
                          unsigned long long records, uint8_t *out, cudaStream_t stream) {
   const OctoTemp o = octo_temp(temp, n);
-  const unsigned long long *m = reinterpret_cast<const unsigned long long *>(static_cast<uint8_t *>(temp) +
-                                                                             align_up((size_t)n * 8));
-  const uint32_t *v = reinterpret_cast<const uint32_t *>(static_cast<uint8_t *>(temp) + 2 * align_up((size_t)n * 8) +
-                                                         align_up((size_t)n * 4));
+  const unsigned long long *m;
+  const uint32_t *v;
+  sorted_of(temp, n, &m, &v);
   const size_t bytes = binary ? records * 2 : records * 5;
   uint32_t *vmax = binary ? nullptr : reinterpret_cast<uint32_t *>(out + align_up(bytes + 4));
   cudaError_t e = cudaMemsetAsync(out, 0, bytes, stream);
@@ -555,6 +572,163 @@ cudaError_t octomap_emit(const MapTable &t, uint32_t n, bool binary, float occ_t
       octo_max_kernel<<<grid, kOctoThreads, 0, stream>>>(v, o.sl, o.off, o.up, n, L, vmax);
     octo_emit_kernel<<<grid, kOctoThreads, 0, stream>>>(v, o.sl, o.off, vmax, n, out);
   }
+  return cudaGetLastError();
+}
+
+// ---- octomap_server's projected 2-D map, nav_msgs/OccupancyGrid (the recipe is in include/d2pc_b200.h)
+//
+// On the voxels octo_front sorted and levelled, one thread per voxel with its leaf level lambda_i.  Every voxel of a
+// leaf has the leaf's level and value, and the leaf's voxels fill it, so what each voxel does with its leaf's extent,
+// height test and value over its own column is, over all of them, what octomap does with the leaf.
+//   proj_extent  the leaf's lo and hi per axis, reduced over the warp and the block, then one atomicMin per block
+//                into 6 words: ordered encodings of the minima, complemented ones of the maxima (so one 0xff memset
+//                starts all six).  The host reads them (the call's one extra wait) and sizes the grid
+//   proj_fill    a leaf that passes the height test ORs 1 (free) or 2 (occupied) into its voxel's cell byte; the
+//                byte is read first, as most voxels share their column with others
+//   proj_emit    the codes into OccupancyGrid values: 2 or 3 -> 100, 1 -> 0, 0 -> -1
+namespace {
+
+constexpr int kProjThreads = 256;
+
+__device__ __forceinline__ unsigned long long ordered64(double d) {
+  const unsigned long long b = (unsigned long long)__double_as_longlong(d);
+  return (b >> 63) ? ~b : b | 0x8000000000000000ull;
+}
+double unordered64(unsigned long long o) {
+  const unsigned long long b = (o >> 63) ? o & 0x7fffffffffffffffull : ~o;
+  double d;
+  memcpy(&d, &b, 8);
+  return d;
+}
+__device__ __forceinline__ unsigned long long umin64(unsigned long long a, unsigned long long b) { return b < a ? b : a; }
+
+__global__ void __launch_bounds__(kProjThreads) proj_extent_kernel(const unsigned long long *__restrict__ m,
+                                                                   const uint16_t *__restrict__ sl, uint32_t n,
+                                                                   double res, unsigned long long *ext) {
+  const uint32_t i = blockIdx.x * kProjThreads + threadIdx.x;
+  unsigned long long e[6];
+  for (int a = 0; a < 6; ++a) e[a] = ~0ull;
+  if (i < n) {
+    uint16_t k[3];
+    demorton(m[i], k);
+    const uint32_t lam = leaf_of(sl[i]);
+    // calcMinMax: lo = c - size / 2, hi = lo + size
+    const double size = d2pc_map_node_size(lam, res), half = __ddiv_rn(size, 2.0);
+    for (int a = 0; a < 3; ++a) {
+      const double lo = __dsub_rn(d2pc_map_node_centre(k[a], lam, res), half);
+      e[a] = ordered64(lo);
+      e[3 + a] = ~ordered64(__dadd_rn(lo, size));
+    }
+  }
+  __shared__ unsigned long long part[6][kProjThreads / 32];
+  const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  for (int a = 0; a < 6; ++a) {
+    for (int s = 16; s > 0; s >>= 1) e[a] = umin64(e[a], __shfl_xor_sync(0xffffffffu, e[a], s));
+    if (lane == 0) part[a][warp] = e[a];
+  }
+  __syncthreads();
+  if (threadIdx.x < 6) {
+    unsigned long long r = part[threadIdx.x][0];
+    for (int w = 1; w < kProjThreads / 32; ++w) r = umin64(r, part[threadIdx.x][w]);
+    if (r != ~0ull) atomicMin(ext + threadIdx.x, r);
+  }
+}
+
+__global__ void __launch_bounds__(kProjThreads) proj_fill_kernel(const unsigned long long *__restrict__ m,
+                                                                 const uint32_t *__restrict__ v,
+                                                                 const uint16_t *__restrict__ sl, uint32_t n,
+                                                                 double res, double min_z, double max_z,
+                                                                 float occ_thres, const ProjGrid g, uint8_t *cells) {
+  const uint32_t i = blockIdx.x * kProjThreads + threadIdx.x;
+  if (i >= n) return;
+  uint16_t k[3];
+  demorton(m[i], k);
+  const uint32_t lam = leaf_of(sl[i]);
+  const double half = __ddiv_rn(d2pc_map_node_size(lam, res), 2.0), cz = d2pc_map_node_centre(k[2], lam, res);
+  if (!(__dadd_rn(cz, half) > min_z && __dsub_rn(cz, half) < max_z)) return;
+  const uint32_t code = __uint_as_float(v[i]) >= occ_thres ? 2u : 1u;
+  // the padded min key is at most the least key of the map on each axis and the padded max at least the largest
+  // (both come within one key of a leaf's face), so the cell is inside the grid
+  const unsigned long long at =
+      (unsigned long long)(k[1] - g.min_key[1]) * g.width + (unsigned long long)(k[0] - g.min_key[0]);
+  if (!(cells[at] & code)) or_byte(cells, at, code);
+}
+
+__global__ void __launch_bounds__(kProjThreads) proj_emit_kernel(uint4 *cells, unsigned long long vecs) {
+  for (unsigned long long j = (unsigned long long)blockIdx.x * kProjThreads + threadIdx.x; j < vecs;
+       j += (unsigned long long)gridDim.x * kProjThreads) {
+    uint4 c = cells[j];
+    uint32_t *w = &c.x;
+    for (int q = 0; q < 4; ++q) {
+      uint32_t out = 0;
+      for (int b = 0; b < 4; ++b) {
+        const uint32_t code = (w[q] >> (8 * b)) & 3u;
+        out |= (code & 2u ? 100u : code ? 0u : 0xffu) << (8 * b);
+      }
+      w[q] = out;
+    }
+    cells[j] = c;
+  }
+}
+
+}  // namespace
+
+cudaError_t projmap_extent(const MapTable &t, uint32_t n, double res, void *temp, uint32_t *d_pos,
+                           unsigned long long *d_ext, unsigned long long *h_ext, cudaStream_t stream) {
+  const OctoTemp o = octo_temp(temp, n);
+  // the front also writes the binary format's record counts into o.cnt; the projection needs only the leaf levels
+  cudaError_t e = octo_front(t, n, true, temp, d_pos, o, stream);
+  if (e != cudaSuccess) return e;
+  if ((e = cudaMemsetAsync(d_ext, 0xff, 6 * 8, stream)) != cudaSuccess) return e;
+  const unsigned long long *m;
+  const uint32_t *v;
+  sorted_of(temp, n, &m, &v);
+  proj_extent_kernel<<<(n + kProjThreads - 1) / kProjThreads, kProjThreads, 0, stream>>>(m, o.sl, n, res, d_ext);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  return cudaMemcpyAsync(h_ext, d_ext, 6 * 8, cudaMemcpyDeviceToHost, stream);
+}
+
+bool projmap_grid(const unsigned long long ext[6], double res, double min_x_size, double min_y_size, ProjGrid *g) {
+  double mn[3], mx[3];
+  for (int a = 0; a < 3; ++a) mn[a] = unordered64(ext[a]), mx[a] = unordered64(~ext[3 + a]);
+  // the padding: std::min(a, b) is (b < a) ? b : a, std::max(a, b) is (a < b) ? b : a
+  const double half[2] = {0.5 * min_x_size, 0.5 * min_y_size};
+  for (int a = 0; a < 2; ++a) {
+    if (-half[a] < mn[a]) mn[a] = -half[a];
+    if (mx[a] < half[a]) mx[a] = half[a];
+  }
+  // float point3d corners, coordToKeyChecked on all three axes
+  const double rf = 1.0 / res;
+  uint16_t lo[3], hi[3];
+  if (!d2pc_map_key3(rf, (float)mn[0], (float)mn[1], (float)mn[2], lo) ||
+      !d2pc_map_key3(rf, (float)mx[0], (float)mx[1], (float)mx[2], hi))
+    return false;
+  for (int a = 0; a < 2; ++a) {
+    g->min_key[a] = lo[a];
+    g->origin[a] = (double)(float)d2pc_map_centre(lo[a], res) - res * 0.5;
+  }
+  g->width = (uint32_t)(hi[0] - lo[0]) + 1u;
+  g->height = (uint32_t)(hi[1] - lo[1]) + 1u;
+  return true;
+}
+
+size_t projmap_cells_bytes(const ProjGrid &g) { return ((size_t)g.width * g.height + 15) & ~(size_t)15; }
+
+cudaError_t projmap_fill(const MapTable &t, uint32_t n, double res, double min_z, double max_z, float occ_thres,
+                         void *temp, const ProjGrid &g, uint8_t *cells, cudaStream_t stream) {
+  const size_t bytes = projmap_cells_bytes(g);
+  cudaError_t e = cudaMemsetAsync(cells, 0, bytes, stream);
+  if (e != cudaSuccess) return e;
+  const OctoTemp o = octo_temp(temp, n);
+  const unsigned long long *m;
+  const uint32_t *v;
+  sorted_of(temp, n, &m, &v);
+  proj_fill_kernel<<<(n + kProjThreads - 1) / kProjThreads, kProjThreads, 0, stream>>>(m, v, o.sl, n, res, min_z,
+                                                                                        max_z, occ_thres, g, cells);
+  if ((e = cudaGetLastError()) != cudaSuccess) return e;
+  const unsigned long long vecs = bytes / 16, want = (vecs + kProjThreads - 1) / kProjThreads;
+  const uint32_t grid = (uint32_t)(want < 65536 ? want : 65536);
+  proj_emit_kernel<<<grid, kProjThreads, 0, stream>>>(reinterpret_cast<uint4 *>(cells), vecs);
   return cudaGetLastError();
 }
 

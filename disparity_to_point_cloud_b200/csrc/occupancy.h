@@ -70,4 +70,21 @@ size_t octomap_out_bytes(unsigned long long records, bool binary);
 cudaError_t octomap_emit(const MapTable &t, uint32_t n, bool binary, float occ_thres, void *temp,
                          unsigned long long records, uint8_t *out, cudaStream_t stream);
 
+// octomap_server's projected 2-D map of the n known voxels (> 0), on one temp of octomap_temp_bytes(n), in three
+// steps.  projmap_extent (asynchronous on `stream`): sorts and levels the voxels as octomap_plan does and reads the
+// tree's extent into the host's h_ext[6] through d_ext[6].  projmap_grid (host, once h_ext is there): the padded grid,
+// false when a padded corner has no key.  projmap_fill (asynchronous): the grid's int8 cells into `cells`, which
+// holds projmap_cells_bytes(g).
+struct ProjGrid {
+  uint16_t min_key[2];  // the padded min key on x and y: cell (0, 0)
+  uint32_t width, height;
+  double origin[2];     // OccupancyGrid's info.origin.position x and y
+};
+cudaError_t projmap_extent(const MapTable &t, uint32_t n, double res, void *temp, uint32_t *d_pos,
+                           unsigned long long *d_ext, unsigned long long *h_ext, cudaStream_t stream);
+bool projmap_grid(const unsigned long long ext[6], double res, double min_x_size, double min_y_size, ProjGrid *g);
+size_t projmap_cells_bytes(const ProjGrid &g);
+cudaError_t projmap_fill(const MapTable &t, uint32_t n, double res, double min_z, double max_z, float occ_thres,
+                         void *temp, const ProjGrid &g, uint8_t *cells, cudaStream_t stream);
+
 }  // namespace d2pc

@@ -588,6 +588,69 @@ typedef struct d2pc_octomap {
  * leaving the map and the previous result as they were. */
 int d2pc_occupancy_octomap(d2pc_ctx *ctx, int binary, d2pc_octomap *out);
 
+/* ---- the map projected to 2-D as nav_msgs/OccupancyGrid (octomap_server's /projected_map) -----------------------------
+ *
+ * Reference: OctomapServer::publishAll -> handlePreNodeTraversal, then per leaf handleOccupiedNode / handleFreeNode ->
+ * update2DMap, restated from memory like the recipes above, for max_depth 16 (the default), incremental_2D_projection
+ * false (the complete map is projected every time), filter_speckles and filter_ground off.  The leaves are the pruned
+ * tree's (d2pc_occupancy_octomap's recipe, item 2): a leaf at depth d has a key k per axis (any key inside it).
+ *   1. empty map: publishAll returns early when octree.size() <= 1, so no known voxel gives no grid.
+ *   2. extent (OcTreeBaseImpl::calcMinMax over the leaves, in double): size = getNodeSize(d) = res * (double)(1 << (16
+ *      - d)); c = keyToCoord(k, d), which is ((double)(k - 32768) + 0.5) * res at d = 16 and otherwise
+ *      (floor(((double)k - 32768.0) / (double)(1 << (16 - d))) + 0.5) * size (0 at d = 0); lo = c - size / 2.0 and hi =
+ *      lo + size (two roundings, not c + size / 2).  min = the least lo, max = the greatest hi, per axis.
+ *   3. padding: minX = std::min(minX, -0.5 * min_x_size), maxX = std::max(maxX, 0.5 * min_x_size), the same on y with
+ *      min_y_size (so with the default 0 the grid always holds key 32768, the world origin, on x and y; -0.0 and 0.0
+ *      give the same key).  The corners become float point3d (z the unpadded min / max) and coordToKeyChecked runs on
+ *      all three axes; when either corner has no valid key octomap_server logs an error and this library returns
+ *      D2PC_ERR_BAD_DIMS (a voxel at key 65535 can put the max face out of range).
+ *   4. grid: width = paddedMax.x - paddedMin.x + 1, height likewise on y; resolution = (float)res; origin.position.x =
+ *      (double)(float)keyToCoord(paddedMin.x) - res * 0.5, likewise y; z 0, the orientation left at the message's
+ *      default; map_load_time 0.
+ *   5. cells, row-major, index (kx - paddedMin.x) + (ky - paddedMin.y) * width, all -1 first.  A leaf passes when c_z
+ *      + h > occupancy_min_z && c_z - h < occupancy_max_z (its double centre and h = size / 2.0, strict); it then
+ *      covers its 2^(16-d) x 2^(16-d) square of cells: an occupied leaf (log_odds >= the current occupancy_thres) sets
+ *      100, a free one sets 0 where the cell is still -1.  So a cell is 100 when a passing occupied leaf covers it,
+ *      else 0 when a passing free leaf covers it, else -1, in any leaf order.
+ * Per voxel: every known voxel inside a leaf has the leaf's depth and value, and the leaf is complete (all its voxels
+ * are known), so the union of its voxels' columns is the leaf's square.  Items 2 and 5 are therefore each voxel doing
+ * its own leaf's extent, height test and value over its own column.  A full-depth voxel's own centre and size would
+ * not do: they differ from the leaf's in the height test at finite z limits and in the last bit of the extent, which
+ * can move a padded key by one.  tests/test_oracle_projected_map.py checks the per-voxel recipe against a pointer tree.
+ * What rests on recollection and is not verified against the sources: the early return on size() <= 1; calcMinMax's
+ * lo-then-add-size arithmetic; keyToCoord(k, d)'s floor form and its 0 at the root; the padding with std::min /
+ * std::max and the float point3d corners; coordToKeyChecked on z too; the origin's float round trip; the height test
+ * on the leaf's extent (some older octomap_server releases test the centre alone); occupied overriding free; that the
+ * orientation is all four components 0; the param names occupancy_min_z / occupancy_max_z (default -DBL_MAX /
+ * DBL_MAX) and min_x_size / min_y_size (default 0).
+ * On the device: the known voxels are sorted and each one's leaf level found as for d2pc_occupancy_octomap; one thread
+ * per voxel reduces the extent (the host reads six values back and sizes the grid), then ORs a free or occupied code
+ * into its cell, and the codes become the cell values (csrc/occupancy.cu).  The library does this work only when this
+ * call is made. */
+typedef struct d2pc_projected_map_params {
+  uint32_t struct_size;   /* sizeof(d2pc_projected_map_params) */
+  double occupancy_min_z; /* -DBL_MAX (m): a leaf must reach above it; not NaN (+-inf allowed) */
+  double occupancy_max_z; /* DBL_MAX (m): a leaf must reach below it; not NaN (+-inf allowed) */
+  double min_x_size;      /* 0 (m): the grid spans at least [-min_x_size / 2, min_x_size / 2]; finite, >= 0 */
+  double min_y_size;      /* 0 (m): likewise on y */
+} d2pc_projected_map_params;
+
+typedef struct d2pc_grid_map {
+  const int8_t *data; /* width * height cells, row-major (row y, column x), each -1, 0 or 100: page-locked memory the
+                         library owns, valid until the next call on the context or d2pc_destroy; NULL when empty */
+  uint32_t width, height;      /* cells; 0 for an empty map.  width * height can reach 2^32 */
+  float resolution;            /* info.resolution (m), the map's resolution as float */
+  double origin_x, origin_y;   /* info.origin.position x and y (m) of cell (0, 0)'s corner */
+} d2pc_grid_map;
+
+/* octomap_server's defaults above. */
+void d2pc_projected_map_params_default(d2pc_projected_map_params *p);
+/* The map projected to 2-D (recipe above).  Synchronous; reflects every frame submitted before the call.  An empty map
+ * gives width = height = 0, data NULL and D2PC_OK.  D2PC_ERR_INVALID_ARG for a NaN z limit, a min size that is
+ * negative or not finite, or a wrong struct_size; D2PC_ERR_BAD_DIMS when a padded corner has no key (item 3);
+ * D2PC_ERR_NOMEM when a host or device allocation fails.  The previous result is left as it was on every error. */
+int d2pc_occupancy_projected_map(d2pc_ctx *ctx, const d2pc_projected_map_params *p, d2pc_grid_map *out);
+
 /* ---- the disparity callback, host buffers (the reference-facing calls) ------ */
 
 /* Whole DisparityCb (src/disparity_to_point_cloud.cpp:46-92) on one mono8

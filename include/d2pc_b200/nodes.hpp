@@ -44,6 +44,7 @@ class Bus {
   using CloudCb = std::function<void(const sensor_msgs::PointCloud2 &)>;
   using ScanCb = std::function<void(const sensor_msgs::LaserScan &)>;
   using OctomapCb = std::function<void(const ros_lite::octomap_msgs::Octomap &)>;
+  using GridCb = std::function<void(const ros_lite::nav_msgs::OccupancyGrid &)>;
 
   // <remap from="/disparity" to="/throttled_depth_map"/>
   void remap(const std::string &from, const std::string &to) { remaps_[from] = to; }
@@ -86,6 +87,9 @@ class Bus {
   void subscribe_octomap(const std::string &topic, uint32_t queue_size, OctomapCb cb) {
     octomap_subs_[resolve(topic)].push_back({queue_size, std::move(cb)});
   }
+  void subscribe_grid(const std::string &topic, uint32_t queue_size, GridCb cb) {
+    grid_subs_[resolve(topic)].push_back({queue_size, std::move(cb)});
+  }
   struct Advertised {
     std::string topic;
     uint32_t queue_size;
@@ -118,11 +122,18 @@ class Bus {
     if (it != octomap_subs_.end())
       for (auto &s : it->second) s.cb(msg);
   }
+  void publish(const std::string &resolved_topic, const ros_lite::nav_msgs::OccupancyGrid &msg) {
+    auto it = grid_subs_.find(resolved_topic);
+    if (it != grid_subs_.end())
+      for (auto &s : it->second) s.cb(msg);
+  }
   const std::vector<Advertised> &advertised() const { return advertised_; }
   bool has_subscribers(const std::string &resolved_topic) const {  // ros::Publisher::getNumSubscribers() > 0
     auto it = image_subs_.find(resolved_topic);
     auto ot = octomap_subs_.find(resolved_topic);
-    return (it != image_subs_.end() && !it->second.empty()) || (ot != octomap_subs_.end() && !ot->second.empty());
+    auto gt = grid_subs_.find(resolved_topic);
+    return (it != image_subs_.end() && !it->second.empty()) || (ot != octomap_subs_.end() && !ot->second.empty()) ||
+           (gt != grid_subs_.end() && !gt->second.empty());
   }
 
   // Reads <remap from= to=/> and <param name= value=/> out of a roslaunch file (launch/*.launch).  A value that
@@ -175,6 +186,7 @@ class Bus {
   std::map<std::string, std::vector<Sub<CloudCb>>> cloud_subs_;
   std::map<std::string, std::vector<Sub<ScanCb>>> scan_subs_;
   std::map<std::string, std::vector<Sub<OctomapCb>>> octomap_subs_;
+  std::map<std::string, std::vector<Sub<GridCb>>> grid_subs_;
   std::map<std::string, sensor_msgs::PointCloud2> latched_clouds_;
   std::vector<Advertised> advertised_;
 };
@@ -248,6 +260,9 @@ class Disparity2PCloud {
   sensor_msgs::PointCloud2 centres_;
   std::string p_octomap_topic_[2];  // "/octomap_full", "/octomap_binary" when map_enable != 0
   ros_lite::octomap_msgs::Octomap octomap_;
+  std::string p_grid_topic_;  // "/projected_map" when map_enable != 0
+  d2pc_projected_map_params grid_params_;
+  ros_lite::nav_msgs::OccupancyGrid grid_;
 
   // make output_.data hold `bytes` bytes in page-locked storage without touching bytes it already has
   void reserve_output(size_t bytes) {
@@ -379,7 +394,10 @@ class Disparity2PCloud {
     // its defaults; map_max_bricks sizes the device map; map_keep_cloud 0 leaves the cloud on the device and
     // /point_cloud unpublished.  The sensor origin is the transform's translation: set the transform params.
     // The map also goes out as octomap_msgs/Octomap on /octomap_full and /octomap_binary (octomap_server with
-    // latch false), each serialized only while somebody subscribes to it.
+    // latch false), each serialized only while somebody subscribes to it, and projected to 2-D as
+    // nav_msgs/OccupancyGrid on /projected_map (latch false), built only while somebody subscribes to it;
+    // map_occupancy_min_z, map_occupancy_max_z, map_min_x_size and map_min_y_size are octomap_server's occupancy_min_z,
+    // occupancy_max_z, min_x_size and min_y_size with its defaults.
     int map_on = 0;
     nh_.param<int>("map_enable", map_on, 0);
     if (map_on) {
@@ -402,6 +420,12 @@ class Disparity2PCloud {
       p_map_topic_ = nh_.advertise("/octomap_point_cloud_centers", 1);
       p_octomap_topic_[0] = nh_.advertise("/octomap_full", 1);
       p_octomap_topic_[1] = nh_.advertise("/octomap_binary", 1);
+      d2pc_projected_map_params_default(&grid_params_);
+      nh_.param<double>("map_occupancy_min_z", grid_params_.occupancy_min_z, grid_params_.occupancy_min_z);
+      nh_.param<double>("map_occupancy_max_z", grid_params_.occupancy_max_z, grid_params_.occupancy_max_z);
+      nh_.param<double>("map_min_x_size", grid_params_.min_x_size, grid_params_.min_x_size);
+      nh_.param<double>("map_min_y_size", grid_params_.min_y_size, grid_params_.min_y_size);
+      p_grid_topic_ = nh_.advertise("/projected_map", 1);
     }
   }
   ~Disparity2PCloud() {
@@ -465,6 +489,21 @@ class Disparity2PCloud {
         octomap_.data.resize(m.size);
         if (m.size) std::memcpy(octomap_.data.data(), m.data, m.size);
         nh_.publish(p_octomap_topic_[binary], octomap_);
+      }
+      if (nh_.has_subscribers(p_grid_topic_)) {
+        // nothing while the map is empty (publishAll's early return), nor when a padded corner has no key (octomap_server
+        // logs an error and publishes no valid grid)
+        d2pc_grid_map g;
+        const int rc = d2pc_occupancy_projected_map(ctx_, &grid_params_, &g);
+        if (rc != D2PC_ERR_BAD_DIMS) d2pc_b200::check(rc, "d2pc_occupancy_projected_map", ctx_);
+        if (rc == D2PC_OK && g.width) {
+          grid_.header = output.header;
+          grid_.info.resolution = g.resolution;
+          grid_.info.width = g.width, grid_.info.height = g.height;
+          grid_.info.origin.position.x = g.origin_x, grid_.info.origin.position.y = g.origin_y;
+          grid_.data.assign(g.data, g.data + static_cast<size_t>(g.width) * g.height);
+          nh_.publish(p_grid_topic_, grid_);
+        }
       }
     }
   }

@@ -3,7 +3,8 @@
 // Field order and types follow the message definitions the reference uses:
 //   std_msgs/Header, sensor_msgs/Image, sensor_msgs/PointField, sensor_msgs/PointCloud2, and sensor_msgs/LaserScan
 //   (pointcloud_to_laserscan's output, which the point cloud node can publish next to its cloud), and
-//   octomap_msgs/Octomap (octomap_server's /octomap_full and /octomap_binary, published next to it with the map on)
+//   octomap_msgs/Octomap (octomap_server's /octomap_full and /octomap_binary, published next to it with the map on),
+//   nav_msgs/OccupancyGrid with nav_msgs/MapMetaData and geometry_msgs/Pose (octomap_server's /projected_map)
 //   (src/disparity_to_point_cloud.cpp:46-92, src/depth_map_fusion.cpp:46-136).
 // With a real ROS1 the ros1_shim/ sources use the genuine sensor_msgs types instead; the layouts are identical.
 #pragma once
@@ -77,6 +78,38 @@ struct Octomap {
 };
 
 }  // namespace octomap_msgs
+
+namespace geometry_msgs {
+
+struct Point {
+  double x = 0, y = 0, z = 0;
+};
+struct Quaternion {
+  double x = 0, y = 0, z = 0, w = 0;
+};
+struct Pose {
+  Point position;
+  Quaternion orientation;
+};
+
+}  // namespace geometry_msgs
+
+namespace nav_msgs {
+
+struct MapMetaData {
+  Time map_load_time;
+  float resolution = 0;
+  uint32_t width = 0, height = 0;
+  geometry_msgs::Pose origin;
+};
+
+struct OccupancyGrid {
+  Header header;
+  MapMetaData info;
+  std::vector<int8_t> data;
+};
+
+}  // namespace nav_msgs
 
 // ---- ROS1 serialisation: little endian, strings and arrays prefixed by a uint32 length --------------------
 class Writer {
@@ -248,6 +281,30 @@ inline std::vector<uint8_t> serialize(const octomap_msgs::Octomap &m) {
   w.header(m.header);
   w.u8(m.binary), w.str(m.id), w.f64(m.resolution), w.int8s(m.data);
   return std::move(w.buf);
+}
+inline std::vector<uint8_t> serialize(const nav_msgs::OccupancyGrid &m) {
+  Writer w;
+  w.header(m.header);
+  const nav_msgs::MapMetaData &i = m.info;
+  w.u32(i.map_load_time.sec), w.u32(i.map_load_time.nsec), w.f32(i.resolution), w.u32(i.width), w.u32(i.height);
+  w.f64(i.origin.position.x), w.f64(i.origin.position.y), w.f64(i.origin.position.z);
+  w.f64(i.origin.orientation.x), w.f64(i.origin.orientation.y), w.f64(i.origin.orientation.z);
+  w.f64(i.origin.orientation.w);
+  w.int8s(m.data);
+  return std::move(w.buf);
+}
+inline nav_msgs::OccupancyGrid deserialize_grid(const uint8_t *p, size_t n) {
+  Reader r(p, n);
+  nav_msgs::OccupancyGrid m;
+  m.header = r.header();
+  nav_msgs::MapMetaData &i = m.info;
+  i.map_load_time.sec = r.u32(), i.map_load_time.nsec = r.u32(), i.resolution = r.f32();
+  i.width = r.u32(), i.height = r.u32();
+  i.origin.position.x = r.f64(), i.origin.position.y = r.f64(), i.origin.position.z = r.f64();
+  i.origin.orientation.x = r.f64(), i.origin.orientation.y = r.f64(), i.origin.orientation.z = r.f64();
+  i.origin.orientation.w = r.f64();
+  m.data = r.int8s();
+  return m;
 }
 inline octomap_msgs::Octomap deserialize_octomap(const uint8_t *p, size_t n) {
   Reader r(p, n);

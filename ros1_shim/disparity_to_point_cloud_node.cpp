@@ -4,6 +4,7 @@
 // Topic names, queue sizes, the (accidentally) latched publisher, parameter names and defaults follow
 // include/disparity_to_point_cloud/disparity_to_point_cloud.hpp:75-106 of the reference, so
 // launch/d2pcloud.launch works unchanged.
+#include <nav_msgs/OccupancyGrid.h>
 #include <octomap_msgs/Octomap.h>
 #include <ros/ros.h>
 #include <sensor_msgs/Image.h>
@@ -169,7 +170,9 @@ class Disparity2PCloudGpu {
     // map_occupancy_thres, map_max_range), map_max_bricks and map_keep_cloud (0: /point_cloud is not published).
     // The sensor origin is the transform's translation: set transform_*.  The map also goes out as
     // octomap_msgs/Octomap on /octomap_full and /octomap_binary (octomap_server with latch false), each serialized
-    // only while somebody subscribes to it.
+    // only while somebody subscribes to it, and projected to 2-D as nav_msgs/OccupancyGrid on /projected_map (latch
+    // false), built only while somebody subscribes to it; map_occupancy_min_z, map_occupancy_max_z, map_min_x_size and
+    // map_min_y_size are octomap_server's occupancy_min_z, occupancy_max_z, min_x_size and min_y_size.
     int map_on = 0;
     nh_.param<int>("map_enable", map_on, 0);
     if (map_on) {
@@ -196,6 +199,12 @@ class Disparity2PCloudGpu {
         map_pub_ = nh_.advertise<sensor_msgs::PointCloud2>("/octomap_point_cloud_centers", 1);
         octomap_pub_[0] = nh_.advertise<octomap_msgs::Octomap>("/octomap_full", 1);
         octomap_pub_[1] = nh_.advertise<octomap_msgs::Octomap>("/octomap_binary", 1);
+        d2pc_projected_map_params_default(&grid_params_);
+        nh_.param<double>("map_occupancy_min_z", grid_params_.occupancy_min_z, grid_params_.occupancy_min_z);
+        nh_.param<double>("map_occupancy_max_z", grid_params_.occupancy_max_z, grid_params_.occupancy_max_z);
+        nh_.param<double>("map_min_x_size", grid_params_.min_x_size, grid_params_.min_x_size);
+        nh_.param<double>("map_min_y_size", grid_params_.min_y_size, grid_params_.min_y_size);
+        grid_pub_ = nh_.advertise<nav_msgs::OccupancyGrid>("/projected_map", 1);
         map_on_ = true;
       }
     }
@@ -278,6 +287,23 @@ class Disparity2PCloudGpu {
       if (m.size) std::memcpy(octomap_.data.data(), m.data, m.size);
       octomap_pub_[binary].publish(octomap_);
     }
+    if (grid_pub_.getNumSubscribers() > 0) {
+      // nothing while the map is empty (publishAll's early return); a padded corner without a key skips the frame
+      d2pc_grid_map g;
+      const int grc = d2pc_occupancy_projected_map(ctx_, &grid_params_, &g);
+      if (grc == D2PC_ERR_BAD_DIMS) {
+        ROS_ERROR("d2pc_occupancy_projected_map: the padded map leaves the key range");
+      } else if (grc != D2PC_OK) {
+        ROS_ERROR("d2pc_occupancy_projected_map: %s (%s)", d2pc_strerror(grc), d2pc_last_cuda_error(ctx_));
+      } else if (g.width) {
+        grid_.header = out.header;
+        grid_.info.resolution = g.resolution;
+        grid_.info.width = g.width, grid_.info.height = g.height;
+        grid_.info.origin.position.x = g.origin_x, grid_.info.origin.position.y = g.origin_y;
+        grid_.data.assign(g.data, g.data + static_cast<size_t>(g.width) * g.height);
+        grid_pub_.publish(grid_);
+      }
+    }
   }
 
   // a PointCloud2's fields from the library's d2pc_cloud; data keeps its storage and shows the cloud's bytes
@@ -304,6 +330,9 @@ class Disparity2PCloudGpu {
   ros::Publisher pub_, scan_pub_, map_pub_;
   ros::Publisher octomap_pub_[2];          // /octomap_full, /octomap_binary
   octomap_msgs::Octomap octomap_;
+  ros::Publisher grid_pub_;  // /projected_map
+  d2pc_projected_map_params grid_params_;
+  nav_msgs::OccupancyGrid grid_;
   bool scan_on_ = false, map_on_ = false;  // scan_enable, map_enable
   bool publish_cloud_ = true;              // scan_keep_cloud and map_keep_cloud
   sensor_msgs::PointCloud2 centres_;       // /octomap_point_cloud_centers

@@ -4,6 +4,8 @@
 //       CPU only: serialises a small hand-made PointCloud2 and Image with ros_lite (self-test of the wire code).
 //   d2pc_offline wire-octomap <out.bin>
 //       CPU only: a small hand-made octomap_msgs/Octomap through ros_lite's serialize / deserialize; its wire bytes.
+//   d2pc_offline wire-grid <out.bin>
+//       CPU only: a small hand-made nav_msgs/OccupancyGrid through ros_lite's serialize / deserialize; its wire bytes.
 //   d2pc_offline params <launch file> <name>...
 //       CPU only: loads the launch file into a Bus and prints one line per name: "<name> number <value>" (%.17g),
 //       "<name> string <value>" or "<name> missing" (the launch-file loader's number / string rule).
@@ -20,6 +22,10 @@
 //       node1map with /octomap_full and /octomap_binary subscribed too: the last message of each (an empty file when
 //       none was published); a path of "-" leaves that topic without a subscriber.  With map_enable 0 in the launch file nothing is subscribed but /point_cloud, and the
 //       harness fails if the node advertised any octomap topic.
+//   d2pc_offline node1projmap <launch file> <w> <h> <cloud.bin> <grid.bin> <count.txt> <in.raw> [<in.raw> ...]
+//       node1 with the map on and /projected_map subscribed: the last PointCloud2 and the last OccupancyGrid (an empty
+//       file when none was published), and the number of grids published.  With map_enable 0 in the launch file
+//       only /point_cloud is subscribed, and the harness fails if the node advertised /projected_map.
 //   d2pc_offline fusion <fusion launch> <w> <h> <d1.raw> <d2.raw> <s1.raw> <s2.raw> <fused.bin> [<cloud.bin> [<debug dir>]]
 //       BASELINE config 5 shape: four mono8 frames into DepthMapFusion; the fused Image is written, and when
 //       <cloud.bin> is given it is also fed to a Disparity2PCloud node whose /disparity is remapped to
@@ -170,6 +176,48 @@ int main(int argc, char **argv) {
       write_file(argv[6], centres);
       if (std::string(argv[7]) != "-") write_file(argv[7], full);
       if (std::string(argv[8]) != "-") write_file(argv[8], binary);
+      return 0;
+    }
+    if (mode == "wire-grid" && argc == 3) {
+      ros_lite::nav_msgs::OccupancyGrid m;
+      m.header.seq = 7, m.header.stamp.sec = 11, m.header.stamp.nsec = 13, m.header.frame_id = "/map";
+      m.info.map_load_time.sec = 17, m.info.map_load_time.nsec = 19;
+      m.info.resolution = 0.05f, m.info.width = 3, m.info.height = 2;
+      m.info.origin.position.x = -1.25, m.info.origin.position.y = 2.5, m.info.origin.position.z = 0.125;
+      m.info.origin.orientation.w = 1.0;
+      m.data = {-1, 0, 100, 100, 0, -1};
+      auto bytes = ros_lite::serialize(m);
+      auto back = ros_lite::deserialize_grid(bytes.data(), bytes.size());
+      if (ros_lite::serialize(back) != bytes || back.info.width != 3 || back.data.size() != 6)
+        throw std::runtime_error("OccupancyGrid round trip differs");
+      write_file(argv[2], bytes);
+      return 0;
+    }
+    if (mode == "node1projmap" && argc >= 9) {
+      const uint32_t w = (uint32_t)std::atoi(argv[3]), h = (uint32_t)std::atoi(argv[4]);
+      d2pc_b200::Bus bus;
+      if (!bus.load_launch_file(argv[2])) throw std::runtime_error(std::string("cannot read ") + argv[2]);
+      d2pc::Disparity2PCloud node(bus);
+      bool map_on = false;
+      for (const auto &a : bus.advertised()) map_on = map_on || a.topic == "/octomap_point_cloud_centers";
+      std::vector<uint8_t> cloud, grid;
+      int grids = 0;
+      bus.subscribe_cloud("/point_cloud", 1, [&](const sm::PointCloud2 &c) { cloud = ros_lite::serialize(c); });
+      if (map_on) {
+        bus.subscribe_grid("/projected_map", 1, [&](const ros_lite::nav_msgs::OccupancyGrid &m) {
+          grid = ros_lite::serialize(m);
+          ++grids;
+        });
+      } else {
+        for (const auto &a : bus.advertised())
+          if (a.topic == "/projected_map") throw std::runtime_error("map off, " + a.topic + " advertised");
+      }
+      for (int i = 8; i < argc; ++i)  // frame i - 8 stamped (3 + i - 8, 4)
+        bus.publish(bus.resolve("/disparity"), make_image(read_file(argv[i], (size_t)w * h), w, h, 3 + (i - 8), 4));
+      write_file(argv[5], cloud);
+      write_file(argv[6], grid);
+      const std::string count = std::to_string(grids) + "\n";
+      write_file(argv[7], std::vector<uint8_t>(count.begin(), count.end()));
       return 0;
     }
     if (mode == "params" && argc >= 3) {
