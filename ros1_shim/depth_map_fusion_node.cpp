@@ -11,10 +11,10 @@
 #include <sensor_msgs/Image.h>
 #include <sensor_msgs/image_encodings.h>
 
-#include <cstring>
 #include <vector>
 
 #include "d2pc_b200.h"
+#include "d2pc_b200/node_params.hpp"
 
 namespace {
 
@@ -63,24 +63,15 @@ class DepthMapFusionGpu {
       out.encoding = sensor_msgs::image_encodings::RGB8;
     }
     out.step = row_bytes;
-    out.data.resize(static_cast<size_t>(row_bytes) * h);
-    for (uint32_t y = 0; y < h; ++y)
-      std::memcpy(&out.data[static_cast<size_t>(y) * row_bytes], src + static_cast<size_t>(y) * src_step, row_bytes);
+    d2pc_b200::dense_rows(src, src_step, row_bytes, h, out.data);
     pub.publish(out);
   }
   // cropToSquare(+-offset) [after rotateMat for map 2] as a dense copy -- debug views only
   void PublishCroppedDepth(const sensor_msgs::ImageConstPtr &m, int which, ros::Publisher &pub) {
     if (pub.getNumSubscribers() == 0) return;
-    int r1[4], r2[4], rc[4], dims[3];
-    if (d2pc_fuse_geometry(ctx_, m->width, m->height, r1, r2, rc, dims) != D2PC_OK) return;
-    const uint32_t n = static_cast<uint32_t>(dims[0]);
-    const int *r = which == 1 ? r1 : r2;
-    std::vector<uint8_t> v(static_cast<size_t>(n) * n);
-    for (uint32_t i = 0; i < n; ++i)
-      for (uint32_t j = 0; j < n; ++j)
-        v[static_cast<size_t>(i) * n + j] =
-            which == 1 ? m->data[static_cast<size_t>(r[1] + i) * m->step + r[0] + j]
-                       : m->data[static_cast<size_t>(m->height - 1 - (r[0] + j)) * m->step + r[1] + i];
+    uint32_t n = 0;
+    std::vector<uint8_t> v;
+    if (d2pc_b200::cropped_view(ctx_, *m, which, v, n) != D2PC_OK) return;
     PublishView(m, v.data(), n, n, n, pub, true);
   }
 
@@ -99,9 +90,7 @@ class DepthMapFusionGpu {
   void Preprocess(const sensor_msgs::ImageConstPtr &m, int which, std::vector<uint8_t> &slot, uint32_t &n) {
     d2pc_image out;
     if (d2pc_preprocess_score(ctx_, m->data.data(), m->width, m->height, m->step, which, &out) != D2PC_OK) return;
-    slot.resize(static_cast<size_t>(out.width) * out.height);
-    for (uint32_t y = 0; y < out.height; ++y)
-      std::memcpy(&slot[static_cast<size_t>(y) * out.width], out.data + static_cast<size_t>(y) * out.step, out.width);
+    d2pc_b200::dense_rows(out.data, out.step, out.width, out.height, slot);
     n = out.width;
   }
   void DisparityCb2(const sensor_msgs::ImageConstPtr &m) {
@@ -117,9 +106,7 @@ class DepthMapFusionGpu {
       return;
     }
     // the reference's combined score aliases its cached score 1 (src/depth_map_fusion.cpp:113)
-    for (uint32_t y = 0; y < combined.height; ++y)
-      std::memcpy(&s1_[static_cast<size_t>(y) * combined.width], combined.data + static_cast<size_t>(y) * combined.step,
-                  combined.width);
+    d2pc_b200::dense_rows(combined.data, combined.step, combined.width, combined.height, s1_);
     sensor_msgs::Image out;
     out.header = m->header;
     out.height = fused.height;
@@ -127,10 +114,7 @@ class DepthMapFusionGpu {
     out.encoding = sensor_msgs::image_encodings::MONO8;
     out.is_bigendian = 0;
     out.step = fused.width;
-    out.data.resize(static_cast<size_t>(fused.width) * fused.height);
-    for (uint32_t y = 0; y < fused.height; ++y)
-      std::memcpy(&out.data[static_cast<size_t>(y) * fused.width], fused.data + static_cast<size_t>(y) * fused.step,
-                  fused.width);
+    d2pc_b200::dense_rows(fused.data, fused.step, fused.width, fused.height, out.data);
     PublishView(m, s1_.data(), n1_, n1_, n1_, cropped_score_combined_pub_, false);   // :126-127
     PublishView(m, out.data.data(), out.width, out.height, out.step, grad_pub_, true);  // :132
     fused_pub_.publish(out);

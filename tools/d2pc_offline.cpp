@@ -9,6 +9,9 @@
 //   d2pc_offline params <launch file> <name>...
 //       CPU only: loads the launch file into a Bus and prints one line per name: "<name> number <value>" (%.17g),
 //       "<name> string <value>" or "<name> missing" (the launch-file loader's number / string rule).
+//   d2pc_offline node1settings <launch file>
+//       CPU only: the point cloud node's settings as read from the launch file (d2pc_b200::read_cloud_settings), one
+//       "<field> <value>" line per field of d2pc_b200::CloudSettings (numbers %.17g, arrays as <field>.<index>).
 //   d2pc_offline node1  <launch file> <w> <h> <in.raw> <out.bin> [sec nsec]
 //       BASELINE config 1/2 shape: one mono8 frame published on the node's (remapped) input topic; the
 //       PointCloud2 received on the (remapped) output topic is written in ROS1 wire format.
@@ -233,6 +236,34 @@ int main(int argc, char **argv) {
         else
           std::printf("%s missing\n", argv[i]);
       }
+      return 0;
+    }
+    if (mode == "node1settings" && argc == 3) {
+      d2pc_b200::Bus bus;
+      if (!bus.load_launch_file(argv[2])) throw std::runtime_error(std::string("cannot read ") + argv[2]);
+      const d2pc_b200::CloudSettings s = d2pc_b200::read_cloud_settings(bus);
+      auto put = [](const std::string &name, double v) { std::printf("%s %.17g\n", name.c_str(), v); };
+      auto put_n = [&put](const std::string &name, const float *v, int n) {
+        for (int i = 0; i < n; ++i) put(name + "." + std::to_string(i), v[i]);
+      };
+#define D2PC_PUT(field) put(#field, s.field)
+      D2PC_PUT(config.fx), D2PC_PUT(config.fy), D2PC_PUT(config.cx), D2PC_PUT(config.cy), D2PC_PUT(config.baseline);
+      D2PC_PUT(voxel_on), D2PC_PUT(voxel.leaf_x), D2PC_PUT(voxel.leaf_y), D2PC_PUT(voxel.leaf_z);
+      D2PC_PUT(voxel.min_points_per_voxel), D2PC_PUT(voxel.limit_field), D2PC_PUT(voxel.limit_min);
+      D2PC_PUT(voxel.limit_max), D2PC_PUT(ror_radius), D2PC_PUT(ror_min_neighbors), D2PC_PUT(crop_box.enabled);
+      put_n("crop_box.min_pt", s.crop_box.min_pt, 3), put_n("crop_box.max_pt", s.crop_box.max_pt, 3);
+      put_n("crop_box.transform", s.crop_box.transform, 12);
+      D2PC_PUT(transform.enabled), put_n("transform.matrix", s.transform.matrix, 12);
+      D2PC_PUT(scan.enabled), D2PC_PUT(scan.min_height), D2PC_PUT(scan.max_height), D2PC_PUT(scan.angle_min);
+      D2PC_PUT(scan.angle_max), D2PC_PUT(scan.angle_increment), D2PC_PUT(scan.scan_time), D2PC_PUT(scan.range_min);
+      D2PC_PUT(scan.range_max), D2PC_PUT(scan.use_inf), D2PC_PUT(scan.inf_epsilon), D2PC_PUT(scan.keep_cloud);
+      D2PC_PUT(map.enabled), D2PC_PUT(map.resolution), D2PC_PUT(map.prob_hit), D2PC_PUT(map.prob_miss);
+      D2PC_PUT(map.clamp_min), D2PC_PUT(map.clamp_max), D2PC_PUT(map.occupancy_thres), D2PC_PUT(map.max_range);
+      D2PC_PUT(map.max_bricks), D2PC_PUT(map.keep_cloud), D2PC_PUT(projected_map.occupancy_min_z);
+      D2PC_PUT(projected_map.occupancy_max_z), D2PC_PUT(projected_map.min_x_size), D2PC_PUT(projected_map.min_y_size);
+      D2PC_PUT(publish_cloud);
+#undef D2PC_PUT
+      std::printf("frame_id %s\n", s.frame_id.c_str());
       return 0;
     }
     if (mode == "node1" && argc >= 7) {
